@@ -5,6 +5,7 @@ ray pass at 2400 x 1800 (BASELINE.json `metric`, configs[2]: synthetic 8M-tet gr
 
     python bench.py [--gpus N] [--steps K] [--warmup W]                    # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   # the reference's OpenMP path
+    python bench.py [...] --dump-outputs DIR                               # + the last timed view's image
 
 A "step" is one view: rotate -> BVH refit -> solid mask -> entry + tet walk -> grazing rays (at N > 1
 each rank renders a row band and the walk kernels store their pixels into rank 0's image over NVLink).
@@ -40,6 +41,8 @@ from course5_b200 import api, synth  # noqa: E402
 BYTES_PER_STEP = 72      # 16 B connectivity + 16 B neighbours + 24 B one new vertex + 16 B (alpha, Q)
 BYTES_PER_PIXEL = 16     # {tau, I} doubles written
 REL_TOL, ABS_FLOOR = 1e-9, 1e-13   # the parity gate (tests/parity.py, BASELINE.json north_star)
+DUMP_LIMIT_BYTES = 64_000_000      # --dump-outputs: an image larger than this (64 MB) is written as a sample
+DUMP_SAMPLE_PIXELS = 1 << 21       # (42 MB: tau and I doubles, solid mask floats)
 
 
 def E2E_AUTO(world: int) -> str:
@@ -187,6 +190,27 @@ def reference_solids(D):
     return hostlib.make_solids(D)
 
 
+def dump_outputs(directory, image):
+    """Writes the (res_y, res_x, 2) image {tau, I} of the last timed view, so that two builds run with the same
+    arguments can be compared value for value, as finite arrays: directory/tau.npy and intensity.npy (float64)
+    and solid.npy (float32, 1 where a solid covers the pixel, 0 elsewhere). The image marks a solid pixel with
+    NaN in both components; those pixels are written as 0 in tau and intensity, so the image is
+    np.where(solid, nan, value) of the three. When the three arrays together exceed DUMP_LIMIT_BYTES they hold
+    a fixed sample instead: the DUMP_SAMPLE_PIXELS pixels np.random.default_rng(0) draws from the row-major
+    image without replacement, as 1-D arrays in ascending pixel order (the same pixels on every run at that
+    resolution)."""
+    os.makedirs(directory, exist_ok=True)
+    image = np.asarray(image, dtype=np.float64)
+    tau, inten = image[..., 0], image[..., 1]
+    if tau.size * (8 + 8 + 4) > DUMP_LIMIT_BYTES:
+        pick = np.sort(np.random.default_rng(0).choice(tau.size, DUMP_SAMPLE_PIXELS, replace=False))
+        tau, inten = tau.reshape(-1)[pick], inten.reshape(-1)[pick]
+    solid = np.isnan(tau) | np.isnan(inten)
+    np.save(os.path.join(directory, "tau.npy"), np.where(solid, 0.0, tau))
+    np.save(os.path.join(directory, "intensity.npy"), np.where(solid, 0.0, inten))
+    np.save(os.path.join(directory, "solid.npy"), solid.astype(np.float32))
+
+
 def config_dict(name, mesh, view):
     """The workload, in the same words for both arms (what ran it goes under `execution`)."""
     return {
@@ -276,7 +300,9 @@ def run_reference_arm(args):
     dog = Watchdog(0, limit_s=1800.0)
     dog.start()
     mesh, view = synth.make_config(args.workload)
-    r = time_reference(mesh, view, steps=args.steps, warmup=args.warmup, tick=dog.tick)
+    r = time_reference(mesh, view, steps=args.steps, warmup=args.warmup, keep_image=bool(args.dump_outputs), tick=dog.tick)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.stack([r["image"].tau, r["image"].inten], axis=-1))
     sample_txt = (f"{args.workload} mesh ({mesh.n_tets} tets) + reference solids at {view['res_x']}x{view['res_y']}, the whole "
                   f"workload: {r['tet_steps']} tet-steps per step; timed region = plane ctor + find_intersections + "
                   "trace_rays (main.cpp:126-130)")
@@ -435,7 +461,7 @@ def run_ours(args):
     ev0.record()
     t_host0 = time.perf_counter()
     for _ in range(args.steps):
-        br.render(v, rebalance=False, stats=False, pipeline=True, gather=not args.experiment_no_exchange)
+        last_image, _, _ = br.render(v, rebalance=False, stats=False, pipeline=True, gather=not args.experiment_no_exchange)
         host_t.append(time.perf_counter() - t_host0)
     br.finish()
     ev1.record()
@@ -444,6 +470,8 @@ def run_ours(args):
     launches = br.kernel_launches() - launches0
     elapsed_ms = max(ev0.elapsed_time(ev1), 1e-6)
     host_enqueue_ms = 1e3 * host_t[-1] / args.steps
+    if args.dump_outputs and last_image is not None:      # rank 0 holds the assembled image
+        dump_outputs(args.dump_outputs, last_image.cpu().numpy())
     timeline = None
     if args.timeline:
         lanes_tl = br.timeline(ev0.cuda_event)
@@ -693,7 +721,11 @@ def main():
     ap.add_argument("--no-clock-sampler", action="store_true", help="experiments: no NVML polling at all")
     ap.add_argument("--timeline", default=None, metavar="FILE",
                     help="write per-rank, per-view phase times of the timed region (CUDA events) and host enqueue times as JSON")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed views, write the image the last one computed to DIR as .npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     elif int(os.environ.get("WORLD_SIZE", "1")) > 1 and os.environ.get("C5_BENCH_CHILD") is None:
@@ -743,6 +775,8 @@ def run_with_fallback(args):
             cmd.append("--no-cpu-baseline")
         if args.timeline:
             cmd += ["--timeline", args.timeline]
+        if args.dump_outputs:
+            cmd += ["--dump-outputs", args.dump_outputs]
         if args.no_clock_sampler:
             cmd.append("--no-clock-sampler")
         if args.no_numa_bind:

@@ -440,9 +440,9 @@ def check_output_alignment(lib, device_buffer=None):
 # ---- the UNMODIFIED reference at the benchmarked sizes -------------------------------------------
 
 def reference_process(name, overrides, out_path, timeout=1500):
-    """oracle/_ref on configuration `name` (one view per dict of flag overrides) in a process of its
-    own (tests/ref_runner.py: the reference reports a degenerate ray by std::terminate). Returns the
-    saved arrays."""
+    """oracle/_ref (where it was built, else the C restatement: tests/ref_runner.py) on configuration
+    `name` (one view per dict of flag overrides) in a process of its own (the reference reports a
+    degenerate ray by std::terminate). Returns the saved arrays."""
     import json
     import os
     import subprocess

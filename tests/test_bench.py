@@ -1,12 +1,14 @@
 """bench.py on CPU: what can be checked without a GPU — the reference arm (the one place besides
 tests/ that may execute oracle/), the parity record it attaches to a line, and that both arms
-describe the workload in the same words. The CUDA arm itself refuses to run without a device."""
+describe the workload in the same words. The CUDA arm itself refuses to run without a device; on a
+B200, its --dump-outputs image is checked against a render of the same view."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -52,6 +54,76 @@ def test_cuda_arm_refuses_to_run_without_a_device(built):
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1"],
                        capture_output=True, text=True, timeout=300)
     assert p.returncode != 0 and "no CPU path" in (p.stderr + p.stdout) and "{" not in p.stdout
+
+
+def _load_dump(directory):
+    """(image with NaN under solids, as bench.py's image is, rebuilt from the dump; the dumped arrays)."""
+    arrays = {n: np.load(os.path.join(directory, n + ".npy")) for n in ("tau", "intensity", "solid")}
+    for name, a in arrays.items():
+        assert np.isfinite(a).all(), f"{name}.npy is not finite"
+    assert arrays["tau"].dtype == arrays["intensity"].dtype == np.float64 and arrays["solid"].dtype == np.float32
+    assert set(np.unique(arrays["solid"]).tolist()) <= {0.0, 1.0}
+    solid = arrays["solid"] == 1.0
+    image = np.stack([np.where(solid, np.nan, arrays["tau"]), np.where(solid, np.nan, arrays["intensity"])], axis=-1)
+    return image, arrays
+
+
+def test_reference_arm_dumps_the_last_image(built, port, tmp_path):
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "C1",
+                        "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path / "out")],
+                       capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    got, arrays = _load_dump(tmp_path / "out")
+    assert got.shape == (450, 600, 2)
+    if _line(p.stdout)["cpu_baseline"]["kind"] == "port":
+        import bench
+        from course5_b200 import synth
+        mesh, view = synth.make_config("C1")
+        roche, sphere = bench.reference_solids(view["D"])
+        want = port.render(mesh.tet_points(), mesh.alpha, mesh.q, res_x=600, res_y=450, X=view["X"], Y=view["Y"],
+                           I=view["I"], alpha_limit=view["alpha_limit"], solid_rot=roche, solid_static=sphere)
+        assert np.array_equal(got, np.stack([want.tau, want.inten], axis=-1), equal_nan=True)
+    assert arrays["solid"].any() and (arrays["intensity"] > 0).any()
+
+
+@pytest.mark.gpu
+def test_cuda_arm_dump_equals_a_render_of_the_benchmark_view(gpu_lib, tmp_path):
+    """bench.py's render plus the dump round trip. Every timed step renders the same view, so this cannot
+    tell the last step's image from an earlier one's."""
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "C1", "--steps", "3", "--warmup", "1",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path / "out")],
+                       capture_output=True, text=True, timeout=900)
+    assert p.returncode == 0, p.stderr[-2000:]
+    assert _line(p.stdout)["steps"] == 3
+    got, arrays = _load_dump(tmp_path / "out")
+    import bench
+    from course5_b200 import api, synth
+    mesh, view = synth.make_config("C1")
+    roche, sphere = bench.reference_solids(view["D"])
+    with api.Context(devices=(0,), lib=gpu_lib) as ctx:
+        ctx.upload_mesh(mesh.points, mesh.tets, mesh.alpha, mesh.q)
+        ctx.upload_solids(roche, True)
+        ctx.upload_solids(sphere, False)
+        want, _ = ctx.render(api.make_view(view["res_x"], view["res_y"], X=view["X"], Y=view["Y"], I=view["I"],
+                                           alpha_limit=view["alpha_limit"], lib=gpu_lib))
+    assert got.shape == (450, 600, 2) and arrays["solid"].any()
+    assert np.array_equal(got, want, equal_nan=True)
+
+
+def test_dump_of_a_large_image_is_a_fixed_sample(tmp_path):
+    import bench
+    image = np.random.default_rng(7).normal(size=(1800, 2400, 2))
+    image[100:300, 200:900] = np.nan                  # a solid
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), image)
+        assert sorted(os.listdir(tmp_path / run)) == ["intensity.npy", "solid.npy", "tau.npy"]
+        assert sum(os.path.getsize(tmp_path / run / n) for n in os.listdir(tmp_path / run)) <= 64_000_000
+    a, arrays = _load_dump(tmp_path / "a")
+    b, _ = _load_dump(tmp_path / "b")
+    assert a.shape == (bench.DUMP_SAMPLE_PIXELS, 2) and np.array_equal(a, b, equal_nan=True)
+    assert arrays["solid"].any()
+    pick = np.sort(np.random.default_rng(0).choice(1800 * 2400, bench.DUMP_SAMPLE_PIXELS, replace=False))
+    assert np.array_equal(a, image.reshape(-1, 2)[pick], equal_nan=True)
 
 
 def test_parity_record(hostsim_lib, port):
