@@ -185,20 +185,6 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     d.row_cost.ensure(static_cast<size_t>(v->res_y));
     if (solids) d.mask.ensure(n_pix);
 
-    // c5_debug_set("prep_priority", 1): rotate / refit / mask go to a high-priority stream of their own, so
-    // that their (small, latency-bound) blocks are dispatched ahead of the queued blocks of other lanes'
-    // pixel kernels instead of behind them; the walk waits for them by event.
-    struct StreamSwap {
-        DeviceState& d;
-        cudaStream_t main;
-        ~StreamSwap() { d.stream = main; }
-    } swap{d, d.stream};
-    const bool prep = !kHostSim && (d.opt_prep_priority & 1) && d.prep_stream != nullptr;
-    if (prep) {
-        C5_CUDA(cudaEventRecord(d.ev_fork, swap.main)); // after whatever the caller's stream holds (this lane's previous view)
-        C5_CUDA(cudaStreamWaitEvent(d.prep_stream, d.ev_fork, 0));
-        d.stream = d.prep_stream;
-    }
     record(d, 0);
     timeline_mark(d, 0);
     launch_prepare_cells(d, v->alpha_limit); // no-op unless --alpha_limit changed since the last view
@@ -214,11 +200,6 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     }
     record(d, 3);
     timeline_mark(d, 3);
-    if (prep) {
-        C5_CUDA(cudaEventRecord(d.ev_join, d.prep_stream));
-        d.stream = swap.main;
-        C5_CUDA(cudaStreamWaitEvent(d.stream, d.ev_join, 0));
-    }
     dev_zero(d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
     dev_zero(d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
     WalkLaunch w{};
@@ -234,8 +215,6 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     w.out = out_override ? out_override : d.out.p;
     w.mark_walk_done = d.ev_walk;
     w.mark_walk_done_tl = nullptr;
-    w.graze_stream = (!kHostSim && (d.opt_prep_priority & 2) && d.prep_stream) ? d.prep_stream : nullptr;
-    w.graze_join = d.ev_join;
     if (!kHostSim && !d.tl_events.empty()) {
         const size_t n = d.tl_events.size() / kTimelinePhases;
         w.mark_walk_done_tl = d.tl_events[(d.tl_views % n) * kTimelinePhases + 4];
@@ -803,11 +782,6 @@ int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out) {
                 for (auto& e : d->ev) C5_CUDA(cudaEventCreate(&e));
                 C5_CUDA(cudaEventCreate(&d->ev_walk));
                 C5_CUDA(cudaEventCreateWithFlags(&d->ev_done, cudaEventDisableTiming));
-                int prio_lo = 0, prio_hi = 0;
-                C5_CUDA(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-                C5_CUDA(cudaStreamCreateWithPriority(&d->prep_stream, cudaStreamNonBlocking, prio_hi));
-                C5_CUDA(cudaEventCreateWithFlags(&d->ev_fork, cudaEventDisableTiming));
-                C5_CUDA(cudaEventCreateWithFlags(&d->ev_join, cudaEventDisableTiming));
             }
         }
         if (n_dev > 1 && !kHostSim) {
@@ -841,9 +815,6 @@ int c5_create_sibling(c5_ctx* parent, c5_ctx** out) {
     to.opt_graze_list = from.opt_graze_list;
     to.opt_query_budget = from.opt_query_budget;
     to.opt_serial_list = from.opt_serial_list;
-    to.opt_graze_blocks = from.opt_graze_blocks;
-    to.opt_prep_priority = from.opt_prep_priority;
-    to.opt_mask_per_face = from.opt_mask_per_face;
     to.opt_no_static_mask = from.opt_no_static_mask;
     to.opt_mask_tile = from.opt_mask_tile;
     to.opt_no_zero_copy = from.opt_no_zero_copy;
@@ -888,37 +859,12 @@ void c5_destroy(c5_ctx* ctx) {
             cudaSetDevice(d.device);
             if (d.stream) cudaStreamSynchronize(d.stream);
         }
-#ifdef C5_EXPERIMENTS
-        if (!kHostSim && d.trace_launches > 0) {
-            if (const char* path = std::getenv("C5_TRACE_FILE")) {
-                cudaDeviceSynchronize();
-                std::vector<unsigned long long> h(d.trace.n);
-                if (cudaMemcpy(h.data(), d.trace.p, d.trace.bytes(), cudaMemcpyDeviceToHost) == cudaSuccess) {
-                    if (FILE* f = std::fopen(path, "a")) {
-                        for (int l = 0; l < d.trace_launches; l++) {
-                            for (unsigned b = 0; b < d.trace_grid[l]; b++) {
-                                const unsigned long long* r = h.data() + (static_cast<size_t>(l) * kTraceBlocks + b) * 4;
-                                std::fprintf(f, "%p %d %u %llu %llu %llu\n", static_cast<void*>(ctx), l, b, r[2], r[0], r[1]);
-                            }
-                        }
-                        std::fclose(f);
-                    }
-                }
-            }
-        }
-#endif
         host_pinned_free(d.h_counters);
         host_pinned_free(d.h_row_cost);
         if (!kHostSim) {
             for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
             if (d.ev_walk) cudaEventDestroy(d.ev_walk);
             if (d.ev_done) cudaEventDestroy(d.ev_done);
-            if (d.ev_fork) cudaEventDestroy(d.ev_fork);
-            if (d.ev_join) cudaEventDestroy(d.ev_join);
-            if (d.prep_stream) {
-                cudaStreamSynchronize(d.prep_stream);
-                cudaStreamDestroy(d.prep_stream);
-            }
             for (auto& e : d.ev) {
                 if (e) cudaEventDestroy(e);
             }
@@ -1227,10 +1173,7 @@ int c5_debug_set(c5_ctx* ctx, const char* key, int64_t value) {
                 if (k == "graze_list") d.opt_graze_list = static_cast<int>(value);
                 else if (k == "query_budget") d.opt_query_budget = static_cast<int>(value);
                 else if (k == "serial_list") d.opt_serial_list = static_cast<int>(value);
-                else if (k == "graze_blocks") d.opt_graze_blocks = static_cast<int>(value);
-                else if (k == "prep_priority") d.opt_prep_priority = static_cast<int>(value & 3);
                 else if (k == "mask_tile") d.opt_mask_tile = static_cast<int>(value);
-                else if (k == "mask_per_face") d.opt_mask_per_face = static_cast<int>(value < 0 ? 0 : value > 6 ? 6 : value);
                 else if (k == "no_static_mask") {
                     d.opt_no_static_mask = value != 0;
                     d.mask_static_valid = false;

@@ -271,16 +271,6 @@ C5_HD bool tile_row_covered(const MaskGrid& g, const TileGrid& tg, const FaceSca
     return covered;
 }
 
-// One face, tile row by tile row, by one thread (the CPU test build, and the experiments' per-face kernel).
-C5_HD void mark_face_by_tile_rows(const MaskGrid& g, const TileGrid& tg, const FaceScan& S, int lane, int n_lanes) {
-    const long long c_lo = S.j_lo / tg.h, c_hi = S.j_hi / tg.h;
-    for (long long c = c_lo + lane; c <= c_hi; c += n_lanes) {
-        long long ja, jb;
-        if (tile_row_covered(g, tg, S, c, ja, jb)) continue;
-        for (long long j = ja; j <= jb; j++) scan_row(g, S, j);
-    }
-}
-
 // face f of a solid tet: 0 = (v0,v1,v2), 1 = (v0,v1,v3), 2 = (v0,v2,v3), 3 = (v1,v2,v3) (plane.cpp:30-37)
 C5_HD void face_corners(int64_t f, const double* pts, const double*& a, const double*& b, const double*& c) {
     const double* p = pts + 12 * (f >> 2);
@@ -288,18 +278,6 @@ C5_HD void face_corners(int64_t f, const double* pts, const double*& a, const do
     a = p + (k == 3 ? 3 : 0);
     b = p + (k >= 2 ? 6 : 3);
     c = p + (k == 0 ? 6 : 9);
-}
-
-// pass 1 for one face: draws it if it is small; returns whether it is tall (to be listed)
-C5_HD bool small_face_body(uint32_t f, const double* pts, const MaskGrid& g) {
-    const double *a, *b, *c;
-    face_corners(f, pts, a, b, c);
-    const FaceRows R = scan_rows(g, a, b, c);
-    if (R.j_lo > R.j_hi) return false;
-    if (R.j_hi - R.j_lo >= kSmallRows) return true;
-    const FaceScan S = scan_edges(R);
-    for (long long j = S.j_lo; j <= S.j_hi; j++) scan_row(g, S, j);
-    return false;
 }
 
 // pass 2 for one tile
@@ -320,15 +298,6 @@ C5_HD void tile_flag_body(int ty, int tx, const MaskGrid& g, const TileGrid& tg)
     tg.full[static_cast<size_t>(ty) * tg.tiles_x + tx] = all ? 1 : 0;
 }
 
-// pass 3 for one tall face
-C5_HD void tall_face_body(uint32_t f, const double* pts, const MaskGrid& g, const TileGrid& tg, int lane, int n_lanes) {
-    const double *a, *b, *c;
-    face_corners(f, pts, a, b, c);
-    const FaceRows R = scan_rows(g, a, b, c);
-    if (R.j_lo > R.j_hi) return;
-    mark_face_by_tile_rows(g, tg, scan_edges(R), lane, n_lanes);
-}
-
 // ---- a warp's 32 faces, shared ---------------------------------------------------------------------
 // One face per thread leaves most lanes idle: faces differ in height by two orders of magnitude, two
 // thirds of a pass-1 warp hold faces that are only listed, and the rare tile row that does have to be
@@ -336,7 +305,7 @@ C5_HD void tall_face_body(uint32_t f, const double* pts, const MaskGrid& g, cons
 // profiles/r02_mask_*). So a warp sets up its 32 faces one per lane, parks the FaceScans in shared
 // memory and deals out the ITEMS (rows in pass 1, tile rows in pass 3, rows of uncovered tile rows in
 // its drain) lane by lane, whoever the face belongs to. The arithmetic per item is the same
-// functions on the same operands as the per-face form, so the mask cannot differ.
+// functions on the same operands whichever lane runs it, so the mask cannot differ.
 #define C5_HDN __host__ __device__ // (not force-inlined, unlike C5_HD)
 constexpr int kFaceFields = 17; // p1x p1y + 3 x {x1 y1 dx dy rdy}
 struct WarpFaces {
@@ -526,43 +495,6 @@ __global__ void __launch_bounds__(256) mask_tile_flags(MaskGrid g, TileGrid tg, 
     if (k >= n) return;
     tile_flag_body(tile_row_begin + static_cast<int>(k / tg.tiles_x), static_cast<int>(k % tg.tiles_x), g, tg);
 }
-
-#ifdef C5_EXPERIMENTS
-// The per-face form of passes 1 and 3 (one face per thread; pass 3 optionally 2^lane_shift lanes per face
-// sharing its tile rows round-robin), kept for scripts/ to measure against (c5_debug_set "mask_per_face").
-__global__ void __launch_bounds__(256)
-solid_mask_small_per_face(int64_t n_faces, const uint32_t* __restrict__ faces, const double* __restrict__ pts, MaskGrid g,
-                          uint32_t* __restrict__ tall, unsigned* n_tall) {
-    const unsigned full = 0xFFFFFFFFu;
-    const int lane = threadIdx.x & 31;
-    const int64_t k = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-    uint32_t f = 0;
-    bool is_tall = false;
-    if (k < n_faces) {
-        f = faces[k];
-        is_tall = small_face_body(f, pts, g);
-    }
-    const unsigned m = __ballot_sync(full, is_tall);
-    if (m) {
-        unsigned base = 0;
-        if (lane == 0) base = atomicAdd(n_tall, static_cast<unsigned>(__popc(m)));
-        base = __shfl_sync(full, base, 0);
-        if (is_tall) tall[base + __popc(m & ((1u << lane) - 1u))] = f;
-    }
-}
-__global__ void __launch_bounds__(256)
-solid_mask_tall_per_face(const uint32_t* __restrict__ tall, const unsigned* __restrict__ n_tall, const double* __restrict__ pts,
-                         MaskGrid g, TileGrid tg, int lane_shift) {
-    const unsigned n = *n_tall;
-    const int group_lanes = 1 << lane_shift;
-    const unsigned groups_per_block = blockDim.x >> lane_shift;
-    const unsigned group = threadIdx.x >> lane_shift;
-    const int group_lane = static_cast<int>(threadIdx.x) & (group_lanes - 1);
-    for (unsigned idx = blockIdx.x * groups_per_block + group; idx < n; idx += gridDim.x * groups_per_block) {
-        tall_face_body(tall[idx], pts, g, tg, group_lane, group_lanes);
-    }
-}
-#endif
 
 namespace {
 
@@ -894,23 +826,10 @@ void mask_passes(DeviceState& d, SolidSet& ss, const MaskGrid& g, const TileGrid
     }
     if (d.sm_count == 0) C5_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, d.device));
     constexpr int kBlock = 32 * kMaskWarps;
-#ifdef C5_EXPERIMENTS
-    const bool per_face = d.opt_mask_per_face > 0;
-#else
-    const bool per_face = false;
-#endif
     // pass 1: small faces are drawn, tall ones listed
     count_launch();
-    if (!per_face) {
-        solid_mask_small<<<grid_for(ss.n_faces, kBlock), kBlock, 0, d.stream>>>(ss.n_faces, ss.faces.p, ss.pts_view.p, g,
-                                                                                 d.mask_tall.p, d.mask_counts.p);
-    }
-#ifdef C5_EXPERIMENTS
-    else {
-        solid_mask_small_per_face<<<grid_for(ss.n_faces, 256), 256, 0, d.stream>>>(ss.n_faces, ss.faces.p, ss.pts_view.p, g,
-                                                                                    d.mask_tall.p, d.mask_counts.p);
-    }
-#endif
+    solid_mask_small<<<grid_for(ss.n_faces, kBlock), kBlock, 0, d.stream>>>(ss.n_faces, ss.faces.p, ss.pts_view.p, g,
+                                                                             d.mask_tall.p, d.mask_counts.p);
     C5_CUDA(cudaGetLastError());
     // pass 2: which tiles of the band are solid already
     count_launch();
@@ -918,16 +837,8 @@ void mask_passes(DeviceState& d, SolidSet& ss, const MaskGrid& g, const TileGrid
     C5_CUDA(cudaGetLastError());
     // pass 3: tall faces, skipping tile rows that are solid already
     count_launch();
-    if (!per_face) {
-        solid_mask_tall<<<static_cast<unsigned>(d.sm_count) * 16u, kBlock, 0, d.stream>>>(d.mask_tall.p, d.mask_counts.p,
-                                                                                          ss.pts_view.p, g, tg);
-    }
-#ifdef C5_EXPERIMENTS
-    else {
-        solid_mask_tall_per_face<<<static_cast<unsigned>(d.sm_count) * 8u, 256, 0, d.stream>>>(
-            d.mask_tall.p, d.mask_counts.p, ss.pts_view.p, g, tg, d.opt_mask_per_face - 1);
-    }
-#endif
+    solid_mask_tall<<<static_cast<unsigned>(d.sm_count) * 16u, kBlock, 0, d.stream>>>(d.mask_tall.p, d.mask_counts.p,
+                                                                                      ss.pts_view.p, g, tg);
     C5_CUDA(cudaGetLastError());
 }
 

@@ -50,16 +50,6 @@ struct DeviceState {
     DeviceState* origin = nullptr;   // sibling context: the device state that owns the mesh (and these two flags)
     uint64_t mesh_version = 0;       // bumped by every upload; a sibling re-aliases when it falls behind
     bool mesh_shared = false;        // some sibling aliases this state's arrays
-#ifdef C5_EXPERIMENTS
-    DevBuf<StepRec> recs;            // experimental "rec" walk variant: 4 step records per tet, built on first use
-    double recs_limit = 0.0;
-    bool recs_valid = false;
-    // C5_TRACE_FILE: start / end time and SM of every block of the first pixel-kernel launches,
-    // written to that file when the context is destroyed (scripts/trace_blocks.py reads it)
-    DevBuf<unsigned long long> trace;
-    int trace_launches = 0;
-    unsigned trace_grid[64] = {};
-#endif
     DevBuf<BFace> bfaces;            // Morton-sorted boundary faces (BVH leaves)
     DevBuf<BvhNode> nodes;           // n_bfaces - 1 internal nodes, BFS order (root = 0)
     DevBuf<int32_t> node_parent;     // per internal node: (parent << 1) | which child, -1 for the root
@@ -94,11 +84,8 @@ struct DeviceState {
     uint64_t* h_row_cost = nullptr;             // [h_row_cost_n]
     size_t h_row_cost_n = 0;
     // c5_debug_set (tests, diagnostics); 0 = default
-    int opt_graze_list = 0, opt_query_budget = 0, opt_serial_list = 0, opt_graze_blocks = 0, opt_mask_per_face = 0, opt_mask_tile = 0;
+    int opt_graze_list = 0, opt_query_budget = 0, opt_serial_list = 0, opt_mask_tile = 0;
     bool opt_no_zero_copy = false, opt_no_static_mask = false;
-    int opt_prep_priority = 0;                  // bit 0: rotate / refit / mask, bit 1: the grazing-ray kernel, on prep_stream
-    cudaStream_t prep_stream = nullptr;         // high priority (see opt_prep_priority)
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     // c5_debug_set("timeline", n): phase events of the last n views, read by c5_timeline_read
     std::vector<cudaEvent_t> tl_events;         // [n][kTimelinePhases]
     uint64_t tl_views = 0;                      // views recorded since the timeline was enabled
@@ -162,7 +149,6 @@ void dedupe_solid_faces(DeviceState& d, SolidSet& ss); // fills ss.faces / ss.n_
 void launch_prepare_cells(DeviceState& d, double alpha_limit); // cells[t].s = q0[t] / min(alpha, limit)
 
 // c5_walk.cu
-constexpr int kTraceLaunches = 64, kTraceBlocks = 40960;
 struct WalkLaunch {
     int res_x, res_y, row_begin, row_end;
     int i_begin, i_end, j_begin, j_end; // pixel rectangle that can see the mesh (clipped to the band by the launch)
@@ -174,8 +160,6 @@ struct WalkLaunch {
     double* out; // {tau, I} per pixel of the band, x fastest
     cudaEvent_t mark_walk_done;    // recorded between the pixel kernel and the grazing-ray kernel (may be null)
     cudaEvent_t mark_walk_done_tl; // the same moment for the timeline ring (may be null)
-    cudaStream_t graze_stream;     // non-null: the grazing-ray kernel goes there (after mark_walk_done) and is joined back
-    cudaEvent_t graze_join;
 };
 void launch_walk(DeviceState& d, const WalkLaunch& w);
 

@@ -216,8 +216,7 @@ struct BFaceOp {
         bf.c = cc;
         bf.tet = static_cast<int32_t>(f >> 2);
         bf.apex = d;
-        bf.pad[0] = k; // local index of the apex in its tet == index of this face as an ENTRY face (StepRec)
-        bf.pad[1] = bf.pad[2] = 0;
+        bf.pad[0] = bf.pad[1] = bf.pad[2] = 0;
         out[i] = bf;
         keys[i] = morton3((px[a] + px[b] + px[cc]) / 3.0, (py[a] + py[b] + py[cc]) / 3.0,
                           (pz[a] + pz[b] + pz[cc]) / 3.0, box.lo, box.inv);
@@ -483,10 +482,6 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
     d.n_tets = n_tets;
     d.n_bfaces = static_cast<int64_t>(n_b);
     d.cells_limit_valid = false;
-#ifdef C5_EXPERIMENTS
-    d.recs.release();
-    d.recs_valid = false;
-#endif
 }
 
 } // namespace c5

@@ -69,67 +69,6 @@ struct alignas(32) DeferredRay {
 };
 static_assert(sizeof(DeferredRay) == 32, "DeferredRay must be 32 bytes");
 
-// ---- step records (experimental walk variant "rec", libc5gpu_exp.so only; DESIGN.md §4) ----------
-// The walk is bound by L1 data-pipe wavefronts: one per lane and load instruction, and the 64-byte
-// Cell costs two. A StepRec is everything a step needs in ONE 256-bit load: there is one per
-// (tet t, entry face e), index 4 t + e, holding for each of the three faces the ray can leave
-// through the next record's index and the next tet's apex vertex, plus the tet's alpha and s cut to
-// 48 bits (sign, exponent, 36 mantissa bits: 7e-12 relative, far inside the 1e-9 parity gate).
-// Exit slots are ordered by the GLOBAL id of the entry-face vertex the exit face drops, ascending:
-// the ray carries those ids anyway, so it finds its slot with three compares and needs no stored
-// permutation. Limits: 4 n_tets < 2^28 - 1, n_pts < 2^25 (C5: 50.2 M tets, 8.5 M points).
-//   w[i], i < 3:  bits 0..27 next record (kRecNoFace: the ray leaves the mesh), 28..52 next apex,
-//                 53..63 eleven more bits of s (bits 15 + 11 i ... of its 48)
-//   w[3]:         bits 0..47 alpha, 48..62 the low 15 bits of s
-constexpr uint32_t kRecNoFace = (1u << 28) - 1u;
-constexpr uint64_t kRecVtxLimit = 1ull << 25;
-struct alignas(32) StepRec {
-    uint64_t w[4];
-};
-static_assert(sizeof(StepRec) == 32, "StepRec must be 32 bytes");
-
-C5_HD uint64_t bits_of_double(double v) {
-#ifdef __CUDA_ARCH__
-    return static_cast<uint64_t>(__double_as_longlong(v));
-#else
-    uint64_t b;
-    memcpy(&b, &v, sizeof(b));
-    return b;
-#endif
-}
-C5_HD double double_of_bits(uint64_t b) {
-#ifdef __CUDA_ARCH__
-    return __longlong_as_double(static_cast<long long>(b));
-#else
-    double v;
-    memcpy(&v, &b, sizeof(v));
-    return v;
-#endif
-}
-C5_HD uint64_t to_48(double v) { // round to nearest on the 16 dropped bits (finite inputs)
-    return (bits_of_double(v) + 0x8000ull) >> 16;
-}
-C5_HD double from_48(uint64_t x) {
-    return double_of_bits(x << 16);
-}
-C5_HD StepRec pack_rec(const uint32_t next_face[3], const uint32_t next_apex[3], double alpha, double s) {
-    const uint64_t a48 = to_48(alpha), s48 = to_48(s);
-    StepRec r;
-    for (int i = 0; i < 3; i++) {
-        r.w[i] = static_cast<uint64_t>(next_face[i]) | (static_cast<uint64_t>(next_apex[i]) << 28) |
-                 (((s48 >> (15 + 11 * i)) & 0x7FFull) << 53);
-    }
-    r.w[3] = a48 | ((s48 & 0x7FFFull) << 48);
-    return r;
-}
-C5_HD double rec_alpha(const StepRec& r) {
-    return from_48(r.w[3] & 0xFFFFFFFFFFFFull);
-}
-C5_HD double rec_s(const StepRec& r) {
-    const uint64_t s48 = ((r.w[3] >> 48) & 0x7FFFull) | ((r.w[0] >> 53) << 15) | ((r.w[1] >> 53) << 26) | ((r.w[2] >> 53) << 37);
-    return from_48(s48);
-}
-
 struct Rot {       // one rotation with the trig evaluated on the host by libm (so it is the same
     int32_t axis;  // cos/sin the reference's host code multiplies by, tetra.cpp:44-62)
     int32_t pad;

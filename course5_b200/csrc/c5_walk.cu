@@ -64,18 +64,7 @@ struct WalkParams {
     int max_steps;
     int round_float;
     double alpha_limit;
-#ifdef C5_EXPERIMENTS     // libc5gpu_exp.so only (scripts/): block timeline, shared-memory BVH top, step records
-    unsigned long long* trace; // per block {start ns, end ns, sm, block}
-    int top_nodes;        // BVH nodes [0, top_nodes) are staged in shared memory
-    const StepRec* recs;
-#endif
 };
-
-#ifdef C5_EXPERIMENTS
-C5_HD int staged_nodes(const WalkParams& P) { return P.top_nodes; }
-#else
-C5_HD int staged_nodes(const WalkParams&) { return 0; }
-#endif
 
 // ---- loads through the read-only path ----------------------------------------------------------
 struct CellData {
@@ -85,36 +74,22 @@ struct CellData {
 
 // sm_100 has 256-bit global loads (SASS LDG.E.ENL2.256): a 64-byte cell is two of them and a
 // 32-byte vertex one, i.e. 3 load instructions per tet-step instead of 6 LDG.128.
-template <bool kWide>
 C5_HD CellData load_cell(const Cell* cells, int t) {
     CellData c;
 #ifdef __CUDA_ARCH__
-    if (kWide) {
-        const char* p = reinterpret_cast<const char*>(cells + t);
-        long long as0, as1;
-        asm volatile("ld.global.nc.v8.s32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                     : "=r"(c.v.x), "=r"(c.v.y), "=r"(c.v.z), "=r"(c.v.w), "=r"(c.nbr.x), "=r"(c.nbr.y), "=r"(c.nbr.z),
-                       "=r"(c.nbr.w)
-                     : "l"(p));
-        int a0, a1, a2, a3;
-        int lo0, hi0, lo1, hi1;
-        asm volatile("ld.global.nc.v8.s32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                     : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(a3), "=r"(lo0), "=r"(hi0), "=r"(lo1), "=r"(hi1)
-                     : "l"(p + 32));
-        c.apex = make_int4(a0, a1, a2, a3);
-        c.alpha = __hiloint2double(hi0, lo0);
-        c.s = __hiloint2double(hi1, lo1);
-        (void)as0;
-        (void)as1;
-    } else {
-        const int4* p = reinterpret_cast<const int4*>(cells + t);
-        c.v = __ldg(p);
-        c.nbr = __ldg(p + 1);
-        c.apex = __ldg(p + 2);
-        const double2 as = __ldg(reinterpret_cast<const double2*>(p + 3));
-        c.alpha = as.x;
-        c.s = as.y;
-    }
+    const char* p = reinterpret_cast<const char*>(cells + t);
+    asm volatile("ld.global.nc.v8.s32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(c.v.x), "=r"(c.v.y), "=r"(c.v.z), "=r"(c.v.w), "=r"(c.nbr.x), "=r"(c.nbr.y), "=r"(c.nbr.z),
+                   "=r"(c.nbr.w)
+                 : "l"(p));
+    int a0, a1, a2, a3;
+    int lo0, hi0, lo1, hi1;
+    asm volatile("ld.global.nc.v8.s32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(a3), "=r"(lo0), "=r"(hi0), "=r"(lo1), "=r"(hi1)
+                 : "l"(p + 32));
+    c.apex = make_int4(a0, a1, a2, a3);
+    c.alpha = __hiloint2double(hi0, lo0);
+    c.s = __hiloint2double(hi1, lo1);
 #else
     const Cell& s = cells[t];
     c.v = make_int4(s.v[0], s.v[1], s.v[2], s.v[3]);
@@ -134,31 +109,6 @@ C5_HD void load_vtx(const Vtx* vrot, int id, double& x, double& y, double& z) {
     x = vrot[id].x;
     y = vrot[id].y;
     z = vrot[id].z;
-#endif
-}
-
-#ifdef C5_EXPERIMENTS
-C5_HD StepRec load_rec(const StepRec* recs, uint32_t face) {
-    StepRec r;
-#ifdef __CUDA_ARCH__
-    asm volatile("ld.global.nc.v4.u64 {%0,%1,%2,%3}, [%4];"
-                 : "=l"(r.w[0]), "=l"(r.w[1]), "=l"(r.w[2]), "=l"(r.w[3])
-                 : "l"(recs + face));
-#else
-    r = recs[face];
-#endif
-    return r;
-}
-#endif
-
-// Next step's cell and vertex are known as soon as the exit face is (Cell::nbr / Cell::apex), long
-// before this step's divide and exp have retired: asking L1 for them now overlaps their L2/DRAM
-// latency with that math at no register cost.
-C5_HD void prefetch_l1(const void* p) {
-#ifdef __CUDA_ARCH__
-    asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
-#else
-    (void)p;
 #endif
 }
 
@@ -244,8 +194,8 @@ C5_HD void insert_entry(EntryList<kCap>& L, int cap, double z, int leaf) {
 // (block timeline, profiles/r01_trace_band_c3.txt). A search that exceeds its budget returns false
 // and the ray is handed to the grazing-ray kernel, where 32 lanes share the traversal.
 template <int kCap>
-C5_HD bool bvh_collect_entries(const WalkParams& P, const BvhNode* top, double px, double py, double z_after,
-                               EntryList<kCap>& L, int cap, int budget) {
+C5_HD bool bvh_collect_entries(const WalkParams& P, double px, double py, double z_after, EntryList<kCap>& L, int cap,
+                               int budget) {
     int stack[kStack];
     int sp = 0;
     L.n = 0;
@@ -260,7 +210,9 @@ C5_HD bool bvh_collect_entries(const WalkParams& P, const BvhNode* top, double p
             complete = false;
             break;
         }
-        const BvhNode* n = (top && node < staged_nodes(P)) ? (top + node) : (P.nodes + node);
+        // (staging the top BVH levels in shared memory was measured slower than letting L1 serve them:
+        // C3 6.38 ms with 0 nodes, 6.54 with 63, 6.88 with 255; profiles/r01_exp_c3_variants_b.jsonl)
+        const BvhNode* n = P.nodes + node;
 #ifdef __CUDA_ARCH__
         const float4 bx = *reinterpret_cast<const float4*>(n->xlo); // xlo0 xlo1 xhi0 xhi1
         const float4 by = *reinterpret_cast<const float4*>(n->ylo);
@@ -316,7 +268,7 @@ C5_HD bool bvh_collect_entries(const WalkParams& P, const BvhNode* top, double p
 // grazing-ray kernel walks the crossings of one ray in parallel); inten then starts at 0 and gain at
 // 1, and the crossing maps an arriving I to inten + gain * I (the recurrence of line.cpp:206-225 is
 // affine in I: s - (s - I) e = s (1 - e) + e I).
-template <bool kWide, int kPipe, bool kAffine>
+template <bool kAffine>
 C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau,
                           double& inten, double& gain, uint32_t& steps, uint32_t& error) {
 #ifdef __CUDA_ARCH__
@@ -338,15 +290,6 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
     cx -= px; cy -= py;
     int t = f.w;
     double z_cur = z_in;
-    // kPipe == 2 (software-pipelined loop): the cell and the vertex of step k+1 are requested as soon as
-    // step k knows its exit face, BEFORE its divide and exp — the loads' latency overlaps that math.
-    // Costs the registers of one cell + one vertex in flight next to the math's temporaries.
-    CellData c;
-    double dx, dy, dz;
-    if (kPipe == 2) {
-        c = load_cell<kWide>(P.cells, t);
-        load_vtx(P.vrot, id, dx, dy, dz);
-    }
     while (true) {
         if (steps >= static_cast<uint32_t>(P.max_steps)) {
             error = 1;
@@ -355,10 +298,9 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
         // id = the vertex of tet t that is not on the entry face. It is known BEFORE t's cell is
         // read (Cell::apex of the previous tet, BFace::apex at entry), so the cell load and the
         // vertex load of a step are independent and overlap: one memory latency per step, not two.
-        if (kPipe != 2) {
-            c = load_cell<kWide>(P.cells, t);
-            load_vtx(P.vrot, id, dx, dy, dz);
-        }
+        const CellData c = load_cell(P.cells, t);
+        double dx, dy, dz;
+        load_vtx(P.vrot, id, dx, dy, dz);
         dx -= px;
         dy -= py;
         const double sa = orient2(dx, dy, ax, ay);
@@ -371,11 +313,6 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
         const bool k0 = c.v.x == dropped, k1 = c.v.y == dropped, k2 = c.v.z == dropped;
         const int t_next = k0 ? c.nbr.x : k1 ? c.nbr.y : k2 ? c.nbr.z : c.nbr.w;
         const int id_next = k0 ? c.apex.x : k1 ? c.apex.y : k2 ? c.apex.z : c.apex.w;
-        if (kPipe == 1 && t_next >= 0) {
-            prefetch_l1(P.cells + t_next);
-            prefetch_l1(reinterpret_cast<const char*>(P.cells + t_next) + 32);
-            prefetch_l1(P.vrot + id_next);
-        }
         // Barycentric weights of the pixel in the exit face (weight of a vertex = orient2 of the
         // other two, in cyclic order). Two of them are s values; the third belongs to d and is the
         // orient2 of the two vertices that stay — recomputed here (3 flops) rather than carried
@@ -397,22 +334,17 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
             wa = sc;
             wb = orient2(cx, cy, ax, ay);
         }
-        const double alpha_t = c.alpha, s_t = c.s;
-        if (kPipe == 2 && t_next >= 0) { // the next step's operands, on their way while this step finishes
-            c = load_cell<kWide>(P.cells, t_next);
-            load_vtx(P.vrot, id_next, dx, dy, dz);
-        }
         const double wsum = wa + wb + wc;
         const double z_exit = (wsum != 0.0) ? (wa * az + wb * bz + wc * cz) / wsum : z_cur;
         const double dzv = fabs(z_exit - z_cur);
         // tau: line.cpp:176-193 (alpha not clamped)
-        tau += dzv * alpha_t;
+        tau += dzv * c.alpha;
         // I: line.cpp:206-225 with s = Q / a^:  (Q - (Q - a^ I) e) / a^  ==  s - (s - I) e
-        double a_c = alpha_t;
+        double a_c = c.alpha;
         if (a_c > P.alpha_limit) a_c = P.alpha_limit;
         if (!(a_c < DBL_EPSILON)) {
             const double e = exp(-a_c * dzv);
-            inten = s_t - (s_t - inten) * e;
+            inten = c.s - (c.s - inten) * e;
             if (kAffine) gain *= e;
         }
         steps++;
@@ -423,92 +355,6 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
     }
     return z_cur;
 }
-
-#ifdef C5_EXPERIMENTS
-// Experimental variant "rec" (C5_WALK_VARIANT=rec, libc5gpu_exp.so only; measured: 3 % faster on the C3
-// README view, 6 % slower on an oblique one, profiles/r02_exp_rec_vs_cells.jsonl — not adopted): the same crossing on step records
-// (c5_types.h) — one 256-bit load for the tet instead of two, so two L1 data-pipe wavefronts per
-// lane and step instead of three. The exit slot is the rank of the dropped vertex's id among the
-// three entry-face ids. alpha and s arrive cut to 48 bits (7e-12 relative).
-C5_HD double crossing_rec_f64(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau,
-                              double& inten, uint32_t& steps, uint32_t& error) {
-#ifdef __CUDA_ARCH__
-    const int4 f = __ldg(reinterpret_cast<const int4*>(P.bfaces + leaf));
-    const int2 ae = __ldg(reinterpret_cast<const int2*>(&P.bfaces[leaf].apex)); // apex, entry-face index
-    int id = ae.x;
-    uint32_t face = 4u * static_cast<uint32_t>(f.w) + static_cast<uint32_t>(ae.y);
-#else
-    const BFace& bf = P.bfaces[leaf];
-    const int4 f = make_int4(bf.a, bf.b, bf.c, bf.tet);
-    int id = bf.apex;
-    uint32_t face = 4u * static_cast<uint32_t>(bf.tet) + static_cast<uint32_t>(bf.pad[0]);
-#endif
-    int ia = f.x, ib = f.z, ic = f.y;
-    double ax, ay, az, bx, by, bz, cx, cy, cz;
-    load_vtx(P.vrot, ia, ax, ay, az);
-    load_vtx(P.vrot, ib, bx, by, bz);
-    load_vtx(P.vrot, ic, cx, cy, cz);
-    ax -= px; ay -= py;
-    bx -= px; by -= py;
-    cx -= px; cy -= py;
-    double z_cur = z_in;
-    while (true) {
-        if (steps >= static_cast<uint32_t>(P.max_steps)) {
-            error = 1;
-            break;
-        }
-        const StepRec r = load_rec(P.recs, face);
-        double dx, dy, dz;
-        load_vtx(P.vrot, id, dx, dy, dz);
-        dx -= px;
-        dy -= py;
-        const double sa = orient2(dx, dy, ax, ay);
-        const double sb = orient2(dx, dy, bx, by);
-        const double sc = orient2(dx, dy, cx, cy);
-        const bool drop_c = sa >= 0 && sb < 0;
-        const bool drop_a = !drop_c && sb >= 0 && sc < 0;
-        const int dropped = drop_c ? ic : drop_a ? ia : ib;
-        const int slot = (ia < dropped ? 1 : 0) + (ib < dropped ? 1 : 0) + (ic < dropped ? 1 : 0);
-        const uint64_t w = slot == 0 ? r.w[0] : slot == 1 ? r.w[1] : r.w[2];
-        const uint32_t face_next = static_cast<uint32_t>(w) & kRecNoFace;
-        const int id_next = static_cast<int>((w >> 28) & (kRecVtxLimit - 1));
-        double wa, wb, wc;
-        if (drop_c) {
-            ic = id; cx = dx; cy = dy; cz = dz;
-            wa = -sb;
-            wb = sa;
-            wc = orient2(ax, ay, bx, by);
-        } else if (drop_a) {
-            ia = id; ax = dx; ay = dy; az = dz;
-            wb = -sc;
-            wc = sb;
-            wa = orient2(bx, by, cx, cy);
-        } else {
-            ib = id; bx = dx; by = dy; bz = dz;
-            wc = -sa;
-            wa = sc;
-            wb = orient2(cx, cy, ax, ay);
-        }
-        const double wsum = wa + wb + wc;
-        const double z_exit = (wsum != 0.0) ? (wa * az + wb * bz + wc * cz) / wsum : z_cur;
-        const double dzv = fabs(z_exit - z_cur);
-        const double alpha = rec_alpha(r);
-        tau += dzv * alpha;
-        double a_c = alpha;
-        if (a_c > P.alpha_limit) a_c = P.alpha_limit;
-        if (!(a_c < DBL_EPSILON)) {
-            const double sf = rec_s(r);
-            inten = sf - (sf - inten) * exp(-a_c * dzv);
-        }
-        steps++;
-        z_cur = z_exit;
-        face = face_next;
-        id = id_next;
-        if (face == kRecNoFace) break;
-    }
-    return z_cur;
-}
-#endif
 
 // ---- FP32 variant -----------------------------------------------------------------------------------
 // Same crossing with the per-step geometry in single precision: FP32 orientation tests (still exactly
@@ -537,7 +383,7 @@ C5_HD float orient2f(float ux, float uy, float vx, float vy) {
     return fsub_rn(fmul_rn(ux, vy), fmul_rn(uy, vx));
 }
 
-template <bool kWide, int kPipe, bool kAffine>
+template <bool kAffine>
 C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau,
                           double& inten, double& gain, uint32_t& steps, uint32_t& error) {
     const float limit = static_cast<float>(P.alpha_limit);
@@ -571,7 +417,7 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
             error = 1;
             break;
         }
-        const CellData c = load_cell<kWide>(P.cells, t);
+        const CellData c = load_cell(P.cells, t);
         float dx, dy, dz;
         {
             double x, y, z;
@@ -589,11 +435,6 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
         const bool k0 = c.v.x == dropped, k1 = c.v.y == dropped, k2 = c.v.z == dropped;
         const int t_next = k0 ? c.nbr.x : k1 ? c.nbr.y : k2 ? c.nbr.z : c.nbr.w;
         const int id_next = k0 ? c.apex.x : k1 ? c.apex.y : k2 ? c.apex.z : c.apex.w;
-        if (kPipe == 1 && t_next >= 0) {
-            prefetch_l1(P.cells + t_next);
-            prefetch_l1(reinterpret_cast<const char*>(P.cells + t_next) + 32);
-            prefetch_l1(P.vrot + id_next);
-        }
         if (drop_c) {
             ic = id; cx = dx; cy = dy; cz = dz;
             wa = -sb;
@@ -630,47 +471,12 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
     return z_exit_abs > z0 ? z_exit_abs : z0;
 }
 
-template <bool kF32, bool kWide, int kPipe, bool kAffine, bool kRec = false>
+template <bool kF32, bool kAffine>
 C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau, double& inten,
                       double& gain, uint32_t& steps, uint32_t& error) {
-#ifdef C5_EXPERIMENTS
-    if (kRec) return crossing_rec_f64(P, px, py, leaf, z_in, tau, inten, steps, error);
-#endif
-    return kF32 ? crossing_f32<kWide, kPipe, kAffine>(P, px, py, leaf, z_in, tau, inten, gain, steps, error)
-                : crossing_f64<kWide, kPipe, kAffine>(P, px, py, leaf, z_in, tau, inten, gain, steps, error);
+    return kF32 ? crossing_f32<kAffine>(P, px, py, leaf, z_in, tau, inten, gain, steps, error)
+                : crossing_f64<kAffine>(P, px, py, leaf, z_in, tau, inten, gain, steps, error);
 }
-
-#ifdef C5_EXPERIMENTS
-// Step record of (tet, entry face) f = 4 t + e: the three faces the ray can leave through, ordered by
-// the global id of the entry-face vertex each one drops.
-C5_HD StepRec make_step_record(const Cell* cells, int64_t f) {
-    const Cell& c = cells[f >> 2];
-    const int e = static_cast<int>(f & 3);
-    int k[3], n = 0;
-    for (int j = 0; j < 4; j++) {
-        if (j != e) k[n++] = j;
-    }
-    // sort the three local indices by global vertex id
-    if (c.v[k[1]] < c.v[k[0]]) { const int t = k[0]; k[0] = k[1]; k[1] = t; }
-    if (c.v[k[2]] < c.v[k[1]]) { const int t = k[1]; k[1] = k[2]; k[2] = t; }
-    if (c.v[k[1]] < c.v[k[0]]) { const int t = k[0]; k[0] = k[1]; k[1] = t; }
-    uint32_t next_face[3], next_apex[3];
-    for (int i = 0; i < 3; i++) {
-        const int nb = c.nbr[k[i]]; // across the face that drops vertex k[i]
-        if (nb < 0) {
-            next_face[i] = kRecNoFace;
-            next_apex[i] = 0;
-        } else {
-            const Cell& o = cells[nb];
-            const int apex = c.apex[k[i]];
-            const int e2 = o.v[0] == apex ? 0 : o.v[1] == apex ? 1 : o.v[2] == apex ? 2 : 3;
-            next_face[i] = 4u * static_cast<uint32_t>(nb) + static_cast<uint32_t>(e2);
-            next_apex[i] = static_cast<uint32_t>(apex);
-        }
-    }
-    return pack_rec(next_face, next_apex, c.alpha, c.s);
-}
-#endif
 
 // ---- one ray (pixel kernel) ------------------------------------------------------------------------
 
@@ -701,9 +507,8 @@ C5_HD void sync_lanes(unsigned lanes) {
 #endif
 }
 
-template <bool kF32, bool kWide, int kPipe, bool kRec = false>
-C5_HD RayResult trace_ray(const WalkParams& P, const BvhNode* top, double px, double py, uint32_t pixel,
-                          unsigned tracing) {
+template <bool kF32>
+C5_HD RayResult trace_ray(const WalkParams& P, double px, double py, uint32_t pixel, unsigned tracing) {
     RayResult r;
     r.tau = 0.0;
     r.inten = 0.0;
@@ -715,19 +520,18 @@ C5_HD RayResult trace_ray(const WalkParams& P, const BvhNode* top, double px, do
     EntryList<kInline> L;
 
     // A: nearest entry
-    bool defer = !bvh_collect_entries(P, top, px, py, z_after, L, 1, P.query_budget);
+    bool defer = !bvh_collect_entries(P, px, py, z_after, L, 1, P.query_budget);
     sync_lanes(tracing);
     // B: first crossing
     const bool entered = !defer && L.n > 0;
     if (entered) {
-        z_after = crossing<kF32, kWide, kPipe, false, kRec>(P, px, py, L.leaf[0], L.z[0], r.tau, r.inten, gain_unused,
-                                                            r.steps, r.error);
+        z_after = crossing<kF32, false>(P, px, py, L.leaf[0], L.z[0], r.tau, r.inten, gain_unused, r.steps, r.error);
     }
     sync_lanes(tracing);
     // C: anything above the exit?
     L.n = 0;
     if (entered && !r.error) {
-        const bool searched = bvh_collect_entries(P, top, px, py, z_after, L, kInline, P.query_budget);
+        const bool searched = bvh_collect_entries(P, px, py, z_after, L, kInline, P.query_budget);
         defer = !searched || L.n == kInline; // too many boxes in the way, or too many entries
     }
     sync_lanes(tracing);
@@ -736,8 +540,7 @@ C5_HD RayResult trace_ray(const WalkParams& P, const BvhNode* top, double px, do
         // an entry at or below the ray's position is already behind it (two boundary faces sharing
         // the edge the ray passes through report the same depth)
         if (!defer && e < L.n && L.z[e] > z_after && !r.error) {
-            z_after = crossing<kF32, kWide, kPipe, false, kRec>(P, px, py, L.leaf[e], L.z[e], r.tau, r.inten, gain_unused,
-                                                                r.steps, r.error);
+            z_after = crossing<kF32, false>(P, px, py, L.leaf[e], L.z[e], r.tau, r.inten, gain_unused, r.steps, r.error);
         }
         sync_lanes(tracing);
     }
@@ -796,13 +599,12 @@ C5_HD RayAcc graze_ray_serial(const WalkParams& P, const DeferredRay& q, double 
     EntryList<kSerialList> L;
     int crossings = 0;
     while (!a.error) {
-        if (!bvh_collect_entries(P, nullptr, px, py, a.z_after, L, P.serial_cap, 0x7FFFFFFF)) a.error = 1; // stack overflow
+        if (!bvh_collect_entries(P, px, py, a.z_after, L, P.serial_cap, 0x7FFFFFFF)) a.error = 1; // stack overflow
         for (int e = 0; e < L.n; e++) {
             if (!(L.z[e] > a.z_after)) continue;
             double tau_k = 0.0, inten_k = 0.0, gain_k = 1.0;
             uint32_t steps_k = 0, error_k = 0;
-            const double z_out = crossing<kF32, false, 0, true>(P, px, py, L.leaf[e], L.z[e], tau_k, inten_k, gain_k,
-                                                                steps_k, error_k);
+            const double z_out = crossing<kF32, true>(P, px, py, L.leaf[e], L.z[e], tau_k, inten_k, gain_k, steps_k, error_k);
             compose_crossing(a, L.z[e], z_out, tau_k, inten_k, gain_k, steps_k, error_k);
             if (++crossings > 65536) a.error = 1;
         }
@@ -997,8 +799,7 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
                 double z_out = z_in, tau_k = 0.0, inten_k = 0.0, gain_k = 1.0;
                 uint32_t steps_k = 0, error_k = 0;
                 if (have && z_in > a.z_after) { // a is the same in every lane
-                    z_out = crossing<kF32, true, 0, true>(P, px, py, S.leaf[k], z_in, tau_k, inten_k, gain_k, steps_k,
-                                                          error_k);
+                    z_out = crossing<kF32, true>(P, px, py, S.leaf[k], z_in, tau_k, inten_k, gain_k, steps_k, error_k);
                 }
                 const int cnt = n - base < 32 ? n - base : 32;
                 for (int l = 0; l < cnt; l++) {
@@ -1032,19 +833,8 @@ __device__ __forceinline__ int compact3(int v) {
     return (v & 1) | ((v >> 1) & 2) | ((v >> 2) & 4);
 }
 
-template <bool kF32, bool kWide, int kPipe, int kWarpsX = 2, int kWarpsY = 2, bool kRec = false>
-__device__ __forceinline__ void walk_block_body(const WalkParams& P) {
-    constexpr int kTx = 8 * kWarpsX, kTy = 4 * kWarpsY;
-    [[maybe_unused]] constexpr int kThreads = 32 * kWarpsX * kWarpsY;
-#ifdef C5_EXPERIMENTS
-    extern __shared__ __align__(64) unsigned char smem_raw[];
-    BvhNode* top = reinterpret_cast<BvhNode*>(smem_raw);
-#else
-    // (staging the top BVH levels in shared memory was measured slower than letting L1 serve them:
-    // C3 6.38 ms with 0 nodes, 6.54 with 63, 6.88 with 255; profiles/r01_exp_c3_variants_b.jsonl)
-    const BvhNode* top = nullptr;
-#endif
-
+template <bool kF32>
+__device__ __forceinline__ void walk_block(const WalkParams& P) {
     // screen-space order: macro tiles of 8 x 8 block tiles in row-major order, Morton inside, so that
     // concurrently resident blocks cover a compact patch of the image and share tets in L2
     const int b = blockIdx.x;
@@ -1053,9 +843,9 @@ __device__ __forceinline__ void walk_block_body(const WalkParams& P) {
     const int tile_y = (macro / P.n_macro_x) * 8 + compact3(r >> 1);
     if (tile_x >= P.n_tiles_x || tile_y >= P.n_tiles_y) return;
 
-    // Tiles that cannot see the mesh (outside the root's two boxes) skip the staging and the rays.
-    const int i_lo = P.i0 + tile_x * kTx, j_lo = P.j0 + tile_y * kTy;
-    const int i_hi = min(i_lo + kTx, P.i1) - 1, j_hi = min(j_lo + kTy, P.j1) - 1;
+    // Tiles that cannot see the mesh (outside the root's two boxes) skip the rays.
+    const int i_lo = P.i0 + tile_x * kTileX, j_lo = P.j0 + tile_y * kTileY;
+    const int i_hi = min(i_lo + kTileX, P.i1) - 1, j_hi = min(j_lo + kTileY, P.j1) - 1;
     bool tile_sees_mesh;
     {
         const BvhNode* root = P.nodes;
@@ -1065,18 +855,10 @@ __device__ __forceinline__ void walk_block_body(const WalkParams& P) {
         const bool s1 = x1 >= root->xlo[1] && x0 <= root->xhi[1] && y1 >= root->ylo[1] && y0 <= root->yhi[1];
         tile_sees_mesh = s0 || s1;
     }
-#ifdef C5_EXPERIMENTS
-    if (tile_sees_mesh && P.top_nodes > 0) {
-        const int4* src = reinterpret_cast<const int4*>(P.nodes);
-        int4* dst = reinterpret_cast<int4*>(top);
-        for (int k = threadIdx.x; k < P.top_nodes * 4; k += kThreads) dst[k] = src[k];
-        __syncthreads();
-    }
-#endif
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int i = P.i0 + tile_x * kTx + (warp % kWarpsX) * 8 + (lane & 7);
-    const int j = P.j0 + tile_y * kTy + (warp / kWarpsX) * 4 + (lane >> 3);
+    const int i = P.i0 + tile_x * kTileX + (warp % 2) * 8 + (lane & 7);
+    const int j = P.j0 + tile_y * kTileY + (warp / 2) * 4 + (lane >> 3);
     const bool live = i < P.i1 && j < P.j1;
 
     RayResult res;
@@ -1095,9 +877,9 @@ __device__ __forceinline__ void walk_block_body(const WalkParams& P) {
             store_pixel(P, i, j, nan, nan, 0);
         } else {
             if (tile_sees_mesh) {
-                res = trace_ray<kF32, kWide, kPipe, kRec>(P, top, P.xs[i], P.ys[j],
-                                                    static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
-                                                    tracing);
+                res = trace_ray<kF32>(P, P.xs[i], P.ys[j],
+                                      static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
+                                      tracing);
             }
             if (!res.deferred) store_pixel(P, i, j, res.tau, res.inten, res.steps);
         }
@@ -1124,65 +906,14 @@ __device__ __forceinline__ void walk_block_body(const WalkParams& P) {
     }
 }
 
-#ifdef C5_EXPERIMENTS
-__device__ __forceinline__ unsigned long long global_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#endif
-
-template <bool kF32, bool kWide, int kPipe, int kWarpsX = 2, int kWarpsY = 2, bool kRec = false>
-__device__ __forceinline__ void walk_block(const WalkParams& P) {
-#ifdef C5_EXPERIMENTS   // block timeline (C5_TRACE_FILE)
-    if (P.trace && threadIdx.x == 0) P.trace[4ull * blockIdx.x] = global_ns(); // stored at once: nothing stays live
-#endif
-    walk_block_body<kF32, kWide, kPipe, kWarpsX, kWarpsY, kRec>(P);
-#ifdef C5_EXPERIMENTS
-    if (P.trace) {
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            unsigned sm;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
-            unsigned long long* rec = P.trace + 4ull * blockIdx.x;
-            rec[1] = global_ns();
-            rec[2] = sm;
-            rec[3] = blockIdx.x;
-        }
-    }
-#endif
-}
-
 } // namespace
 
 // The product kernels. 7 blocks of 128 threads per SM = 72 registers: one more resident block than the
 // 80 the compiler picks on its own, measured faster (5.41 vs 5.64 ms on C3) despite a few spilled words
 // outside the step loop.
-__global__ void __launch_bounds__(kBlock, 7) tet_walk_fp64(const WalkParams P) { walk_block<false, true, 0>(P); }
+__global__ void __launch_bounds__(kBlock, 7) tet_walk_fp64(const WalkParams P) { walk_block<false>(P); }
 // optional single-precision step geometry (north-star item (d)); entry search and accumulators stay FP64
-__global__ void __launch_bounds__(kBlock, 8) tet_walk_fp32(const WalkParams P) { walk_block<true, true, 0>(P); }
-
-#ifdef C5_EXPERIMENTS
-// Variants measured and NOT adopted (C5_WALK_VARIANT selects one in libc5gpu_exp.so; results under
-// profiles/): 128-bit loads, L1 prefetch of the next step, 64-thread blocks, other register caps,
-// step records.
-__global__ void __launch_bounds__(kBlock) tet_walk_fp64_l128(const WalkParams P) { walk_block<false, false, 0>(P); }
-__global__ void __launch_bounds__(kBlock) tet_walk_fp64_pf(const WalkParams P) { walk_block<false, true, 1>(P); }
-__global__ void __launch_bounds__(64) tet_walk_fp64_b64(const WalkParams P) { walk_block<false, true, 0, 1, 2>(P); }
-__global__ void __launch_bounds__(kBlock, 6) tet_walk_fp64_r80(const WalkParams P) { walk_block<false, true, 0>(P); }
-__global__ void __launch_bounds__(kBlock, 8) tet_walk_fp64_r64(const WalkParams P) { walk_block<false, true, 0>(P); }
-__global__ void __launch_bounds__(kBlock, 5) tet_walk_fp64_r96(const WalkParams P) { walk_block<false, true, 0>(P); }
-__global__ void __launch_bounds__(kBlock, 7) tet_walk_fp64_rec(const WalkParams P) { walk_block<false, true, 0, 2, 2, true>(P); }
-// software-pipelined step loop (kPipe == 2) at 5, 6 and 7 resident blocks per SM (96 / 80 / 72 registers)
-__global__ void __launch_bounds__(kBlock, 5) tet_walk_fp64_sp5(const WalkParams P) { walk_block<false, true, 2>(P); }
-__global__ void __launch_bounds__(kBlock, 6) tet_walk_fp64_sp6(const WalkParams P) { walk_block<false, true, 2>(P); }
-__global__ void __launch_bounds__(kBlock, 7) tet_walk_fp64_sp7(const WalkParams P) { walk_block<false, true, 2>(P); }
-// Builds the four step records of every tet from its Cell (after prepare_cells: s depends on --alpha_limit).
-__global__ void __launch_bounds__(256) build_step_records(int64_t n_faces, const Cell* __restrict__ cells, StepRec* __restrict__ recs) {
-    const int64_t f = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-    if (f < n_faces) recs[f] = make_step_record(cells, f);
-}
-#endif
+__global__ void __launch_bounds__(kBlock, 8) tet_walk_fp32(const WalkParams P) { walk_block<true>(P); }
 
 // The walk's grid only covers the pixel rectangle that can see the mesh (a one-wave row band whose
 // grid is 60 % empty tiles fills the SMs unevenly: measured 1.60 M busy cycles on the fullest SM
@@ -1240,13 +971,7 @@ void walk_on_host(const WalkParams& P, bool f32) {
                 continue;
             }
             const uint32_t pixel = static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i);
-            RayResult r;
-#ifdef C5_EXPERIMENTS
-            if (!f32 && P.recs) r = trace_ray<false, false, 0, true>(P, nullptr, P.xs[i], P.ys[j], pixel, 0);
-            else
-#endif
-            r = f32 ? trace_ray<true, false, 0>(P, nullptr, P.xs[i], P.ys[j], pixel, 0)
-                    : trace_ray<false, false, 0>(P, nullptr, P.xs[i], P.ys[j], pixel, 0);
+            const RayResult r = f32 ? trace_ray<true>(P, P.xs[i], P.ys[j], pixel, 0) : trace_ray<false>(P, P.xs[i], P.ys[j], pixel, 0);
             if (!r.deferred) store_pixel(P, i, j, r.tau, r.inten, r.steps);
             P.counters[kSteps] += r.steps;
             P.row_cost[j] += r.steps;
@@ -1257,33 +982,6 @@ void walk_on_host(const WalkParams& P, bool f32) {
 }
 
 } // namespace
-
-#ifdef C5_EXPERIMENTS
-// The step records of the mesh `d` renders (its own, or its parent's for a sibling context), (re)built when
-// --alpha_limit changed.
-const StepRec* step_records(DeviceState& dd, double alpha_limit) {
-    DeviceState& d = dd.origin ? *dd.origin : dd;
-    if (d.recs_valid && d.recs_limit == alpha_limit && d.recs.n == static_cast<size_t>(4 * d.n_tets)) return d.recs.p;
-    if (4 * d.n_tets >= static_cast<int64_t>(kRecNoFace) || d.n_pts >= static_cast<int64_t>(kRecVtxLimit)) {
-        fail(C5_E_INVALID, "walk variant 'rec': mesh too large for 28-bit record / 25-bit vertex indices");
-    }
-    const bool shared = dd.origin != nullptr || d.mesh_shared;
-    if (shared && !kHostSim) C5_CUDA(cudaDeviceSynchronize()); // other lanes may be walking the old records
-    d.recs.ensure(static_cast<size_t>(4 * d.n_tets));
-    const int64_t n = 4 * d.n_tets;
-    count_launch();
-    if (kHostSim) {
-        for (int64_t f = 0; f < n; f++) d.recs.p[f] = make_step_record(d.cells.p, f);
-    } else {
-        build_step_records<<<static_cast<unsigned>((n + 255) / 256), 256, 0, dd.stream>>>(n, d.cells.p, d.recs.p);
-        C5_CUDA(cudaGetLastError());
-        if (shared) C5_CUDA(cudaDeviceSynchronize());
-    }
-    d.recs_limit = alpha_limit;
-    d.recs_valid = true;
-    return d.recs.p;
-}
-#endif
 
 // One view's rays on d.stream: background fill, the pixel kernel, then the grazing-ray kernel for the
 // rays it deferred — three launches in stream order, no kernel ever waits for another one. (Round 1
@@ -1310,14 +1008,6 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     P.res_y = w.res_y;
     P.row_begin = w.row_begin;
     P.row_end = w.row_end;
-    int tile_x = kTileX, tile_y = kTileY;
-#ifdef C5_EXPERIMENTS
-    const char* variant = std::getenv("C5_WALK_VARIANT");
-    const std::string var = variant ? variant : "";
-    const bool small_blocks = !f32 && var == "b64"; // 8 x 8 pixel tiles, 64 threads
-    if (small_blocks) tile_x = tile_y = 8;
-    P.recs = (!f32 && var == "rec") ? step_records(d, w.alpha_limit) : nullptr;
-#endif
     // the walk covers [i0,i1) x [j0,j1): the caller's estimate of where the mesh can be, cut to the band
     P.i0 = w.i_begin < 0 ? 0 : w.i_begin;
     P.i1 = w.i_end > w.res_x ? w.res_x : w.i_end;
@@ -1326,8 +1016,8 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     const bool empty_rect = P.i0 >= P.i1 || P.j0 >= P.j1;
     if (empty_rect) P.i0 = P.i1 = P.j0 = P.j1 = 0;
     const bool whole_band = P.i0 == 0 && P.i1 == w.res_x && P.j0 == w.row_begin && P.j1 == w.row_end;
-    P.n_tiles_x = (P.i1 - P.i0 + tile_x - 1) / tile_x;
-    P.n_tiles_y = (P.j1 - P.j0 + tile_y - 1) / tile_y;
+    P.n_tiles_x = (P.i1 - P.i0 + kTileX - 1) / kTileX;
+    P.n_tiles_y = (P.j1 - P.j0 + kTileY - 1) / kTileY;
     P.n_macro_x = (P.n_tiles_x + 7) / 8;
     const int n_macro_y = (P.n_tiles_y + 7) / 8;
     // c5_debug_set (tests shrink these to reach the overflow paths on small meshes); defaults otherwise
@@ -1357,81 +1047,25 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
         return;
     }
     const unsigned grid = static_cast<unsigned>(P.n_macro_x) * static_cast<unsigned>(n_macro_y) * 64u;
-    size_t smem = 0;
-#ifdef C5_EXPERIMENTS
-    const int64_t n_nodes = d.n_bfaces - 1;
-    int top = 0;
-    if (const char* e = std::getenv("C5_TOP_NODES")) top = std::atoi(e);
-    top = top < 0 ? 0 : top > 1023 ? 1023 : top;
-    P.top_nodes = static_cast<int>(n_nodes < top ? n_nodes : top);
-    smem = static_cast<size_t>(P.top_nodes) * sizeof(BvhNode);
-    P.trace = nullptr;
-    if (std::getenv("C5_TRACE_FILE") && d.trace_launches < kTraceLaunches) { // block timeline of the first launches
-        if (d.trace.n == 0) {
-            d.trace.alloc(static_cast<size_t>(kTraceLaunches) * kTraceBlocks * 4);
-            dev_zero(d.trace.p, d.trace.bytes(), d.stream);
-        }
-        if (grid <= kTraceBlocks) {
-            P.trace = d.trace.p + static_cast<size_t>(d.trace_launches) * kTraceBlocks * 4;
-            d.trace_grid[d.trace_launches] = grid;
-            d.trace_launches++;
-        }
-    }
     if (f32) {
-        tet_walk_fp32<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (small_blocks) {
-        tet_walk_fp64_b64<<<grid, 64, smem, d.stream>>>(P);
-    } else if (P.recs) {
-        tet_walk_fp64_rec<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "l128") {
-        tet_walk_fp64_l128<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "pf") {
-        tet_walk_fp64_pf<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "r80") {
-        tet_walk_fp64_r80<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "r64") {
-        tet_walk_fp64_r64<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "r96") {
-        tet_walk_fp64_r96<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "sp5") {
-        tet_walk_fp64_sp5<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "sp6") {
-        tet_walk_fp64_sp6<<<grid, kBlock, smem, d.stream>>>(P);
-    } else if (var == "sp7") {
-        tet_walk_fp64_sp7<<<grid, kBlock, smem, d.stream>>>(P);
+        tet_walk_fp32<<<grid, kBlock, 0, d.stream>>>(P);
     } else {
-        tet_walk_fp64<<<grid, kBlock, smem, d.stream>>>(P);
+        tet_walk_fp64<<<grid, kBlock, 0, d.stream>>>(P);
     }
-#else
-    if (f32) {
-        tet_walk_fp32<<<grid, kBlock, smem, d.stream>>>(P);
-    } else {
-        tet_walk_fp64<<<grid, kBlock, smem, d.stream>>>(P);
-    }
-#endif
     C5_CUDA(cudaGetLastError());
     if (w.mark_walk_done) C5_CUDA(cudaEventRecord(w.mark_walk_done, d.stream));
     if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
 
     // Rays the pixel kernel deferred: a fixed grid of persistent warps that draw tickets.
     if (d.sm_count == 0) C5_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, d.device));
-    const unsigned graze_grid = static_cast<unsigned>(d.sm_count) * static_cast<unsigned>(d.opt_graze_blocks > 0 ? d.opt_graze_blocks : kGrazeBlocksPerSm);
+    const unsigned graze_grid = static_cast<unsigned>(d.sm_count) * static_cast<unsigned>(kGrazeBlocksPerSm);
     count_launch();
-    cudaStream_t gs = d.stream;
-    if (w.graze_stream && w.mark_walk_done) { // c5_debug_set("prep_priority", 2): on the high-priority stream, still AFTER the pixel kernel
-        gs = w.graze_stream;
-        C5_CUDA(cudaStreamWaitEvent(gs, w.mark_walk_done, 0));
-    }
     if (f32) {
-        grazing_rays_fp32<<<graze_grid, 32 * kGrazeWarps, 0, gs>>>(P);
+        grazing_rays_fp32<<<graze_grid, 32 * kGrazeWarps, 0, d.stream>>>(P);
     } else {
-        grazing_rays_fp64<<<graze_grid, 32 * kGrazeWarps, 0, gs>>>(P);
+        grazing_rays_fp64<<<graze_grid, 32 * kGrazeWarps, 0, d.stream>>>(P);
     }
     C5_CUDA(cudaGetLastError());
-    if (gs != d.stream) {
-        C5_CUDA(cudaEventRecord(w.graze_join, gs));
-        C5_CUDA(cudaStreamWaitEvent(d.stream, w.graze_join, 0));
-    }
 }
 
 } // namespace c5

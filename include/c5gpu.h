@@ -210,14 +210,9 @@ uint64_t c5_kernel_launches(const c5_ctx* ctx);
  *   "query_budget"  BVH nodes a thread of the pixel kernel may visit per search before it hands the
  *                   ray to the grazing-ray kernel (>= 1, 0 = default 64)
  *   "serial_list"   the same for the serial form of the CPU test build (2..64)
- *   "graze_blocks"  blocks per SM of the grazing-ray kernel's grid (tuning experiments; 0 = default)
  *   "mask_tile"     100 w + h: tile size of the solid mask's "already solid" flags (0 = default)
- *   "mask_per_face" n > 0: the solid mask's face passes run one face per thread, 2^(n-1) lanes per tall face
- *                   (only in the experiments build, libc5gpu_exp.so; the product library ignores it)
  *   "no_static_mask" 1: solids that do not follow the view are scan-converted in every view, like the
  *                   others, instead of once per pixel grid (tests compare the two)
- *   "prep_priority" bit 0: rotate / refit / mask of a view run on a high-priority stream of their own;
- *                   bit 1: so does the grazing-ray kernel (still after the pixel kernel, by event)
  *   "no_zero_copy"  1: page-locked output buffers get a device-to-host copy like pageable ones
  *   "timeline"      n > 0: keep the phase events of the last n views of every lane (0 = off)
  * Unknown keys return C5_E_INVALID.

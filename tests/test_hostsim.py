@@ -98,6 +98,18 @@ def test_static_solid_mask_cache(hostsim_lib, port):
     rc.check_static_solid_mask_cache(hostsim_lib, port)
 
 
+def test_debug_set_rejects_unknown_keys(hostsim_lib):
+    """Keys c5gpu.h does not list return C5_E_INVALID instead of being ignored; the first three
+    selected kernel variants and a second stream that have been removed."""
+    from course5_b200 import api
+    with api.Context(lib=hostsim_lib) as ctx:
+        for key in ("prep_priority", "graze_blocks", "mask_per_face", "no_such_key"):
+            with pytest.raises(api.C5Error) as e:
+                ctx.debug_set(key, 1)
+            assert e.value.code == api.E_INVALID, key
+        ctx.debug_set("query_budget", 0)  # a listed key is still accepted
+
+
 def test_image_handles_and_host_register(hostsim_lib):
     """c5_image_create / open / close and c5_host_register bookkeeping (the CUDA IPC mapping itself
     needs two processes and two GPUs: test_gpu_dist.py)."""
