@@ -24,7 +24,7 @@ const double kPi = 3.14159265358979323846; // config.hpp:45
 template <class Fn>
 int guarded(c5_ctx* ctx, Fn&& fn) {
     try {
-        if (ctx) g_launch_counter = &ctx->dev[0]->launches;
+        if (ctx) g_launch_counter = &ctx->dev.launches;
         fn();
         return C5_OK;
     } catch (const Error& e) {
@@ -43,8 +43,15 @@ void use_device(const DeviceState& d) {
     if (!kHostSim) C5_CUDA(cudaSetDevice(d.device));
 }
 
+// The context and, for a multi-device context, its parts: one context per device.
+std::vector<c5_ctx*> with_parts(c5_ctx* ctx) {
+    std::vector<c5_ctx*> all{ctx};
+    all.insert(all.end(), ctx->parts.begin(), ctx->parts.end());
+    return all;
+}
+
 // Phase events of the view being enqueued: 0 start, 1 rotated, 2 BVH refitted, 3 mask done,
-// 4 walk done (pixel + grazing-ray kernel), 5 band gathered (multi-device), 6 image on the host;
+// 4 walk done (pixel + grazing-ray kernel), 5 image copy starts, 6 image on the host;
 // ev_walk sits between the two walk kernels.
 void record(DeviceState& d, int k) {
     if (!kHostSim) C5_CUDA(cudaEventRecord(d.ev[k], d.stream));
@@ -230,62 +237,6 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     if (!d.tl_events.empty()) d.tl_views++;
 }
 
-// ---- NCCL, loaded lazily: only multi-device contexts need it ---------------------------------------
-struct NcclApi {
-    void* handle = nullptr;
-    int (*CommInitAll)(void**, int, const int*) = nullptr;
-    int (*CommDestroy)(void*) = nullptr;
-    int (*GroupStart)() = nullptr;
-    int (*GroupEnd)() = nullptr;
-    int (*Send)(const void*, size_t, int, int, void*, cudaStream_t) = nullptr;
-    int (*Recv)(void*, size_t, int, int, void*, cudaStream_t) = nullptr;
-    const char* (*GetErrorString)(int) = nullptr;
-};
-constexpr int kNcclFloat64 = 8; // ncclDouble
-
-struct NcclGroup {
-    NcclApi api;
-    std::vector<void*> comms;
-};
-
-void nccl_check(const NcclApi& api, int rc, const char* what) {
-    if (rc != 0) fail(C5_E_NCCL, std::string(what) + ": " + (api.GetErrorString ? api.GetErrorString(rc) : "error"));
-}
-
-NcclGroup* nccl_open(const std::vector<int>& devices) {
-    auto g = std::make_unique<NcclGroup>();
-    NcclApi& a = g->api;
-    for (const char* name : {"libnccl.so.2", "libnccl.so"}) {
-        a.handle = dlopen(name, RTLD_NOW | RTLD_GLOBAL);
-        if (a.handle) break;
-    }
-    if (!a.handle) fail(C5_E_NCCL, std::string("cannot load libnccl.so.2: ") + dlerror());
-    auto sym = [&](const char* n) {
-        void* p = dlsym(a.handle, n);
-        if (!p) fail(C5_E_NCCL, std::string("libnccl lacks ") + n);
-        return p;
-    };
-    a.CommInitAll = reinterpret_cast<decltype(a.CommInitAll)>(sym("ncclCommInitAll"));
-    a.CommDestroy = reinterpret_cast<decltype(a.CommDestroy)>(sym("ncclCommDestroy"));
-    a.GroupStart = reinterpret_cast<decltype(a.GroupStart)>(sym("ncclGroupStart"));
-    a.GroupEnd = reinterpret_cast<decltype(a.GroupEnd)>(sym("ncclGroupEnd"));
-    a.Send = reinterpret_cast<decltype(a.Send)>(sym("ncclSend"));
-    a.Recv = reinterpret_cast<decltype(a.Recv)>(sym("ncclRecv"));
-    a.GetErrorString = reinterpret_cast<decltype(a.GetErrorString)>(sym("ncclGetErrorString"));
-    g->comms.assign(devices.size(), nullptr);
-    nccl_check(a, a.CommInitAll(g->comms.data(), static_cast<int>(devices.size()), devices.data()), "ncclCommInitAll");
-    return g.release();
-}
-
-void nccl_close(void* p) {
-    auto* g = static_cast<NcclGroup*>(p);
-    if (!g) return;
-    for (void* c : g->comms) {
-        if (c) g->api.CommDestroy(c);
-    }
-    delete g;
-}
-
 // Contiguous row bands of [row_begin,row_end) with equal estimated cost (previous view's per-row
 // tet-steps plus a constant per row), one per device; equal heights when there is no history.
 std::vector<std::pair<int, int>> cut_bands(const c5_ctx* ctx, const c5_view* v, const ViewPlan& p, int n) {
@@ -320,180 +271,7 @@ std::vector<std::pair<int, int>> cut_bands(const c5_ctx* ctx, const c5_view* v, 
     return bands;
 }
 
-struct Counters {
-    unsigned long long c[kNumCounters] = {};
-};
-
-void follow_parent(c5_ctx* ctx);
-
-// Multi-device contexts (c5_create with several devices, one process): plane ctor + find_intersections
-// + trace_rays for one view into a HOST buffer; device r renders band r, the bands land in device 0's
-// image by one grouped NCCL send/recv, device 0 copies the image to the host. Synchronous.
-void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, c5_stats* st) {
-    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    if (!out) fail(C5_E_INVALID, "render: out is NULL");
-    const ViewPlan p = plan_view(v);
-    const int n_dev = static_cast<int>(ctx->dev.size());
-    if ((p.row_end - p.row_begin) < n_dev) fail(C5_E_INVALID, "render: fewer rows than devices");
-    const auto bands = cut_bands(ctx, v, p, n_dev);
-    DeviceState& d0 = *ctx->dev[0];
-    const size_t row_doubles = static_cast<size_t>(v->res_x) * 2;
-    const size_t n_pix_view = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
-    use_device(d0);
-    d0.out.ensure(2 * n_pix_view); // device 0 assembles the whole view here
-    const size_t view_off = static_cast<size_t>(p.row_begin) * v->res_x;
-
-    // enqueue every device's band (asynchronous; devices run concurrently). With several devices
-    // one host thread per device issues the launches, so launch latency is not serialised.
-    auto enqueue_band = [&](int r) {
-        DeviceState& d = *ctx->dev[static_cast<size_t>(r)];
-        ViewPlan pr = p;
-        pr.row_begin = bands[static_cast<size_t>(r)].first;
-        pr.row_end = bands[static_cast<size_t>(r)].second;
-        double* target = nullptr;
-        if (r == 0) target = d0.out.p + static_cast<size_t>(pr.row_begin - p.row_begin) * row_doubles;
-        enqueue_view(d, v, pr, steps != nullptr, target);
-    };
-    if (kHostSim) {
-        for (int r = 0; r < n_dev; r++) enqueue_band(r);
-    } else {
-        std::vector<std::thread> workers;
-        std::vector<std::exception_ptr> errors(static_cast<size_t>(n_dev));
-        for (int r = 0; r < n_dev; r++) {
-            workers.emplace_back([&, r] {
-                try {
-                    enqueue_band(r);
-                } catch (...) {
-                    errors[static_cast<size_t>(r)] = std::current_exception();
-                }
-            });
-        }
-        for (auto& w : workers) w.join();
-        for (auto& e : errors) {
-            if (e) std::rethrow_exception(e);
-        }
-        g_launch_counter = &d0.launches;
-    }
-
-    // gather-v of the bands into device 0's image
-    {
-        if (kHostSim) {
-            for (int r = 1; r < n_dev; r++) {
-                const auto& b = bands[static_cast<size_t>(r)];
-                std::memcpy(d0.out.p + static_cast<size_t>(b.first - p.row_begin) * row_doubles,
-                            ctx->dev[static_cast<size_t>(r)]->out.p, static_cast<size_t>(b.second - b.first) * row_doubles * sizeof(double));
-            }
-        } else {
-            auto* g = static_cast<NcclGroup*>(ctx->nccl);
-            nccl_check(g->api, g->api.GroupStart(), "ncclGroupStart");
-            for (int r = 1; r < n_dev; r++) {
-                const auto& b = bands[static_cast<size_t>(r)];
-                const size_t count = static_cast<size_t>(b.second - b.first) * row_doubles;
-                DeviceState& d = *ctx->dev[static_cast<size_t>(r)];
-                nccl_check(g->api, g->api.Send(d.out.p, count, kNcclFloat64, 0, g->comms[static_cast<size_t>(r)], d.stream), "ncclSend");
-                nccl_check(g->api, g->api.Recv(d0.out.p + static_cast<size_t>(b.first - p.row_begin) * row_doubles, count, kNcclFloat64, r,
-                                               g->comms[0], d0.stream), "ncclRecv");
-            }
-            nccl_check(g->api, g->api.GroupEnd(), "ncclGroupEnd");
-        }
-    }
-    use_device(d0);
-    record(d0, 5);
-    d2h(out + 2 * view_off, d0.out.p, 2 * n_pix_view * sizeof(double), d0.stream);
-    record(d0, 6);
-
-    // per-device extras (steps, mask), counters, row costs
-    const bool solids = v->use_solids && (d0.solid_follow.n + d0.solid_static.n) > 0;
-    std::vector<Counters> counters(static_cast<size_t>(n_dev));
-    std::vector<std::vector<uint64_t>> row_cost(static_cast<size_t>(n_dev));
-    for (int r = 0; r < n_dev; r++) {
-        DeviceState& d = *ctx->dev[static_cast<size_t>(r)];
-        use_device(d);
-        const auto& b = bands[static_cast<size_t>(r)];
-        const size_t band_off = static_cast<size_t>(b.first) * v->res_x;
-        const size_t n_pix_band = static_cast<size_t>(b.second - b.first) * v->res_x;
-        if (steps) d2h(steps + band_off, d.steps.p, n_pix_band * sizeof(uint32_t), d.stream);
-        if (solid_mask) {
-            if (solids) d2h(solid_mask + band_off, d.mask.p + band_off, n_pix_band, d.stream);
-            else std::memset(solid_mask + band_off, 0, n_pix_band);
-        }
-        d2h(counters[static_cast<size_t>(r)].c, d.counters.p, sizeof(Counters), d.stream);
-        row_cost[static_cast<size_t>(r)].assign(static_cast<size_t>(v->res_y), 0);
-        d2h(row_cost[static_cast<size_t>(r)].data(), d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
-    }
-    for (auto& dp : ctx->dev) {
-        use_device(*dp);
-        stream_sync(dp->stream);
-    }
-    use_device(d0);
-
-    Counters total;
-    ctx->last_row_cost.assign(static_cast<size_t>(v->res_y), 0);
-    for (int r = 0; r < n_dev; r++) {
-        for (int k = 0; k < kNumCounters; k++) total.c[k] += counters[static_cast<size_t>(r)].c[k];
-        for (int j = 0; j < v->res_y; j++) ctx->last_row_cost[static_cast<size_t>(j)] += row_cost[static_cast<size_t>(r)][static_cast<size_t>(j)];
-    }
-    if (st) {
-        std::memset(st, 0, sizeof(*st));
-        st->pixels = static_cast<uint64_t>(n_pix_view);
-        st->tet_steps = total.c[kSteps];
-        st->hit_pixels = total.c[kHitPixels];
-        st->solid_pixels = total.c[kSolidPixels];
-        st->walk_errors = total.c[kWalkErrors];
-        st->grazing_rays = static_cast<int32_t>(total.c[kDeferred]);
-        for (auto& dp : ctx->dev) { // phase times: the slowest device
-            use_device(*dp);
-            st->ms_rotate = std::max(st->ms_rotate, elapsed(*dp, 0, 1));
-            st->ms_bvh = std::max(st->ms_bvh, elapsed(*dp, 1, 2));
-            st->ms_mask = std::max(st->ms_mask, elapsed(*dp, 2, 3));
-            st->ms_walk = std::max(st->ms_walk, elapsed(*dp, 3, 4));
-            if (!kHostSim) {
-                float g = 0.f;
-                C5_CUDA(cudaEventElapsedTime(&g, dp->ev_walk, dp->ev[4]));
-                st->ms_graze = std::max(st->ms_graze, g);
-            }
-        }
-        use_device(d0);
-        st->ms_gather = elapsed(d0, 4, 5);
-        st->ms_d2h = elapsed(d0, 5, 6);
-        st->ms_total = elapsed(d0, 0, 6);
-        st->n_devices = n_dev;
-    }
-    if (total.c[kWalkErrors]) {
-        fail(C5_E_WALK, "render: " + std::to_string(total.c[kWalkErrors]) + " ray(s) exceeded the step cap");
-    }
-}
-
-// Single-device, device-resident output (the caller's buffer), no host copy of the image.
-void collect_stats(c5_ctx* ctx, DeviceState& d, const c5_view* v, const ViewPlan& p, c5_stats* st, int ev_last) {
-    unsigned long long c[kNumCounters] = {};
-    d2h(c, d.counters.p, sizeof(c), d.stream);
-    ctx->last_row_cost.assign(static_cast<size_t>(v->res_y), 0);
-    static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "row cost width");
-    d2h(ctx->last_row_cost.data(), d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
-    stream_sync(d.stream);
-    if (st) {
-        std::memset(st, 0, sizeof(*st));
-        st->pixels = static_cast<uint64_t>(p.row_end - p.row_begin) * static_cast<uint64_t>(v->res_x);
-        st->tet_steps = c[kSteps];
-        st->hit_pixels = c[kHitPixels];
-        st->solid_pixels = c[kSolidPixels];
-        st->walk_errors = c[kWalkErrors];
-        st->grazing_rays = static_cast<int32_t>(c[kDeferred]);
-        st->ms_rotate = elapsed(d, 0, 1);
-        st->ms_bvh = elapsed(d, 1, 2);
-        st->ms_mask = elapsed(d, 2, 3);
-        st->ms_walk = elapsed(d, 3, 4);
-        if (!kHostSim) C5_CUDA(cudaEventElapsedTime(&st->ms_graze, d.ev_walk, d.ev[4]));
-        st->ms_total = elapsed(d, 0, ev_last);
-        st->n_devices = 1;
-    }
-    if (c[kWalkErrors]) {
-        fail(C5_E_WALK, "render: " + std::to_string(c[kWalkErrors]) + " ray(s) exceeded the step cap");
-    }
-}
-
-// ---- single-device contexts: submit / wait -----------------------------------------------------------
+// ---- one device: submit / wait -----------------------------------------------------------------------
 // A view is enqueued on the context's stream together with the copies that bring its results to the
 // host (image unless it is stored in place, counters, per-row costs -> page-locked staging), then an
 // event; waiting for the view is waiting for that event. Nothing in between touches the host, so
@@ -510,6 +288,8 @@ void ensure_host_staging(DeviceState& d, size_t rows) {
     }
 }
 
+void follow_parent(c5_ctx* ctx);
+
 void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, uint64_t ticket,
                  bool in_place_allowed = true) {
     follow_parent(ctx);
@@ -517,7 +297,7 @@ void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, ui
     if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
     if (!out) fail(C5_E_INVALID, "render: out is NULL");
     const ViewPlan p = plan_view(v);
-    DeviceState& d = *ctx->dev[0];
+    DeviceState& d = ctx->dev;
     use_device(d);
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
     const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
@@ -560,38 +340,123 @@ void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, ui
     ctx->pending.d2h_copy = host_direct == nullptr;
 }
 
-// Waits for the view `lane` has in flight; row costs and errors are reported through `owner`
-// (the context the caller holds: lane itself, or the context whose lane it is).
-void finish_view(c5_ctx* owner, c5_ctx* lane, c5_stats* st) {
+// What one device reports for a view: its stats and per-row tet-steps.
+struct ViewResult {
+    c5_stats st{};
+    std::vector<uint64_t> row_cost;
+};
+
+// Reads d's last view (planned as p) from the page-locked staging, once the stream has passed the
+// copies into it. A submitted view ends with the image on the host (event 6); a view of
+// c5_render_device ends with the walk (event 4) and has no ms_d2h.
+ViewResult read_view(DeviceState& d, const c5_view& v, const ViewPlan& p, bool submitted) {
+    ViewResult r;
+    c5_stats& st = r.st;
+    const unsigned long long* c = d.h_counters;
+    st.pixels = static_cast<uint64_t>(p.row_end - p.row_begin) * static_cast<uint64_t>(v.res_x);
+    st.tet_steps = c[kSteps];
+    st.hit_pixels = c[kHitPixels];
+    st.solid_pixels = c[kSolidPixels];
+    st.walk_errors = c[kWalkErrors];
+    st.grazing_rays = static_cast<int32_t>(c[kDeferred]);
+    st.ms_rotate = elapsed(d, 0, 1);
+    st.ms_bvh = elapsed(d, 1, 2);
+    st.ms_mask = elapsed(d, 2, 3);
+    st.ms_walk = elapsed(d, 3, 4);
+    if (!kHostSim) C5_CUDA(cudaEventElapsedTime(&st.ms_graze, d.ev_walk, d.ev[4]));
+    if (submitted) st.ms_d2h = elapsed(d, 5, 6);
+    st.ms_total = elapsed(d, 0, submitted ? 6 : 4);
+    st.n_devices = 1;
+    r.row_cost.assign(d.h_row_cost, d.h_row_cost + v.res_y);
+    return r;
+}
+
+// Row costs go to `owner` (the context the caller holds), stats to *st (may be NULL); a ray stopped
+// by the step cap is C5_E_WALK.
+void report(c5_ctx* owner, ViewResult& r, c5_stats* st) {
+    owner->last_row_cost = std::move(r.row_cost);
+    if (st) *st = r.st;
+    if (r.st.walk_errors) {
+        fail(C5_E_WALK, "render: " + std::to_string(r.st.walk_errors) + " ray(s) exceeded the step cap");
+    }
+}
+
+// Waits for the view `lane` has in flight and reads it.
+ViewResult wait_view(c5_ctx* lane) {
     if (!lane->pending.active) fail(C5_E_STATE, "render_wait: no view in flight");
-    DeviceState& d = *lane->dev[0];
+    DeviceState& d = lane->dev;
     use_device(d);
     lane->pending.active = false; // whatever happens below, the lane is free again
     if (!kHostSim) C5_CUDA(cudaEventSynchronize(d.ev_done));
-    const c5_view& v = lane->pending.view;
-    const ViewPlan& p = lane->pending.plan;
-    owner->last_row_cost.assign(d.h_row_cost, d.h_row_cost + v.res_y);
-    const unsigned long long* c = d.h_counters;
-    if (st) {
-        std::memset(st, 0, sizeof(*st));
-        st->pixels = static_cast<uint64_t>(p.row_end - p.row_begin) * static_cast<uint64_t>(v.res_x);
-        st->tet_steps = c[kSteps];
-        st->hit_pixels = c[kHitPixels];
-        st->solid_pixels = c[kSolidPixels];
-        st->walk_errors = c[kWalkErrors];
-        st->grazing_rays = static_cast<int32_t>(c[kDeferred]);
-        st->ms_rotate = elapsed(d, 0, 1);
-        st->ms_bvh = elapsed(d, 1, 2);
-        st->ms_mask = elapsed(d, 2, 3);
-        st->ms_walk = elapsed(d, 3, 4);
-        if (!kHostSim) C5_CUDA(cudaEventElapsedTime(&st->ms_graze, d.ev_walk, d.ev[4]));
-        st->ms_d2h = elapsed(d, 5, 6);
-        st->ms_total = elapsed(d, 0, 6);
-        st->n_devices = 1;
+    return read_view(d, lane->pending.view, lane->pending.plan, true);
+}
+
+// Multi-device contexts (c5_create with several devices): the context and each of its parts render
+// one cost-balanced row band, as c5_render does for a row band, straight into its final rows of the
+// caller's buffers. One host thread per device submits: a copy into pageable memory blocks the
+// submitting thread until its device is done, so one thread would render the bands one after another.
+void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, c5_stats* st) {
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    const ViewPlan p = plan_view(v);
+    const std::vector<c5_ctx*> parts = with_parts(ctx);
+    const size_t n = parts.size();
+    if (static_cast<size_t>(p.row_end - p.row_begin) < n) fail(C5_E_INVALID, "render: fewer rows than devices");
+    const auto bands = cut_bands(ctx, v, p, static_cast<int>(n));
+    std::vector<c5_view> band_views(n, *v);
+    std::vector<std::exception_ptr> errors(n);
+    auto submit = [&](size_t r) {
+        try {
+            band_views[r].row_begin = bands[r].first;
+            band_views[r].row_end = bands[r].second;
+            submit_view(parts[r], &band_views[r], out, steps, solid_mask, 0);
+        } catch (...) {
+            errors[r] = std::current_exception();
+        }
+    };
+    if (kHostSim) {
+        for (size_t r = 0; r < n; r++) submit(r);
+    } else {
+        std::vector<std::thread> workers;
+        for (size_t r = 0; r < n; r++) workers.emplace_back(submit, r);
+        for (auto& w : workers) w.join();
     }
-    if (c[kWalkErrors]) {
-        fail(C5_E_WALK, "render: " + std::to_string(c[kWalkErrors]) + " ray(s) exceeded the step cap");
+    // every band that was submitted is waited for, also when another failed: none may still be
+    // writing into the caller's buffers once this returns
+    std::vector<ViewResult> results(n);
+    for (size_t r = 0; r < n; r++) {
+        if (!parts[r]->pending.active) continue;
+        try {
+            results[r] = wait_view(parts[r]);
+        } catch (...) {
+            if (!errors[r]) errors[r] = std::current_exception();
+        }
     }
+    for (auto& e : errors) {
+        if (e) std::rethrow_exception(e);
+    }
+    // counters and row costs add up, phase times are the slowest device's
+    ViewResult total;
+    c5_stats& t = total.st;
+    total.row_cost.assign(static_cast<size_t>(v->res_y), 0);
+    for (const ViewResult& r : results) {
+        const c5_stats& s = r.st;
+        t.pixels += s.pixels;
+        t.tet_steps += s.tet_steps;
+        t.hit_pixels += s.hit_pixels;
+        t.solid_pixels += s.solid_pixels;
+        t.walk_errors += s.walk_errors;
+        t.grazing_rays += s.grazing_rays;
+        t.ms_rotate = std::max(t.ms_rotate, s.ms_rotate);
+        t.ms_bvh = std::max(t.ms_bvh, s.ms_bvh);
+        t.ms_mask = std::max(t.ms_mask, s.ms_mask);
+        t.ms_walk = std::max(t.ms_walk, s.ms_walk);
+        t.ms_graze = std::max(t.ms_graze, s.ms_graze);
+        t.ms_d2h = std::max(t.ms_d2h, s.ms_d2h);
+        t.ms_total = std::max(t.ms_total, s.ms_total);
+        for (size_t j = 0; j < total.row_cost.size(); j++) total.row_cost[j] += r.row_cost[j];
+    }
+    t.n_devices = static_cast<int32_t>(n);
+    report(ctx, total, st);
 }
 
 // The lanes of c5_render_submit: lane 0 is the context itself, the others are sibling contexts the
@@ -612,8 +477,8 @@ void ensure_lanes(c5_ctx* ctx) {
 void upload_solids(c5_ctx* ctx, const double* pts, int64_t n, int follows) {
     if (n < 0 || (n > 0 && !pts)) fail(C5_E_INVALID, "upload_solids: bad arguments");
     if (n == 0) return;
-    for (auto& dp : ctx->dev) {
-        DeviceState& d = *dp;
+    for (c5_ctx* c : with_parts(ctx)) {
+        DeviceState& d = c->dev;
         use_device(d);
         SolidSet& ss = follows ? d.solid_follow : d.solid_static;
         const size_t old_n = static_cast<size_t>(ss.n), add = static_cast<size_t>(n);
@@ -691,8 +556,8 @@ void alias_mesh(DeviceState& s, DeviceState& o) {
 void follow_parent(c5_ctx* ctx) {
     if (!ctx->parent) return;
     c5_ctx* par = ctx->parent;
-    DeviceState& s = *ctx->dev[0];
-    DeviceState& o = *par->dev[0];
+    DeviceState& s = ctx->dev;
+    DeviceState& o = par->dev;
     if (par->has_mesh && (s.origin != &o || s.mesh_version != o.mesh_version)) alias_mesh(s, o);
     ctx->has_mesh = par->has_mesh;
     ctx->info = par->info;
@@ -755,7 +620,7 @@ int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out) {
             std::lock_guard<std::mutex> lock(g_create_err_mu);
             g_create_err = text;
         }
-        c5_destroy(ctx); // the same teardown as a finished context: streams, events, NCCL, device memory
+        c5_destroy(ctx); // the same teardown as a finished context: parts, streams, events, device memory
         return code;
     };
     try {
@@ -772,21 +637,20 @@ int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out) {
                 if (devices[k] < 0 || devices[k] >= count) fail(C5_E_INVALID, "c5_create: device ordinal out of range");
             }
         }
-        for (int k = 0; k < n_dev; k++) {
-            ctx->dev.push_back(std::make_unique<DeviceState>());
-            DeviceState* d = ctx->dev.back().get(); // in the context before anything is created: a failure below is torn down
-            d->device = devices[k];
-            if (!kHostSim) {
-                C5_CUDA(cudaSetDevice(d->device));
-                C5_CUDA(cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking));
-                for (auto& e : d->ev) C5_CUDA(cudaEventCreate(&e));
-                C5_CUDA(cudaEventCreate(&d->ev_walk));
-                C5_CUDA(cudaEventCreateWithFlags(&d->ev_done, cudaEventDisableTiming));
-            }
+        DeviceState& d = ctx->dev;
+        d.device = devices[0];
+        if (!kHostSim) {
+            C5_CUDA(cudaSetDevice(d.device));
+            C5_CUDA(cudaStreamCreateWithFlags(&d.stream, cudaStreamNonBlocking));
+            for (auto& e : d.ev) C5_CUDA(cudaEventCreate(&e));
+            C5_CUDA(cudaEventCreate(&d.ev_walk));
+            C5_CUDA(cudaEventCreateWithFlags(&d.ev_done, cudaEventDisableTiming));
         }
-        if (n_dev > 1 && !kHostSim) {
-            ctx->nccl = nccl_open(std::vector<int>(devices, devices + n_dev));
-            // peers are only touched by NCCL; each device keeps its own replica of the mesh
+        for (int k = 1; k < n_dev; k++) { // every further device: a single-device context of its own
+            c5_ctx* part = nullptr;
+            const int rc = c5_create(&devices[k], 1, &part);
+            if (rc != C5_OK) fail(rc, c5_last_error(nullptr));
+            ctx->parts.push_back(part);
         }
         *out = ctx;
         return C5_OK;
@@ -800,18 +664,18 @@ int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out) {
 int c5_create_sibling(c5_ctx* parent, c5_ctx** out) {
     if (!parent || !out) return C5_E_INVALID;
     *out = nullptr;
-    if (parent->parent || parent->dev.size() != 1) {
+    if (parent->parent || !parent->parts.empty()) {
         parent->err = "create_sibling: the parent must be a single-device context that is not itself a sibling";
         return C5_E_INVALID;
     }
-    const int32_t device = parent->dev[0]->device;
+    const int32_t device = parent->dev.device;
     c5_ctx* ctx = nullptr;
     const int rc = c5_create(&device, 1, &ctx);
     if (rc != C5_OK) return rc;
     ctx->parent = parent;
     parent->siblings.push_back(ctx);
-    DeviceState& from = *parent->dev[0];
-    DeviceState& to = *ctx->dev[0];
+    DeviceState& from = parent->dev;
+    DeviceState& to = ctx->dev;
     to.opt_graze_list = from.opt_graze_list;
     to.opt_query_budget = from.opt_query_budget;
     to.opt_serial_list = from.opt_serial_list;
@@ -826,25 +690,26 @@ void c5_destroy(c5_ctx* ctx) {
     if (!ctx) return;
     for (c5_ctx* lane : ctx->lanes) c5_destroy(lane); // our own lanes go first (each leaves ctx->siblings)
     ctx->lanes.clear();
+    for (c5_ctx* part : ctx->parts) c5_destroy(part);
+    ctx->parts.clear();
     if (ctx->parent) { // a sibling leaves its parent's list
         auto& sib = ctx->parent->siblings;
         sib.erase(std::remove(sib.begin(), sib.end(), ctx), sib.end());
     }
     for (c5_ctx* s : ctx->siblings) { // a parent going first takes the shared mesh with it
-        if (!kHostSim && !s->dev.empty()) {
-            cudaSetDevice(s->dev[0]->device);
+        if (!kHostSim) {
+            cudaSetDevice(s->dev.device);
             cudaDeviceSynchronize();
         }
         s->parent = nullptr;
         s->has_mesh = false;
-        if (!s->dev.empty()) s->dev[0]->origin = nullptr;
+        s->dev.origin = nullptr;
     }
     ctx->siblings.clear();
-    nccl_close(ctx->nccl);
-    ctx->nccl = nullptr;
-    if (!kHostSim && !ctx->dev.empty() && ctx->dev[0]->stream) {
-        cudaSetDevice(ctx->dev[0]->device);
-        cudaStreamSynchronize(ctx->dev[0]->stream);
+    DeviceState& d = ctx->dev;
+    if (!kHostSim && d.stream) {
+        cudaSetDevice(d.device);
+        cudaStreamSynchronize(d.stream);
     }
     for (void* p : ctx->registered) {
         if (!kHostSim) cudaHostUnregister(p);
@@ -853,27 +718,18 @@ void c5_destroy(c5_ctx* ctx) {
         if (im.second) dev_free(im.first);
         else if (!kHostSim) cudaIpcCloseMemHandle(im.first);
     }
-    for (auto& dp : ctx->dev) {
-        DeviceState& d = *dp;
-        if (!kHostSim) {
-            cudaSetDevice(d.device);
-            if (d.stream) cudaStreamSynchronize(d.stream);
+    host_pinned_free(d.h_counters);
+    host_pinned_free(d.h_row_cost);
+    if (!kHostSim) {
+        for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
+        if (d.ev_walk) cudaEventDestroy(d.ev_walk);
+        if (d.ev_done) cudaEventDestroy(d.ev_done);
+        for (auto& e : d.ev) {
+            if (e) cudaEventDestroy(e);
         }
-        host_pinned_free(d.h_counters);
-        host_pinned_free(d.h_row_cost);
-        if (!kHostSim) {
-            for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
-            if (d.ev_walk) cudaEventDestroy(d.ev_walk);
-            if (d.ev_done) cudaEventDestroy(d.ev_done);
-            for (auto& e : d.ev) {
-                if (e) cudaEventDestroy(e);
-            }
-            if (d.stream) cudaStreamDestroy(d.stream);
-        }
-        // DevBuf destructors free on the current device
-        dp.reset();
+        if (d.stream) cudaStreamDestroy(d.stream);
     }
-    delete ctx;
+    delete ctx; // DevBuf destructors free on the current device, d.device
 }
 
 const char* c5_last_error(const c5_ctx* ctx) {
@@ -891,20 +747,21 @@ int c5_upload_mesh(c5_ctx* ctx, const double* points_xyz, int64_t n_points, cons
         if (ctx->parent) fail(C5_E_STATE, "upload_mesh: a sibling context shares its parent's mesh; upload through the parent");
         if (!points_xyz || !tet_vertices || !alpha || !q) fail(C5_E_INVALID, "upload_mesh: NULL array");
         if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize()); // siblings may be rendering from it
-        ctx->dev[0]->mesh_version++;
-        ctx->has_mesh = false;
+        ctx->dev.mesh_version++;
+        const std::vector<c5_ctx*> all = with_parts(ctx);
+        for (c5_ctx* c : all) c->has_mesh = false;
         const size_t before = dev_bytes_in_use();
-        for (auto& dp : ctx->dev) {
-            use_device(*dp);
-            g_launch_counter = &dp->launches;
-            build_mesh(*dp, points_xyz, n_points, tet_vertices, n_tets, alpha, q);
+        for (c5_ctx* c : all) {
+            use_device(c->dev);
+            g_launch_counter = &c->dev.launches;
+            build_mesh(c->dev, points_xyz, n_points, tet_vertices, n_tets, alpha, q);
         }
         ctx->info.n_points = n_points;
         ctx->info.n_tets = n_tets;
-        ctx->info.n_boundary_faces = ctx->dev[0]->n_bfaces;
-        ctx->info.n_bvh_nodes = ctx->dev[0]->n_bfaces - 1;
-        ctx->info.device_bytes = static_cast<int64_t>((dev_bytes_in_use() - before) / ctx->dev.size());
-        ctx->has_mesh = true;
+        ctx->info.n_boundary_faces = ctx->dev.n_bfaces;
+        ctx->info.n_bvh_nodes = ctx->dev.n_bfaces - 1;
+        ctx->info.device_bytes = static_cast<int64_t>((dev_bytes_in_use() - before) / all.size());
+        for (c5_ctx* c : all) c->has_mesh = true;
     });
 }
 
@@ -913,7 +770,7 @@ int c5_upload_solids(c5_ctx* ctx, const double* tet_points, int64_t n_tets, int3
     return guarded(ctx, [&] {
         if (ctx->parent) fail(C5_E_STATE, "upload_solids: upload through the parent context");
         if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize());
-        ctx->dev[0]->mesh_version++;
+        ctx->dev.mesh_version++;
         upload_solids(ctx, tet_points, n_tets, follows_view);
     });
 }
@@ -923,10 +780,11 @@ int c5_clear_solids(c5_ctx* ctx) {
     return guarded(ctx, [&] {
         if (ctx->parent) fail(C5_E_STATE, "clear_solids: clear through the parent context");
         if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize());
-        ctx->dev[0]->mesh_version++;
-        for (auto& dp : ctx->dev) {
-            use_device(*dp);
-            for (SolidSet* ss : {&dp->solid_follow, &dp->solid_static}) {
+        ctx->dev.mesh_version++;
+        for (c5_ctx* c : with_parts(ctx)) {
+            DeviceState& d = c->dev;
+            use_device(d);
+            for (SolidSet* ss : {&d.solid_follow, &d.solid_static}) {
                 ss->pts0.release();
                 ss->pts_view.release();
                 ss->faces.release();
@@ -934,7 +792,7 @@ int c5_clear_solids(c5_ctx* ctx) {
                 ss->n_faces = 0;
                 ss->extent = 0.0;
             }
-            dp->mask_static_valid = false;
+            d.mask_static_valid = false;
         }
         ctx->info.n_solid_tets = 0;
     });
@@ -954,12 +812,13 @@ int c5_render_raw(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* steps
                   c5_stats* stats) {
     if (!ctx) return C5_E_INVALID;
     return guarded(ctx, [&] {
-        if (ctx->dev.size() > 1) {
+        if (!ctx->parts.empty()) {
             render_multi_device(ctx, view, out, steps, solid_mask, stats);
             return;
         }
         submit_view(ctx, view, out, steps, solid_mask, 0);
-        finish_view(ctx, ctx, stats);
+        ViewResult r = wait_view(ctx);
+        report(ctx, r, stats);
     });
 }
 
@@ -967,7 +826,7 @@ int c5_set_views_in_flight(c5_ctx* ctx, int32_t n) {
     if (!ctx) return C5_E_INVALID;
     return guarded(ctx, [&] {
         if (n < 1 || n > C5_MAX_IN_FLIGHT) fail(C5_E_INVALID, "set_views_in_flight: 1 .. C5_MAX_IN_FLIGHT");
-        if (ctx->parent || ctx->dev.size() != 1) fail(C5_E_INVALID, "set_views_in_flight: single-device contexts that are not siblings");
+        if (ctx->parent || !ctx->parts.empty()) fail(C5_E_INVALID, "set_views_in_flight: single-device contexts that are not siblings");
         for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
             if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "set_views_in_flight: views are in flight");
         }
@@ -983,7 +842,7 @@ int c5_set_views_in_flight(c5_ctx* ctx, int32_t n) {
 int c5_render_submit(c5_ctx* ctx, const c5_view* view, double* out, uint64_t* ticket) {
     if (!ctx || !ticket) return C5_E_INVALID;
     return guarded(ctx, [&] {
-        if (ctx->parent || ctx->dev.size() != 1) fail(C5_E_INVALID, "render_submit: single-device contexts that are not siblings");
+        if (ctx->parent || !ctx->parts.empty()) fail(C5_E_INVALID, "render_submit: single-device contexts that are not siblings");
         ensure_lanes(ctx);
         // the next lane in turn, or any free one
         const unsigned n = static_cast<unsigned>(ctx->lanes.size()) + 1;
@@ -998,7 +857,7 @@ int c5_render_submit(c5_ctx* ctx, const c5_view* view, double* out, uint64_t* ti
         if (!lane) fail(C5_E_STATE, "render_submit: " + std::to_string(n) + " views are in flight already (c5_render_wait one first)");
         const uint64_t t = ctx->next_ticket++;
         try {
-            g_launch_counter = &lane->dev[0]->launches;
+            g_launch_counter = &lane->dev.launches;
             submit_view(lane, view, out, nullptr, nullptr, t, /*in_place_allowed=*/ctx->views_in_flight == 1);
         } catch (const Error& e) {
             if (lane != ctx) ctx->err = e.text; // (guarded() reports through ctx)
@@ -1014,7 +873,8 @@ int c5_render_wait(c5_ctx* ctx, uint64_t ticket, c5_stats* stats) {
         for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
             c5_ctx* lane = lane_of(ctx, k);
             if (lane->pending.active && lane->pending.ticket == ticket && ticket != 0) {
-                finish_view(ctx, lane, stats);
+                ViewResult r = wait_view(lane);
+                report(ctx, r, stats);
                 return;
             }
         }
@@ -1029,10 +889,11 @@ int c5_render_device(c5_ctx* ctx, const c5_view* view, void* d_out, void* stream
         if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
         if (!d_out) fail(C5_E_INVALID, "render_device: d_out is NULL");
         if (reinterpret_cast<uintptr_t>(d_out) & 15u) fail(C5_E_INVALID, "render_device: d_out must be 16-byte aligned");
-        if (ctx->dev.size() != 1) fail(C5_E_INVALID, "render_device: single-device contexts only");
+        if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_device: single-device contexts only");
         if (ctx->pending.active) fail(C5_E_STATE, "render_device: this context has a submitted view in flight");
         const ViewPlan p = plan_view(view);
-        DeviceState& d = *ctx->dev[0];
+        DeviceState& d = ctx->dev;
+        if (stats) ensure_host_staging(d, static_cast<size_t>(view->res_y));
         // run on the CALLER's stream (NULL = the legacy default stream, which is what torch's
         // default "current stream" is) so the result is ordered with the caller's later work
         cudaStream_t own = d.stream;
@@ -1041,7 +902,13 @@ int c5_render_device(c5_ctx* ctx, const c5_view* view, void* d_out, void* stream
             enqueue_view(d, view, p, false, static_cast<double*>(d_out)); // the walk stores into the caller's buffer
             // stats == NULL: fire and forget — nothing is read back and the stream is not synchronised,
             // so successive views (and the caller's gather) pipeline on the device
-            if (stats) collect_stats(ctx, d, view, p, stats, 4);
+            if (stats) {
+                d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
+                d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(view->res_y) * sizeof(uint64_t), d.stream);
+                stream_sync(d.stream);
+                ViewResult r = read_view(d, *view, p, false);
+                report(ctx, r, stats);
+            }
         } catch (...) {
             d.stream = own;
             throw;
@@ -1062,7 +929,7 @@ int c5_image_create(c5_ctx* ctx, uint64_t bytes, void** d_ptr, uint8_t handle[C5
     if (!ctx || !d_ptr || !handle) return C5_E_INVALID;
     return guarded(ctx, [&] {
         if (bytes == 0) fail(C5_E_INVALID, "image_create: zero bytes");
-        use_device(*ctx->dev[0]);
+        use_device(ctx->dev);
         void* p = dev_alloc(bytes);
         std::memset(handle, 0, C5_IPC_HANDLE_BYTES);
         uint64_t offset = 0;
@@ -1090,7 +957,7 @@ int c5_image_create(c5_ctx* ctx, uint64_t bytes, void** d_ptr, uint8_t handle[C5
 int c5_image_open(c5_ctx* ctx, const uint8_t handle[C5_IPC_HANDLE_BYTES], void** d_ptr) {
     if (!ctx || !d_ptr || !handle) return C5_E_INVALID;
     return guarded(ctx, [&] {
-        use_device(*ctx->dev[0]);
+        use_device(ctx->dev);
         void* p = nullptr;
         if (kHostSim) {
             std::memcpy(&p, handle, sizeof(p));
@@ -1121,7 +988,7 @@ int c5_image_close(c5_ctx* ctx, void* d_ptr) {
             if (ctx->images[k].first != d_ptr) continue;
             const bool owner = ctx->images[k].second;
             ctx->images.erase(ctx->images.begin() + static_cast<long>(k));
-            use_device(*ctx->dev[0]);
+            use_device(ctx->dev);
             if (owner) dev_free(d_ptr);
             else if (!kHostSim) C5_CUDA(cudaIpcCloseMemHandle(d_ptr));
             return;
@@ -1133,7 +1000,7 @@ int c5_image_close(c5_ctx* ctx, void* d_ptr) {
 int c5_host_register(c5_ctx* ctx, void* ptr, uint64_t bytes) {
     if (!ctx || !ptr || bytes == 0) return C5_E_INVALID;
     return guarded(ctx, [&] {
-        use_device(*ctx->dev[0]);
+        use_device(ctx->dev);
         if (!kHostSim) C5_CUDA(cudaHostRegister(ptr, bytes, cudaHostRegisterPortable | cudaHostRegisterMapped));
         ctx->registered.push_back(ptr);
     });
@@ -1155,8 +1022,9 @@ int c5_host_unregister(c5_ctx* ctx, void* ptr) {
 uint64_t c5_kernel_launches(const c5_ctx* ctx) {
     uint64_t n = 0;
     if (ctx) {
-        for (const auto& d : ctx->dev) n += d->launches;
+        n = ctx->dev.launches;
         for (const c5_ctx* lane : ctx->lanes) n += c5_kernel_launches(lane);
+        for (const c5_ctx* part : ctx->parts) n += c5_kernel_launches(part);
     }
     return n;
 }
@@ -1165,36 +1033,34 @@ int c5_debug_set(c5_ctx* ctx, const char* key, int64_t value) {
     if (!ctx || !key) return C5_E_INVALID;
     return guarded(ctx, [&] {
         const std::string k = key;
-        std::vector<c5_ctx*> all{ctx};
+        std::vector<c5_ctx*> all = with_parts(ctx);
         all.insert(all.end(), ctx->siblings.begin(), ctx->siblings.end()); // the caller's siblings and our lanes
         for (c5_ctx* c : all) {
-            for (auto& dp : c->dev) {
-                DeviceState& d = *dp;
-                if (k == "graze_list") d.opt_graze_list = static_cast<int>(value);
-                else if (k == "query_budget") d.opt_query_budget = static_cast<int>(value);
-                else if (k == "serial_list") d.opt_serial_list = static_cast<int>(value);
-                else if (k == "mask_tile") d.opt_mask_tile = static_cast<int>(value);
-                else if (k == "no_static_mask") {
-                    d.opt_no_static_mask = value != 0;
-                    d.mask_static_valid = false;
+            DeviceState& d = c->dev;
+            if (k == "graze_list") d.opt_graze_list = static_cast<int>(value);
+            else if (k == "query_budget") d.opt_query_budget = static_cast<int>(value);
+            else if (k == "serial_list") d.opt_serial_list = static_cast<int>(value);
+            else if (k == "mask_tile") d.opt_mask_tile = static_cast<int>(value);
+            else if (k == "no_static_mask") {
+                d.opt_no_static_mask = value != 0;
+                d.mask_static_valid = false;
+            }
+            else if (k == "no_zero_copy") d.opt_no_zero_copy = value != 0;
+            else if (k == "timeline") {
+                if (value < 0 || value > 4096) fail(C5_E_INVALID, "debug_set: timeline 0 .. 4096 views");
+                if (kHostSim) continue;
+                use_device(d);
+                C5_CUDA(cudaStreamSynchronize(d.stream));
+                for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
+                d.tl_events.clear();
+                d.tl_views = 0;
+                for (int64_t i = 0; i < value * kTimelinePhases; i++) {
+                    cudaEvent_t e = nullptr;
+                    C5_CUDA(cudaEventCreate(&e));
+                    d.tl_events.push_back(e);
                 }
-                else if (k == "no_zero_copy") d.opt_no_zero_copy = value != 0;
-                else if (k == "timeline") {
-                    if (value < 0 || value > 4096) fail(C5_E_INVALID, "debug_set: timeline 0 .. 4096 views");
-                    if (kHostSim) continue;
-                    use_device(d);
-                    C5_CUDA(cudaStreamSynchronize(d.stream));
-                    for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
-                    d.tl_events.clear();
-                    d.tl_views = 0;
-                    for (int64_t i = 0; i < value * kTimelinePhases; i++) {
-                        cudaEvent_t e = nullptr;
-                        C5_CUDA(cudaEventCreate(&e));
-                        d.tl_events.push_back(e);
-                    }
-                } else {
-                    fail(C5_E_INVALID, "debug_set: unknown key '" + k + "'");
-                }
+            } else {
+                fail(C5_E_INVALID, "debug_set: unknown key '" + k + "'");
             }
         }
     });
@@ -1206,7 +1072,7 @@ int c5_timeline_read(c5_ctx* ctx, void* origin, float* ms_out, int32_t max_views
         *n_views = 0;
         if (kHostSim) return;
         if (!origin) fail(C5_E_INVALID, "timeline_read: origin event is NULL");
-        DeviceState& d = *ctx->dev[0];
+        DeviceState& d = ctx->dev;
         use_device(d);
         const uint64_t cap = d.tl_events.size() / kTimelinePhases;
         if (cap == 0) return;

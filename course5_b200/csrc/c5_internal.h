@@ -1,7 +1,6 @@
 // c5_internal.h — context and the entry points shared between the library's translation units.
 #pragma once
 
-#include <memory>
 #include <string>
 #include <utility>
 #include <vector>
@@ -114,12 +113,12 @@ struct PendingView {   // the view a context has in flight between c5_render_sub
 } // namespace c5
 
 struct c5_ctx {
-    std::vector<std::unique_ptr<c5::DeviceState>> dev;
+    c5::DeviceState dev;             // siblings point DeviceState::origin at it: a context is never moved
     std::string err;
     bool has_mesh = false;
     c5_mesh_info info{};
     std::vector<uint64_t> last_row_cost;
-    void* nccl = nullptr; // NcclGroup*, multi-device contexts only
+    std::vector<c5_ctx*> parts;      // multi-device context: one context per further device (owned)
     c5_ctx* parent = nullptr;        // sibling context (c5_create_sibling): shares parent's mesh and solids
     std::vector<c5_ctx*> siblings;   // contexts created from this one (the caller's, and our own lanes)
     std::vector<c5_ctx*> lanes;      // lanes of c5_render_submit beyond this context itself (owned; also in siblings)

@@ -39,7 +39,7 @@ enum c5_status {
     C5_E_TOPOLOGY = -4, /* mesh is not a conforming manifold partition (a face shared by >2 tets) */
     C5_E_STATE = -5,    /* call order (render before upload_mesh, ...) */
     C5_E_WALK = -6,     /* a ray exceeded the step cap (reported in c5_stats.walk_errors too) */
-    C5_E_NCCL = -7
+    C5_E_NCCL = -7      /* no longer returned; the value stays reserved */
 };
 
 /* One rigid rotation, the unit of object3d_base::rotate_around_{x,y}_axis
@@ -86,9 +86,9 @@ typedef struct c5_stats {
     float ms_bvh;
     float ms_mask;
     float ms_walk;
-    float ms_gather;        /* NCCL band gather (multi-device contexts) */
+    float ms_gather;        /* always 0 (nothing is gathered); kept for the struct's layout */
     float ms_d2h;
-    float ms_total;         /* whole call on the device timeline */
+    float ms_total;         /* whole call on the device timeline, max over devices */
     int32_t n_devices;
     int32_t grazing_rays;   /* rays with so many crossings that the grazing-ray kernel finished them */
     float ms_graze;         /* the grazing-ray kernel's share of ms_walk */
@@ -101,7 +101,8 @@ typedef struct c5_mesh_info {
 } c5_mesh_info;
 
 /* devices: CUDA ordinals, n_dev >= 1. With n_dev > 1 the mesh is replicated, each device
- * renders a contiguous band of rows and one NCCL gather assembles the image on devices[0]. */
+ * renders a contiguous band of rows (cut by the previous view's cost) and stores it in its rows
+ * of the caller's buffers: in place if `out` is page-locked, else by its own device-to-host copy. */
 int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out);
 void c5_destroy(c5_ctx* ctx);
 const char* c5_last_error(const c5_ctx* ctx); /* ctx may be NULL: text of the last failed c5_create */

@@ -167,7 +167,8 @@ def check_scaling_properties(lib, mesh, res_x, res_y, flags):
 
 
 def check_multi_device_context(lib, devices):
-    """One context over several devices: cost-balanced row bands + gather == single-device image."""
+    """One context over several devices: each device renders a cost-balanced row band into its rows
+    of the caller's buffers, which must give the single-device image."""
     mesh = synth.kuhn_cube(8, seed=36)
     solids = reference_solids(0.0)
     views = [api.make_view(160, 120, X=0.4, Y=y, lib=lib, round_through_float=0) for y in (0.1, 0.8, 0.8)]
@@ -176,6 +177,9 @@ def check_multi_device_context(lib, devices):
         one.upload_solids(solids[0], True)
         one.upload_solids(solids[1], False)
         want = [one.render_raw(v) for v in views]
+        one.debug_set("query_budget", 1)     # nearly every ray goes to the grazing-ray kernel
+        want_budget = one.render_raw(views[0])
+    assert want_budget.stats["grazing_rays"] > want[0].stats["grazing_rays"]
     with api.Context(devices=devices, lib=lib) as many:
         many.upload_mesh(mesh.points, mesh.tets, mesh.alpha, mesh.q)
         many.upload_solids(solids[0], True)
@@ -187,6 +191,17 @@ def check_multi_device_context(lib, devices):
             assert got.stats["tet_steps"] == w.stats["tet_steps"]
             assert got.stats["n_devices"] == len(devices)
             assert int(many.last_row_cost(120).sum()) == w.stats["tet_steps"]
+        pinned = np.full((120, 160, 2), -7.0)
+        many.host_register(pinned)           # page-locked: on GPUs every device stores its band in place
+        try:
+            many.render(views[1], out=pinned)
+        finally:
+            many.host_unregister(pinned)
+        assert np.array_equal(pinned, want[1].image, equal_nan=True)
+        many.debug_set("query_budget", 1)    # must reach every device
+        got = many.render_raw(views[0])
+        assert np.array_equal(got.image, want_budget.image, equal_nan=True)
+        assert got.stats["grazing_rays"] == want_budget.stats["grazing_rays"]
 
 
 def check_fp32_variant(lib, port, mesh, res_x, res_y, flags):
