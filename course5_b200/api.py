@@ -23,6 +23,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # C5GPU_LIBRARY: another build of the same library (A/B runs of two builds in one process-per-build experiment)
 DEFAULT_SO = os.environ.get("C5GPU_LIBRARY") or os.path.join(HERE, "libc5gpu.so")
 C5_MAX_ROT = 8
+MAX_CHANNELS = 8       # C5_MAX_CHANNELS
 PI = 3.14159265358979323846  # config.hpp:45
 
 OK, E_INVALID, E_CUDA, E_NOMEM, E_TOPOLOGY, E_STATE, E_WALK, E_NCCL = 0, -1, -2, -3, -4, -5, -6, -7
@@ -84,6 +85,8 @@ SYMBOLS = {
     "c5_mesh_info_get": (C.c_int, [C.c_void_p, C.POINTER(MeshInfo)]),
     "c5_render": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, C.POINTER(Stats)]),
     "c5_render_raw": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _u32p, _u8p, C.POINTER(Stats)]),
+    "c5_upload_channels": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int32]),
+    "c5_render_channels": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _u32p, _u8p, C.POINTER(Stats)]),
     "c5_render_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_last_row_cost": (C.c_int, [C.c_void_p, _u64p, C.c_int32]),
     "c5_kernel_launches": (C.c_uint64, [C.c_void_p]),
@@ -100,7 +103,7 @@ SYMBOLS = {
 }
 IPC_HANDLE_BYTES = 80
 MAX_IN_FLIGHT = 8
-ABI_VERSION = 2        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
+ABI_VERSION = 3        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
 TIMELINE_PHASES = 6
 
 
@@ -227,6 +230,7 @@ class Context:
             raise ValueError("points must be (n,3) and tets (m,4)")
         if alpha.shape != (tets.shape[0],) or q.shape != (tets.shape[0],):
             raise ValueError("alpha and q must have one value per tet")
+        self._n_channels = 0  # a new mesh drops the channels, also when its upload fails
         self._check(self.lib.c5_upload_mesh(self._h, _ptr(points, _dp), points.shape[0], _ptr(tets, _i32p),
                                             tets.shape[0], _ptr(alpha, _dp), _ptr(q, _dp)))
         return self.mesh_info()
@@ -253,6 +257,45 @@ class Context:
             out = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64)
         st = Stats()
         self._check(self.lib.c5_render(self._h, C.byref(view), _ptr(out, _dp), C.byref(st)))
+        return out, st.as_dict()
+
+    def upload_channels(self, alpha, q):
+        """Several pairs of cell fields for render_channels: alpha and q of shape (n, n_tets), tets in
+        the order given to upload_mesh (c5_upload_channels). n = 0 removes them."""
+        alpha = np.ascontiguousarray(alpha, dtype=np.float64)
+        q = np.ascontiguousarray(q, dtype=np.float64)
+        if alpha.ndim != 2 or alpha.shape != q.shape:
+            raise ValueError("alpha and q must both have shape (n_channels, n_tets)")
+        n_tets = self.mesh_info().n_tets  # 0 before upload_mesh: the library reports that
+        if n_tets and alpha.shape[0] and alpha.shape[1] != n_tets:
+            raise ValueError("alpha and q need one value per tet of the uploaded mesh")
+        self._n_channels = 0  # a failed upload leaves no channels
+        self._check(self.lib.c5_upload_channels(self._h, alpha.ctypes.data_as(_dp), q.ctypes.data_as(_dp),
+                                                alpha.shape[0]))
+        self._n_channels = alpha.shape[0]
+
+    @property
+    def n_channels(self) -> int:
+        """Channels uploaded through this context (a sibling's are its parent's)."""
+        owner = getattr(self, "_parent", None) or self
+        return getattr(owner, "_n_channels", 0)
+
+    def render_channels(self, view: View, out: np.ndarray | None = None, *, raw: bool = False):
+        """All uploaded channels of one view in one walk (c5_render_channels): returns (image, stats)
+        with image of shape (res_y, res_x, n, 2), [..., c, 0] = tau and [..., c, 1] = I of channel c;
+        with raw=True (image, steps, solid mask, stats)."""
+        shape = (view.res_y, view.res_x, self.n_channels, 2)
+        if out is None:
+            out = np.zeros(shape, dtype=np.float64)
+        if out.dtype != np.float64 or not out.flags["C_CONTIGUOUS"] or out.shape != shape:
+            raise ValueError(f"out must be a C-contiguous float64 array of shape {shape}")
+        steps = np.zeros((view.res_y, view.res_x), dtype=np.uint32) if raw else None
+        solid = np.zeros((view.res_y, view.res_x), dtype=np.uint8) if raw else None
+        st = Stats()
+        self._check(self.lib.c5_render_channels(self._h, C.byref(view), _ptr(out, _dp), _ptr(steps, _u32p),
+                                                _ptr(solid, _u8p), C.byref(st)))
+        if raw:
+            return out, steps, solid, st.as_dict()
         return out, st.as_dict()
 
     def render_submit(self, view: View, out: np.ndarray) -> int:

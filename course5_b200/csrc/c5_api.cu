@@ -176,7 +176,9 @@ void mesh_pixel_rect(const DeviceState& d, const c5_view* v, const ViewPlan& p, 
 
 // Enqueues one view's kernels for rows [row_begin,row_end) on device d. Events:
 // 0 start, 1 rotated, 2 bvh, 3 mask, 4 walk.
-void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want_steps, double* out_override = nullptr) {
+// channels > 0: the walk integrates that many uploaded channels (c5_render_channels).
+void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want_steps, double* out_override = nullptr,
+                  int channels = 0) {
     use_device(d);
     g_launch_counter = &d.launches;
     ensure_pixel_tables(d, v, p);
@@ -185,16 +187,19 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     // synchronisation) and a cudaMalloc on the spot.
     const size_t n_pix = static_cast<size_t>(v->res_y) * v->res_x;
     const bool solids = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0;
-    if (!out_override) d.out.ensure(2 * n_pix);
+    const size_t words = 2 * static_cast<size_t>(channels ? channels : 1); // doubles per pixel
+    if (!out_override) d.out.ensure(words * n_pix);
     if (want_steps) d.steps.ensure(n_pix);
     d.counters.ensure(kNumCounters);
     d.queue.ensure(n_pix); // every ray may be deferred (reserved, hardly ever touched)
+    if (channels) d.ch_queue.ensure(words * n_pix);
     d.row_cost.ensure(static_cast<size_t>(v->res_y));
     if (solids) d.mask.ensure(n_pix);
 
     record(d, 0);
     timeline_mark(d, 0);
     launch_prepare_cells(d, v->alpha_limit); // no-op unless --alpha_limit changed since the last view
+    if (channels) launch_prepare_channels(d, v->alpha_limit); // the same for the channels
     launch_rotate_vertices(d, p.rot, p.n_rot);
     if (solids) launch_rotate_solids(d, p.rot, p.n_rot);
     record(d, 1);
@@ -219,6 +224,7 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     w.use_mask = solids ? 1 : 0;
     w.write_steps = want_steps ? 1 : 0;
     w.precision = v->precision ? v->precision : 64;
+    w.channels = channels;
     w.out = out_override ? out_override : d.out.p;
     w.mark_walk_done = d.ev_walk;
     w.mark_walk_done_tl = nullptr;
@@ -291,13 +297,16 @@ void ensure_host_staging(DeviceState& d, size_t rows) {
 void follow_parent(c5_ctx* ctx);
 
 void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, uint64_t ticket,
-                 bool in_place_allowed = true) {
+                 bool in_place_allowed = true, bool channels = false) {
     follow_parent(ctx);
     if (ctx->pending.active) fail(C5_E_STATE, "render: this context still has a view in flight (c5_render_wait it first)");
     if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
     if (!out) fail(C5_E_INVALID, "render: out is NULL");
     const ViewPlan p = plan_view(v);
     DeviceState& d = ctx->dev;
+    if (channels && d.n_channels == 0) fail(C5_E_STATE, "render_channels: no channels uploaded");
+    const int n_ch = channels ? d.n_channels : 0;
+    const size_t words = 2 * static_cast<size_t>(channels ? n_ch : 1); // doubles per pixel of `out`
     use_device(d);
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
     const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
@@ -314,15 +323,15 @@ void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, ui
     if (!kHostSim && in_place_allowed && !d.opt_no_zero_copy && (reinterpret_cast<uintptr_t>(out) & 15u) == 0) {
         cudaPointerAttributes attr{};
         if (cudaPointerGetAttributes(&attr, out) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer) {
-            host_direct = static_cast<double*>(attr.devicePointer) + 2 * band_off;
+            host_direct = static_cast<double*>(attr.devicePointer) + words * band_off;
         } else {
             cudaGetLastError(); // pageable memory reports an error on some drivers: not ours
         }
     }
     ensure_host_staging(d, static_cast<size_t>(v->res_y));
-    enqueue_view(d, v, p, steps != nullptr, host_direct);
+    enqueue_view(d, v, p, steps != nullptr, host_direct, n_ch);
     record(d, 5);
-    if (!host_direct) d2h(out + 2 * band_off, d.out.p, 2 * n_pix_band * sizeof(double), d.stream);
+    if (!host_direct) d2h(out + words * band_off, d.out.p, words * n_pix_band * sizeof(double), d.stream);
     record(d, 6);
     const bool solids = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0;
     if (steps) d2h(steps + band_off, d.steps.p, n_pix_band * sizeof(uint32_t), d.stream);
@@ -395,7 +404,8 @@ ViewResult wait_view(c5_ctx* lane) {
 // one cost-balanced row band, as c5_render does for a row band, straight into its final rows of the
 // caller's buffers. One host thread per device submits: a copy into pageable memory blocks the
 // submitting thread until its device is done, so one thread would render the bands one after another.
-void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, c5_stats* st) {
+void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, c5_stats* st,
+                         bool channels = false) {
     if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
     const ViewPlan p = plan_view(v);
     const std::vector<c5_ctx*> parts = with_parts(ctx);
@@ -408,7 +418,7 @@ void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* s
         try {
             band_views[r].row_begin = bands[r].first;
             band_views[r].row_end = bands[r].second;
-            submit_view(parts[r], &band_views[r], out, steps, solid_mask, 0);
+            submit_view(parts[r], &band_views[r], out, steps, solid_mask, 0, true, channels);
         } catch (...) {
             errors[r] = std::current_exception();
         }
@@ -529,6 +539,9 @@ void alias_mesh(DeviceState& s, DeviceState& o) {
     s.pz.alias(o.pz);
     s.cells.alias(o.cells);
     s.q0.alias(o.q0);
+    s.n_channels = o.n_channels;
+    s.ch_rec.alias(o.ch_rec);
+    s.ch_q0.alias(o.ch_q0);
     s.bfaces.alias(o.bfaces);
     s.node_parent.alias(o.node_parent);
     s.leaf_parent.alias(o.leaf_parent);
@@ -749,7 +762,13 @@ int c5_upload_mesh(c5_ctx* ctx, const double* points_xyz, int64_t n_points, cons
         if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize()); // siblings may be rendering from it
         ctx->dev.mesh_version++;
         const std::vector<c5_ctx*> all = with_parts(ctx);
-        for (c5_ctx* c : all) c->has_mesh = false;
+        for (c5_ctx* c : all) {
+            c->has_mesh = false;
+            use_device(c->dev);
+            upload_channels(c->dev, nullptr, nullptr, 0); // a new mesh drops the channels
+        }
+        ctx->info.device_bytes -= ctx->channel_bytes;
+        ctx->channel_bytes = 0;
         const size_t before = dev_bytes_in_use();
         for (c5_ctx* c : all) {
             use_device(c->dev);
@@ -817,6 +836,61 @@ int c5_render_raw(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* steps
             return;
         }
         submit_view(ctx, view, out, steps, solid_mask, 0);
+        ViewResult r = wait_view(ctx);
+        report(ctx, r, stats);
+    });
+}
+
+int c5_upload_channels(c5_ctx* ctx, const double* alpha, const double* q, int32_t n_channels) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (ctx->parent) fail(C5_E_STATE, "upload_channels: a sibling context shares its parent's channels; upload through the parent");
+        if (!alpha || !q) fail(C5_E_INVALID, "upload_channels: NULL array");
+        if (n_channels < 0 || n_channels > C5_MAX_CHANNELS) fail(C5_E_INVALID, "upload_channels: n_channels must be 0 .. C5_MAX_CHANNELS");
+        if (!ctx->has_mesh) fail(C5_E_STATE, "upload_channels: no mesh uploaded");
+        for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
+            if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "upload_channels: a submitted view is in flight");
+        }
+        if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize()); // siblings may be rendering from them
+        ctx->dev.mesh_version++; // siblings and lanes re-alias at their next render
+        const std::vector<c5_ctx*> all = with_parts(ctx);
+        // the old channels go first: a failed upload leaves none anywhere, and the sizes say so
+        ctx->info.device_bytes -= ctx->channel_bytes;
+        ctx->channel_bytes = 0;
+        try {
+            for (c5_ctx* c : all) {
+                use_device(c->dev);
+                g_launch_counter = &c->dev.launches;
+                upload_channels(c->dev, alpha, q, n_channels);
+            }
+        } catch (...) {
+            for (c5_ctx* c : all) {
+                use_device(c->dev);
+                upload_channels(c->dev, nullptr, nullptr, 0);
+            }
+            throw;
+        }
+        ctx->channel_bytes = static_cast<int64_t>(ctx->dev.ch_rec.bytes() + ctx->dev.ch_q0.bytes());
+        ctx->info.device_bytes += ctx->channel_bytes;
+    });
+}
+
+int c5_render_channels(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* steps, uint8_t* solid_mask,
+                       c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (view && view->precision == 32) fail(C5_E_INVALID, "render_channels: FP64 only (precision 64)");
+        follow_parent(ctx);
+        if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+        if (ctx->dev.n_channels == 0) fail(C5_E_STATE, "render_channels: no channels uploaded");
+        for (const c5_ctx* part : ctx->parts) { // every band must be as wide as the caller's image
+            if (part->dev.n_channels != ctx->dev.n_channels) fail(C5_E_STATE, "render_channels: the devices hold different channels");
+        }
+        if (!ctx->parts.empty()) {
+            render_multi_device(ctx, view, out, steps, solid_mask, stats, true);
+            return;
+        }
+        submit_view(ctx, view, out, steps, solid_mask, 0, true, true);
         ViewResult r = wait_view(ctx);
         report(ctx, r, stats);
     });

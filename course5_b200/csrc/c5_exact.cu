@@ -672,6 +672,17 @@ C5_HD void prepare_cell_body(int64_t t, Cell* cells, const double* q0, double li
     cells[t].s = (a < DBL_EPSILON) ? 0.0 : q0[t] / a;
 }
 
+// The same arithmetic for channel c of tet t (k = t * n + c): s_c from ch_q0[c][t] and the alpha_c
+// beside it in the record.
+C5_HD void prepare_channel_body(int64_t k, double* rec, const double* q0, int64_t n_tets, int n, double limit) {
+    const int64_t t = k / n;
+    const int c = static_cast<int>(k - t * n);
+    double* r = rec + t * channel_stride(n) + 2 * c;
+    double a = r[0];
+    if (a > limit) a = limit;
+    r[1] = (a < DBL_EPSILON) ? 0.0 : q0[c * n_tets + t] / a;
+}
+
 } // namespace
 
 // Source function s = Q / min(alpha, limit) per cell; rerun only when --alpha_limit changes.
@@ -679,6 +690,13 @@ __global__ void __launch_bounds__(256)
 prepare_cells(int64_t n, Cell* __restrict__ cells, const double* __restrict__ q0, double limit) {
     const int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
     if (t < n) prepare_cell_body(t, cells, q0, limit);
+}
+
+// The same for the uploaded channels (n_tets * n_channels records).
+__global__ void __launch_bounds__(256)
+prepare_channels(int64_t n_tets, int n_channels, double* __restrict__ rec, const double* __restrict__ q0, double limit) {
+    const int64_t k = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+    if (k < n_tets * n_channels) prepare_channel_body(k, rec, q0, n_tets, n_channels, limit);
 }
 
 namespace {
@@ -908,6 +926,30 @@ void launch_prepare_cells(DeviceState& dd, double alpha_limit) {
     }
     d.cells_limit = alpha_limit;
     d.cells_limit_valid = true;
+}
+
+void launch_prepare_channels(DeviceState& dd, double alpha_limit) {
+    // fenced like launch_prepare_cells: siblings read the owner's records
+    DeviceState& d = dd.origin ? *dd.origin : dd;
+    if (d.n_channels == 0 || (d.ch_limit_valid && d.ch_limit == alpha_limit)) return;
+    const bool shared = dd.origin != nullptr || d.mesh_shared;
+    if (shared && !kHostSim) C5_CUDA(cudaDeviceSynchronize());
+    struct SyncAfter {
+        bool on;
+        ~SyncAfter() {
+            if (on) cudaDeviceSynchronize();
+        }
+    } sync_after{shared && !kHostSim};
+    const int64_t n = d.n_tets * d.n_channels;
+    count_launch();
+    if (kHostSim) {
+        for (int64_t k = 0; k < n; k++) prepare_channel_body(k, d.ch_rec.p, d.ch_q0.p, d.n_tets, d.n_channels, alpha_limit);
+    } else {
+        prepare_channels<<<grid_for(n, 256), 256, 0, dd.stream>>>(d.n_tets, d.n_channels, d.ch_rec.p, d.ch_q0.p, alpha_limit);
+        C5_CUDA(cudaGetLastError());
+    }
+    d.ch_limit = alpha_limit;
+    d.ch_limit_valid = true;
 }
 
 void dedupe_solid_faces(DeviceState& d, SolidSet& ss) {

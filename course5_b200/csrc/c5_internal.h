@@ -54,6 +54,14 @@ struct DeviceState {
     DevBuf<int32_t> node_parent;     // per internal node: (parent << 1) | which child, -1 for the root
     DevBuf<int32_t> leaf_parent;     // per leaf: (parent << 1) | which child
     DevBuf<uint32_t> refit_flags;    // per internal node arrival counter
+    std::vector<uint32_t> tperm;     // new -> old tet (host): places the file-order fields of c5_upload_channels
+
+    // channels (c5_upload_channels; aliased by siblings like the mesh)
+    int n_channels = 0;
+    DevBuf<double> ch_rec;           // [n_tets][channel_stride(n)]: {alpha_c, s_c} per channel, Morton order
+    DevBuf<double> ch_q0;            // [n][n_tets]: Q per channel and tet (Morton order); s_c is derived from it
+    double ch_limit = 0.0;           // the alpha_limit ch_rec's s_c were last prepared for
+    bool ch_limit_valid = false;
 
     // solids
     SolidSet solid_follow, solid_static;
@@ -75,6 +83,7 @@ struct DeviceState {
     DevBuf<unsigned long long> counters;
     DevBuf<unsigned long long> row_cost;
     DevBuf<DeferredRay> queue;       // grazing rays of the current view (capacity: pixels of the band)
+    DevBuf<double> ch_queue;         // their channel values {tau, I} (channel renders only)
     int sm_count = 0;
     cudaEvent_t ev_walk = nullptr;   // between the pixel kernel and the grazing-ray kernel (phase times)
     cudaEvent_t ev_done = nullptr;   // after the view's last copy: what c5_render_wait waits for
@@ -117,6 +126,7 @@ struct c5_ctx {
     std::string err;
     bool has_mesh = false;
     c5_mesh_info info{};
+    int64_t channel_bytes = 0;       // device bytes of the uploaded channels (included in info.device_bytes)
     std::vector<uint64_t> last_row_cost;
     std::vector<c5_ctx*> parts;      // multi-device context: one context per further device (owned)
     c5_ctx* parent = nullptr;        // sibling context (c5_create_sibling): shares parent's mesh and solids
@@ -146,6 +156,10 @@ void launch_solid_mask(DeviceState& d, int res_x, int res_y, double x_min, doubl
 void launch_bvh_refit(DeviceState& d);
 void dedupe_solid_faces(DeviceState& d, SolidSet& ss); // fills ss.faces / ss.n_faces from ss.pts0
 void launch_prepare_cells(DeviceState& d, double alpha_limit); // cells[t].s = q0[t] / min(alpha, limit)
+void launch_prepare_channels(DeviceState& d, double alpha_limit); // the same for every channel of ch_rec
+
+// c5_topology.cu — places n channels of file-order fields (channel-major) in ch_rec / ch_q0.
+void upload_channels(DeviceState& d, const double* alpha, const double* q, int n);
 
 // c5_walk.cu
 struct WalkLaunch {
@@ -156,10 +170,13 @@ struct WalkLaunch {
     int use_mask;
     int write_steps;
     int precision;
-    double* out; // {tau, I} per pixel of the band, x fastest
+    int channels; // 0: the cells' own fields; n: the n uploaded channels, n {tau, I} per pixel
+    double* out; // {tau, I} per pixel (per channel) of the band, x fastest
     cudaEvent_t mark_walk_done;    // recorded between the pixel kernel and the grazing-ray kernel (may be null)
     cudaEvent_t mark_walk_done_tl; // the same moment for the timeline ring (may be null)
 };
 void launch_walk(DeviceState& d, const WalkLaunch& w);
+// doubles per tet of ch_rec: n {alpha, s} pairs padded to 32 bytes (read with 256-bit loads)
+C5_HD constexpr int channel_stride(int n_channels) { return 4 * ((n_channels + 1) / 2); }
 
 } // namespace c5

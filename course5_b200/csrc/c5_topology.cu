@@ -292,6 +292,28 @@ int bits_for(uint64_t n) {
     return b;
 }
 
+// Channel records from channel-major file-order fields: record t holds {alpha_c, 0} (s_c is set by
+// prepare_channels) of old tet tperm[t] for every channel c, and zeros in the padding.
+struct ChannelGatherOp {
+    const double* alpha;   // [n][n_tets], file order
+    const double* q;
+    const uint32_t* tperm; // new -> old tet
+    int64_t n_tets;
+    int n;
+    double* rec;           // [n_tets][channel_stride(n)]
+    double* q0;            // [n][n_tets], Morton order
+    C5_HD void operator()(int64_t t) const {
+        const int64_t old = tperm[t];
+        double* r = rec + t * channel_stride(n);
+        for (int k = 2 * n; k < channel_stride(n); k++) r[k] = 0.0;
+        for (int c = 0; c < n; c++) {
+            r[2 * c] = alpha[c * n_tets + old];
+            r[2 * c + 1] = 0.0;
+            q0[c * n_tets + t] = q[c * n_tets + old];
+        }
+    }
+};
+
 } // namespace
 
 void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t* tets, int64_t n_tets,
@@ -360,6 +382,8 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
         sort_pairs_u64(keys.p, tperm.p, static_cast<size_t>(n_tets), 63, s);
         d.q0.alloc(static_cast<size_t>(n_tets));
         for_each(s, n_tets, CellFillOp{tets_in.p, alpha_in.p, q_in.p, tperm.p, vinv.p, d.cells.p, d.q0.p});
+        d.tperm.resize(static_cast<size_t>(n_tets));
+        d2h(d.tperm.data(), tperm.p, tperm.bytes(), s);
         stream_sync(s);
     }
     xyz.release();
@@ -482,6 +506,29 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
     d.n_tets = n_tets;
     d.n_bfaces = static_cast<int64_t>(n_b);
     d.cells_limit_valid = false;
+}
+
+void upload_channels(DeviceState& d, const double* alpha, const double* q, int n) {
+    d.ch_rec.release();
+    d.ch_q0.release();
+    d.n_channels = 0;
+    d.ch_limit_valid = false;
+    if (n == 0) return;
+    cudaStream_t s = d.stream;
+    const size_t n_t = static_cast<size_t>(d.n_tets), n_all = n_t * static_cast<size_t>(n);
+    DevBuf<double> alpha_in, q_in;
+    DevBuf<uint32_t> tperm;
+    alpha_in.alloc(n_all);
+    q_in.alloc(n_all);
+    tperm.alloc(n_t);
+    h2d(alpha_in.p, alpha, alpha_in.bytes(), s);
+    h2d(q_in.p, q, q_in.bytes(), s);
+    h2d(tperm.p, d.tperm.data(), tperm.bytes(), s);
+    d.ch_rec.alloc(n_t * static_cast<size_t>(channel_stride(n)));
+    d.ch_q0.alloc(n_all);
+    for_each(s, d.n_tets, ChannelGatherOp{alpha_in.p, q_in.p, tperm.p, d.n_tets, n, d.ch_rec.p, d.ch_q0.p});
+    stream_sync(s);
+    d.n_channels = n;
 }
 
 } // namespace c5

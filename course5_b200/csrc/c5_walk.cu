@@ -268,9 +268,13 @@ C5_HD bool bvh_collect_entries(const WalkParams& P, double px, double py, double
 // grazing-ray kernel walks the crossings of one ray in parallel); inten then starts at 0 and gain at
 // 1, and the crossing maps an arriving I to inten + gain * I (the recurrence of line.cpp:206-225 is
 // affine in I: s - (s - I) e = s (1 - e) + e I).
-template <bool kAffine>
-C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau,
-                          double& inten, double& gain, uint32_t& steps, uint32_t& error) {
+//
+// `acc` integrates the fields along the crossing: fetch(t) is issued with tet t's cell load and
+// step(c, dz) adds one segment. CellFields below integrates the cells' own alpha and s; the
+// channel walk (further down) integrates several field pairs over the same steps.
+template <bool kAffine, class Acc>
+C5_HD double crossing_walk(const WalkParams& P, double px, double py, int leaf, double z_in, Acc& acc,
+                           uint32_t& steps, uint32_t& error) {
 #ifdef __CUDA_ARCH__
     const int4 f = __ldg(reinterpret_cast<const int4*>(P.bfaces + leaf));
     int id = __ldg(&P.bfaces[leaf].apex);
@@ -299,6 +303,7 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
         // read (Cell::apex of the previous tet, BFace::apex at entry), so the cell load and the
         // vertex load of a step are independent and overlap: one memory latency per step, not two.
         const CellData c = load_cell(P.cells, t);
+        acc.fetch(t);
         double dx, dy, dz;
         load_vtx(P.vrot, id, dx, dy, dz);
         dx -= px;
@@ -337,16 +342,7 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
         const double wsum = wa + wb + wc;
         const double z_exit = (wsum != 0.0) ? (wa * az + wb * bz + wc * cz) / wsum : z_cur;
         const double dzv = fabs(z_exit - z_cur);
-        // tau: line.cpp:176-193 (alpha not clamped)
-        tau += dzv * c.alpha;
-        // I: line.cpp:206-225 with s = Q / a^:  (Q - (Q - a^ I) e) / a^  ==  s - (s - I) e
-        double a_c = c.alpha;
-        if (a_c > P.alpha_limit) a_c = P.alpha_limit;
-        if (!(a_c < DBL_EPSILON)) {
-            const double e = exp(-a_c * dzv);
-            inten = c.s - (c.s - inten) * e;
-            if (kAffine) gain *= e;
-        }
+        acc.step(P, c, dzv);
         steps++;
         z_cur = z_exit;
         t = t_next;
@@ -354,6 +350,39 @@ C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, d
         if (t < 0) break;
     }
     return z_cur;
+}
+
+// One segment of length dz through a medium (alpha, s):
+// tau: line.cpp:176-193 (alpha not clamped);
+// I: line.cpp:206-225 with s = Q / a^:  (Q - (Q - a^ I) e) / a^  ==  s - (s - I) e
+template <bool kAffine>
+C5_HD void segment(double alpha, double s, double limit, double dzv, double& tau, double& inten, double& gain) {
+    tau += dzv * alpha;
+    double a_c = alpha;
+    if (a_c > limit) a_c = limit;
+    if (!(a_c < DBL_EPSILON)) {
+        const double e = exp(-a_c * dzv);
+        inten = s - (s - inten) * e;
+        if (kAffine) gain *= e;
+    }
+}
+
+template <bool kAffine>
+struct CellFields {
+    double& tau;
+    double& inten;
+    double& gain;
+    C5_HD void fetch(int) {}
+    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
+        segment<kAffine>(c.alpha, c.s, P.alpha_limit, dzv, tau, inten, gain);
+    }
+};
+
+template <bool kAffine>
+C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau,
+                          double& inten, double& gain, uint32_t& steps, uint32_t& error) {
+    CellFields<kAffine> acc{tau, inten, gain};
+    return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
 }
 
 // ---- FP32 variant -----------------------------------------------------------------------------------
@@ -953,11 +982,13 @@ void graze_on_host(const WalkParams& P, bool f32) {
     P.counters[kTicket] = n_rays;
 }
 
-void background_on_host(const WalkParams& P) {
+C5_HD bool background_pixel_ch(const WalkParams& P, int n, int i, int j);
+
+void background_on_host(const WalkParams& P, int n_channels) {
     for (int j = P.row_begin; j < P.row_end; j++) {
         for (int i = 0; i < P.res_x; i++) {
             if (i >= P.i0 && i < P.i1 && j >= P.j0 && j < P.j1) continue;
-            if (background_pixel(P, i, j)) P.counters[kSolidPixels]++;
+            if (n_channels ? background_pixel_ch(P, n_channels, i, j) : background_pixel(P, i, j)) P.counters[kSolidPixels]++;
         }
     }
 }
@@ -979,6 +1010,432 @@ void walk_on_host(const WalkParams& P, bool f32) {
             if (r.error) P.counters[kWalkErrors]++;
         }
     }
+}
+
+} // namespace
+
+// ---- several field pairs in one walk (c5_render_channels) ----------------------------------------
+// The rays, their entry searches, deferrals and steps are those of the FP64 walk above: only what is
+// integrated differs. A step reads tet t's record of K {alpha_c, s_c} pairs (padded to 32-byte
+// sectors) together with t's cell, since t is known at the top of the step, so a channel adds FP64
+// work and a store but no further round trip. Channel c of a pixel is stored at
+// out[((j - row_begin) * res_x + i) * K + c] as {tau, I}.
+
+namespace {
+
+struct ChanParams {
+    WalkParams W;
+    const double* rec;   // [n_tets][channel_stride(K)]: {alpha_c, s_c} per channel
+    double* queue;       // [deferred ray][K] {tau, I}: the channel values DeferredRay::tau/inten hold otherwise
+};
+
+C5_HD void store2(double* p, double a, double b) {
+#ifdef __CUDA_ARCH__
+    *reinterpret_cast<double2*>(p) = make_double2(a, b);
+#else
+    p[0] = a;
+    p[1] = b;
+#endif
+}
+
+// K channels integrated along one crossing (the accumulator of crossing_walk).
+template <int K, bool kAffine>
+struct ChanFields {
+    const double* rec;
+    double tau[K], inten[K], gain[K];
+    double f[channel_stride(K)]; // the record of the tet being crossed
+
+    C5_HD void reset() {
+#pragma unroll
+        for (int c = 0; c < K; c++) {
+            tau[c] = 0.0;
+            inten[c] = 0.0;
+            gain[c] = 1.0;
+        }
+    }
+    C5_HD void fetch(int t) {
+        const double* p = rec + static_cast<size_t>(t) * channel_stride(K);
+#ifdef __CUDA_ARCH__
+#pragma unroll
+        for (int k = 0; k < channel_stride(K); k += 4) {
+            asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];"
+                         : "=d"(f[k]), "=d"(f[k + 1]), "=d"(f[k + 2]), "=d"(f[k + 3])
+                         : "l"(p + k));
+        }
+#else
+        for (int k = 0; k < channel_stride(K); k++) f[k] = p[k];
+#endif
+    }
+    C5_HD void step(const WalkParams& P, const CellData&, double dzv) {
+#pragma unroll
+        for (int c = 0; c < K; c++) segment<kAffine>(f[2 * c], f[2 * c + 1], P.alpha_limit, dzv, tau[c], inten[c], gain[c]);
+    }
+};
+
+template <int K>
+struct ChanRay {
+    ChanFields<K, false> f;
+    uint32_t steps, error, deferred;
+};
+
+template <int K>
+C5_HD void store_pixel_ch(const WalkParams& P, int i, int j, const double* tau, const double* inten, uint32_t steps) {
+    const size_t o = static_cast<size_t>(j - P.row_begin) * P.res_x + i;
+#pragma unroll
+    for (int c = 0; c < K; c++) {
+        double t = tau[c], v = inten[c];
+        if (P.round_float) {
+            t = static_cast<double>(static_cast<float>(t));
+            v = static_cast<double>(static_cast<float>(v));
+        }
+        store2(P.out + 2 * (o * K + c), t, v);
+    }
+    if (P.steps) P.steps[o] = steps;
+}
+
+// Background or solid pixel outside the walk's rectangle, n channels wide.
+C5_HD bool background_pixel_ch(const WalkParams& P, int n, int i, int j) {
+    const bool solid = P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i];
+    const double v = solid ? __longlong_as_double_hd(0x7FF8000000000000ll) : 0.0;
+    const size_t o = static_cast<size_t>(j - P.row_begin) * P.res_x + i;
+    for (int c = 0; c < n; c++) store2(P.out + 2 * (o * n + c), v, v);
+    if (P.steps) P.steps[o] = 0;
+    return solid;
+}
+
+// trace_ray with K channels: the same four phases, searches and deferral rule.
+template <int K>
+C5_HD void trace_ray_ch(const ChanParams& CP, double px, double py, uint32_t pixel, unsigned tracing, ChanRay<K>& r) {
+    const WalkParams& P = CP.W;
+    r.f.rec = CP.rec;
+    r.f.reset();
+    r.steps = 0;
+    r.error = 0;
+    r.deferred = 0;
+    double z_after = -INFINITY;
+    EntryList<kInline> L;
+
+    bool defer = !bvh_collect_entries(P, px, py, z_after, L, 1, P.query_budget);
+    sync_lanes(tracing);
+    const bool entered = !defer && L.n > 0;
+    if (entered) z_after = crossing_walk<false>(P, px, py, L.leaf[0], L.z[0], r.f, r.steps, r.error);
+    sync_lanes(tracing);
+    L.n = 0;
+    if (entered && !r.error) {
+        const bool searched = bvh_collect_entries(P, px, py, z_after, L, kInline, P.query_budget);
+        defer = !searched || L.n == kInline;
+    }
+    sync_lanes(tracing);
+    for (int e = 0; e < kInline - 1; e++) {
+        if (!defer && e < L.n && L.z[e] > z_after && !r.error) {
+            z_after = crossing_walk<false>(P, px, py, L.leaf[e], L.z[e], r.f, r.steps, r.error);
+        }
+        sync_lanes(tracing);
+    }
+    if (defer) {
+#ifdef __CUDA_ARCH__
+        const unsigned long long slot = atomicAdd(&P.counters[kDeferred], 1ull);
+#else
+        const unsigned long long slot = P.counters[kDeferred]++;
+#endif
+        DeferredRay& q = P.queue[slot];
+        q.tau = 0.0;
+        q.inten = 0.0;
+        q.z_after = z_after;
+        q.pixel = pixel;
+        q.steps = r.steps;
+#pragma unroll
+        for (int c = 0; c < K; c++) store2(CP.queue + 2 * (slot * K + c), r.f.tau[c], r.f.inten[c]);
+        r.deferred = 1;
+    }
+}
+
+// A deferred ray's K channels and geometry, as RayAcc holds one.
+template <int K>
+struct ChanAcc {
+    double tau[K], inten[K];
+    double z_after;
+    uint32_t steps, error;
+};
+
+template <int K>
+C5_HD void load_deferred_ch(const ChanParams& CP, unsigned long long slot, ChanAcc<K>& a) {
+    const DeferredRay& q = CP.W.queue[slot];
+    a.z_after = q.z_after;
+    a.steps = q.steps;
+    a.error = 0;
+#pragma unroll
+    for (int c = 0; c < K; c++) {
+        a.tau[c] = CP.queue[2 * (slot * K + c)];
+        a.inten[c] = CP.queue[2 * (slot * K + c) + 1];
+    }
+}
+
+// compose_crossing, per channel.
+template <int K>
+C5_HD void compose_crossing_ch(ChanAcc<K>& a, double z_in, double z_out, const ChanFields<K, true>& k, uint32_t steps_k,
+                               uint32_t error_k) {
+    if (!(z_in > a.z_after)) return;
+#pragma unroll
+    for (int c = 0; c < K; c++) {
+        a.tau[c] += k.tau[c];
+        a.inten[c] = k.inten[c] + k.gain[c] * a.inten[c];
+    }
+    a.steps += steps_k;
+    a.error |= error_k;
+    a.z_after = z_out;
+}
+
+// graze_ray_serial with K channels (host-loop build).
+template <int K>
+C5_HD ChanAcc<K> graze_ray_serial_ch(const ChanParams& CP, unsigned long long slot, double px, double py) {
+    const WalkParams& P = CP.W;
+    ChanAcc<K> a;
+    load_deferred_ch<K>(CP, slot, a);
+    EntryList<kSerialList> L;
+    int crossings = 0;
+    while (!a.error) {
+        if (!bvh_collect_entries(P, px, py, a.z_after, L, P.serial_cap, 0x7FFFFFFF)) a.error = 1;
+        for (int e = 0; e < L.n; e++) {
+            if (!(L.z[e] > a.z_after)) continue;
+            ChanFields<K, true> k;
+            k.rec = CP.rec;
+            k.reset();
+            uint32_t steps_k = 0, error_k = 0;
+            const double z_out = crossing_walk<true>(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
+            compose_crossing_ch<K>(a, L.z[e], z_out, k, steps_k, error_k);
+            if (++crossings > 65536) a.error = 1;
+        }
+        if (L.n < P.serial_cap) break;
+    }
+    return a;
+}
+
+// graze_block with K channels: the same collection, and crossings folded per channel in z order.
+template <int K>
+__device__ __forceinline__ void graze_block_ch(const ChanParams& CP) {
+    const WalkParams& P = CP.W;
+    __shared__ GrazeSmem smem[kGrazeWarps];
+    const unsigned full = 0xFFFFFFFFu;
+    const int lane = threadIdx.x & 31;
+    GrazeSmem& S = smem[threadIdx.x >> 5];
+    const unsigned long long n_rays = P.counters[kDeferred];
+    while (true) {
+        unsigned long long ticket = 0;
+        if (lane == 0) ticket = atomicAdd(&P.counters[kTicket], 1ull);
+        ticket = __shfl_sync(full, ticket, 0);
+        if (ticket >= n_rays) break;
+        const uint32_t q_pixel = P.queue[ticket].pixel;
+        const int i = static_cast<int>(q_pixel % static_cast<uint32_t>(P.res_x));
+        const int j = static_cast<int>(q_pixel / static_cast<uint32_t>(P.res_x));
+        const double px = P.xs[i], py = P.ys[j];
+        ChanAcc<K> a;
+        load_deferred_ch<K>(CP, ticket, a);
+        const uint32_t q_steps = a.steps;
+        int crossings = 0;
+        bool truncated = true;
+        while (truncated && !a.error) {
+            const int n = graze_collect(P, S, px, py, a.z_after, lane, truncated);
+            for (int base = 0; base < n; base += 32) {
+                const int k = base + lane;
+                const bool have = k < n;
+                const double z_in = have ? S.z[k] : INFINITY;
+                double z_out = z_in;
+                ChanFields<K, true> f;
+                f.rec = CP.rec;
+                f.reset();
+                uint32_t steps_k = 0, error_k = 0;
+                if (have && z_in > a.z_after) z_out = crossing_walk<true>(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
+                const int cnt = n - base < 32 ? n - base : 32;
+                for (int l = 0; l < cnt; l++) {
+                    ChanFields<K, true> g;
+#pragma unroll
+                    for (int c = 0; c < K; c++) {
+                        g.tau[c] = __shfl_sync(full, f.tau[c], l);
+                        g.inten[c] = __shfl_sync(full, f.inten[c], l);
+                        g.gain[c] = __shfl_sync(full, f.gain[c], l);
+                    }
+                    compose_crossing_ch<K>(a, __shfl_sync(full, z_in, l), __shfl_sync(full, z_out, l), g,
+                                           __shfl_sync(full, steps_k, l), __shfl_sync(full, error_k, l));
+                }
+            }
+            crossings += n;
+            if (crossings > 65536) a.error = 1;
+            __syncwarp();
+        }
+        if (lane == 0) {
+            store_pixel_ch<K>(P, i, j, a.tau, a.inten, a.steps);
+            const unsigned long long more = a.steps - q_steps;
+            if (more) {
+                atomicAdd(&P.counters[kSteps], more);
+                atomicAdd(&P.row_cost[j], more);
+                if (q_steps == 0) atomicAdd(&P.counters[kHitPixels], 1ull);
+            }
+            if (a.error) atomicAdd(&P.counters[kWalkErrors], 1ull);
+        }
+    }
+}
+
+// walk_block with K channels: same tiles, same statistics.
+template <int K>
+__device__ __forceinline__ void walk_block_ch(const ChanParams& CP) {
+    const WalkParams& P = CP.W;
+    const int b = blockIdx.x;
+    const int macro = b >> 6, r = b & 63;
+    const int tile_x = (macro % P.n_macro_x) * 8 + compact3(r);
+    const int tile_y = (macro / P.n_macro_x) * 8 + compact3(r >> 1);
+    if (tile_x >= P.n_tiles_x || tile_y >= P.n_tiles_y) return;
+
+    const int i_lo = P.i0 + tile_x * kTileX, j_lo = P.j0 + tile_y * kTileY;
+    const int i_hi = min(i_lo + kTileX, P.i1) - 1, j_hi = min(j_lo + kTileY, P.j1) - 1;
+    bool tile_sees_mesh;
+    {
+        const BvhNode* root = P.nodes;
+        const float x0 = f_round_down(P.xs[i_lo]), x1 = f_round_up(P.xs[i_hi]);
+        const float y0 = f_round_down(P.ys[j_lo]), y1 = f_round_up(P.ys[j_hi]);
+        const bool s0 = x1 >= root->xlo[0] && x0 <= root->xhi[0] && y1 >= root->ylo[0] && y0 <= root->yhi[0];
+        const bool s1 = x1 >= root->xlo[1] && x0 <= root->xhi[1] && y1 >= root->ylo[1] && y0 <= root->yhi[1];
+        tile_sees_mesh = s0 || s1;
+    }
+
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int i = P.i0 + tile_x * kTileX + (warp % 2) * 8 + (lane & 7);
+    const int j = P.j0 + tile_y * kTileY + (warp / 2) * 4 + (lane >> 3);
+    const bool live = i < P.i1 && j < P.j1;
+
+    ChanRay<K> res;
+    res.f.reset();
+    res.steps = 0;
+    res.error = 0;
+    res.deferred = 0;
+    bool solid = false;
+    if (live) solid = P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i];
+    const unsigned tracing = __ballot_sync(0xFFFFFFFFu, live && !solid && tile_sees_mesh);
+    if (live) {
+        if (solid) {
+            double nan[K];
+#pragma unroll
+            for (int c = 0; c < K; c++) nan[c] = __longlong_as_double(0x7FF8000000000000ll);
+            store_pixel_ch<K>(P, i, j, nan, nan, 0);
+        } else {
+            if (tile_sees_mesh) {
+                trace_ray_ch<K>(CP, P.xs[i], P.ys[j],
+                                static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
+                                tracing, res);
+            }
+            if (!res.deferred) store_pixel_ch<K>(P, i, j, res.f.tau, res.f.inten, res.steps);
+        }
+    }
+
+    const unsigned full = 0xFFFFFFFFu;
+    unsigned row_steps = res.steps;
+    row_steps += __shfl_xor_sync(full, row_steps, 1);
+    row_steps += __shfl_xor_sync(full, row_steps, 2);
+    row_steps += __shfl_xor_sync(full, row_steps, 4);
+    if ((lane & 7) == 0 && live && row_steps) atomicAdd(&P.row_cost[j], static_cast<unsigned long long>(row_steps));
+    unsigned warp_steps = row_steps;
+    warp_steps += __shfl_xor_sync(full, warp_steps, 8);
+    warp_steps += __shfl_xor_sync(full, warp_steps, 16);
+    const unsigned hits = __popc(__ballot_sync(full, live && res.steps > 0));
+    const unsigned solids = __popc(__ballot_sync(full, solid));
+    const unsigned errors = __popc(__ballot_sync(full, res.error != 0));
+    if (lane == 0) {
+        if (warp_steps) atomicAdd(&P.counters[kSteps], static_cast<unsigned long long>(warp_steps));
+        if (hits) atomicAdd(&P.counters[kHitPixels], static_cast<unsigned long long>(hits));
+        if (solids) atomicAdd(&P.counters[kSolidPixels], static_cast<unsigned long long>(solids));
+        if (errors) atomicAdd(&P.counters[kWalkErrors], static_cast<unsigned long long>(errors));
+    }
+}
+
+// Resident blocks of 128 threads per SM for the K-channel pixel kernel. K = 1, 2: the most blocks
+// whose register cap (72, 80) leaves the kernel free of spills. K >= 3: the occupancy the registers
+// ptxas needs without a cap allow (110..128 registers: 4 blocks, 136..150: 3), so the bound only
+// records it (-Xptxas -v; the registers per K are in DESIGN.md).
+constexpr int chan_blocks_per_sm(int K) {
+    return K <= 1 ? 7 : K <= 2 ? 6 : K <= 5 ? 4 : 3;
+}
+
+} // namespace
+
+template <int K>
+__global__ void __launch_bounds__(kBlock, chan_blocks_per_sm(K)) tet_walk_ch(const ChanParams P) { walk_block_ch<K>(P); }
+template <int K>
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_ch(const ChanParams P) { graze_block_ch<K>(P); }
+
+__global__ void __launch_bounds__(256) fill_background_ch(const WalkParams P, int n_channels) {
+    const int n_rows = P.row_end - P.row_begin;
+    const int64_t k = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+    bool solid = false;
+    if (k < static_cast<int64_t>(n_rows) * P.res_x) {
+        const int j = P.row_begin + static_cast<int>(k / P.res_x), i = static_cast<int>(k % P.res_x);
+        if (!(i >= P.i0 && i < P.i1 && j >= P.j0 && j < P.j1)) solid = background_pixel_ch(P, n_channels, i, j);
+    }
+    const unsigned solids = __popc(__ballot_sync(0xFFFFFFFFu, solid));
+    if ((threadIdx.x & 31) == 0 && solids) atomicAdd(&P.counters[kSolidPixels], static_cast<unsigned long long>(solids));
+}
+
+namespace {
+
+template <int K>
+void walk_on_host_ch(const ChanParams& CP) {
+    const WalkParams& P = CP.W;
+    for (int j = P.j0; j < P.j1; j++) {
+        for (int i = P.i0; i < P.i1; i++) {
+            if (P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i]) {
+                double nan[K];
+                for (int c = 0; c < K; c++) nan[c] = NAN;
+                store_pixel_ch<K>(P, i, j, nan, nan, 0);
+                P.counters[kSolidPixels]++;
+                continue;
+            }
+            const uint32_t pixel = static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i);
+            ChanRay<K> r;
+            trace_ray_ch<K>(CP, P.xs[i], P.ys[j], pixel, 0, r);
+            if (!r.deferred) store_pixel_ch<K>(P, i, j, r.f.tau, r.f.inten, r.steps);
+            P.counters[kSteps] += r.steps;
+            P.row_cost[j] += r.steps;
+            if (r.steps) P.counters[kHitPixels]++;
+            if (r.error) P.counters[kWalkErrors]++;
+        }
+    }
+}
+
+template <int K>
+void graze_on_host_ch(const ChanParams& CP) {
+    const WalkParams& P = CP.W;
+    const unsigned long long n_rays = P.counters[kDeferred];
+    for (unsigned long long k = 0; k < n_rays; k++) {
+        const DeferredRay& q = P.queue[k];
+        const int i = static_cast<int>(q.pixel % static_cast<uint32_t>(P.res_x));
+        const int j = static_cast<int>(q.pixel / static_cast<uint32_t>(P.res_x));
+        const ChanAcc<K> a = graze_ray_serial_ch<K>(CP, k, P.xs[i], P.ys[j]);
+        store_pixel_ch<K>(P, i, j, a.tau, a.inten, a.steps);
+        P.counters[kSteps] += a.steps - q.steps;
+        P.row_cost[j] += a.steps - q.steps;
+        if (q.steps == 0 && a.steps > 0) P.counters[kHitPixels]++;
+        if (a.error) P.counters[kWalkErrors]++;
+    }
+    P.counters[kTicket] = n_rays;
+}
+
+template <int K>
+void launch_walk_ch(DeviceState& d, const WalkLaunch& w, const WalkParams& P, unsigned grid) {
+    ChanParams CP{P, d.ch_rec.p, d.ch_queue.p};
+    if (kHostSim) {
+        walk_on_host_ch<K>(CP);
+        count_launch();
+        graze_on_host_ch<K>(CP);
+        return;
+    }
+    tet_walk_ch<K><<<grid, kBlock, 0, d.stream>>>(CP);
+    C5_CUDA(cudaGetLastError());
+    if (w.mark_walk_done) C5_CUDA(cudaEventRecord(w.mark_walk_done, d.stream));
+    if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
+    if (d.sm_count == 0) C5_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, d.device));
+    count_launch();
+    grazing_rays_ch<K><<<static_cast<unsigned>(d.sm_count) * static_cast<unsigned>(kGrazeBlocksPerSm), 32 * kGrazeWarps, 0,
+                         d.stream>>>(CP);
+    C5_CUDA(cudaGetLastError());
 }
 
 } // namespace
@@ -1028,18 +1485,39 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     P.round_float = w.round_through_float;
     P.alpha_limit = w.alpha_limit;
 
+    if (w.channels < 0 || w.channels > C5_MAX_CHANNELS || (w.channels && f32)) {
+        fail(C5_E_INVALID, "render: channels need precision 64 and 1 .. C5_MAX_CHANNELS channels");
+    }
     if (!whole_band) {
         count_launch();
         if (kHostSim) {
-            background_on_host(P);
+            background_on_host(P, w.channels);
         } else {
             const int64_t n = static_cast<int64_t>(w.row_end - w.row_begin) * w.res_x;
-            fill_background<<<static_cast<unsigned>((n + 255) / 256), 256, 0, d.stream>>>(P);
+            if (w.channels) {
+                fill_background_ch<<<static_cast<unsigned>((n + 255) / 256), 256, 0, d.stream>>>(P, w.channels);
+            } else {
+                fill_background<<<static_cast<unsigned>((n + 255) / 256), 256, 0, d.stream>>>(P);
+            }
             C5_CUDA(cudaGetLastError());
         }
     }
     if (empty_rect) return; // the mesh is not in this band: no rays
     count_launch();
+    if (w.channels) {
+        const unsigned grid = static_cast<unsigned>(P.n_macro_x) * static_cast<unsigned>(n_macro_y) * 64u;
+        switch (w.channels) {
+        case 1: launch_walk_ch<1>(d, w, P, grid); break;
+        case 2: launch_walk_ch<2>(d, w, P, grid); break;
+        case 3: launch_walk_ch<3>(d, w, P, grid); break;
+        case 4: launch_walk_ch<4>(d, w, P, grid); break;
+        case 5: launch_walk_ch<5>(d, w, P, grid); break;
+        case 6: launch_walk_ch<6>(d, w, P, grid); break;
+        case 7: launch_walk_ch<7>(d, w, P, grid); break;
+        default: launch_walk_ch<8>(d, w, P, grid); break;
+        }
+        return;
+    }
     if (kHostSim) {
         walk_on_host(P, f32);
         count_launch();

@@ -2,6 +2,7 @@
 #include "cli.hpp"
 
 #include <algorithm>
+#include <array>
 #include <cstdlib>
 #include <iostream>
 #include <stdexcept>
@@ -25,8 +26,27 @@ const option kOptions[] = {
     {"initial_system_angle", 'I', true}, {"alpha_limit", 0, true},
     // additions of this build (absent from the reference)
     {"devices", 0, true},          {"stats", 0, false},           {"precision", 0, true},
-    {"frames", 0, true},           {"sweep_y_to", 0, true},
+    {"frames", 0, true},           {"sweep_y_to", 0, true},       {"channels", 0, true},
 };
+
+// --channels A:Q[,A:Q...]: pairs of CELL_DATA array names, at most C5_MAX_CHANNELS (8)
+std::vector<std::array<std::string, 2>> parse_channels(const std::string& value) {
+    std::vector<std::array<std::string, 2>> out;
+    std::size_t at = 0;
+    while (at <= value.size()) {
+        const std::size_t comma = std::min(value.find(',', at), value.size());
+        const std::string item = value.substr(at, comma - at);
+        const std::size_t colon = item.find(':');
+        if (colon == std::string::npos || colon == 0 || colon + 1 == item.size() ||
+            item.find(':', colon + 1) != std::string::npos) {
+            throw std::runtime_error("--channels: '" + item + "' is not of the form ALPHA:Q");
+        }
+        out.push_back({item.substr(0, colon), item.substr(colon + 1)});
+        at = comma + 1;
+    }
+    if (out.size() > 8) throw std::runtime_error("--channels: at most 8 channels");
+    return out;
+}
 
 const option* find_long(const std::string& name, std::string& err) {
     const option* exact = nullptr;
@@ -94,6 +114,9 @@ void print_usage(std::ostream& out) {
            "                                         uses Y + (sweep_y_to - Y) k / frames and is\n"
            "                                         written to <destination stem>_<k>.vti\n"
            "  --sweep_y_to arg (=2)                  end angle of the sweep (exclusive)\n"
+           "  --channels arg                         A:Q[,A:Q...]: also render these pairs of cell\n"
+           "                                         arrays of the input file in the same walk, each\n"
+           "                                         as a further array named A:Q (not with --frames)\n"
         << std::endl;
 }
 
@@ -151,7 +174,9 @@ cli_result program_options(int argc, char** argv, config_str& cfg, std::ostream&
             else if (name == "precision") cfg.precision = static_cast<int>(to_integer(name, value));
             else if (name == "frames") cfg.frames = static_cast<int>(to_integer(name, value));
             else if (name == "sweep_y_to") cfg.sweep_y_to = to_double(name, value);
+            else if (name == "channels") cfg.channels = parse_channels(value);
         }
+        if (!cfg.channels.empty() && cfg.frames > 1) throw std::runtime_error("--channels cannot be combined with --frames > 1");
     } catch (const std::exception& e) {
         out << "Error! " << e.what() << std::endl;
         print_usage(out);

@@ -3,9 +3,11 @@
 // bit-identical (they feed the solid-object generators and the view rotations).
 #pragma once
 
+#include <array>
 #include <cstddef>
 #include <limits>
 #include <string>
+#include <vector>
 
 namespace c5host {
 
@@ -29,6 +31,7 @@ struct config_str {
     int precision = 64;
     int frames = 1;                            // --frames N: in-process sweep of -Y (replaces utility/rotate_traces.py)
     double sweep_y_to = 2.0;                   // --sweep_y_to: end angle (exclusive), units of pi
+    std::vector<std::array<std::string, 2>> channels; // --channels A:Q,...: (alpha, Q) cell array names
 };
 
 constexpr double PI = 3.14159265358979323846;  // config.hpp:45

@@ -80,7 +80,36 @@ long long c5host_write_vti(const char* filename, const double* image, long long 
     });
 }
 
+// write_vti with n_extra further arrays: names[k] and data[k] (res_y * res_x * 2 doubles each).
+long long c5host_write_vti_arrays(const char* filename, const double* image, long long res_x, long long res_y, int compress,
+                                  int n_extra, const char* const* names, const double* const* data) {
+    return guarded([&]() -> long long {
+        std::vector<vti_array> extra;
+        for (int k = 0; k < n_extra; k++) extra.push_back(vti_array{names[k], data[k]});
+        write_vti(filename, image, static_cast<std::size_t>(res_x), static_cast<std::size_t>(res_y),
+                  compress == 2 ? vti_encoding::zlib_base64 : compress == 1 ? vti_encoding::zlib_raw : vti_encoding::raw,
+                  extra);
+        return 0;
+    });
+}
+
 // Returns the number of doubles (res_x * res_y * comps), fills dims; call again with `out` to copy.
+// `name`: the PointData array (NULL or empty: the first one, ImageScalars).
+long long c5host_read_vti_array(const char* filename, const char* name, long long* res_x, long long* res_y,
+                                long long* comps, double* out) {
+    return guarded([&]() -> long long {
+        std::size_t x, y, c;
+        double* img = nullptr;
+        read_vti(filename, x, y, c, img, name ? name : "");
+        *res_x = static_cast<long long>(x);
+        *res_y = static_cast<long long>(y);
+        *comps = static_cast<long long>(c);
+        if (out) std::memcpy(out, img, x * y * c * sizeof(double));
+        delete[] img;
+        return static_cast<long long>(x * y * c);
+    });
+}
+
 long long c5host_read_vti(const char* filename, long long* res_x, long long* res_y, long long* comps, double* out) {
     return guarded([&]() -> long long {
         std::size_t x, y, c;

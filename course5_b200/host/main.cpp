@@ -75,6 +75,13 @@ int main(int argc, char** argv) {
         auto acc_sphere = object3d_sphere{{ACC_X0, ACC_Y0, ACC_Z0}, ACC_DISK_R}; // not rotated, main.cpp:116
         loader.join();
         if (!load_error.empty()) throw std::runtime_error(load_error);
+        for (const auto& pair : config.channels) {
+            for (const std::string& name : pair) {
+                if (!acc_disk.get_pointer()->grid.cell_scalars.count(name)) {
+                    throw std::runtime_error(config.file + ": no cell scalar named '" + name + "' (--channels)");
+                }
+            }
+        }
         auto t2 = std::chrono::steady_clock::now();
         std::cout << "Loading data with VTK lib and other preparations completed in " << ms_between(t1, t2) << " ms. "
                   << std::endl;
@@ -83,16 +90,24 @@ int main(int argc, char** argv) {
         options.devices = parse_devices(config.devices);
         options.alpha_limit = config.limit_alpha_value;
         options.precision = config.precision;
+        options.channels = config.channels;
 
         t1 = std::chrono::steady_clock::now();
         plane base_plane{config.resolution_x, config.resolution_y, {acc_disk, roche_lobe, acc_sphere}, domain, options};
         base_plane.find_intersections();
         object2d result = base_plane.trace_rays(tetra_value::alpha, tetra_value::Q);
+        // --channels: the named pairs in one further walk, written beside ImageScalars as "A:Q"
+        const std::vector<std::vector<double>> channels =
+            config.channels.empty() ? std::vector<std::vector<double>>{} : base_plane.trace_channels();
         t2 = std::chrono::steady_clock::now();
         std::cout << "Ray-tracing completed in " << ms_between(t1, t2) << " ms. " << std::endl;
 
         if (config.frames <= 1) {
-            result.export_to_vti(config.destination);
+            std::vector<vti_array> extra;
+            for (std::size_t c = 0; c < channels.size(); c++) {
+                extra.push_back(vti_array{config.channels[c][0] + ":" + config.channels[c][1], channels[c].data()});
+            }
+            result.export_to_vti(config.destination, false, extra);
         } else {
             // in-process sweep: the scene stays on the device, only the rotations change
             std::string stem = config.destination, ext = ".vti";

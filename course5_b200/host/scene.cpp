@@ -112,8 +112,8 @@ object3d_sphere::object3d_sphere(const point& center, double R) {
     _data->solid = make_sphere(center, R);
 }
 
-void object2d::export_to_vti(const std::string& filename, bool compress) const {
-    write_vti(filename, _image.data(), _x, _y, compress);
+void object2d::export_to_vti(const std::string& filename, bool compress, const std::vector<vti_array>& extra) const {
+    write_vti(filename, _image.data(), _x, _y, compress ? vti_encoding::zlib_raw : vti_encoding::raw, extra);
 }
 
 void image_ref::export_to_vti(const std::string& filename, bool compress) const {
@@ -205,6 +205,20 @@ void plane::find_intersections() {
                                grid.grid.tets.data(), static_cast<int64_t>(grid.grid.n_tets()), alpha.data(), q.data()),
           "c5_upload_mesh");
     check(_ctx, c5_clear_solids(_ctx), "c5_clear_solids");
+    if (!_options.channels.empty()) { // channel-major, in the file's tet order
+        const std::size_t n_t = grid.grid.n_tets(), n = _options.channels.size();
+        std::vector<double> ch_alpha(n * n_t), ch_q(n * n_t);
+        for (std::size_t c = 0; c < n; c++) {
+            for (int k = 0; k < 2; k++) {
+                const auto it = grid.grid.cell_scalars.find(_options.channels[c][static_cast<std::size_t>(k)]);
+                if (it == grid.grid.cell_scalars.end() || it->second.size() != n_t) {
+                    throw std::runtime_error("no cell scalar named '" + _options.channels[c][static_cast<std::size_t>(k)] + "'");
+                }
+                std::copy(it->second.begin(), it->second.end(), (k ? ch_q : ch_alpha).begin() + static_cast<std::ptrdiff_t>(c * n_t));
+            }
+        }
+        check(_ctx, c5_upload_channels(_ctx, ch_alpha.data(), ch_q.data(), static_cast<int32_t>(n)), "c5_upload_channels");
+    }
 
     // the grid's recorded rotations define the view; solids that recorded the same list follow it
     // on the device, the others are baked on the host and uploaded as static
@@ -262,6 +276,21 @@ object2d plane::trace_rays(tetra_value value_alpha, tetra_value value_Q) {
     std::vector<double> image(_x * _y * 2);
     check(_ctx, c5_render(_ctx, &_view, image.data(), &_stats), "c5_render");
     return object2d{std::move(image), _x, _y};
+}
+
+std::vector<std::vector<double>> plane::trace_channels() {
+    if (!_uploaded) find_intersections();
+    const std::size_t n = _options.channels.size(), n_pix = _x * _y;
+    std::vector<double> all(n_pix * n * 2);
+    check(_ctx, c5_render_channels(_ctx, &_view, all.data(), nullptr, nullptr, nullptr), "c5_render_channels");
+    std::vector<std::vector<double>> out(n, std::vector<double>(n_pix * 2));
+    for (std::size_t p = 0; p < n_pix; p++) {
+        for (std::size_t c = 0; c < n; c++) {
+            out[c][2 * p] = all[(p * n + c) * 2];
+            out[c][2 * p + 1] = all[(p * n + c) * 2 + 1];
+        }
+    }
+    return out;
 }
 
 } // namespace c5host

@@ -23,6 +23,7 @@
 #include "../../include/c5gpu.h"
 #include "config.hpp"
 #include "solids.hpp"
+#include "vti_writer.hpp"
 #include "vtk_reader.hpp"
 
 namespace c5host {
@@ -80,7 +81,8 @@ class object2d {
 public:
     object2d(std::vector<double> image, std::size_t res_x, std::size_t res_y)
         : _image(std::move(image)), _x(res_x), _y(res_y) {}
-    void export_to_vti(const std::string& filename, bool compress = false) const;
+    // extra: further arrays beside ImageScalars (course --channels)
+    void export_to_vti(const std::string& filename, bool compress = false, const std::vector<vti_array>& extra = {}) const;
     const std::vector<double>& data() const { return _image; } // res_y * res_x * {tau, I}, x fastest
     std::size_t get_x() const { return _x; }
     std::size_t get_y() const { return _y; }
@@ -101,6 +103,7 @@ struct render_options {
     std::vector<int> devices{0};
     double alpha_limit = 2.5; // the reference reads app::instance().config.limit_alpha_value (line.cpp:204)
     int precision = 64;
+    std::vector<std::array<std::string, 2>> channels; // (alpha, Q) cell scalar names uploaded as channels
 };
 
 class plane {
@@ -114,6 +117,9 @@ public:
 
     void find_intersections();
     object2d trace_rays(tetra_value value_alpha, tetra_value value_Q);
+    // The pairs of render_options::channels for the same view, in one walk (c5_render_channels):
+    // one (res_y, res_x, 2) image per channel.
+    std::vector<std::vector<double>> trace_channels();
     // Sweeps: replace the recorded view rotations (grid and view-following solids) without
     // re-uploading anything; the next trace_rays() renders the new view in milliseconds.
     void set_view_rotations(const std::vector<c5_rotation>& rotations);

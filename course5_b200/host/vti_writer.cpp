@@ -106,8 +106,59 @@ void write_vti(const std::string& filename, const double* image, std::size_t res
     write_vti(filename, image, res_x, res_y, compress ? vti_encoding::zlib_raw : vti_encoding::raw);
 }
 
+namespace {
+
+// One array's appended data in VTK's compressed block layout: [n_blocks][block_size][last_block_size]
+// [compressed sizes...] then the blocks; with b64 the table and the blocks as two base64 streams.
+std::string compressed_payload(const double* data, std::uint64_t n_bytes, bool b64, const std::string& filename) {
+    const std::uint64_t block = 1u << 20;
+    const std::uint64_t n_blocks = (n_bytes + block - 1) / block;
+    const std::uint64_t last = n_bytes - (n_blocks - 1) * block;
+    std::vector<std::vector<unsigned char>> packed(n_blocks);
+    std::vector<std::uint64_t> header(3 + n_blocks);
+    header[0] = n_blocks;
+    header[1] = block;
+    header[2] = (last == block) ? 0 : last;
+    const unsigned char* src = reinterpret_cast<const unsigned char*>(data);
+    std::atomic<std::uint64_t> next{0};
+    std::atomic<bool> failed{false};
+    auto deflate_blocks = [&] {   // blocks are handed out one at a time: the last, short one does not unbalance anyone
+        for (std::uint64_t b = next.fetch_add(1); b < n_blocks && !failed.load(); b = next.fetch_add(1)) {
+            const uLong in_size = static_cast<uLong>(b + 1 == n_blocks ? last : block);
+            uLongf out_size = compressBound(in_size);
+            packed[b].resize(out_size);
+            if (compress2(packed[b].data(), &out_size, src + b * block, in_size, Z_BEST_SPEED) != Z_OK) {
+                failed.store(true);
+                return;
+            }
+            packed[b].resize(out_size);
+            header[3 + b] = out_size;
+        }
+    };
+    const unsigned n_threads = compressor_threads(n_blocks);
+    if (n_threads <= 1) {
+        deflate_blocks();
+    } else {
+        std::vector<std::thread> pool;
+        for (unsigned t = 1; t < n_threads; t++) pool.emplace_back(deflate_blocks);
+        deflate_blocks();
+        for (auto& t : pool) t.join();
+    }
+    if (failed.load()) throw std::runtime_error("zlib failed while writing " + filename);
+    std::vector<unsigned char> all(reinterpret_cast<const unsigned char*>(header.data()),
+                                   reinterpret_cast<const unsigned char*>(header.data() + header.size()));
+    const std::size_t table = all.size();
+    for (const auto& p : packed) all.insert(all.end(), p.begin(), p.end());
+    if (!b64) return std::string(all.begin(), all.end());
+    // vtkXMLWriter's default (EncodeAppendedData on): the block table is one base64 stream, the
+    // concatenated compressed blocks another
+    return base64(all.data(), table) + base64(all.data() + table, all.size() - table);
+}
+
+} // namespace
+
 void write_vti(const std::string& filename, const double* image, std::size_t res_x, std::size_t res_y,
-               vti_encoding encoding) {
+               vti_encoding encoding, const std::vector<vti_array>& extra) {
     const bool compress = encoding != vti_encoding::raw;
     const bool b64 = encoding == vti_encoding::zlib_base64;
     FILE* fp = std::fopen(filename.c_str(), "wb");
@@ -115,26 +166,42 @@ void write_vti(const std::string& filename, const double* image, std::size_t res
     file_closer closer{fp};
     const std::uint64_t n_bytes = static_cast<std::uint64_t>(res_x) * res_y * 2 * sizeof(double);
     const int ex = static_cast<int>(res_x) - 1, ey = static_cast<int>(res_y) - 1;
+    std::vector<vti_array> arrays{{"ImageScalars", image}};
+    arrays.insert(arrays.end(), extra.begin(), extra.end());
+    // compressed arrays are packed first: their sizes give the offsets the header lists
+    std::vector<std::string> payload(compress ? arrays.size() : 0);
+    for (std::size_t a = 0; a < payload.size(); a++) payload[a] = compressed_payload(arrays[a].data, n_bytes, b64, filename);
+    std::string data_arrays;
+    std::uint64_t offset = 0;
+    for (std::size_t a = 0; a < arrays.size(); a++) {
+        data_arrays += "        <DataArray type=\"Float64\" Name=\"" + arrays[a].name +
+                       "\" NumberOfComponents=\"2\" format=\"appended\" offset=\"" + std::to_string(offset) + "\"/>\n";
+        offset += compress ? payload[a].size() : sizeof(n_bytes) + n_bytes;
+    }
     std::fprintf(fp,
                  "<?xml version=\"1.0\"?>\n"
                  "<VTKFile type=\"ImageData\" version=\"1.0\" byte_order=\"LittleEndian\" header_type=\"UInt64\"%s>\n"
                  "  <ImageData WholeExtent=\"0 %d 0 %d 0 0\" Origin=\"0 0 0\" Spacing=\"1 1 1\">\n"
                  "    <Piece Extent=\"0 %d 0 %d 0 0\">\n"
                  "      <PointData Scalars=\"ImageScalars\">\n"
-                 "        <DataArray type=\"Float64\" Name=\"ImageScalars\" NumberOfComponents=\"2\" "
-                 "format=\"appended\" offset=\"0\"/>\n"
+                 "%s"
                  "      </PointData>\n"
                  "      <CellData/>\n"
                  "    </Piece>\n"
                  "  </ImageData>\n"
                  "  <AppendedData encoding=\"%s\">\n   _",
-                 compress ? " compressor=\"vtkZLibDataCompressor\"" : "", ex, ey, ex, ey, b64 ? "base64" : "raw");
-    if (!compress) {
+                 compress ? " compressor=\"vtkZLibDataCompressor\"" : "", ex, ey, ex, ey, data_arrays.c_str(),
+                 b64 ? "base64" : "raw");
+    for (std::size_t a = 0; a < arrays.size(); a++) {
+        if (compress) {
+            std::fwrite(payload[a].data(), 1, payload[a].size(), fp);
+            continue;
+        }
         std::fwrite(&n_bytes, sizeof(n_bytes), 1, fp);
         // the pixels go straight from the caller's buffer to the file descriptor: stdio would copy 69 MB through its
         // own buffer first
         std::fflush(fp);
-        const char* at = reinterpret_cast<const char*>(image);
+        const char* at = reinterpret_cast<const char*>(arrays[a].data);
         std::uint64_t left = n_bytes;
         while (left > 0) {
             const ssize_t w = ::write(fileno(fp), at, left > (1u << 30) ? (1u << 30) : left);
@@ -142,61 +209,12 @@ void write_vti(const std::string& filename, const double* image, std::size_t res
             at += w;
             left -= static_cast<std::uint64_t>(w);
         }
-    } else {
-        // VTK compressed block layout: [n_blocks][block_size][last_block_size][compressed sizes...] data...
-        const std::uint64_t block = 1u << 20;
-        const std::uint64_t n_blocks = (n_bytes + block - 1) / block;
-        const std::uint64_t last = n_bytes - (n_blocks - 1) * block;
-        std::vector<std::vector<unsigned char>> packed(n_blocks);
-        std::vector<std::uint64_t> header(3 + n_blocks);
-        header[0] = n_blocks;
-        header[1] = block;
-        header[2] = (last == block) ? 0 : last;
-        const unsigned char* src = reinterpret_cast<const unsigned char*>(image);
-        std::atomic<std::uint64_t> next{0};
-        std::atomic<bool> failed{false};
-        auto deflate_blocks = [&] {   // blocks are handed out one at a time: the last, short one does not unbalance anyone
-            for (std::uint64_t b = next.fetch_add(1); b < n_blocks && !failed.load(); b = next.fetch_add(1)) {
-                const uLong in_size = static_cast<uLong>(b + 1 == n_blocks ? last : block);
-                uLongf out_size = compressBound(in_size);
-                packed[b].resize(out_size);
-                if (compress2(packed[b].data(), &out_size, src + b * block, in_size, Z_BEST_SPEED) != Z_OK) {
-                    failed.store(true);
-                    return;
-                }
-                packed[b].resize(out_size);
-                header[3 + b] = out_size;
-            }
-        };
-        const unsigned n_threads = compressor_threads(n_blocks);
-        if (n_threads <= 1) {
-            deflate_blocks();
-        } else {
-            std::vector<std::thread> pool;
-            for (unsigned t = 1; t < n_threads; t++) pool.emplace_back(deflate_blocks);
-            deflate_blocks();
-            for (auto& t : pool) t.join();
-        }
-        if (failed.load()) throw std::runtime_error("zlib failed while writing " + filename);
-        if (!b64) {
-            std::fwrite(header.data(), sizeof(std::uint64_t), header.size(), fp);
-            for (const auto& p : packed) std::fwrite(p.data(), 1, p.size(), fp);
-        } else {
-            // vtkXMLWriter's default (EncodeAppendedData on): the block table is one base64 stream, the
-            // concatenated compressed blocks another
-            const std::string h = base64(reinterpret_cast<const unsigned char*>(header.data()), header.size() * sizeof(std::uint64_t));
-            std::fwrite(h.data(), 1, h.size(), fp);
-            std::vector<unsigned char> all;
-            for (const auto& p : packed) all.insert(all.end(), p.begin(), p.end());
-            const std::string d = base64(all.data(), all.size());
-            std::fwrite(d.data(), 1, d.size(), fp);
-        }
     }
     std::fprintf(fp, "\n  </AppendedData>\n</VTKFile>\n");
 }
 
 void read_vti(const std::string& filename, std::size_t& res_x, std::size_t& res_y, std::size_t& comps,
-              double*& image_out) {
+              double*& image_out, const std::string& name) {
     std::ifstream in(filename, std::ios::binary);
     if (!in) throw std::runtime_error("cannot open " + filename);
     std::stringstream ss;
@@ -217,12 +235,29 @@ void read_vti(const std::string& filename, std::size_t& res_x, std::size_t& res_
     }
     res_x = static_cast<std::size_t>(x1 - x0 + 1);
     res_y = static_cast<std::size_t>(y1 - y0 + 1);
-    comps = static_cast<std::size_t>(std::stoul(attr("DataArray", "NumberOfComponents")));
+    // the array: its element (by name, or the first one) and where its data starts in the appended section
+    std::size_t array_at = all.find("<DataArray");
+    if (!name.empty()) {
+        const std::size_t named = all.find("Name=\"" + name + "\"");
+        if (named == std::string::npos) throw std::runtime_error(filename + ": no array named '" + name + "'");
+        array_at = all.rfind("<DataArray", named);
+    }
+    if (array_at == std::string::npos) throw std::runtime_error(filename + ": no <DataArray>");
+    auto array_attr = [&](const std::string& key) -> std::string {
+        const std::size_t e = all.find('>', array_at);
+        const std::size_t a = all.find(" " + key + "=\"", array_at);
+        if (a == std::string::npos || a > e) return "";
+        const std::size_t s = a + key.size() + 3;
+        return all.substr(s, all.find('"', s) - s);
+    };
+    comps = static_cast<std::size_t>(std::stoul(array_attr("NumberOfComponents")));
+    const std::string off = array_attr("offset");
+    const std::size_t array_offset = off.empty() ? 0 : static_cast<std::size_t>(std::stoull(off));
     const bool compressed = !attr("VTKFile", "compressor").empty();
     const bool b64 = attr("AppendedData", "encoding") == "base64";
     const std::size_t marker = all.find("<AppendedData");
     const std::size_t under = all.find('_', all.find('>', marker));
-    const unsigned char* p = reinterpret_cast<const unsigned char*>(all.data()) + under + 1;
+    const unsigned char* p = reinterpret_cast<const unsigned char*>(all.data()) + under + 1 + array_offset;
     const unsigned char* file_end = reinterpret_cast<const unsigned char*>(all.data()) + all.size();
     const std::size_t n_values = res_x * res_y * comps;
     std::vector<unsigned char> decoded; // base64: the appended section turned back into the raw layout

@@ -37,6 +37,12 @@ def lib() -> C.CDLL:
         l.c5host_read_vti.restype = C.c_longlong
         l.c5host_read_vti.argtypes = [C.c_char_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong),
                                       C.POINTER(C.c_longlong), _dp]
+        l.c5host_write_vti_arrays.restype = C.c_longlong
+        l.c5host_write_vti_arrays.argtypes = [C.c_char_p, _dp, C.c_longlong, C.c_longlong, C.c_int, C.c_int,
+                                              C.POINTER(C.c_char_p), C.POINTER(_dp)]
+        l.c5host_read_vti_array.restype = C.c_longlong
+        l.c5host_read_vti_array.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong),
+                                            C.POINTER(C.c_longlong), _dp]
         l.c5host_parse_cli.restype = C.c_int
         l.c5host_parse_cli.argtypes = [C.c_int, C.POINTER(C.c_char_p), C.c_char_p, C.c_int, _dp, C.c_char_p,
                                        C.c_char_p, C.c_int]
@@ -76,24 +82,36 @@ def read_vtk(path: str, alpha_name="AbsorpCoef", q_name="radEnLooseRate"):
     return pts, tets, alpha, q
 
 
-def write_vti(path: str, image: np.ndarray, compress=False, base64=False):
+def write_vti(path: str, image: np.ndarray, compress=False, base64=False, extra: dict | None = None):
     """compress: vtkZLibDataCompressor blocks; base64 (with compress): the appended section as base64
-    streams — together what vtkXMLImageDataWriter writes by default."""
+    streams — together what vtkXMLImageDataWriter writes by default. extra: {name: (res_y, res_x, 2)
+    array} written as further PointData arrays beside ImageScalars."""
     image = np.ascontiguousarray(image, dtype=np.float64)
     res_y, res_x, comps = image.shape
     assert comps == 2
     mode = 2 if (compress and base64) else 1 if compress else 0
-    if lib().c5host_write_vti(path.encode(), image.ctypes.data_as(_dp), res_x, res_y, mode) < 0:
+    if not extra:
+        rc = lib().c5host_write_vti(path.encode(), image.ctypes.data_as(_dp), res_x, res_y, mode)
+    else:
+        arrays = [np.ascontiguousarray(a, dtype=np.float64) for a in extra.values()]
+        assert all(a.shape == image.shape for a in arrays)
+        names = (C.c_char_p * len(arrays))(*[n.encode() for n in extra])
+        data = (_dp * len(arrays))(*[a.ctypes.data_as(_dp) for a in arrays])
+        rc = lib().c5host_write_vti_arrays(path.encode(), image.ctypes.data_as(_dp), res_x, res_y, mode, len(arrays),
+                                           names, data)
+    if rc < 0:
         raise RuntimeError(_err())
 
 
-def read_vti(path: str) -> np.ndarray:
+def read_vti(path: str, name: str | None = None) -> np.ndarray:
+    """The PointData array `name` (default: the first, ImageScalars) as (res_y, res_x, components)."""
     x, y, c = C.c_longlong(), C.c_longlong(), C.c_longlong()
-    n = lib().c5host_read_vti(path.encode(), C.byref(x), C.byref(y), C.byref(c), None)
+    nm = name.encode() if name else None
+    n = lib().c5host_read_vti_array(path.encode(), nm, C.byref(x), C.byref(y), C.byref(c), None)
     if n < 0:
         raise RuntimeError(_err())
     out = np.zeros((y.value, x.value, c.value))
-    lib().c5host_read_vti(path.encode(), C.byref(x), C.byref(y), C.byref(c), out.ctypes.data_as(_dp))
+    lib().c5host_read_vti_array(path.encode(), nm, C.byref(x), C.byref(y), C.byref(c), out.ctypes.data_as(_dp))
     return out
 
 

@@ -25,9 +25,10 @@
 extern "C" {
 #endif
 
-#define C5_ABI_VERSION 2
+#define C5_ABI_VERSION 3
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
+#define C5_MAX_CHANNELS 8
 
 typedef struct c5_ctx c5_ctx;
 
@@ -154,6 +155,27 @@ int c5_set_views_in_flight(c5_ctx* ctx, int32_t n);
  * the doubles are the pre-cast values the parity gate is defined on. */
 int c5_render_raw(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* steps, uint8_t* solid_mask,
                   c5_stats* stats);
+
+/* ---- several field pairs from one view ------------------------------------------------------------
+ * c5_upload_channels replaces the context's channels: n_channels (0 .. C5_MAX_CHANNELS) pairs of cell
+ * fields, alpha and q each n_channels * n_tets doubles, channel-major (alpha[c * n_tets + k] for tet k
+ * in the order given to c5_upload_mesh). n_channels = 0 removes them. Needs a mesh (C5_E_STATE
+ * otherwise); goes through the parent like every upload (C5_E_STATE on a sibling) and reaches the
+ * parts of a multi-device context; siblings and lanes see it at their next render. C5_E_STATE while
+ * the context or one of its lanes has a submitted view. No topology or BVH is rebuilt;
+ * c5_upload_mesh drops the channels. While channels are uploaded, c5_mesh_info.device_bytes
+ * includes them.
+ *
+ * c5_render_channels is c5_render_raw over the uploaded channels, in ONE walk: out holds
+ * res_y * res_x * n * 2 doubles, x fastest, {tau_0, I_0, ..., tau_{n-1}, I_{n-1}} per pixel (a row
+ * band writes only its rows). Channel c is the image c5_render_raw gives for a mesh uploaded with
+ * (alpha_c, q_c): the same rays, hit set, solid mask and steps. steps, solid_mask and stats mean what
+ * they mean for c5_render_raw (counts are the geometry's, not multiplied by n); steps and solid_mask
+ * may be NULL. A page-locked, 16-byte aligned `out` is written in place. FP64 only: precision 32 is
+ * C5_E_INVALID; no channels uploaded is C5_E_STATE. Single- and multi-device contexts and siblings. */
+int c5_upload_channels(c5_ctx* ctx, const double* alpha, const double* q, int32_t n_channels);
+int c5_render_channels(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* steps, uint8_t* solid_mask,
+                       c5_stats* stats);
 
 /* Device-resident variant for callers that own device memory (e.g. a torch tensor that an NCCL
  * gather will read): d_out is a DEVICE pointer on the context's first device to
