@@ -665,22 +665,24 @@ bvh_refit(int64_t n_leaves, const BFace* __restrict__ faces, const Vtx* __restri
 
 namespace {
 
-C5_HD void prepare_cell_body(int64_t t, Cell* cells, const double* q0, double limit) {
-    double a = cells[t].alpha;
-    if (a > limit) a = limit;                 // line.cpp:216-218
+// Source function s = Q / min(alpha, limit) of one cell or channel, Q read from q[k]. Channel renders
+// are bitwise equal to plain renders because cells and channels both get s from here.
+C5_HD double source_fn(double alpha, const double* q, int64_t k, double limit) {
+    if (alpha > limit) alpha = limit;         // line.cpp:216-218
     // alpha^ < DBL_EPSILON leaves I unchanged (line.cpp:221); the walk tests alpha itself, s is unused
-    cells[t].s = (a < DBL_EPSILON) ? 0.0 : q0[t] / a;
+    return (alpha < DBL_EPSILON) ? 0.0 : q[k] / alpha;
 }
 
-// The same arithmetic for channel c of tet t (k = t * n + c): s_c from ch_q0[c][t] and the alpha_c
-// beside it in the record.
+C5_HD void prepare_cell_body(int64_t t, Cell* cells, const double* q0, double limit) {
+    cells[t].s = source_fn(cells[t].alpha, q0, t, limit);
+}
+
+// Channel c of tet t (k = t * n + c): s_c from ch_q0[c][t] and the alpha_c beside it in the record.
 C5_HD void prepare_channel_body(int64_t k, double* rec, const double* q0, int64_t n_tets, int n, double limit) {
     const int64_t t = k / n;
     const int c = static_cast<int>(k - t * n);
     double* r = rec + t * channel_stride(n) + 2 * c;
-    double a = r[0];
-    if (a > limit) a = limit;
-    r[1] = (a < DBL_EPSILON) ? 0.0 : q0[c * n_tets + t] / a;
+    r[1] = source_fn(r[0], q0 + c * n_tets, t, limit);
 }
 
 } // namespace
@@ -904,11 +906,20 @@ void launch_solid_mask(DeviceState& d, int res_x, int res_y, double x_min, doubl
     mask_passes(d, d.solid_follow, g, tg);
 }
 
-void launch_prepare_cells(DeviceState& dd, double alpha_limit) {
-    // cells[].s belongs to the context that owns the mesh; its siblings read the same array, possibly
-    // on other streams right now, so a change of --alpha_limit (rare) is fenced by device-wide syncs
-    DeviceState& d = dd.origin ? *dd.origin : dd;
-    if (d.cells_limit_valid && d.cells_limit == alpha_limit) return;
+namespace {
+
+DeviceState& mesh_owner(DeviceState& dd) {
+    return dd.origin ? *dd.origin : dd;
+}
+
+// Runs `prepare` on the context that owns the mesh unless its `limit` already holds alpha_limit.
+// What it writes belongs to that owner; its siblings read the same array, possibly on other streams
+// right now, so a change of --alpha_limit (rare) is fenced by device-wide syncs.
+template <class Prepare>
+void prepare_for_limit(DeviceState& dd, double alpha_limit, double DeviceState::*limit, bool DeviceState::*valid,
+                       Prepare prepare) {
+    DeviceState& d = mesh_owner(dd);
+    if (d.*valid && d.*limit == alpha_limit) return;
     const bool shared = dd.origin != nullptr || d.mesh_shared;
     if (shared && !kHostSim) C5_CUDA(cudaDeviceSynchronize());
     struct SyncAfter {
@@ -918,38 +929,36 @@ void launch_prepare_cells(DeviceState& dd, double alpha_limit) {
         }
     } sync_after{shared && !kHostSim};
     count_launch();
-    if (kHostSim) {
-        for (int64_t t = 0; t < d.n_tets; t++) prepare_cell_body(t, d.cells.p, d.q0.p, alpha_limit);
-    } else {
-        prepare_cells<<<grid_for(d.n_tets, 256), 256, 0, dd.stream>>>(d.n_tets, d.cells.p, d.q0.p, alpha_limit);
-        C5_CUDA(cudaGetLastError());
-    }
-    d.cells_limit = alpha_limit;
-    d.cells_limit_valid = true;
+    prepare(d);
+    d.*limit = alpha_limit;
+    d.*valid = true;
+}
+
+} // namespace
+
+void launch_prepare_cells(DeviceState& dd, double alpha_limit) {
+    prepare_for_limit(dd, alpha_limit, &DeviceState::cells_limit, &DeviceState::cells_limit_valid, [&](DeviceState& d) {
+        if (kHostSim) {
+            for (int64_t t = 0; t < d.n_tets; t++) prepare_cell_body(t, d.cells.p, d.q0.p, alpha_limit);
+        } else {
+            prepare_cells<<<grid_for(d.n_tets, 256), 256, 0, dd.stream>>>(d.n_tets, d.cells.p, d.q0.p, alpha_limit);
+            C5_CUDA(cudaGetLastError());
+        }
+    });
 }
 
 void launch_prepare_channels(DeviceState& dd, double alpha_limit) {
-    // fenced like launch_prepare_cells: siblings read the owner's records
-    DeviceState& d = dd.origin ? *dd.origin : dd;
-    if (d.n_channels == 0 || (d.ch_limit_valid && d.ch_limit == alpha_limit)) return;
-    const bool shared = dd.origin != nullptr || d.mesh_shared;
-    if (shared && !kHostSim) C5_CUDA(cudaDeviceSynchronize());
-    struct SyncAfter {
-        bool on;
-        ~SyncAfter() {
-            if (on) cudaDeviceSynchronize();
+    if (mesh_owner(dd).n_channels == 0) return;
+    prepare_for_limit(dd, alpha_limit, &DeviceState::ch_limit, &DeviceState::ch_limit_valid, [&](DeviceState& d) {
+        const int64_t n = d.n_tets * d.n_channels;
+        if (kHostSim) {
+            for (int64_t k = 0; k < n; k++) prepare_channel_body(k, d.ch_rec.p, d.ch_q0.p, d.n_tets, d.n_channels, alpha_limit);
+        } else {
+            prepare_channels<<<grid_for(n, 256), 256, 0, dd.stream>>>(d.n_tets, d.n_channels, d.ch_rec.p, d.ch_q0.p,
+                                                                      alpha_limit);
+            C5_CUDA(cudaGetLastError());
         }
-    } sync_after{shared && !kHostSim};
-    const int64_t n = d.n_tets * d.n_channels;
-    count_launch();
-    if (kHostSim) {
-        for (int64_t k = 0; k < n; k++) prepare_channel_body(k, d.ch_rec.p, d.ch_q0.p, d.n_tets, d.n_channels, alpha_limit);
-    } else {
-        prepare_channels<<<grid_for(n, 256), 256, 0, dd.stream>>>(d.n_tets, d.n_channels, d.ch_rec.p, d.ch_q0.p, alpha_limit);
-        C5_CUDA(cudaGetLastError());
-    }
-    d.ch_limit = alpha_limit;
-    d.ch_limit_valid = true;
+    });
 }
 
 void dedupe_solid_faces(DeviceState& d, SolidSet& ss) {

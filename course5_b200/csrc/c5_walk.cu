@@ -15,9 +15,11 @@
 // with cavities or a bumpy silhouette are crossed several times). Rays with many crossings, or
 // whose searches are expensive, are deferred to grazing_rays_* (one warp per ray, further down).
 //
-// File map: loads -> entry search (one thread) -> one crossing (FP64, FP32) -> one ray, in
-// warp-synchronised phases (trace_ray) -> grazing rays: composition, serial form, warp-cooperative
-// collection / sort / walk -> kernels (walk_block, fill_background, graze_block) -> launch_walk.
+// File map: loads -> entry search (one thread) -> one crossing (FP64 over cell fields or channels,
+// FP32) -> field policies -> one ray, in warp-synchronised phases (trace_ray) -> grazing rays:
+// composition, serial form, warp-cooperative collection / sort / walk -> kernels (walk_block,
+// fill_background, graze_block) -> host loops -> launch_walk. Everything from trace_ray on is one
+// body over a field policy: FP64 cell fields, FP32 cell fields or K uploaded channels.
 //
 // Geometry of one step. All rays are parallel to z, so "which face does the ray leave through"
 // is a 2-D question about the projected tet. The entry face (a,b,c) is kept counter-clockwise in
@@ -33,6 +35,8 @@
 // Per step the thread reads one 64-byte Cell and ONE new 32-byte vertex; the other three
 // vertices and their ids stay in registers (the 72 B/step algorithmic figure of SURVEY.md §8d).
 #include "c5_internal.h"
+
+#include <utility>
 
 namespace c5 {
 
@@ -64,6 +68,9 @@ struct WalkParams {
     int max_steps;
     int round_float;
     double alpha_limit;
+    // channel renders only (null otherwise)
+    const double* rec;    // [n_tets][channel_stride(K)]: {alpha_c, s_c} per channel
+    double* ch_queue;     // [deferred ray][K] {tau, I}: the channel values DeferredRay::tau/inten hold otherwise
 };
 
 // ---- loads through the read-only path ----------------------------------------------------------
@@ -270,8 +277,8 @@ C5_HD bool bvh_collect_entries(const WalkParams& P, double px, double py, double
 // affine in I: s - (s - I) e = s (1 - e) + e I).
 //
 // `acc` integrates the fields along the crossing: fetch(t) is issued with tet t's cell load and
-// step(c, dz) adds one segment. CellFields below integrates the cells' own alpha and s; the
-// channel walk (further down) integrates several field pairs over the same steps.
+// step(c, dz) adds one segment. CellFields below integrates the cells' own alpha and s; ChanFields
+// integrates K uploaded field pairs over the same steps.
 template <bool kAffine, class Acc>
 C5_HD double crossing_walk(const WalkParams& P, double px, double py, int leaf, double z_in, Acc& acc,
                            uint32_t& steps, uint32_t& error) {
@@ -367,23 +374,70 @@ C5_HD void segment(double alpha, double s, double limit, double dzv, double& tau
     }
 }
 
-template <bool kAffine>
-struct CellFields {
-    double& tau;
-    double& inten;
-    double& gain;
-    C5_HD void fetch(int) {}
-    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
-        segment<kAffine>(c.alpha, c.s, P.alpha_limit, dzv, tau, inten, gain);
+// K {tau, I} pairs, of one ray or of one crossing. A crossing walked without the I it arrives with
+// (kAffine) also yields gain[c], the factor it puts on that I; elsewhere gain stays 1 and is not read.
+// Loops over K are unrolled with fixed bounds, so the arrays live in registers.
+// The pixel kernel's pairs are value-initialised and stored by fold expressions over c = 0 .. K-1 of
+// force-inlined calls. A loop, even of one trip, is unrolled only after the compiler's early passes,
+// which then see the arrays in memory: the FP64 pixel kernel came out slower that way (C3 on one
+// B200: 4.416 against 4.401 ms per view).
+template <int K, int... C>
+C5_HD void fill_pairs(double (&a)[K], double v, std::integer_sequence<int, C...>) {
+    ((a[C] = v), ...);
+}
+
+template <int K>
+struct Pairs {
+    double tau[K], inten[K], gain[K];
+    C5_HD void reset() {
+#pragma unroll
+        for (int c = 0; c < K; c++) {
+            tau[c] = 0.0;
+            inten[c] = 0.0;
+            gain[c] = 1.0;
+        }
     }
 };
 
 template <bool kAffine>
-C5_HD double crossing_f64(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau,
-                          double& inten, double& gain, uint32_t& steps, uint32_t& error) {
-    CellFields<kAffine> acc{tau, inten, gain};
-    return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
-}
+struct CellFields {
+    Pairs<1>& v;
+    C5_HD void fetch(int) {}
+    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
+        segment<kAffine>(c.alpha, c.s, P.alpha_limit, dzv, v.tau[0], v.inten[0], v.gain[0]);
+    }
+};
+
+// K uploaded field pairs. A step reads tet t's record of K {alpha_c, s_c} pairs (padded to 32-byte
+// sectors) together with t's cell, since t is known at the top of the step, so a channel adds FP64
+// work and a store but no further round trip.
+template <int K, bool kAffine>
+struct ChanFields {
+    const double* rec;
+    Pairs<K>& v;
+    double f[channel_stride(K)]; // the record of the tet being crossed
+
+    // f stays uninitialised: fetch fills it before every step (zeroing it costs the K = 3 grazing-ray
+    // kernel 24 more bytes of spills)
+    C5_HD ChanFields(const double* rec_, Pairs<K>& v_) : rec(rec_), v(v_) {}
+    C5_HD void fetch(int t) {
+        const double* p = rec + static_cast<size_t>(t) * channel_stride(K);
+#ifdef __CUDA_ARCH__
+#pragma unroll
+        for (int k = 0; k < channel_stride(K); k += 4) {
+            asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];"
+                         : "=d"(f[k]), "=d"(f[k + 1]), "=d"(f[k + 2]), "=d"(f[k + 3])
+                         : "l"(p + k));
+        }
+#else
+        for (int k = 0; k < channel_stride(K); k++) f[k] = p[k];
+#endif
+    }
+    C5_HD void step(const WalkParams& P, const CellData&, double dzv) {
+#pragma unroll
+        for (int c = 0; c < K; c++) segment<kAffine>(f[2 * c], f[2 * c + 1], P.alpha_limit, dzv, v.tau[c], v.inten[c], v.gain[c]);
+    }
+};
 
 // ---- FP32 variant -----------------------------------------------------------------------------------
 // Same crossing with the per-step geometry in single precision: FP32 orientation tests (still exactly
@@ -500,17 +554,61 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
     return z_exit_abs > z0 ? z_exit_abs : z0;
 }
 
-template <bool kF32, bool kAffine>
-C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, double& tau, double& inten,
-                      double& gain, uint32_t& steps, uint32_t& error) {
-    return kF32 ? crossing_f32<kAffine>(P, px, py, leaf, z_in, tau, inten, gain, steps, error)
-                : crossing_f64<kAffine>(P, px, py, leaf, z_in, tau, inten, gain, steps, error);
+// ---- field policies ----------------------------------------------------------------------------------
+// What a ray integrates. Everything from trace_ray on is written once over a policy F:
+//   F::K                   {tau, I} pairs per pixel, stored at out[((j - row_begin) * res_x + i) * K + c];
+//   F::crossing<kAffine>   the crossing that integrates them into a Pairs<K>;
+//   F::kChanQueue          a deferred ray's values wait in WalkParams::ch_queue and DeferredRay::tau/inten
+//                          stay 0; otherwise they wait in DeferredRay::tau/inten.
+struct CellsF64 { // the cells' own fields
+    static constexpr int K = 1;
+    static constexpr bool kChanQueue = false;
+    template <bool kAffine>
+    static C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<1>& v,
+                                 uint32_t& steps, uint32_t& error) {
+        CellFields<kAffine> acc{v};
+        return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
+    }
+};
+
+struct CellsF32 { // the cells' own fields, FP32 step geometry
+    static constexpr int K = 1;
+    static constexpr bool kChanQueue = false;
+    template <bool kAffine>
+    static C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<1>& v,
+                                 uint32_t& steps, uint32_t& error) {
+        return crossing_f32<kAffine>(P, px, py, leaf, z_in, v.tau[0], v.inten[0], v.gain[0], steps, error);
+    }
+};
+
+// Several field pairs in one walk (c5_render_channels): the rays, their entry searches, deferrals and
+// steps are those of CellsF64; only what is integrated differs.
+template <int N>
+struct Channels {
+    static constexpr int K = N;
+    static constexpr bool kChanQueue = true;
+    template <bool kAffine>
+    static C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<K>& v,
+                                 uint32_t& steps, uint32_t& error) {
+        ChanFields<K, kAffine> acc{P.rec, v};
+        return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
+    }
+};
+
+C5_HD void store2(double* p, double a, double b) {
+#ifdef __CUDA_ARCH__
+    *reinterpret_cast<double2*>(p) = make_double2(a, b);
+#else
+    p[0] = a;
+    p[1] = b;
+#endif
 }
 
 // ---- one ray (pixel kernel) ------------------------------------------------------------------------
 
+template <int K>
 struct RayResult {
-    double tau, inten;
+    Pairs<K> v;
     uint32_t steps;
     uint32_t error;
     uint32_t deferred; // handed to the grazing-ray kernel: the pixel is stored there
@@ -536,16 +634,10 @@ C5_HD void sync_lanes(unsigned lanes) {
 #endif
 }
 
-template <bool kF32>
-C5_HD RayResult trace_ray(const WalkParams& P, double px, double py, uint32_t pixel, unsigned tracing) {
-    RayResult r;
-    r.tau = 0.0;
-    r.inten = 0.0;
-    r.steps = 0;
-    r.error = 0;
-    r.deferred = 0;
+template <class F>
+C5_HD RayResult<F::K> trace_ray(const WalkParams& P, double px, double py, uint32_t pixel, unsigned tracing) {
+    RayResult<F::K> r{};
     double z_after = -INFINITY;
-    double gain_unused = 1.0;
     EntryList<kInline> L;
 
     // A: nearest entry
@@ -554,7 +646,7 @@ C5_HD RayResult trace_ray(const WalkParams& P, double px, double py, uint32_t pi
     // B: first crossing
     const bool entered = !defer && L.n > 0;
     if (entered) {
-        z_after = crossing<kF32, false>(P, px, py, L.leaf[0], L.z[0], r.tau, r.inten, gain_unused, r.steps, r.error);
+        z_after = F::template crossing<false>(P, px, py, L.leaf[0], L.z[0], r.v, r.steps, r.error);
     }
     sync_lanes(tracing);
     // C: anything above the exit?
@@ -569,7 +661,7 @@ C5_HD RayResult trace_ray(const WalkParams& P, double px, double py, uint32_t pi
         // an entry at or below the ray's position is already behind it (two boundary faces sharing
         // the edge the ray passes through report the same depth)
         if (!defer && e < L.n && L.z[e] > z_after && !r.error) {
-            z_after = crossing<kF32, false>(P, px, py, L.leaf[e], L.z[e], r.tau, r.inten, gain_unused, r.steps, r.error);
+            z_after = F::template crossing<false>(P, px, py, L.leaf[e], L.z[e], r.v, r.steps, r.error);
         }
         sync_lanes(tracing);
     }
@@ -581,11 +673,15 @@ C5_HD RayResult trace_ray(const WalkParams& P, double px, double py, uint32_t pi
 #endif
         // read by the grazing-ray kernel, which is launched after this one on the same stream
         DeferredRay& q = P.queue[slot];
-        q.tau = r.tau;
-        q.inten = r.inten;
+        q.tau = F::kChanQueue ? 0.0 : r.v.tau[0];
+        q.inten = F::kChanQueue ? 0.0 : r.v.inten[0];
         q.z_after = z_after;
         q.pixel = pixel;
         q.steps = r.steps;
+        if (F::kChanQueue) {
+#pragma unroll
+            for (int c = 0; c < F::K; c++) store2(P.ch_queue + 2 * (slot * F::K + c), r.v.tau[c], r.v.inten[c]);
+        }
         r.deferred = 1;
     }
     return r;
@@ -599,17 +695,44 @@ C5_HD RayResult trace_ray(const WalkParams& P, double px, double py, uint32_t pi
 // frontier. So one WARP takes one ray: the lanes expand 32 BVH nodes per round from a shared stack,
 // rank-sort the entries found, walk 32 crossings at a time and fold the results in order.
 
+template <int K>
 struct RayAcc {
-    double tau, inten, z_after;
+    Pairs<K> v; // gain unused
+    double z_after;
     uint32_t steps, error;
 };
 
+// A deferred ray as trace_ray left it.
+template <class F>
+C5_HD RayAcc<F::K> load_deferred(const WalkParams& P, unsigned long long slot) {
+    const DeferredRay& q = P.queue[slot];
+    RayAcc<F::K> a;
+    if (F::kChanQueue) {
+#pragma unroll
+        for (int c = 0; c < F::K; c++) {
+            a.v.tau[c] = P.ch_queue[2 * (slot * F::K + c)];
+            a.v.inten[c] = P.ch_queue[2 * (slot * F::K + c) + 1];
+        }
+    } else {
+        a.v.tau[0] = q.tau;
+        a.v.inten[0] = q.inten;
+    }
+    a.z_after = q.z_after;
+    a.steps = q.steps;
+    a.error = 0;
+    return a;
+}
+
 // Folds crossing (z_in -> z_out) into the ray unless the ray is already past its entry.
-C5_HD void compose_crossing(RayAcc& a, double z_in, double z_out, double tau_k, double inten_k, double gain_k,
-                            uint32_t steps_k, uint32_t error_k) {
+template <int K>
+C5_HD void compose_crossing(RayAcc<K>& a, double z_in, double z_out, const Pairs<K>& k, uint32_t steps_k,
+                            uint32_t error_k) {
     if (!(z_in > a.z_after)) return;
-    a.tau += tau_k;
-    a.inten = inten_k + gain_k * a.inten;
+#pragma unroll
+    for (int c = 0; c < K; c++) {
+        a.v.tau[c] += k.tau[c];
+        a.v.inten[c] = k.inten[c] + k.gain[c] * a.v.inten[c];
+    }
     a.steps += steps_k;
     a.error |= error_k;
     a.z_after = z_out;
@@ -617,24 +740,20 @@ C5_HD void compose_crossing(RayAcc& a, double z_in, double z_out, double tau_k, 
 
 // Serial form (one thread does everything): the host-loop build, and the reference the warp
 // version is tested against. Same crossing function, same composition.
-template <bool kF32>
-C5_HD RayAcc graze_ray_serial(const WalkParams& P, const DeferredRay& q, double px, double py) {
-    RayAcc a;
-    a.tau = q.tau;
-    a.inten = q.inten;
-    a.z_after = q.z_after;
-    a.steps = q.steps;
-    a.error = 0;
+template <class F>
+C5_HD RayAcc<F::K> graze_ray_serial(const WalkParams& P, unsigned long long slot, double px, double py) {
+    RayAcc<F::K> a = load_deferred<F>(P, slot);
     EntryList<kSerialList> L;
     int crossings = 0;
     while (!a.error) {
         if (!bvh_collect_entries(P, px, py, a.z_after, L, P.serial_cap, 0x7FFFFFFF)) a.error = 1; // stack overflow
         for (int e = 0; e < L.n; e++) {
             if (!(L.z[e] > a.z_after)) continue;
-            double tau_k = 0.0, inten_k = 0.0, gain_k = 1.0;
+            Pairs<F::K> k;
+            k.reset();
             uint32_t steps_k = 0, error_k = 0;
-            const double z_out = crossing<kF32, true>(P, px, py, L.leaf[e], L.z[e], tau_k, inten_k, gain_k, steps_k, error_k);
-            compose_crossing(a, L.z[e], z_out, tau_k, inten_k, gain_k, steps_k, error_k);
+            const double z_out = F::template crossing<true>(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
+            compose_crossing(a, L.z[e], z_out, k, steps_k, error_k);
             if (++crossings > 65536) a.error = 1;
         }
         if (L.n < P.serial_cap) break;
@@ -652,26 +771,36 @@ C5_HD double __longlong_as_double_hd(long long bits) {
 #endif
 }
 
-C5_HD void store_pixel(const WalkParams& P, int i, int j, double tau, double inten, uint32_t steps) {
-    const size_t o = static_cast<size_t>(j - P.row_begin) * P.res_x + i;
+// Pair k of the band buffer.
+C5_HD void store_pair(const WalkParams& P, size_t k, double t, double v) {
     if (P.round_float) { // plane.cpp:165-166 then object2d.cpp:19-20
-        tau = static_cast<double>(static_cast<float>(tau));
-        inten = static_cast<double>(static_cast<float>(inten));
+        t = static_cast<double>(static_cast<float>(t));
+        v = static_cast<double>(static_cast<float>(v));
     }
-#ifdef __CUDA_ARCH__
-    reinterpret_cast<double2*>(P.out)[o] = make_double2(tau, inten);
-#else
-    P.out[2 * o] = tau;
-    P.out[2 * o + 1] = inten;
-#endif
+    store2(P.out + 2 * k, t, v);
+}
+
+template <int K, int... C>
+C5_HD void store_pairs(const WalkParams& P, size_t o, const double (&tau)[K], const double (&inten)[K],
+                       std::integer_sequence<int, C...>) {
+    (store_pair(P, o * K + C, tau[C], inten[C]), ...);
+}
+
+template <int K>
+C5_HD void store_pixel(const WalkParams& P, int i, int j, const double (&tau)[K], const double (&inten)[K],
+                       uint32_t steps) {
+    const size_t o = static_cast<size_t>(j - P.row_begin) * P.res_x + i;
+    store_pairs(P, o, tau, inten, std::make_integer_sequence<int, K>{});
     if (P.steps) P.steps[o] = steps;
 }
 
-// Pixels of the band outside the rectangle the walk covers: background (or solid).
-C5_HD bool background_pixel(const WalkParams& P, int i, int j) {
+// Pixels of the band outside the rectangle the walk covers: background (or solid), n pairs wide.
+C5_HD bool background_pixel(const WalkParams& P, int n, int i, int j) {
     const bool solid = P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i];
     const double v = solid ? __longlong_as_double_hd(0x7FF8000000000000ll) : 0.0; // quiet NaN (config.hpp:26-27)
-    store_pixel(P, i, j, v, v, 0);
+    const size_t o = static_cast<size_t>(j - P.row_begin) * P.res_x + i;
+    for (int c = 0; c < n; c++) store2(P.out + 2 * (o * n + c), v, v);
+    if (P.steps) P.steps[o] = 0;
     return solid;
 }
 
@@ -790,7 +919,7 @@ __device__ __forceinline__ int graze_collect(const WalkParams& P, GrazeSmem& S, 
     return n;
 }
 
-template <bool kF32>
+template <class F>
 __device__ __forceinline__ void graze_block(const WalkParams& P) {
     __shared__ GrazeSmem smem[kGrazeWarps];
     const unsigned full = 0xFFFFFFFFu;
@@ -805,18 +934,12 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
         if (lane == 0) ticket = atomicAdd(&P.counters[kTicket], 1ull);
         ticket = __shfl_sync(full, ticket, 0);
         if (ticket >= n_rays) break;
-        const DeferredRay* qp = P.queue + ticket;
-        const uint32_t q_steps = qp->steps;
-        const uint32_t q_pixel = qp->pixel;
+        const uint32_t q_pixel = P.queue[ticket].pixel;
         const int i = static_cast<int>(q_pixel % static_cast<uint32_t>(P.res_x));
         const int j = static_cast<int>(q_pixel / static_cast<uint32_t>(P.res_x));
         const double px = P.xs[i], py = P.ys[j];
-        RayAcc a;
-        a.tau = qp->tau;
-        a.inten = qp->inten;
-        a.z_after = qp->z_after;
-        a.steps = q_steps;
-        a.error = 0;
+        RayAcc<F::K> a = load_deferred<F>(P, ticket);
+        const uint32_t q_steps = a.steps;
         int crossings = 0;
         bool truncated = true;
         while (truncated && !a.error) {
@@ -825,17 +948,24 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
                 const int k = base + lane;
                 const bool have = k < n;
                 const double z_in = have ? S.z[k] : INFINITY;
-                double z_out = z_in, tau_k = 0.0, inten_k = 0.0, gain_k = 1.0;
+                double z_out = z_in;
+                Pairs<F::K> f;
+                f.reset();
                 uint32_t steps_k = 0, error_k = 0;
                 if (have && z_in > a.z_after) { // a is the same in every lane
-                    z_out = crossing<kF32, true>(P, px, py, S.leaf[k], z_in, tau_k, inten_k, gain_k, steps_k, error_k);
+                    z_out = F::template crossing<true>(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
                 }
                 const int cnt = n - base < 32 ? n - base : 32;
                 for (int l = 0; l < cnt; l++) {
-                    compose_crossing(a, __shfl_sync(full, z_in, l), __shfl_sync(full, z_out, l),
-                                     __shfl_sync(full, tau_k, l), __shfl_sync(full, inten_k, l),
-                                     __shfl_sync(full, gain_k, l), __shfl_sync(full, steps_k, l),
-                                     __shfl_sync(full, error_k, l));
+                    Pairs<F::K> g;
+#pragma unroll
+                    for (int c = 0; c < F::K; c++) {
+                        g.tau[c] = __shfl_sync(full, f.tau[c], l);
+                        g.inten[c] = __shfl_sync(full, f.inten[c], l);
+                        g.gain[c] = __shfl_sync(full, f.gain[c], l);
+                    }
+                    compose_crossing(a, __shfl_sync(full, z_in, l), __shfl_sync(full, z_out, l), g,
+                                     __shfl_sync(full, steps_k, l), __shfl_sync(full, error_k, l));
                 }
             }
             crossings += n;
@@ -843,7 +973,7 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
             __syncwarp();
         }
         if (lane == 0) {
-            store_pixel(P, i, j, a.tau, a.inten, a.steps);
+            store_pixel(P, i, j, a.v.tau, a.v.inten, a.steps);
             const unsigned long long more = a.steps - q_steps;
             if (more) {
                 atomicAdd(&P.counters[kSteps], more);
@@ -862,7 +992,7 @@ __device__ __forceinline__ int compact3(int v) {
     return (v & 1) | ((v >> 1) & 2) | ((v >> 2) & 4);
 }
 
-template <bool kF32>
+template <class F>
 __device__ __forceinline__ void walk_block(const WalkParams& P) {
     // screen-space order: macro tiles of 8 x 8 block tiles in row-major order, Morton inside, so that
     // concurrently resident blocks cover a compact patch of the image and share tets in L2
@@ -890,443 +1020,27 @@ __device__ __forceinline__ void walk_block(const WalkParams& P) {
     const int j = P.j0 + tile_y * kTileY + (warp / 2) * 4 + (lane >> 3);
     const bool live = i < P.i1 && j < P.j1;
 
-    RayResult res;
-    res.tau = 0.0;
-    res.inten = 0.0;
-    res.steps = 0;
-    res.error = 0;
-    res.deferred = 0;
+    RayResult<F::K> res{};
     bool solid = false;
     if (live) solid = P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i];
     // the lanes that will trace a ray, agreed on while the warp is whole (trace_ray synchronises on it)
     const unsigned tracing = __ballot_sync(0xFFFFFFFFu, live && !solid && tile_sees_mesh);
     if (live) {
         if (solid) {
-            const double nan = __longlong_as_double(0x7FF8000000000000ll); // quiet NaN (config.hpp:26-27)
+            double nan[F::K];
+            fill_pairs(nan, __longlong_as_double(0x7FF8000000000000ll), std::make_integer_sequence<int, F::K>{}); // quiet NaN (config.hpp:26-27)
             store_pixel(P, i, j, nan, nan, 0);
         } else {
             if (tile_sees_mesh) {
-                res = trace_ray<kF32>(P, P.xs[i], P.ys[j],
-                                      static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
-                                      tracing);
+                res = trace_ray<F>(P, P.xs[i], P.ys[j],
+                                   static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
+                                   tracing);
             }
-            if (!res.deferred) store_pixel(P, i, j, res.tau, res.inten, res.steps);
+            if (!res.deferred) store_pixel(P, i, j, res.v.tau, res.v.inten, res.steps);
         }
     }
 
     // statistics: one atomic per warp per counter, one per warp-row for the row costs
-    const unsigned full = 0xFFFFFFFFu;
-    unsigned row_steps = res.steps;
-    row_steps += __shfl_xor_sync(full, row_steps, 1);
-    row_steps += __shfl_xor_sync(full, row_steps, 2);
-    row_steps += __shfl_xor_sync(full, row_steps, 4);
-    if ((lane & 7) == 0 && live && row_steps) atomicAdd(&P.row_cost[j], static_cast<unsigned long long>(row_steps));
-    unsigned warp_steps = row_steps;
-    warp_steps += __shfl_xor_sync(full, warp_steps, 8);
-    warp_steps += __shfl_xor_sync(full, warp_steps, 16);
-    const unsigned hits = __popc(__ballot_sync(full, live && res.steps > 0));
-    const unsigned solids = __popc(__ballot_sync(full, solid));
-    const unsigned errors = __popc(__ballot_sync(full, res.error != 0));
-    if (lane == 0) {
-        if (warp_steps) atomicAdd(&P.counters[kSteps], static_cast<unsigned long long>(warp_steps));
-        if (hits) atomicAdd(&P.counters[kHitPixels], static_cast<unsigned long long>(hits));
-        if (solids) atomicAdd(&P.counters[kSolidPixels], static_cast<unsigned long long>(solids));
-        if (errors) atomicAdd(&P.counters[kWalkErrors], static_cast<unsigned long long>(errors));
-    }
-}
-
-} // namespace
-
-// The product kernels. 7 blocks of 128 threads per SM = 72 registers: one more resident block than the
-// 80 the compiler picks on its own, measured faster (5.41 vs 5.64 ms on C3) despite a few spilled words
-// outside the step loop.
-__global__ void __launch_bounds__(kBlock, 7) tet_walk_fp64(const WalkParams P) { walk_block<false>(P); }
-// optional single-precision step geometry (north-star item (d)); entry search and accumulators stay FP64
-__global__ void __launch_bounds__(kBlock, 8) tet_walk_fp32(const WalkParams P) { walk_block<true>(P); }
-
-// The walk's grid only covers the pixel rectangle that can see the mesh (a one-wave row band whose
-// grid is 60 % empty tiles fills the SMs unevenly: measured 1.60 M busy cycles on the fullest SM
-// against 1.07 M on average, profiles/r01_walk_band_c3.csv). Everything else in the band is background
-// or solid and is written by this streaming kernel.
-__global__ void __launch_bounds__(256) fill_background(const WalkParams P) {
-    const int n_rows = P.row_end - P.row_begin;
-    const int64_t k = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-    bool solid = false;
-    if (k < static_cast<int64_t>(n_rows) * P.res_x) {
-        const int j = P.row_begin + static_cast<int>(k / P.res_x), i = static_cast<int>(k % P.res_x);
-        if (!(i >= P.i0 && i < P.i1 && j >= P.j0 && j < P.j1)) solid = background_pixel(P, i, j);
-    }
-    const unsigned solids = __popc(__ballot_sync(0xFFFFFFFFu, solid));
-    if ((threadIdx.x & 31) == 0 && solids) atomicAdd(&P.counters[kSolidPixels], static_cast<unsigned long long>(solids));
-}
-
-// Grazing rays (deferred by the pixel kernel): persistent warps, one ray per warp at a time.
-__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_fp64(const WalkParams P) { graze_block<false>(P); }
-__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_fp32(const WalkParams P) { graze_block<true>(P); }
-
-namespace {
-
-void graze_on_host(const WalkParams& P, bool f32) {
-    const unsigned long long n_rays = P.counters[kDeferred];
-    for (unsigned long long k = 0; k < n_rays; k++) {
-        const DeferredRay& q = P.queue[k];
-        const int i = static_cast<int>(q.pixel % static_cast<uint32_t>(P.res_x));
-        const int j = static_cast<int>(q.pixel / static_cast<uint32_t>(P.res_x));
-        const RayAcc a = f32 ? graze_ray_serial<true>(P, q, P.xs[i], P.ys[j]) : graze_ray_serial<false>(P, q, P.xs[i], P.ys[j]);
-        store_pixel(P, i, j, a.tau, a.inten, a.steps);
-        P.counters[kSteps] += a.steps - q.steps;
-        P.row_cost[j] += a.steps - q.steps;
-        if (q.steps == 0 && a.steps > 0) P.counters[kHitPixels]++;
-        if (a.error) P.counters[kWalkErrors]++;
-    }
-    P.counters[kTicket] = n_rays;
-}
-
-C5_HD bool background_pixel_ch(const WalkParams& P, int n, int i, int j);
-
-void background_on_host(const WalkParams& P, int n_channels) {
-    for (int j = P.row_begin; j < P.row_end; j++) {
-        for (int i = 0; i < P.res_x; i++) {
-            if (i >= P.i0 && i < P.i1 && j >= P.j0 && j < P.j1) continue;
-            if (n_channels ? background_pixel_ch(P, n_channels, i, j) : background_pixel(P, i, j)) P.counters[kSolidPixels]++;
-        }
-    }
-}
-
-void walk_on_host(const WalkParams& P, bool f32) {
-    for (int j = P.j0; j < P.j1; j++) {
-        for (int i = P.i0; i < P.i1; i++) {
-            if (P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i]) {
-                store_pixel(P, i, j, NAN, NAN, 0);
-                P.counters[kSolidPixels]++;
-                continue;
-            }
-            const uint32_t pixel = static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i);
-            const RayResult r = f32 ? trace_ray<true>(P, P.xs[i], P.ys[j], pixel, 0) : trace_ray<false>(P, P.xs[i], P.ys[j], pixel, 0);
-            if (!r.deferred) store_pixel(P, i, j, r.tau, r.inten, r.steps);
-            P.counters[kSteps] += r.steps;
-            P.row_cost[j] += r.steps;
-            if (r.steps) P.counters[kHitPixels]++;
-            if (r.error) P.counters[kWalkErrors]++;
-        }
-    }
-}
-
-} // namespace
-
-// ---- several field pairs in one walk (c5_render_channels) ----------------------------------------
-// The rays, their entry searches, deferrals and steps are those of the FP64 walk above: only what is
-// integrated differs. A step reads tet t's record of K {alpha_c, s_c} pairs (padded to 32-byte
-// sectors) together with t's cell, since t is known at the top of the step, so a channel adds FP64
-// work and a store but no further round trip. Channel c of a pixel is stored at
-// out[((j - row_begin) * res_x + i) * K + c] as {tau, I}.
-
-namespace {
-
-struct ChanParams {
-    WalkParams W;
-    const double* rec;   // [n_tets][channel_stride(K)]: {alpha_c, s_c} per channel
-    double* queue;       // [deferred ray][K] {tau, I}: the channel values DeferredRay::tau/inten hold otherwise
-};
-
-C5_HD void store2(double* p, double a, double b) {
-#ifdef __CUDA_ARCH__
-    *reinterpret_cast<double2*>(p) = make_double2(a, b);
-#else
-    p[0] = a;
-    p[1] = b;
-#endif
-}
-
-// K channels integrated along one crossing (the accumulator of crossing_walk).
-template <int K, bool kAffine>
-struct ChanFields {
-    const double* rec;
-    double tau[K], inten[K], gain[K];
-    double f[channel_stride(K)]; // the record of the tet being crossed
-
-    C5_HD void reset() {
-#pragma unroll
-        for (int c = 0; c < K; c++) {
-            tau[c] = 0.0;
-            inten[c] = 0.0;
-            gain[c] = 1.0;
-        }
-    }
-    C5_HD void fetch(int t) {
-        const double* p = rec + static_cast<size_t>(t) * channel_stride(K);
-#ifdef __CUDA_ARCH__
-#pragma unroll
-        for (int k = 0; k < channel_stride(K); k += 4) {
-            asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];"
-                         : "=d"(f[k]), "=d"(f[k + 1]), "=d"(f[k + 2]), "=d"(f[k + 3])
-                         : "l"(p + k));
-        }
-#else
-        for (int k = 0; k < channel_stride(K); k++) f[k] = p[k];
-#endif
-    }
-    C5_HD void step(const WalkParams& P, const CellData&, double dzv) {
-#pragma unroll
-        for (int c = 0; c < K; c++) segment<kAffine>(f[2 * c], f[2 * c + 1], P.alpha_limit, dzv, tau[c], inten[c], gain[c]);
-    }
-};
-
-template <int K>
-struct ChanRay {
-    ChanFields<K, false> f;
-    uint32_t steps, error, deferred;
-};
-
-template <int K>
-C5_HD void store_pixel_ch(const WalkParams& P, int i, int j, const double* tau, const double* inten, uint32_t steps) {
-    const size_t o = static_cast<size_t>(j - P.row_begin) * P.res_x + i;
-#pragma unroll
-    for (int c = 0; c < K; c++) {
-        double t = tau[c], v = inten[c];
-        if (P.round_float) {
-            t = static_cast<double>(static_cast<float>(t));
-            v = static_cast<double>(static_cast<float>(v));
-        }
-        store2(P.out + 2 * (o * K + c), t, v);
-    }
-    if (P.steps) P.steps[o] = steps;
-}
-
-// Background or solid pixel outside the walk's rectangle, n channels wide.
-C5_HD bool background_pixel_ch(const WalkParams& P, int n, int i, int j) {
-    const bool solid = P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i];
-    const double v = solid ? __longlong_as_double_hd(0x7FF8000000000000ll) : 0.0;
-    const size_t o = static_cast<size_t>(j - P.row_begin) * P.res_x + i;
-    for (int c = 0; c < n; c++) store2(P.out + 2 * (o * n + c), v, v);
-    if (P.steps) P.steps[o] = 0;
-    return solid;
-}
-
-// trace_ray with K channels: the same four phases, searches and deferral rule.
-template <int K>
-C5_HD void trace_ray_ch(const ChanParams& CP, double px, double py, uint32_t pixel, unsigned tracing, ChanRay<K>& r) {
-    const WalkParams& P = CP.W;
-    r.f.rec = CP.rec;
-    r.f.reset();
-    r.steps = 0;
-    r.error = 0;
-    r.deferred = 0;
-    double z_after = -INFINITY;
-    EntryList<kInline> L;
-
-    bool defer = !bvh_collect_entries(P, px, py, z_after, L, 1, P.query_budget);
-    sync_lanes(tracing);
-    const bool entered = !defer && L.n > 0;
-    if (entered) z_after = crossing_walk<false>(P, px, py, L.leaf[0], L.z[0], r.f, r.steps, r.error);
-    sync_lanes(tracing);
-    L.n = 0;
-    if (entered && !r.error) {
-        const bool searched = bvh_collect_entries(P, px, py, z_after, L, kInline, P.query_budget);
-        defer = !searched || L.n == kInline;
-    }
-    sync_lanes(tracing);
-    for (int e = 0; e < kInline - 1; e++) {
-        if (!defer && e < L.n && L.z[e] > z_after && !r.error) {
-            z_after = crossing_walk<false>(P, px, py, L.leaf[e], L.z[e], r.f, r.steps, r.error);
-        }
-        sync_lanes(tracing);
-    }
-    if (defer) {
-#ifdef __CUDA_ARCH__
-        const unsigned long long slot = atomicAdd(&P.counters[kDeferred], 1ull);
-#else
-        const unsigned long long slot = P.counters[kDeferred]++;
-#endif
-        DeferredRay& q = P.queue[slot];
-        q.tau = 0.0;
-        q.inten = 0.0;
-        q.z_after = z_after;
-        q.pixel = pixel;
-        q.steps = r.steps;
-#pragma unroll
-        for (int c = 0; c < K; c++) store2(CP.queue + 2 * (slot * K + c), r.f.tau[c], r.f.inten[c]);
-        r.deferred = 1;
-    }
-}
-
-// A deferred ray's K channels and geometry, as RayAcc holds one.
-template <int K>
-struct ChanAcc {
-    double tau[K], inten[K];
-    double z_after;
-    uint32_t steps, error;
-};
-
-template <int K>
-C5_HD void load_deferred_ch(const ChanParams& CP, unsigned long long slot, ChanAcc<K>& a) {
-    const DeferredRay& q = CP.W.queue[slot];
-    a.z_after = q.z_after;
-    a.steps = q.steps;
-    a.error = 0;
-#pragma unroll
-    for (int c = 0; c < K; c++) {
-        a.tau[c] = CP.queue[2 * (slot * K + c)];
-        a.inten[c] = CP.queue[2 * (slot * K + c) + 1];
-    }
-}
-
-// compose_crossing, per channel.
-template <int K>
-C5_HD void compose_crossing_ch(ChanAcc<K>& a, double z_in, double z_out, const ChanFields<K, true>& k, uint32_t steps_k,
-                               uint32_t error_k) {
-    if (!(z_in > a.z_after)) return;
-#pragma unroll
-    for (int c = 0; c < K; c++) {
-        a.tau[c] += k.tau[c];
-        a.inten[c] = k.inten[c] + k.gain[c] * a.inten[c];
-    }
-    a.steps += steps_k;
-    a.error |= error_k;
-    a.z_after = z_out;
-}
-
-// graze_ray_serial with K channels (host-loop build).
-template <int K>
-C5_HD ChanAcc<K> graze_ray_serial_ch(const ChanParams& CP, unsigned long long slot, double px, double py) {
-    const WalkParams& P = CP.W;
-    ChanAcc<K> a;
-    load_deferred_ch<K>(CP, slot, a);
-    EntryList<kSerialList> L;
-    int crossings = 0;
-    while (!a.error) {
-        if (!bvh_collect_entries(P, px, py, a.z_after, L, P.serial_cap, 0x7FFFFFFF)) a.error = 1;
-        for (int e = 0; e < L.n; e++) {
-            if (!(L.z[e] > a.z_after)) continue;
-            ChanFields<K, true> k;
-            k.rec = CP.rec;
-            k.reset();
-            uint32_t steps_k = 0, error_k = 0;
-            const double z_out = crossing_walk<true>(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
-            compose_crossing_ch<K>(a, L.z[e], z_out, k, steps_k, error_k);
-            if (++crossings > 65536) a.error = 1;
-        }
-        if (L.n < P.serial_cap) break;
-    }
-    return a;
-}
-
-// graze_block with K channels: the same collection, and crossings folded per channel in z order.
-template <int K>
-__device__ __forceinline__ void graze_block_ch(const ChanParams& CP) {
-    const WalkParams& P = CP.W;
-    __shared__ GrazeSmem smem[kGrazeWarps];
-    const unsigned full = 0xFFFFFFFFu;
-    const int lane = threadIdx.x & 31;
-    GrazeSmem& S = smem[threadIdx.x >> 5];
-    const unsigned long long n_rays = P.counters[kDeferred];
-    while (true) {
-        unsigned long long ticket = 0;
-        if (lane == 0) ticket = atomicAdd(&P.counters[kTicket], 1ull);
-        ticket = __shfl_sync(full, ticket, 0);
-        if (ticket >= n_rays) break;
-        const uint32_t q_pixel = P.queue[ticket].pixel;
-        const int i = static_cast<int>(q_pixel % static_cast<uint32_t>(P.res_x));
-        const int j = static_cast<int>(q_pixel / static_cast<uint32_t>(P.res_x));
-        const double px = P.xs[i], py = P.ys[j];
-        ChanAcc<K> a;
-        load_deferred_ch<K>(CP, ticket, a);
-        const uint32_t q_steps = a.steps;
-        int crossings = 0;
-        bool truncated = true;
-        while (truncated && !a.error) {
-            const int n = graze_collect(P, S, px, py, a.z_after, lane, truncated);
-            for (int base = 0; base < n; base += 32) {
-                const int k = base + lane;
-                const bool have = k < n;
-                const double z_in = have ? S.z[k] : INFINITY;
-                double z_out = z_in;
-                ChanFields<K, true> f;
-                f.rec = CP.rec;
-                f.reset();
-                uint32_t steps_k = 0, error_k = 0;
-                if (have && z_in > a.z_after) z_out = crossing_walk<true>(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
-                const int cnt = n - base < 32 ? n - base : 32;
-                for (int l = 0; l < cnt; l++) {
-                    ChanFields<K, true> g;
-#pragma unroll
-                    for (int c = 0; c < K; c++) {
-                        g.tau[c] = __shfl_sync(full, f.tau[c], l);
-                        g.inten[c] = __shfl_sync(full, f.inten[c], l);
-                        g.gain[c] = __shfl_sync(full, f.gain[c], l);
-                    }
-                    compose_crossing_ch<K>(a, __shfl_sync(full, z_in, l), __shfl_sync(full, z_out, l), g,
-                                           __shfl_sync(full, steps_k, l), __shfl_sync(full, error_k, l));
-                }
-            }
-            crossings += n;
-            if (crossings > 65536) a.error = 1;
-            __syncwarp();
-        }
-        if (lane == 0) {
-            store_pixel_ch<K>(P, i, j, a.tau, a.inten, a.steps);
-            const unsigned long long more = a.steps - q_steps;
-            if (more) {
-                atomicAdd(&P.counters[kSteps], more);
-                atomicAdd(&P.row_cost[j], more);
-                if (q_steps == 0) atomicAdd(&P.counters[kHitPixels], 1ull);
-            }
-            if (a.error) atomicAdd(&P.counters[kWalkErrors], 1ull);
-        }
-    }
-}
-
-// walk_block with K channels: same tiles, same statistics.
-template <int K>
-__device__ __forceinline__ void walk_block_ch(const ChanParams& CP) {
-    const WalkParams& P = CP.W;
-    const int b = blockIdx.x;
-    const int macro = b >> 6, r = b & 63;
-    const int tile_x = (macro % P.n_macro_x) * 8 + compact3(r);
-    const int tile_y = (macro / P.n_macro_x) * 8 + compact3(r >> 1);
-    if (tile_x >= P.n_tiles_x || tile_y >= P.n_tiles_y) return;
-
-    const int i_lo = P.i0 + tile_x * kTileX, j_lo = P.j0 + tile_y * kTileY;
-    const int i_hi = min(i_lo + kTileX, P.i1) - 1, j_hi = min(j_lo + kTileY, P.j1) - 1;
-    bool tile_sees_mesh;
-    {
-        const BvhNode* root = P.nodes;
-        const float x0 = f_round_down(P.xs[i_lo]), x1 = f_round_up(P.xs[i_hi]);
-        const float y0 = f_round_down(P.ys[j_lo]), y1 = f_round_up(P.ys[j_hi]);
-        const bool s0 = x1 >= root->xlo[0] && x0 <= root->xhi[0] && y1 >= root->ylo[0] && y0 <= root->yhi[0];
-        const bool s1 = x1 >= root->xlo[1] && x0 <= root->xhi[1] && y1 >= root->ylo[1] && y0 <= root->yhi[1];
-        tile_sees_mesh = s0 || s1;
-    }
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int i = P.i0 + tile_x * kTileX + (warp % 2) * 8 + (lane & 7);
-    const int j = P.j0 + tile_y * kTileY + (warp / 2) * 4 + (lane >> 3);
-    const bool live = i < P.i1 && j < P.j1;
-
-    ChanRay<K> res;
-    res.f.reset();
-    res.steps = 0;
-    res.error = 0;
-    res.deferred = 0;
-    bool solid = false;
-    if (live) solid = P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i];
-    const unsigned tracing = __ballot_sync(0xFFFFFFFFu, live && !solid && tile_sees_mesh);
-    if (live) {
-        if (solid) {
-            double nan[K];
-#pragma unroll
-            for (int c = 0; c < K; c++) nan[c] = __longlong_as_double(0x7FF8000000000000ll);
-            store_pixel_ch<K>(P, i, j, nan, nan, 0);
-        } else {
-            if (tile_sees_mesh) {
-                trace_ray_ch<K>(CP, P.xs[i], P.ys[j],
-                                static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
-                                tracing, res);
-            }
-            if (!res.deferred) store_pixel_ch<K>(P, i, j, res.f.tau, res.f.inten, res.steps);
-        }
-    }
-
     const unsigned full = 0xFFFFFFFFu;
     unsigned row_steps = res.steps;
     row_steps += __shfl_xor_sync(full, row_steps, 1);
@@ -1357,41 +1071,81 @@ constexpr int chan_blocks_per_sm(int K) {
 
 } // namespace
 
+// The product kernels. 7 blocks of 128 threads per SM = 72 registers: one more resident block than the
+// 80 the compiler picks on its own, measured faster (5.41 vs 5.64 ms on C3) despite a few spilled words
+// outside the step loop.
+__global__ void __launch_bounds__(kBlock, 7) tet_walk_fp64(const WalkParams P) { walk_block<CellsF64>(P); }
+// optional single-precision step geometry (north-star item (d)); entry search and accumulators stay FP64
+__global__ void __launch_bounds__(kBlock, 8) tet_walk_fp32(const WalkParams P) { walk_block<CellsF32>(P); }
 template <int K>
-__global__ void __launch_bounds__(kBlock, chan_blocks_per_sm(K)) tet_walk_ch(const ChanParams P) { walk_block_ch<K>(P); }
-template <int K>
-__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_ch(const ChanParams P) { graze_block_ch<K>(P); }
+__global__ void __launch_bounds__(kBlock, chan_blocks_per_sm(K)) tet_walk_ch(const WalkParams P) { walk_block<Channels<K>>(P); }
 
-__global__ void __launch_bounds__(256) fill_background_ch(const WalkParams P, int n_channels) {
+// The walk's grid only covers the pixel rectangle that can see the mesh (a one-wave row band whose
+// grid is 60 % empty tiles fills the SMs unevenly: measured 1.60 M busy cycles on the fullest SM
+// against 1.07 M on average, profiles/r01_walk_band_c3.csv). Everything else in the band is background
+// or solid and is written by this streaming kernel, n {tau, I} pairs per pixel.
+__global__ void __launch_bounds__(256) fill_background(const WalkParams P, int n) {
     const int n_rows = P.row_end - P.row_begin;
     const int64_t k = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
     bool solid = false;
     if (k < static_cast<int64_t>(n_rows) * P.res_x) {
         const int j = P.row_begin + static_cast<int>(k / P.res_x), i = static_cast<int>(k % P.res_x);
-        if (!(i >= P.i0 && i < P.i1 && j >= P.j0 && j < P.j1)) solid = background_pixel_ch(P, n_channels, i, j);
+        if (!(i >= P.i0 && i < P.i1 && j >= P.j0 && j < P.j1)) solid = background_pixel(P, n, i, j);
     }
     const unsigned solids = __popc(__ballot_sync(0xFFFFFFFFu, solid));
     if ((threadIdx.x & 31) == 0 && solids) atomicAdd(&P.counters[kSolidPixels], static_cast<unsigned long long>(solids));
 }
 
+// Grazing rays (deferred by the pixel kernel): persistent warps, one ray per warp at a time.
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_fp64(const WalkParams P) { graze_block<CellsF64>(P); }
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_fp32(const WalkParams P) { graze_block<CellsF32>(P); }
+template <int K>
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_ch(const WalkParams P) { graze_block<Channels<K>>(P); }
+
 namespace {
 
+// The pixel and grazing-ray kernels of each field policy.
+template <class F>
+struct Kernels;
+template <>
+struct Kernels<CellsF64> {
+    static constexpr void (*walk)(WalkParams) = tet_walk_fp64;
+    static constexpr void (*graze)(WalkParams) = grazing_rays_fp64;
+};
+template <>
+struct Kernels<CellsF32> {
+    static constexpr void (*walk)(WalkParams) = tet_walk_fp32;
+    static constexpr void (*graze)(WalkParams) = grazing_rays_fp32;
+};
 template <int K>
-void walk_on_host_ch(const ChanParams& CP) {
-    const WalkParams& P = CP.W;
+struct Kernels<Channels<K>> {
+    static constexpr void (*walk)(WalkParams) = tet_walk_ch<K>;
+    static constexpr void (*graze)(WalkParams) = grazing_rays_ch<K>;
+};
+
+void background_on_host(const WalkParams& P, int n) {
+    for (int j = P.row_begin; j < P.row_end; j++) {
+        for (int i = 0; i < P.res_x; i++) {
+            if (i >= P.i0 && i < P.i1 && j >= P.j0 && j < P.j1) continue;
+            if (background_pixel(P, n, i, j)) P.counters[kSolidPixels]++;
+        }
+    }
+}
+
+template <class F>
+void walk_on_host(const WalkParams& P) {
     for (int j = P.j0; j < P.j1; j++) {
         for (int i = P.i0; i < P.i1; i++) {
             if (P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i]) {
-                double nan[K];
-                for (int c = 0; c < K; c++) nan[c] = NAN;
-                store_pixel_ch<K>(P, i, j, nan, nan, 0);
+                double nan[F::K];
+                fill_pairs(nan, NAN, std::make_integer_sequence<int, F::K>{});
+                store_pixel(P, i, j, nan, nan, 0);
                 P.counters[kSolidPixels]++;
                 continue;
             }
             const uint32_t pixel = static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i);
-            ChanRay<K> r;
-            trace_ray_ch<K>(CP, P.xs[i], P.ys[j], pixel, 0, r);
-            if (!r.deferred) store_pixel_ch<K>(P, i, j, r.f.tau, r.f.inten, r.steps);
+            const RayResult<F::K> r = trace_ray<F>(P, P.xs[i], P.ys[j], pixel, 0);
+            if (!r.deferred) store_pixel(P, i, j, r.v.tau, r.v.inten, r.steps);
             P.counters[kSteps] += r.steps;
             P.row_cost[j] += r.steps;
             if (r.steps) P.counters[kHitPixels]++;
@@ -1400,16 +1154,15 @@ void walk_on_host_ch(const ChanParams& CP) {
     }
 }
 
-template <int K>
-void graze_on_host_ch(const ChanParams& CP) {
-    const WalkParams& P = CP.W;
+template <class F>
+void graze_on_host(const WalkParams& P) {
     const unsigned long long n_rays = P.counters[kDeferred];
     for (unsigned long long k = 0; k < n_rays; k++) {
         const DeferredRay& q = P.queue[k];
         const int i = static_cast<int>(q.pixel % static_cast<uint32_t>(P.res_x));
         const int j = static_cast<int>(q.pixel / static_cast<uint32_t>(P.res_x));
-        const ChanAcc<K> a = graze_ray_serial_ch<K>(CP, k, P.xs[i], P.ys[j]);
-        store_pixel_ch<K>(P, i, j, a.tau, a.inten, a.steps);
+        const RayAcc<F::K> a = graze_ray_serial<F>(P, k, P.xs[i], P.ys[j]);
+        store_pixel(P, i, j, a.v.tau, a.v.inten, a.steps);
         P.counters[kSteps] += a.steps - q.steps;
         P.row_cost[j] += a.steps - q.steps;
         if (q.steps == 0 && a.steps > 0) P.counters[kHitPixels]++;
@@ -1418,23 +1171,25 @@ void graze_on_host_ch(const ChanParams& CP) {
     P.counters[kTicket] = n_rays;
 }
 
-template <int K>
-void launch_walk_ch(DeviceState& d, const WalkLaunch& w, const WalkParams& P, unsigned grid) {
-    ChanParams CP{P, d.ch_rec.p, d.ch_queue.p};
+// Policy F's pixel kernel over `grid` blocks, then its grazing-ray kernel for the rays the pixel
+// kernel deferred: a fixed grid of persistent warps that draw tickets. The host-loop build runs both
+// as loops.
+template <class F>
+void launch_rays(DeviceState& d, const WalkLaunch& w, const WalkParams& P, unsigned grid) {
     if (kHostSim) {
-        walk_on_host_ch<K>(CP);
+        walk_on_host<F>(P);
         count_launch();
-        graze_on_host_ch<K>(CP);
+        graze_on_host<F>(P);
         return;
     }
-    tet_walk_ch<K><<<grid, kBlock, 0, d.stream>>>(CP);
+    Kernels<F>::walk<<<grid, kBlock, 0, d.stream>>>(P);
     C5_CUDA(cudaGetLastError());
     if (w.mark_walk_done) C5_CUDA(cudaEventRecord(w.mark_walk_done, d.stream));
     if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
     if (d.sm_count == 0) C5_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, d.device));
+    const unsigned graze_grid = static_cast<unsigned>(d.sm_count) * static_cast<unsigned>(kGrazeBlocksPerSm);
     count_launch();
-    grazing_rays_ch<K><<<static_cast<unsigned>(d.sm_count) * static_cast<unsigned>(kGrazeBlocksPerSm), 32 * kGrazeWarps, 0,
-                         d.stream>>>(CP);
+    Kernels<F>::graze<<<graze_grid, 32 * kGrazeWarps, 0, d.stream>>>(P);
     C5_CUDA(cudaGetLastError());
 }
 
@@ -1488,62 +1243,41 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     if (w.channels < 0 || w.channels > C5_MAX_CHANNELS || (w.channels && f32)) {
         fail(C5_E_INVALID, "render: channels need precision 64 and 1 .. C5_MAX_CHANNELS channels");
     }
+    if (w.channels) {
+        P.rec = d.ch_rec.p;
+        P.ch_queue = d.ch_queue.p;
+    }
+    const int n_pairs = w.channels ? w.channels : 1;
     if (!whole_band) {
         count_launch();
         if (kHostSim) {
-            background_on_host(P, w.channels);
+            background_on_host(P, n_pairs);
         } else {
             const int64_t n = static_cast<int64_t>(w.row_end - w.row_begin) * w.res_x;
-            if (w.channels) {
-                fill_background_ch<<<static_cast<unsigned>((n + 255) / 256), 256, 0, d.stream>>>(P, w.channels);
-            } else {
-                fill_background<<<static_cast<unsigned>((n + 255) / 256), 256, 0, d.stream>>>(P);
-            }
+            fill_background<<<static_cast<unsigned>((n + 255) / 256), 256, 0, d.stream>>>(P, n_pairs);
             C5_CUDA(cudaGetLastError());
         }
     }
     if (empty_rect) return; // the mesh is not in this band: no rays
     count_launch();
-    if (w.channels) {
-        const unsigned grid = static_cast<unsigned>(P.n_macro_x) * static_cast<unsigned>(n_macro_y) * 64u;
-        switch (w.channels) {
-        case 1: launch_walk_ch<1>(d, w, P, grid); break;
-        case 2: launch_walk_ch<2>(d, w, P, grid); break;
-        case 3: launch_walk_ch<3>(d, w, P, grid); break;
-        case 4: launch_walk_ch<4>(d, w, P, grid); break;
-        case 5: launch_walk_ch<5>(d, w, P, grid); break;
-        case 6: launch_walk_ch<6>(d, w, P, grid); break;
-        case 7: launch_walk_ch<7>(d, w, P, grid); break;
-        default: launch_walk_ch<8>(d, w, P, grid); break;
-        }
-        return;
-    }
-    if (kHostSim) {
-        walk_on_host(P, f32);
-        count_launch();
-        graze_on_host(P, f32);
-        return;
-    }
     const unsigned grid = static_cast<unsigned>(P.n_macro_x) * static_cast<unsigned>(n_macro_y) * 64u;
-    if (f32) {
-        tet_walk_fp32<<<grid, kBlock, 0, d.stream>>>(P);
-    } else {
-        tet_walk_fp64<<<grid, kBlock, 0, d.stream>>>(P);
+    switch (w.channels) {
+    case 0:
+        if (f32) {
+            launch_rays<CellsF32>(d, w, P, grid);
+        } else {
+            launch_rays<CellsF64>(d, w, P, grid);
+        }
+        break;
+    case 1: launch_rays<Channels<1>>(d, w, P, grid); break;
+    case 2: launch_rays<Channels<2>>(d, w, P, grid); break;
+    case 3: launch_rays<Channels<3>>(d, w, P, grid); break;
+    case 4: launch_rays<Channels<4>>(d, w, P, grid); break;
+    case 5: launch_rays<Channels<5>>(d, w, P, grid); break;
+    case 6: launch_rays<Channels<6>>(d, w, P, grid); break;
+    case 7: launch_rays<Channels<7>>(d, w, P, grid); break;
+    default: launch_rays<Channels<8>>(d, w, P, grid); break;
     }
-    C5_CUDA(cudaGetLastError());
-    if (w.mark_walk_done) C5_CUDA(cudaEventRecord(w.mark_walk_done, d.stream));
-    if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
-
-    // Rays the pixel kernel deferred: a fixed grid of persistent warps that draw tickets.
-    if (d.sm_count == 0) C5_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, d.device));
-    const unsigned graze_grid = static_cast<unsigned>(d.sm_count) * static_cast<unsigned>(kGrazeBlocksPerSm);
-    count_launch();
-    if (f32) {
-        grazing_rays_fp32<<<graze_grid, 32 * kGrazeWarps, 0, d.stream>>>(P);
-    } else {
-        grazing_rays_fp64<<<graze_grid, 32 * kGrazeWarps, 0, d.stream>>>(P);
-    }
-    C5_CUDA(cudaGetLastError());
 }
 
 } // namespace c5

@@ -53,7 +53,7 @@ def main():
             break
     if best is None:
         raise SystemExit("step loop not found")
-    print(f"# {kernel}: step loop of the first crossing (course5_b200/csrc/c5_walk.cu crossing_f64), "
+    print(f"# {kernel}: step loop of the first crossing (course5_b200/csrc/c5_walk.cu crossing_walk), "
           f"{len(best)} instructions, 0x{best[0][0]:x} .. 0x{best[-1][0]:x}")
     print(f"# {res[full]}")
     census = collections.Counter()
