@@ -87,6 +87,8 @@ SYMBOLS = {
     "c5_render_raw": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _u32p, _u8p, C.POINTER(Stats)]),
     "c5_upload_channels": (C.c_int, [C.c_void_p, _dp, _dp, C.c_int32]),
     "c5_render_channels": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _u32p, _u8p, C.POINTER(Stats)]),
+    "c5_render_flux": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, _dp, _dp, C.POINTER(Stats)]),
+    "c5_render_flux_submit": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, _dp, _dp, _u64p]),
     "c5_render_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_last_row_cost": (C.c_int, [C.c_void_p, _u64p, C.c_int32]),
     "c5_kernel_launches": (C.c_uint64, [C.c_void_p]),
@@ -103,7 +105,7 @@ SYMBOLS = {
 }
 IPC_HANDLE_BYTES = 80
 MAX_IN_FLIGHT = 8
-ABI_VERSION = 3        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
+ABI_VERSION = 4        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
 TIMELINE_PHASES = 6
 
 
@@ -310,8 +312,38 @@ class Context:
 
     def render_wait(self, ticket: int) -> dict:
         st = Stats()
-        self._check(self.lib.c5_render_wait(self._h, ticket, C.byref(st)))
+        try:
+            self._check(self.lib.c5_render_wait(self._h, ticket, C.byref(st)))
+        finally:
+            getattr(self, "_flux_in_flight", {}).pop(ticket, None)
         return st.as_dict()
+
+    def _flux_arrays(self, view: View, channels: bool):
+        n = self.n_channels if channels else 1
+        return np.zeros((view.res_y, n, 2), dtype=np.float64), np.zeros((n, 2), dtype=np.float64)
+
+    def render_flux(self, view: View, *, channels: bool = False):
+        """Row sums of one view, reduced on the device (c5_render_flux): returns (rows, total, stats) with
+        rows of shape (res_y, n, 2) and total of shape (n, 2), [c, 0] = sum of tau and [c, 1] = sum of I
+        over the pixels outside the solid mask; n = 1 for the cells' own fields, n = n_channels with
+        channels=True. Rows outside the view's band are 0."""
+        rows, total = self._flux_arrays(view, channels)
+        st = Stats()
+        self._check(self.lib.c5_render_flux(self._h, C.byref(view), 1 if channels else 0, _ptr(rows, _dp),
+                                            _ptr(total, _dp), C.byref(st)))
+        return rows, total, st.as_dict()
+
+    def render_flux_submit(self, view: View, *, channels: bool = False):
+        """The pipelined form (c5_render_flux_submit): returns (ticket, rows, total) at once; render_wait(ticket)
+        fills the two arrays. The context keeps them alive until then."""
+        rows, total = self._flux_arrays(view, channels)
+        ticket = C.c_uint64(0)
+        self._check(self.lib.c5_render_flux_submit(self._h, C.byref(view), 1 if channels else 0, _ptr(rows, _dp),
+                                                   _ptr(total, _dp), C.byref(ticket)))
+        if not hasattr(self, "_flux_in_flight"):
+            self._flux_in_flight = {}
+        self._flux_in_flight[int(ticket.value)] = (rows, total)
+        return int(ticket.value), rows, total
 
     def render_raw(self, view: View) -> RawImage:
         out = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64)

@@ -283,7 +283,8 @@ std::vector<std::pair<int, int>> cut_bands(const c5_ctx* ctx, const c5_view* v, 
 // event; waiting for the view is waiting for that event. Nothing in between touches the host, so
 // several contexts that share a mesh (the lanes of c5_render_submit) overlap on the device.
 
-void ensure_host_staging(DeviceState& d, size_t rows) {
+// flux_words: doubles of row sums a flux view copies back (res_y * pairs * 2; 0 for other views)
+void ensure_host_staging(DeviceState& d, size_t rows, size_t flux_words = 0) {
     if (!d.h_counters) d.h_counters = static_cast<unsigned long long*>(host_pinned_alloc(kNumCounters * sizeof(unsigned long long)));
     if (rows > d.h_row_cost_n) {
         host_pinned_free(d.h_row_cost);
@@ -292,16 +293,25 @@ void ensure_host_staging(DeviceState& d, size_t rows) {
         d.h_row_cost = static_cast<uint64_t*>(host_pinned_alloc(rows * sizeof(uint64_t)));
         d.h_row_cost_n = rows;
     }
+    if (flux_words > d.h_row_flux_n) {
+        host_pinned_free(d.h_row_flux);
+        d.h_row_flux = nullptr;
+        d.h_row_flux_n = 0;
+        d.h_row_flux = static_cast<double*>(host_pinned_alloc(flux_words * sizeof(double)));
+        d.h_row_flux_n = flux_words;
+    }
 }
 
 void follow_parent(c5_ctx* ctx);
 
+// flux != null: a flux view. No image leaves the device: the band's rows are summed (launch_reduce_rows)
+// and the sums are copied into page-locked staging; c5_render_wait / the caller hands them to `flux`.
 void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, uint64_t ticket,
-                 bool in_place_allowed = true, bool channels = false) {
+                 bool in_place_allowed = true, bool channels = false, const FluxOut* flux = nullptr) {
     follow_parent(ctx);
     if (ctx->pending.active) fail(C5_E_STATE, "render: this context still has a view in flight (c5_render_wait it first)");
     if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    if (!out) fail(C5_E_INVALID, "render: out is NULL");
+    if (!out && !flux) fail(C5_E_INVALID, "render: out is NULL");
     const ViewPlan p = plan_view(v);
     DeviceState& d = ctx->dev;
     if (channels && d.n_channels == 0) fail(C5_E_STATE, "render_channels: no channels uploaded");
@@ -320,7 +330,7 @@ void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, ui
     // in_place_allowed = false. Pixels are stored as one 128-bit word, so an in-place buffer must be
     // 16-byte aligned; pageable or misaligned buffers take the copy.
     double* host_direct = nullptr;
-    if (!kHostSim && in_place_allowed && !d.opt_no_zero_copy && (reinterpret_cast<uintptr_t>(out) & 15u) == 0) {
+    if (!kHostSim && !flux && in_place_allowed && !d.opt_no_zero_copy && (reinterpret_cast<uintptr_t>(out) & 15u) == 0) {
         cudaPointerAttributes attr{};
         if (cudaPointerGetAttributes(&attr, out) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer) {
             host_direct = static_cast<double*>(attr.devicePointer) + words * band_off;
@@ -328,12 +338,19 @@ void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, ui
             cudaGetLastError(); // pageable memory reports an error on some drivers: not ours
         }
     }
-    ensure_host_staging(d, static_cast<size_t>(v->res_y));
+    ensure_host_staging(d, static_cast<size_t>(v->res_y), flux ? words * static_cast<size_t>(v->res_y) : 0);
     enqueue_view(d, v, p, steps != nullptr, host_direct, n_ch);
-    record(d, 5);
-    if (!host_direct) d2h(out + words * band_off, d.out.p, words * n_pix_band * sizeof(double), d.stream);
-    record(d, 6);
     const bool solids = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0;
+    record(d, 5);
+    if (flux) { // after the grazing-ray kernel: deferred rays are in the sums
+        launch_reduce_rows(d, v->res_x, v->res_y, p.row_begin, p.row_end, static_cast<int>(words / 2), solids);
+        const size_t rows_off = words * static_cast<size_t>(p.row_begin);
+        d2h(d.h_row_flux + rows_off, d.row_flux.p + rows_off, words * static_cast<size_t>(p.row_end - p.row_begin) * sizeof(double),
+            d.stream);
+    } else if (!host_direct) {
+        d2h(out + words * band_off, d.out.p, words * n_pix_band * sizeof(double), d.stream);
+    }
+    record(d, 6);
     if (steps) d2h(steps + band_off, d.steps.p, n_pix_band * sizeof(uint32_t), d.stream);
     if (solid_mask) {
         if (solids) d2h(solid_mask + band_off, d.mask.p + band_off, n_pix_band, d.stream);
@@ -347,18 +364,22 @@ void submit_view(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, ui
     ctx->pending.view = *v;
     ctx->pending.plan = p;
     ctx->pending.d2h_copy = host_direct == nullptr;
+    ctx->pending.flux_pairs = flux ? static_cast<int>(words / 2) : 0;
+    ctx->pending.flux = flux ? *flux : FluxOut{};
 }
 
 // What one device reports for a view: its stats and per-row tet-steps.
 struct ViewResult {
     c5_stats st{};
     std::vector<uint64_t> row_cost;
+    std::vector<double> flux; // flux views: res_y * pairs * 2 row sums, 0 outside the band
 };
 
 // Reads d's last view (planned as p) from the page-locked staging, once the stream has passed the
 // copies into it. A submitted view ends with the image on the host (event 6); a view of
-// c5_render_device ends with the walk (event 4) and has no ms_d2h.
-ViewResult read_view(DeviceState& d, const c5_view& v, const ViewPlan& p, bool submitted) {
+// c5_render_device ends with the walk (event 4) and has no ms_d2h. A flux view (flux_pairs > 0) ends
+// with its row sums on the host (event 6).
+ViewResult read_view(DeviceState& d, const c5_view& v, const ViewPlan& p, bool submitted, int flux_pairs = 0) {
     ViewResult r;
     c5_stats& st = r.st;
     const unsigned long long* c = d.h_counters;
@@ -377,7 +398,24 @@ ViewResult read_view(DeviceState& d, const c5_view& v, const ViewPlan& p, bool s
     st.ms_total = elapsed(d, 0, submitted ? 6 : 4);
     st.n_devices = 1;
     r.row_cost.assign(d.h_row_cost, d.h_row_cost + v.res_y);
+    if (flux_pairs) {
+        const size_t words = 2 * static_cast<size_t>(flux_pairs);
+        r.flux.assign(words * static_cast<size_t>(v.res_y), 0.0);
+        std::copy(d.h_row_flux + words * static_cast<size_t>(p.row_begin), d.h_row_flux + words * static_cast<size_t>(p.row_end),
+                  r.flux.begin() + static_cast<std::ptrdiff_t>(words * static_cast<size_t>(p.row_begin)));
+    }
     return r;
+}
+
+// Hands a flux view's row sums (res_y rows of `words` doubles) to the caller: the rows as they are,
+// total[c] = sum of rows[j][c] in increasing j, accumulated in double.
+void deliver_flux(const std::vector<double>& rows, size_t words, const FluxOut& f) {
+    if (f.rows) std::copy(rows.begin(), rows.end(), f.rows);
+    if (!f.total) return;
+    for (size_t c = 0; c < words; c++) f.total[c] = 0.0;
+    for (size_t j = 0; j < rows.size() / words; j++) {
+        for (size_t c = 0; c < words; c++) f.total[c] += rows[j * words + c];
+    }
 }
 
 // Row costs go to `owner` (the context the caller holds), stats to *st (may be NULL); a ray stopped
@@ -397,15 +435,16 @@ ViewResult wait_view(c5_ctx* lane) {
     use_device(d);
     lane->pending.active = false; // whatever happens below, the lane is free again
     if (!kHostSim) C5_CUDA(cudaEventSynchronize(d.ev_done));
-    return read_view(d, lane->pending.view, lane->pending.plan, true);
+    return read_view(d, lane->pending.view, lane->pending.plan, true, lane->pending.flux_pairs);
 }
 
 // Multi-device contexts (c5_create with several devices): the context and each of its parts render
 // one cost-balanced row band, as c5_render does for a row band, straight into its final rows of the
 // caller's buffers. One host thread per device submits: a copy into pageable memory blocks the
 // submitting thread until its device is done, so one thread would render the bands one after another.
+// A flux render (flux != null) merges the parts' row sums and sums the total over all rows in order.
 void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, c5_stats* st,
-                         bool channels = false) {
+                         bool channels = false, const FluxOut* flux = nullptr) {
     if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
     const ViewPlan p = plan_view(v);
     const std::vector<c5_ctx*> parts = with_parts(ctx);
@@ -418,7 +457,8 @@ void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* s
         try {
             band_views[r].row_begin = bands[r].first;
             band_views[r].row_end = bands[r].second;
-            submit_view(parts[r], &band_views[r], out, steps, solid_mask, 0, true, channels);
+            const FluxOut part_flux{}; // the merged sums are handed over below
+            submit_view(parts[r], &band_views[r], out, steps, solid_mask, 0, true, channels, flux ? &part_flux : nullptr);
         } catch (...) {
             errors[r] = std::current_exception();
         }
@@ -466,6 +506,16 @@ void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* s
         for (size_t j = 0; j < total.row_cost.size(); j++) total.row_cost[j] += r.row_cost[j];
     }
     t.n_devices = static_cast<int32_t>(n);
+    if (flux) {
+        const size_t words = results[0].flux.size() / static_cast<size_t>(v->res_y);
+        std::vector<double> rows(words * static_cast<size_t>(v->res_y), 0.0);
+        for (size_t r = 0; r < n; r++) {
+            const size_t lo = words * static_cast<size_t>(bands[r].first), hi = words * static_cast<size_t>(bands[r].second);
+            std::copy(results[r].flux.begin() + static_cast<std::ptrdiff_t>(lo), results[r].flux.begin() + static_cast<std::ptrdiff_t>(hi),
+                      rows.begin() + static_cast<std::ptrdiff_t>(lo));
+        }
+        deliver_flux(rows, words, *flux);
+    }
     report(ctx, total, st);
 }
 
@@ -482,6 +532,47 @@ void ensure_lanes(c5_ctx* ctx) {
         if (rc != C5_OK) fail(rc, "render_submit: cannot create a lane: " + ctx->err);
         ctx->lanes.push_back(lane);
     }
+}
+
+// c5_render_submit / c5_render_flux_submit: the view goes to the next lane in turn, or any free one.
+void submit_on_lane(c5_ctx* ctx, const c5_view* view, double* out, uint64_t* ticket, bool channels, const FluxOut* flux) {
+    ensure_lanes(ctx);
+    const unsigned n = static_cast<unsigned>(ctx->lanes.size()) + 1;
+    c5_ctx* lane = nullptr;
+    for (unsigned k = 0; k < n && !lane; k++) {
+        c5_ctx* cand = lane_of(ctx, (ctx->next_lane + k) % n);
+        if (!cand->pending.active) {
+            lane = cand;
+            ctx->next_lane = (ctx->next_lane + k + 1) % n;
+        }
+    }
+    if (!lane) fail(C5_E_STATE, "render_submit: " + std::to_string(n) + " views are in flight already (c5_render_wait one first)");
+    const uint64_t t = ctx->next_ticket++;
+    try {
+        g_launch_counter = &lane->dev.launches;
+        submit_view(lane, view, out, nullptr, nullptr, t, /*in_place_allowed=*/ctx->views_in_flight == 1, channels, flux);
+    } catch (const Error& e) {
+        if (lane != ctx) ctx->err = e.text; // (guarded() reports through ctx)
+        throw;
+    }
+    *ticket = t;
+}
+
+// A render over the uploaded channels needs them on the context and, alike, on every part.
+void check_channels_ready(c5_ctx* ctx) {
+    follow_parent(ctx);
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    if (ctx->dev.n_channels == 0) fail(C5_E_STATE, "render_channels: no channels uploaded");
+    for (const c5_ctx* part : ctx->parts) { // every band must be as wide as the caller's image
+        if (part->dev.n_channels != ctx->dev.n_channels) fail(C5_E_STATE, "render_channels: the devices hold different channels");
+    }
+}
+
+// Arguments of c5_render_flux / c5_render_flux_submit.
+void check_flux_args(const c5_view* view, int32_t channels, const double* rows, const double* total) {
+    if (!rows && !total) fail(C5_E_INVALID, "render_flux: rows and total are both NULL");
+    if (channels != 0 && channels != 1) fail(C5_E_INVALID, "render_flux: channels must be 0 or 1");
+    if (channels && view && view->precision == 32) fail(C5_E_INVALID, "render_flux: channels are FP64 only (precision 64)");
 }
 
 void upload_solids(c5_ctx* ctx, const double* pts, int64_t n, int follows) {
@@ -733,6 +824,7 @@ void c5_destroy(c5_ctx* ctx) {
     }
     host_pinned_free(d.h_counters);
     host_pinned_free(d.h_row_cost);
+    host_pinned_free(d.h_row_flux);
     if (!kHostSim) {
         for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
         if (d.ev_walk) cudaEventDestroy(d.ev_walk);
@@ -880,12 +972,7 @@ int c5_render_channels(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* 
     if (!ctx) return C5_E_INVALID;
     return guarded(ctx, [&] {
         if (view && view->precision == 32) fail(C5_E_INVALID, "render_channels: FP64 only (precision 64)");
-        follow_parent(ctx);
-        if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-        if (ctx->dev.n_channels == 0) fail(C5_E_STATE, "render_channels: no channels uploaded");
-        for (const c5_ctx* part : ctx->parts) { // every band must be as wide as the caller's image
-            if (part->dev.n_channels != ctx->dev.n_channels) fail(C5_E_STATE, "render_channels: the devices hold different channels");
-        }
+        check_channels_ready(ctx);
         if (!ctx->parts.empty()) {
             render_multi_device(ctx, view, out, steps, solid_mask, stats, true);
             return;
@@ -917,27 +1004,35 @@ int c5_render_submit(c5_ctx* ctx, const c5_view* view, double* out, uint64_t* ti
     if (!ctx || !ticket) return C5_E_INVALID;
     return guarded(ctx, [&] {
         if (ctx->parent || !ctx->parts.empty()) fail(C5_E_INVALID, "render_submit: single-device contexts that are not siblings");
-        ensure_lanes(ctx);
-        // the next lane in turn, or any free one
-        const unsigned n = static_cast<unsigned>(ctx->lanes.size()) + 1;
-        c5_ctx* lane = nullptr;
-        for (unsigned k = 0; k < n && !lane; k++) {
-            c5_ctx* cand = lane_of(ctx, (ctx->next_lane + k) % n);
-            if (!cand->pending.active) {
-                lane = cand;
-                ctx->next_lane = (ctx->next_lane + k + 1) % n;
-            }
+        submit_on_lane(ctx, view, out, ticket, false, nullptr);
+    });
+}
+
+int c5_render_flux(c5_ctx* ctx, const c5_view* view, int32_t channels, double* rows, double* total, c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        check_flux_args(view, channels, rows, total);
+        if (channels) check_channels_ready(ctx);
+        const FluxOut f{rows, total};
+        if (!ctx->parts.empty()) {
+            render_multi_device(ctx, view, nullptr, nullptr, nullptr, stats, channels != 0, &f);
+            return;
         }
-        if (!lane) fail(C5_E_STATE, "render_submit: " + std::to_string(n) + " views are in flight already (c5_render_wait one first)");
-        const uint64_t t = ctx->next_ticket++;
-        try {
-            g_launch_counter = &lane->dev.launches;
-            submit_view(lane, view, out, nullptr, nullptr, t, /*in_place_allowed=*/ctx->views_in_flight == 1);
-        } catch (const Error& e) {
-            if (lane != ctx) ctx->err = e.text; // (guarded() reports through ctx)
-            throw;
-        }
-        *ticket = t;
+        submit_view(ctx, view, nullptr, nullptr, nullptr, 0, false, channels != 0, &f);
+        ViewResult r = wait_view(ctx);
+        deliver_flux(r.flux, 2 * static_cast<size_t>(ctx->pending.flux_pairs), f);
+        report(ctx, r, stats);
+    });
+}
+
+int c5_render_flux_submit(c5_ctx* ctx, const c5_view* view, int32_t channels, double* rows, double* total,
+                          uint64_t* ticket) {
+    if (!ctx || !ticket) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        check_flux_args(view, channels, rows, total);
+        if (ctx->parent || !ctx->parts.empty()) fail(C5_E_STATE, "render_flux_submit: single-device contexts that are not siblings");
+        const FluxOut f{rows, total};
+        submit_on_lane(ctx, view, nullptr, ticket, channels != 0, &f);
     });
 }
 
@@ -948,6 +1043,7 @@ int c5_render_wait(c5_ctx* ctx, uint64_t ticket, c5_stats* stats) {
             c5_ctx* lane = lane_of(ctx, k);
             if (lane->pending.active && lane->pending.ticket == ticket && ticket != 0) {
                 ViewResult r = wait_view(lane);
+                if (lane->pending.flux_pairs) deliver_flux(r.flux, 2 * static_cast<size_t>(lane->pending.flux_pairs), lane->pending.flux);
                 report(ctx, r, stats);
                 return;
             }

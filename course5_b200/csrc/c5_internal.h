@@ -84,6 +84,7 @@ struct DeviceState {
     DevBuf<unsigned long long> row_cost;
     DevBuf<DeferredRay> queue;       // grazing rays of the current view (capacity: pixels of the band)
     DevBuf<double> ch_queue;         // their channel values {tau, I} (channel renders only)
+    DevBuf<double> row_flux;         // flux renders: [res_y][pairs] {sum tau, sum I} of the band's rows
     int sm_count = 0;
     cudaEvent_t ev_walk = nullptr;   // between the pixel kernel and the grazing-ray kernel (phase times)
     cudaEvent_t ev_done = nullptr;   // after the view's last copy: what c5_render_wait waits for
@@ -91,6 +92,8 @@ struct DeviceState {
     unsigned long long* h_counters = nullptr;   // [kNumCounters]
     uint64_t* h_row_cost = nullptr;             // [h_row_cost_n]
     size_t h_row_cost_n = 0;
+    double* h_row_flux = nullptr;               // [h_row_flux_n]: row_flux of a flux view
+    size_t h_row_flux_n = 0;
     // c5_debug_set (tests, diagnostics); 0 = default
     int opt_graze_list = 0, opt_query_budget = 0, opt_serial_list = 0, opt_mask_tile = 0;
     bool opt_no_zero_copy = false, opt_no_static_mask = false;
@@ -112,12 +115,18 @@ struct ViewPlan {      // a validated c5_view: trig evaluated, band and pixel st
     int row_begin, row_end;
     double x_min, y_min, step_x, step_y;
 };
+struct FluxOut {       // the caller's arrays of a flux render (either may be null)
+    double* rows;      // res_y * pairs * 2
+    double* total;     // pairs * 2
+};
 struct PendingView {   // the view a context has in flight between c5_render_submit and c5_render_wait
     bool active = false;
     uint64_t ticket = 0;
     c5_view view{};
     ViewPlan plan{};
     bool d2h_copy = false; // the image went through the device band buffer and a copy (not stored in place)
+    int flux_pairs = 0;    // flux view: pairs per row sum (0: an image view)
+    FluxOut flux{};
 };
 } // namespace c5
 
@@ -176,6 +185,9 @@ struct WalkLaunch {
     cudaEvent_t mark_walk_done_tl; // the same moment for the timeline ring (may be null)
 };
 void launch_walk(DeviceState& d, const WalkLaunch& w);
+// c5_flux.cu — row_flux[j] for the rows [row_begin,row_end) of d.out (pairs {tau, I} per pixel),
+// skipping pixels under d.mask when use_mask; the summation order is documented there.
+void launch_reduce_rows(DeviceState& d, int res_x, int res_y, int row_begin, int row_end, int pairs, bool use_mask);
 // doubles per tet of ch_rec: n {alpha, s} pairs padded to 32 bytes (read with 256-bit loads)
 C5_HD constexpr int channel_stride(int n_channels) { return 4 * ((n_channels + 1) / 2); }
 

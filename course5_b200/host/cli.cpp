@@ -27,6 +27,7 @@ const option kOptions[] = {
     // additions of this build (absent from the reference)
     {"devices", 0, true},          {"stats", 0, false},           {"precision", 0, true},
     {"frames", 0, true},           {"sweep_y_to", 0, true},       {"channels", 0, true},
+    {"light_curve", 0, false},
 };
 
 // --channels A:Q[,A:Q...]: pairs of CELL_DATA array names, at most C5_MAX_CHANNELS (8)
@@ -116,7 +117,13 @@ void print_usage(std::ostream& out) {
            "  --sweep_y_to arg (=2)                  end angle of the sweep (exclusive)\n"
            "  --channels arg                         A:Q[,A:Q...]: also render these pairs of cell\n"
            "                                         arrays of the input file in the same walk, each\n"
-           "                                         as a further array named A:Q (not with --frames)\n"
+           "                                         as a further array named A:Q (with --frames\n"
+           "                                         only with --light_curve)\n"
+           "  --light_curve                          write the light curve instead of images: -d names\n"
+           "                                         a CSV with one line per frame (frame, Y_pi,\n"
+           "                                         hit_pixels, solid_pixels, tau_sum, I_sum, then\n"
+           "                                         A:Q_tau_sum, A:Q_I_sum per --channels pair), sums\n"
+           "                                         over the pixels outside the solids, printed %.17g\n"
         << std::endl;
 }
 
@@ -175,8 +182,11 @@ cli_result program_options(int argc, char** argv, config_str& cfg, std::ostream&
             else if (name == "frames") cfg.frames = static_cast<int>(to_integer(name, value));
             else if (name == "sweep_y_to") cfg.sweep_y_to = to_double(name, value);
             else if (name == "channels") cfg.channels = parse_channels(value);
+            else if (name == "light_curve") cfg.light_curve = true;
         }
-        if (!cfg.channels.empty() && cfg.frames > 1) throw std::runtime_error("--channels cannot be combined with --frames > 1");
+        if (!cfg.channels.empty() && cfg.frames > 1 && !cfg.light_curve) {
+            throw std::runtime_error("--channels cannot be combined with --frames > 1");
+        }
     } catch (const std::exception& e) {
         out << "Error! " << e.what() << std::endl;
         print_usage(out);

@@ -32,6 +32,7 @@ struct config_str {
     int frames = 1;                            // --frames N: in-process sweep of -Y (replaces utility/rotate_traces.py)
     double sweep_y_to = 2.0;                   // --sweep_y_to: end angle (exclusive), units of pi
     std::vector<std::array<std::string, 2>> channels; // --channels A:Q,...: (alpha, Q) cell array names
+    bool light_curve = false;                  // --light_curve: the destination is a CSV of per-frame sums, no .vti
 };
 
 constexpr double PI = 3.14159265358979323846;  // config.hpp:45

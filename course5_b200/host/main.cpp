@@ -1,6 +1,9 @@
 // main.cpp — the `course` executable: same flags, same stdout lines, same .vti as the reference's
 // main (main.cpp:73-141), with the OpenMP loops replaced by the B200 ray pass behind the C ABI.
+#include <algorithm>
 #include <chrono>
+#include <cstdio>
+#include <fstream>
 #include <iostream>
 #include <sstream>
 #include <thread>
@@ -22,6 +25,12 @@ std::vector<int> parse_devices(const std::string& s) {
     }
     if (out.empty()) out.push_back(0);
     return out;
+}
+
+std::string g17(double v) { // %.17g: parses back to the same double
+    char buf[32];
+    std::snprintf(buf, sizeof(buf), "%.17g", v);
+    return buf;
 }
 
 long long ms_between(std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
@@ -95,48 +104,80 @@ int main(int argc, char** argv) {
         t1 = std::chrono::steady_clock::now();
         plane base_plane{config.resolution_x, config.resolution_y, {acc_disk, roche_lobe, acc_sphere}, domain, options};
         base_plane.find_intersections();
-        object2d result = base_plane.trace_rays(tetra_value::alpha, tetra_value::Q);
-        // --channels: the named pairs in one further walk, written beside ImageScalars as "A:Q"
-        const std::vector<std::vector<double>> channels =
-            config.channels.empty() ? std::vector<std::vector<double>>{} : base_plane.trace_channels();
-        t2 = std::chrono::steady_clock::now();
-        std::cout << "Ray-tracing completed in " << ms_between(t1, t2) << " ms. " << std::endl;
+        // the view of sweep frame k (frame 0 is the view the flags describe)
+        auto y_of = [&](int k) {
+            return config.angle_around_y + (config.sweep_y_to - config.angle_around_y) * k / std::max(config.frames, 1);
+        };
+        auto rotations_of = [&](int k) {
+            return std::vector<c5_rotation>{c5_rotation{0, 0, make_perpendicular_to_y_angle, 0.0},
+                                            c5_rotation{1, 0, y_of(k) * PI, ACC_X0}, c5_rotation{0, 0, last_angle, 0.0}};
+        };
 
-        if (config.frames <= 1) {
-            std::vector<vti_array> extra;
-            for (std::size_t c = 0; c < channels.size(); c++) {
-                extra.push_back(vti_array{config.channels[c][0] + ":" + config.channels[c][1], channels[c].data()});
-            }
-            result.export_to_vti(config.destination, false, extra);
-        } else {
-            // in-process sweep: the scene stays on the device, only the rotations change
-            std::string stem = config.destination, ext = ".vti";
-            const auto dot = stem.rfind('.');
-            if (dot != std::string::npos) {
-                ext = stem.substr(dot);
-                stem = stem.substr(0, dot);
-            }
-            const auto t3 = std::chrono::steady_clock::now();
-            // Frame 0 is the view just rendered. The others go through the pipelined calls: up to three
-            // views are in flight on the device while this thread writes the previous frame's file.
-            auto rotations_of = [&](int k) {
-                const double y = config.angle_around_y + (config.sweep_y_to - config.angle_around_y) * k / config.frames;
-                return std::vector<c5_rotation>{c5_rotation{0, 0, make_perpendicular_to_y_angle, 0.0},
-                                                c5_rotation{1, 0, y * PI, ACC_X0}, c5_rotation{0, 0, last_angle, 0.0}};
-            };
-            result.export_to_vti(stem + "_0" + ext);
-            const int ahead = base_plane.views_in_flight();
-            for (int k = 1; k < config.frames + ahead; k++) {
-                if (k - ahead >= 1) {
-                    base_plane.collect_rays([&](const image_ref& frame) { frame.export_to_vti(stem + "_" + std::to_string(k - ahead) + ext); });
+        if (config.light_curve) {
+            // --light_curve: every frame through the pipelined flux calls; only its sums leave the device
+            std::ofstream csv(config.destination);
+            if (!csv) throw std::runtime_error("cannot write " + config.destination);
+            csv << "frame,Y_pi,hit_pixels,solid_pixels,tau_sum,I_sum";
+            for (const auto& pair : config.channels) csv << "," << pair[0] << ":" << pair[1] << "_tau_sum," << pair[0] << ":" << pair[1] << "_I_sum";
+            csv << "\n";
+            if (!config.channels.empty()) base_plane.set_views_in_flight(4); // two flux views per frame
+            const int frames = config.frames < 1 ? 1 : config.frames;
+            const int ahead = base_plane.flux_frames_in_flight();
+            for (int k = 0; k < frames + ahead; k++) {
+                if (k - ahead >= 0) {
+                    const plane::frame_flux f = base_plane.collect_flux();
+                    csv << (k - ahead) << "," << g17(y_of(k - ahead)) << "," << f.stats.hit_pixels << "," << f.stats.solid_pixels;
+                    for (double v : f.total) csv << "," << g17(v);
+                    csv << "\n";
                 }
-                if (k < config.frames) {
+                if (k < frames) {
                     base_plane.set_view_rotations(rotations_of(k));
-                    base_plane.submit_rays();
+                    base_plane.submit_flux();
                 }
             }
-            std::cout << "Sweep of " << config.frames << " frames completed in "
-                      << ms_between(t3, std::chrono::steady_clock::now()) << " ms. " << std::endl;
+            csv.close();
+            if (!csv) throw std::runtime_error("cannot write " + config.destination);
+            std::cout << "Light curve of " << frames << " frames completed in "
+                      << ms_between(t1, std::chrono::steady_clock::now()) << " ms. " << std::endl;
+        } else {
+            object2d result = base_plane.trace_rays(tetra_value::alpha, tetra_value::Q);
+            // --channels: the named pairs in one further walk, written beside ImageScalars as "A:Q"
+            const std::vector<std::vector<double>> channels =
+                config.channels.empty() ? std::vector<std::vector<double>>{} : base_plane.trace_channels();
+            t2 = std::chrono::steady_clock::now();
+            std::cout << "Ray-tracing completed in " << ms_between(t1, t2) << " ms. " << std::endl;
+
+            if (config.frames <= 1) {
+                std::vector<vti_array> extra;
+                for (std::size_t c = 0; c < channels.size(); c++) {
+                    extra.push_back(vti_array{config.channels[c][0] + ":" + config.channels[c][1], channels[c].data()});
+                }
+                result.export_to_vti(config.destination, false, extra);
+            } else {
+                // in-process sweep: the scene stays on the device, only the rotations change
+                std::string stem = config.destination, ext = ".vti";
+                const auto dot = stem.rfind('.');
+                if (dot != std::string::npos) {
+                    ext = stem.substr(dot);
+                    stem = stem.substr(0, dot);
+                }
+                const auto t3 = std::chrono::steady_clock::now();
+                // Frame 0 is the view just rendered. The others go through the pipelined calls: up to three
+                // views are in flight on the device while this thread writes the previous frame's file.
+                result.export_to_vti(stem + "_0" + ext);
+                const int ahead = base_plane.views_in_flight();
+                for (int k = 1; k < config.frames + ahead; k++) {
+                    if (k - ahead >= 1) {
+                        base_plane.collect_rays([&](const image_ref& frame) { frame.export_to_vti(stem + "_" + std::to_string(k - ahead) + ext); });
+                    }
+                    if (k < config.frames) {
+                        base_plane.set_view_rotations(rotations_of(k));
+                        base_plane.submit_rays();
+                    }
+                }
+                std::cout << "Sweep of " << config.frames << " frames completed in "
+                          << ms_between(t3, std::chrono::steady_clock::now()) << " ms. " << std::endl;
+            }
         }
         std::cout << "Result exported. Calculations completed." << std::endl;
 

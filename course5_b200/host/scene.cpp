@@ -151,6 +151,9 @@ plane::plane(std::size_t res_x, std::size_t res_y, std::vector<object3d_base> ob
 plane::~plane() {
     // views still in flight write into _buffers: wait for them before the memory goes away
     for (const auto& pv : _pending) c5_render_wait(_ctx, pv.ticket, nullptr);
+    for (const auto& pf : _pending_flux) {
+        for (int k = 0; k < pf.n; k++) c5_render_wait(_ctx, pf.tickets[k], nullptr);
+    }
     for (auto& b : _buffers) c5_host_unregister(_ctx, b.data());
     c5_destroy(_ctx);
 }
@@ -195,6 +198,40 @@ object2d plane::collect_rays() {
     std::vector<double> copy;
     collect_rays([&](const image_ref& im) { copy.assign(im.data, im.data + im.x * im.y * 2); });
     return object2d{std::move(copy), _x, _y};
+}
+
+void plane::submit_flux() {
+    if (!_uploaded) find_intersections();
+    if (static_cast<int>(_pending_flux.size()) >= flux_frames_in_flight()) {
+        throw std::runtime_error("submit_flux: collect a frame first (" + std::to_string(_pending_flux.size()) + " are in flight)");
+    }
+    pending_flux pf{{0, 0}, 0, std::vector<double>(2 + 2 * _options.channels.size())};
+    check(_ctx, c5_render_flux_submit(_ctx, &_view, 0, nullptr, pf.total.data(), &pf.tickets[0]), "c5_render_flux_submit");
+    pf.n = 1;
+    if (!_options.channels.empty()) {
+        const int rc = c5_render_flux_submit(_ctx, &_view, 1, nullptr, pf.total.data() + 2, &pf.tickets[1]);
+        if (rc != C5_OK) {
+            const std::string text = c5_last_error(_ctx);
+            c5_render_wait(_ctx, pf.tickets[0], nullptr); // the first view writes into pf.total
+            throw std::runtime_error("c5_render_flux_submit failed (" + std::to_string(rc) + "): " + text);
+        }
+        pf.n = 2;
+    }
+    _pending_flux.push_back(std::move(pf)); // moving the vector keeps its buffer where the views write
+}
+
+plane::frame_flux plane::collect_flux() {
+    if (_pending_flux.empty()) throw std::runtime_error("collect_flux: nothing was submitted");
+    pending_flux pf = std::move(_pending_flux.front());
+    _pending_flux.erase(_pending_flux.begin());
+    c5_stats st{};
+    const int rc = c5_render_wait(_ctx, pf.tickets[0], &st);
+    const std::string text = rc == C5_OK ? "" : c5_last_error(_ctx);
+    const int rc_ch = pf.n > 1 ? c5_render_wait(_ctx, pf.tickets[1], nullptr) : C5_OK; // waited for also when the first failed
+    if (rc != C5_OK) throw std::runtime_error("c5_render_wait failed (" + std::to_string(rc) + "): " + text);
+    check(_ctx, rc_ch, "c5_render_wait");
+    _stats = st;
+    return frame_flux{st, std::move(pf.total)};
 }
 
 void plane::find_intersections() {

@@ -134,6 +134,18 @@ public:
     // handed back to the pool when it returns.
     void collect_rays(const std::function<void(const image_ref&)>& consume);
     object2d collect_rays(); // the same, as a copy
+    // Light curves, pipelined (c5_render_flux_submit): submit_flux() enqueues the current view as a flux
+    // view of the cells' own fields and, with render_options::channels, one more over the channels; no
+    // image leaves the device. collect_flux() returns the OLDEST submitted frame's sums. A frame takes
+    // one lane per flux view, so flux_frames_in_flight() frames may be submitted before the first is
+    // collected.
+    struct frame_flux {
+        c5_stats stats;            // of the cells' own view
+        std::vector<double> total; // {tau, I} sums of the cells' fields, then of each channel
+    };
+    void submit_flux();
+    frame_flux collect_flux();
+    int flux_frames_in_flight() const { return _in_flight_max / (_options.channels.empty() ? 1 : 2); }
     std::size_t pending_views() const { return _pending.size(); }
     std::size_t count_all_intersections() const { return static_cast<std::size_t>(_stats.tet_steps); }
     std::size_t get_x() const { return _x; }
@@ -159,6 +171,12 @@ private:
     std::vector<std::vector<double>> _buffers; // registered with the context (c5_host_register)
     std::vector<std::size_t> _free_buffers;
     std::vector<pending_view> _pending;
+    struct pending_flux {
+        std::uint64_t tickets[2];
+        int n; // flux views of the frame
+        std::vector<double> total; // written by c5_render_wait
+    };
+    std::vector<pending_flux> _pending_flux;
     int _in_flight_max = 3;
 };
 

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define C5_ABI_VERSION 3
+#define C5_ABI_VERSION 4
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
 #define C5_MAX_CHANNELS 8
@@ -176,6 +176,37 @@ int c5_render_raw(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* steps
 int c5_upload_channels(c5_ctx* ctx, const double* alpha, const double* q, int32_t n_channels);
 int c5_render_channels(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* steps, uint8_t* solid_mask,
                        c5_stats* stats);
+
+/* ---- flux: per-row sums of a view, reduced on the device (light curves) ---------------------------
+ * The image stays in device memory; only its row sums reach the host (16 bytes per pair and row).
+ * For a view and its n pairs:
+ *   rows[j][c]  = {sum_i tau_c(i,j), sum_i I_c(i,j)} over the pixels of row j NOT under the solid mask,
+ *                 of exactly the doubles the image would hold for the same view (round_through_float
+ *                 and precision included); background pixels add their 0, and a NaN outside the mask
+ *                 makes the sum NaN;
+ *   total[c]    = the sum of rows[j][c] in increasing j, accumulated in double on the host.
+ * Summation order of a row: one block of 256 threads; thread t adds the pixels x = t, t+256, ... in
+ * increasing x, starting from 0; the 256 partials are folded by a halving tree, p[t] += p[t+s] for
+ * s = 128, 64, ..., 1. The sums are therefore bit-identical for any row band, any number of devices
+ * and any number of views in flight.
+ *
+ * channels: 0 = the cells' own alpha/Q (one pair; precision 64 or 32), 1 = all uploaded channels
+ * (n pairs; FP64 only, like c5_render_channels). rows: res_y * n * 2 doubles, rows outside the
+ * view's band are written as 0; total: n * 2 doubles. Either may be NULL, not both.
+ * Stats mean what they mean for c5_render_raw (the geometry is counted once), except that ms_d2h
+ * is the time from the end of the walk until the row sums are in host memory: the reduction and a
+ * copy of a few KB. C5_E_INVALID: both outputs NULL, channels not 0 or 1, or precision 32 with
+ * channels = 1. C5_E_STATE: no mesh, or channels = 1 with none uploaded.
+ *
+ * c5_render_flux works on single-device, multi-device and sibling contexts; a multi-device context
+ * reduces each device's band on that device and merges the rows. c5_render_flux_submit is the
+ * pipelined form with the scope of c5_render_submit (single-device contexts that are not siblings,
+ * C5_E_STATE otherwise): it shares the lanes, the tickets and c5_render_wait with it, which writes
+ * rows / total (need not be page-locked; they must stay valid until the wait returns). */
+int c5_render_flux(c5_ctx* ctx, const c5_view* view, int32_t channels, double* rows, double* total,
+                   c5_stats* stats);
+int c5_render_flux_submit(c5_ctx* ctx, const c5_view* view, int32_t channels, double* rows, double* total,
+                          uint64_t* ticket);
 
 /* Device-resident variant for callers that own device memory (e.g. a torch tensor that an NCCL
  * gather will read): d_out is a DEVICE pointer on the context's first device to
