@@ -20,7 +20,7 @@ namespace c5 {
 // is not on the shared face. Knowing apex[k] when the ray leaves through face k lets the walk
 // issue the next cell load and the next vertex load together instead of one after the other.
 // s = Q / min(alpha, limit) (the source function) is refreshed when --alpha_limit changes, so the
-// I recurrence needs no divide: I <- s - (s - I) exp(-a dz). Tets are in Morton order of centroids.
+// I recurrence needs no divide: I <- I - (s - I) expm1(-a dz). Tets are in Morton order of centroids.
 struct alignas(64) Cell {
     int32_t v[4];
     int32_t nbr[4];

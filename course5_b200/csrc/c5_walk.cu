@@ -361,16 +361,19 @@ C5_HD double crossing_walk(const WalkParams& P, double px, double py, int leaf, 
 
 // One segment of length dz through a medium (alpha, s):
 // tau: line.cpp:176-193 (alpha not clamped);
-// I: line.cpp:206-225 with s = Q / a^:  (Q - (Q - a^ I) e) / a^  ==  s - (s - I) e
+// I: line.cpp:206-225 with s = Q / a^:  (Q - (Q - a^ I) e) / a^  ==  s - (s - I) e  ==  I - (s - I) m,
+// m = e - 1 = expm1(-a^ dz). The last form does not cancel: s - (s - I) e subtracts two numbers of
+// size s to get an increment of size Q dz, and loses log10(1 / (a^ dz)) digits a step (all of them
+// once exp rounds to 1, below a^ dz ~ 1e-16), while -(s - I) m and I are each exact to a few ulps.
 template <bool kAffine>
 C5_HD void segment(double alpha, double s, double limit, double dzv, double& tau, double& inten, double& gain) {
     tau += dzv * alpha;
     double a_c = alpha;
     if (a_c > limit) a_c = limit;
     if (!(a_c < DBL_EPSILON)) {
-        const double e = exp(-a_c * dzv);
-        inten = s - (s - inten) * e;
-        if (kAffine) gain *= e;
+        const double m = expm1(-a_c * dzv);
+        inten = inten - (s - inten) * m;
+        if (kAffine) gain *= 1.0 + m;
     }
 }
 
@@ -441,7 +444,7 @@ struct ChanFields {
 
 // ---- FP32 variant -----------------------------------------------------------------------------------
 // Same crossing with the per-step geometry in single precision: FP32 orientation tests (still exactly
-// antisymmetric: two rounded products, one rounded difference), FP32 divide and expf — about half
+// antisymmetric: two rounded products, one rounded difference), FP32 divide and expm1f — about half
 // the issue slots and 56 instead of 72 registers. What stays in double: the ENTRY search (so the
 // hit/miss set is the FP64 one, bit for bit), the vertex fetch and its subtraction of the pixel
 // position / entry depth (rounding a coordinate ~1 to float would cost 1e-7, i.e. 1e-5 of a tet;
@@ -538,10 +541,10 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
         float a_c = static_cast<float>(c.alpha);
         if (a_c > limit) a_c = limit;
         const double a_d = c.alpha > P.alpha_limit ? P.alpha_limit : c.alpha;
-        if (!(a_d < DBL_EPSILON)) {
-            const double e = static_cast<double>(expf(-a_c * dzv));
-            inten = c.s - (c.s - inten) * e;
-            if (kAffine) gain *= e;
+        if (!(a_d < DBL_EPSILON)) { // the cancellation-free form of segment(), expm1f's error is relative
+            const double m = static_cast<double>(expm1f(-a_c * dzv));
+            inten = inten - (c.s - inten) * m;
+            if (kAffine) gain *= 1.0 + m;
         }
         steps++;
         z_cur = z_exit;

@@ -255,9 +255,14 @@ static int cmp_seg_desc(const void* a, const void* b) {
     return (x < y) - (x > y);
 }
 
-int c5o_render(const double* tet_pts, const double* alpha, const double* q, int64_t n_tets,
-               const double* solid_pts, int64_t n_solid, const c5o_view* v, double* tau, double* inten,
-               uint32_t* steps, uint8_t* solid, uint64_t* total_steps, uint64_t* anomalies) {
+/* The whole pass, shared by c5o_render and c5o_render_segments. tau and inten may be NULL (not
+ * stored); with seg_tet, each pixel's segments are also stored at seg_start[pix] .. seg_start[pix + 1]
+ * in the order I is integrated (r = n - 1 .. 0), and a pixel whose record count differs from that
+ * span makes the pass return -3. */
+static int render_pass(const double* tet_pts, const double* alpha, const double* q, int64_t n_tets,
+                       const double* solid_pts, int64_t n_solid, const c5o_view* v, double* tau, double* inten,
+                       uint32_t* steps, uint8_t* solid, uint64_t* total_steps, uint64_t* anomalies,
+                       const int64_t* seg_start, int32_t* seg_tet, double* seg_dz) {
     grid g;
     size_t n_pix;
     uint8_t* mask = NULL;
@@ -265,10 +270,10 @@ int c5o_render(const double* tet_pts, const double* alpha, const double* q, int6
     size_t* start = NULL;
     rec* csr = NULL;
     int n_thr = 1, t, rc = 0;
-    uint64_t odd = 0, sum_steps = 0;
+    uint64_t odd = 0, sum_steps = 0, mismatch = 0;
     int64_t k;
 
-    if (!v || v->res_x < 2 || v->res_y < 2 || n_tets < 0 || n_tets >= (1 << 28) || !tau || !inten) return -1;
+    if (!v || v->res_x < 2 || v->res_y < 2 || n_tets < 0 || n_tets >= (1 << 28)) return -1;
     n_pix = (size_t)v->res_x * (size_t)v->res_y;
     if (n_pix >= 0xFFFFFFFFu) return -1;
 
@@ -390,7 +395,7 @@ int c5o_render(const double* tet_pts, const double* alpha, const double* q, int6
     }
 
     /* per pixel: face z's, order, integrate */
-#pragma omp parallel num_threads(n_thr) reduction(+ : sum_steps)
+#pragma omp parallel num_threads(n_thr) reduction(+ : sum_steps, mismatch)
     {
         seg* segs = NULL;
         size_t segs_cap = 0;
@@ -402,9 +407,10 @@ int c5o_render(const double* tet_pts, const double* alpha, const double* q, int6
             size_t r;
             double sum, I;
             if (mask[pix]) {
-                tau[pix] = NAN;
-                inten[pix] = NAN;
+                if (tau) tau[pix] = NAN;
+                if (inten) inten[pix] = NAN;
                 if (steps) steps[pix] = 0;
+                if (seg_tet && seg_start[pix + 1] != seg_start[pix]) mismatch++;
                 continue;
             }
             if (steps) steps[pix] = (uint32_t)n;
@@ -435,6 +441,17 @@ int c5o_render(const double* tet_pts, const double* alpha, const double* q, int6
                 segs[r].tet = id;
             }
             if (n > 1) qsort(segs, n, sizeof(seg), cmp_seg_desc);
+            if (seg_tet) {
+                if (seg_start[pix + 1] - seg_start[pix] != (int64_t)n) {
+                    mismatch++;
+                } else {
+                    int64_t o = seg_start[pix];
+                    for (r = n; r-- > 0; o++) {
+                        seg_tet[o] = (int32_t)segs[r].tet;
+                        seg_dz[o] = segs[r].dz;
+                    }
+                }
+            }
 
             sum = 0;
             for (r = 0; r < n; r++) sum = sum + segs[r].dz * alpha[segs[r].tet];
@@ -448,14 +465,15 @@ int c5o_render(const double* tet_pts, const double* alpha, const double* q, int6
                 Cc = Q - a * I;
                 if (!(a < DBL_EPSILON)) I = (Q - Cc * exp(-a * segs[r].dz)) / a;
             }
-            tau[pix] = sum;
-            inten[pix] = I;
+            if (tau) tau[pix] = sum;
+            if (inten) inten[pix] = I;
         }
         free(segs);
     }
     if (solid) memcpy(solid, mask, n_pix);
     if (total_steps) *total_steps = sum_steps;
     if (anomalies) *anomalies = odd;
+    if (mismatch) rc = -3;
 
 done:
     if (lists) {
@@ -468,4 +486,20 @@ done:
     free(g.xs);
     free(g.ys);
     return rc;
+}
+
+int c5o_render(const double* tet_pts, const double* alpha, const double* q, int64_t n_tets,
+               const double* solid_pts, int64_t n_solid, const c5o_view* v, double* tau, double* inten,
+               uint32_t* steps, uint8_t* solid, uint64_t* total_steps, uint64_t* anomalies) {
+    if (!tau || !inten) return -1;
+    return render_pass(tet_pts, alpha, q, n_tets, solid_pts, n_solid, v, tau, inten, steps, solid, total_steps,
+                       anomalies, NULL, NULL, NULL);
+}
+
+int c5o_render_segments(const double* tet_pts, const double* alpha, const double* q, int64_t n_tets,
+                        const double* solid_pts, int64_t n_solid, const c5o_view* v, const int64_t* seg_start,
+                        int32_t* seg_tet, double* seg_dz) {
+    if (!seg_start || !seg_tet || !seg_dz) return -1;
+    return render_pass(tet_pts, alpha, q, n_tets, solid_pts, n_solid, v, NULL, NULL, NULL, NULL, NULL, NULL,
+                       seg_start, seg_tet, seg_dz);
 }

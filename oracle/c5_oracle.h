@@ -48,6 +48,18 @@ int c5o_render(const double* tet_pts, const double* alpha, const double* q, int6
                const double* solid_pts, int64_t n_solid, const c5o_view* v, double* tau, double* inten,
                uint32_t* steps, uint8_t* solid, uint64_t* total_steps, uint64_t* anomalies);
 
+/* The segments c5o_render integrates, per pixel: the same inputs, and seg_start[n_pix + 1], the prefix
+ * sum of the steps a c5o_render call returned (pixel j * res_x + i crosses seg_start[pix + 1] -
+ * seg_start[pix] tets). Pixel pix's segments go to seg_tet / seg_dz [seg_start[pix] ..] in the order
+ * the I recurrence takes them (line.cpp:206-225: the lowest segment first, where the ray enters); the
+ * sum of seg_dz * alpha[seg_tet] in reverse order is its tau. Test infrastructure for an integration
+ * that does not come from the code under test.
+ * Returns 0, -1 on bad arguments, -2 on allocation failure, -3 when a pixel's record count is not
+ * its span of seg_start. */
+int c5o_render_segments(const double* tet_pts, const double* alpha, const double* q, int64_t n_tets,
+                        const double* solid_pts, int64_t n_solid, const c5o_view* v, const int64_t* seg_start,
+                        int32_t* seg_tet, double* seg_dz);
+
 #ifdef __cplusplus
 }
 #endif

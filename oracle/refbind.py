@@ -125,10 +125,10 @@ ACC_X0 = 1.0                      # config.hpp:55
 class Port:
     """The plain-C restatement (oracle/c5_oracle.c)."""
 
-    def __init__(self):
-        if not os.path.exists(PORT_SO):
+    def __init__(self, so=PORT_SO):
+        if so == PORT_SO and not os.path.exists(PORT_SO):
             build("port")
-        lib = C.CDLL(PORT_SO)
+        lib = C.CDLL(so)
         lib.c5o_render.restype = C.c_int
         lib.c5o_render.argtypes = [_dp, _dp, _dp, C.c_int64, _dp, C.c_int64, C.POINTER(_View), _dp, _dp,
                                    _u32p, _u8p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
@@ -138,6 +138,10 @@ class Port:
         lib.c5o_rotate_axis.argtypes = [_dp, C.c_int64, C.c_int, C.c_double, C.c_double]
         lib.c5o_pixel_coords.restype = None
         lib.c5o_pixel_coords.argtypes = [C.POINTER(_View), _dp, _dp]
+        if hasattr(lib, "c5o_render_segments"):   # absent from a library built before it existed
+            lib.c5o_render_segments.restype = C.c_int
+            lib.c5o_render_segments.argtypes = [_dp, _dp, _dp, C.c_int64, _dp, C.c_int64, C.POINTER(_View),
+                                                C.POINTER(C.c_int64), C.POINTER(C.c_int32), _dp]
         self.lib = lib
 
     def rotate(self, pts, X=0.0, Y=0.0, I=0.0):
@@ -185,3 +189,37 @@ class Port:
                           dict(rotate=t_rot, ctor=0.0, find=0.0, trace=time.perf_counter() - t0))
         img.anomalies = int(odd.value)
         return img
+
+    def segments(self, tet_pts, alpha, q, *, res_x, res_y, X=0.0, Y=0.0, I=0.0, alpha_limit=2.5, threads=None,
+                 solid_rot=None, solid_static=None, window=WINDOW, steps=None):
+        """Each pixel's ordered segments, as the I recurrence takes them (the lowest first): pixel
+        j * res_x + i crosses tets seg_tet[seg_start[p]:seg_start[p + 1]] over depths seg_dz[...].
+        Returns (seg_start (n_pix + 1,) int64, seg_tet int32, seg_dz float64). `steps`: the per-pixel
+        step counts of a render() of the same arguments, if already at hand."""
+        if steps is None:
+            steps = self.render(tet_pts, alpha, q, res_x=res_x, res_y=res_y, X=X, Y=Y, I=I,
+                                alpha_limit=alpha_limit, threads=threads, solid_rot=solid_rot,
+                                solid_static=solid_static, window=window).steps
+        threads = threads or (os.cpu_count() or 1)
+        pts = self.rotate(tet_pts, X, Y, I)
+        sol = []
+        if solid_rot is not None and len(solid_rot):
+            sol.append(self.rotate(solid_rot, X, Y, I))
+        if solid_static is not None and len(solid_static):
+            sol.append(np.ascontiguousarray(solid_static, dtype=np.float64))
+        sol = np.concatenate(sol) if sol else None
+        alpha = np.ascontiguousarray(alpha, dtype=np.float64)
+        q = np.ascontiguousarray(q, dtype=np.float64)
+        seg_start = np.zeros(res_x * res_y + 1, dtype=np.int64)
+        np.cumsum(np.asarray(steps, dtype=np.int64).ravel(), out=seg_start[1:])
+        seg_tet = np.zeros(max(int(seg_start[-1]), 1), dtype=np.int32)
+        seg_dz = np.zeros(max(int(seg_start[-1]), 1))
+        v = _View(res_x, res_y, (C.c_double * 4)(*window), alpha_limit, threads)
+        rc = self.lib.c5o_render_segments(_ptr(pts, _dp), _ptr(alpha, _dp), _ptr(q, _dp), pts.shape[0],
+                                          _ptr(sol, _dp), 0 if sol is None else sol.shape[0], C.byref(v),
+                                          _ptr(seg_start, C.POINTER(C.c_int64)), _ptr(seg_tet, C.POINTER(C.c_int32)),
+                                          _ptr(seg_dz, _dp))
+        if rc != 0:
+            raise RuntimeError(f"c5o_render_segments failed rc={rc}")
+        n = int(seg_start[-1])
+        return seg_start, seg_tet[:n], seg_dz[:n]

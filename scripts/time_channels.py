@@ -11,6 +11,9 @@ is ms_walk(K) / (K * ms_walk(1)), below 1 when one K-channel walk is cheaper tha
 line names the GPU, its power limit and max SM clock, read in the same run.
 
     python scripts/time_channels.py --channels 1,2,4,8 --views 20 > profiles/r04_channels_c3_one_b200.jsonl
+
+--fp32 X,Y adds one line: plain renders of C3 at that view with precision = 32 (the FP32 variant, which
+channel renders do not have), medians as above.
 """
 import argparse
 import json
@@ -46,6 +49,7 @@ def main():
     ap.add_argument("--views", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--seed", type=int, default=2026)
+    ap.add_argument("--fp32", default=None, metavar="X,Y", help="also time FP32 plain renders at this view")
     args = ap.parse_args()
     ks = [int(x) for x in args.channels.split(",")]
     print(json.dumps(gpu_info()), flush=True)
@@ -90,6 +94,21 @@ def main():
             if ms_walk_one is not None:
                 line["vs_k_passes"] = walk / (k * ms_walk_one)
             print(json.dumps(line), flush=True)
+        if args.fp32:
+            x, y = (float(c) for c in args.fp32.split(","))
+            v32 = api.make_view(vk["res_x"], vk["res_y"], X=x, Y=y, I=vk["I"], alpha_limit=vk["alpha_limit"],
+                                precision=32)
+            runs = []
+            for v in range(args.warmup + args.views):
+                _, st = ctx.render(v32, out=plain_out)
+                if v >= args.warmup:
+                    runs.append(st)
+            assert runs[-1]["walk_errors"] == 0
+            print(json.dumps(dict(workload="C3", res=[vk["res_x"], vk["res_y"]], precision=32, X=x, Y=y,
+                                  views=args.views, warmup=args.warmup, no_zero_copy=1,
+                                  tet_steps=int(runs[-1]["tet_steps"]), ms_walk=median(runs, "ms_walk"),
+                                  ms_graze=median(runs, "ms_graze"), ms_total=median(runs, "ms_total"),
+                                  ms_d2h=median(runs, "ms_d2h"))), flush=True)
 
 
 if __name__ == "__main__":

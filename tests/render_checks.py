@@ -140,6 +140,26 @@ def check_uniform_medium_kat(lib, n=6, res=(96, 72)):
         assert np.allclose(img.inten[hit], want, rtol=1e-11, atol=1e-14)
 
 
+def check_constant_medium_decades(lib, alphas, *, precision=64, n=8, res=(96, 72)):
+    """A constant medium (alpha, Q = 0.75, no clamp) has the closed form I = Q L (-expm1(-alpha L)) / (alpha L)
+    with L = tau / alpha, across the optical-depth range. Gates of tests/parity.py against the exact
+    integration; L comes from the same depths as I, so this sees the step, not the FP32 geometry."""
+    from parity import ABS_FLOOR_FP32, FLOOR_EXACT, REL_TOL_EXACT, exact_margin
+    rel, floor = (REL_TOL_FP32, ABS_FLOOR_FP32) if precision == 32 else (REL_TOL_EXACT, FLOOR_EXACT)
+    mesh = synth.kuhn_cube(n, seed=8, scalars="const")
+    for a in alphas:
+        with api.Context(devices=(0,), lib=lib) as ctx:
+            ctx.upload_mesh(mesh.points, mesh.tets, np.full(mesh.n_tets, a), mesh.q)
+            img = ctx.render_raw(api.make_view(res[0], res[1], lib=lib, X=0.35, Y=0.8, alpha_limit=1e30,
+                                               round_through_float=0, precision=precision))
+        hit = img.hit
+        x = img.tau[hit]                   # alpha L
+        want = 0.75 * (x / a) * (-np.expm1(-x) / x)
+        m = exact_margin(img.inten[hit], want, rel=rel, floor=floor)
+        assert m.max() <= 1.0, (f"alpha {a:g}, precision {precision}: {int((m > 1).sum())} pixels off the closed "
+                                f"form, worst relative error {m.max() * rel:.2e}")
+
+
 def check_scaling_properties(lib, mesh, res_x, res_y, flags):
     """Size-independent properties: tau is linear in alpha and I is linear in Q, and scaling by a
     power of two is exact in binary floating point, so both hold BIT FOR BIT."""
