@@ -89,6 +89,8 @@ SYMBOLS = {
     "c5_render_channels": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _u32p, _u8p, C.POINTER(Stats)]),
     "c5_render_flux": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, _dp, _dp, C.POINTER(Stats)]),
     "c5_render_flux_submit": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, _dp, _dp, _u64p]),
+    "c5_update_fields": (C.c_int, [C.c_void_p, _dp, _dp]),
+    "c5_render_grad": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _dp, _dp, _dp, C.POINTER(Stats)]),
     "c5_render_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_last_row_cost": (C.c_int, [C.c_void_p, _u64p, C.c_int32]),
     "c5_kernel_launches": (C.c_uint64, [C.c_void_p]),
@@ -105,7 +107,7 @@ SYMBOLS = {
 }
 IPC_HANDLE_BYTES = 80
 MAX_IN_FLIGHT = 8
-ABI_VERSION = 4        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
+ABI_VERSION = 5        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
 TIMELINE_PHASES = 6
 
 
@@ -233,6 +235,7 @@ class Context:
         if alpha.shape != (tets.shape[0],) or q.shape != (tets.shape[0],):
             raise ValueError("alpha and q must have one value per tet")
         self._n_channels = 0  # a new mesh drops the channels, also when its upload fails
+        self._fields_version = self.fields_version + 1
         self._check(self.lib.c5_upload_mesh(self._h, _ptr(points, _dp), points.shape[0], _ptr(tets, _i32p),
                                             tets.shape[0], _ptr(alpha, _dp), _ptr(q, _dp)))
         return self.mesh_info()
@@ -344,6 +347,45 @@ class Context:
             self._flux_in_flight = {}
         self._flux_in_flight[int(ticket.value)] = (rows, total)
         return int(ticket.value), rows, total
+
+    def update_fields(self, alpha, q):
+        """Replaces the cells' own alpha and Q (one value per tet, in the order given to upload_mesh)
+        without rebuilding topology or BVH (c5_update_fields)."""
+        alpha = np.ascontiguousarray(alpha, dtype=np.float64)
+        q = np.ascontiguousarray(q, dtype=np.float64)
+        n_tets = self.mesh_info().n_tets  # 0 before upload_mesh: the library reports that
+        if alpha.ndim != 1 or alpha.shape != q.shape or (n_tets and alpha.shape[0] != n_tets):
+            raise ValueError("alpha and q need one value per tet of the uploaded mesh")
+        self._fields_version = self.fields_version + 1
+        self._check(self.lib.c5_update_fields(self._h, _ptr(alpha, _dp), _ptr(q, _dp)))
+
+    @property
+    def fields_version(self) -> int:
+        """Counts the uploads of the cells' own fields (upload_mesh, update_fields) through this context
+        (a sibling's are its parent's): autograd.render compares it to know whether its fields are still
+        the context's."""
+        owner = getattr(self, "_parent", None) or self
+        return getattr(owner, "_fields_version", 0)
+
+    def render_grad(self, view: View, g, *, image: bool = False, alpha: bool = True, q: bool = True):
+        """Vector-Jacobian product of the pre-cast image against g, shape (res_y, res_x, 2) with {g_tau, g_I}
+        per pixel (c5_render_grad; the view needs round_through_float = 0). Returns (grad_alpha, grad_q),
+        each of shape (n_tets,) in the order given to upload_mesh (None for one that was not asked for),
+        and with image=True also the (res_y, res_x, 2) {tau, I} image of render_raw. Gradients are summed
+        with atomics: equal to rounding, not bit for bit, from run to run."""
+        g = np.ascontiguousarray(g, dtype=np.float64)
+        if g.size != view.res_y * view.res_x * 2:
+            raise ValueError("g must hold res_y * res_x * 2 doubles")
+        owner = getattr(self, "_parent", None) or self  # a sibling reports its parent's mesh only once it has rendered
+        n_tets = owner.mesh_info().n_tets
+        ga = np.empty(n_tets, dtype=np.float64) if alpha else None
+        gq = np.empty(n_tets, dtype=np.float64) if q else None
+        out = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64) if image else None
+        st = Stats()
+        self._check(self.lib.c5_render_grad(self._h, C.byref(view), _ptr(g, _dp), _ptr(ga, _dp), _ptr(gq, _dp),
+                                            _ptr(out, _dp), C.byref(st)))
+        self.last_stats = st.as_dict()
+        return (ga, gq, out) if image else (ga, gq)
 
     def render_raw(self, view: View) -> RawImage:
         out = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64)

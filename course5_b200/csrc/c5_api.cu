@@ -174,11 +174,27 @@ void mesh_pixel_rect(const DeviceState& d, const c5_view* v, const ViewPlan& p, 
     w.j_end = pixel(hi[1], p.y_min, p.step_y, v->res_y, true) + 1;
 }
 
+// The walk of view v's band: what every pass over its rays shares.
+WalkLaunch view_walk(const DeviceState& d, const c5_view* v, const ViewPlan& p) {
+    WalkLaunch w{};
+    w.res_x = v->res_x;
+    w.res_y = v->res_y;
+    w.row_begin = p.row_begin;
+    w.row_end = p.row_end;
+    w.alpha_limit = v->alpha_limit;
+    w.round_through_float = v->round_through_float;
+    w.use_mask = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0 ? 1 : 0;
+    w.precision = v->precision ? v->precision : 64;
+    mesh_pixel_rect(d, v, p, w);
+    return w;
+}
+
 // Enqueues one view's kernels for rows [row_begin,row_end) on device d. Events:
 // 0 start, 1 rotated, 2 bvh, 3 mask, 4 walk.
 // channels > 0: the walk integrates that many uploaded channels (c5_render_channels).
+// pass = kDepthPass: the first pass of c5_render_grad ({tau, I, lam, 0} per pixel into d.out).
 void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want_steps, double* out_override = nullptr,
-                  int channels = 0) {
+                  int channels = 0, int pass = kImagePass) {
     use_device(d);
     g_launch_counter = &d.launches;
     ensure_pixel_tables(d, v, p);
@@ -187,12 +203,12 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     // synchronisation) and a cudaMalloc on the spot.
     const size_t n_pix = static_cast<size_t>(v->res_y) * v->res_x;
     const bool solids = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0;
-    const size_t words = 2 * static_cast<size_t>(channels ? channels : 1); // doubles per pixel
+    const size_t words = 2 * static_cast<size_t>(channels ? channels : pass == kDepthPass ? 2 : 1); // doubles per pixel
     if (!out_override) d.out.ensure(words * n_pix);
     if (want_steps) d.steps.ensure(n_pix);
     d.counters.ensure(kNumCounters);
     d.queue.ensure(n_pix); // every ray may be deferred (reserved, hardly ever touched)
-    if (channels) d.ch_queue.ensure(words * n_pix);
+    if (channels || pass == kDepthPass) d.ch_queue.ensure(words * n_pix);
     d.row_cost.ensure(static_cast<size_t>(v->res_y));
     if (solids) d.mask.ensure(n_pix);
 
@@ -214,17 +230,10 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     timeline_mark(d, 3);
     dev_zero(d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
     dev_zero(d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
-    WalkLaunch w{};
-    w.res_x = v->res_x;
-    w.res_y = v->res_y;
-    w.row_begin = p.row_begin;
-    w.row_end = p.row_end;
-    w.alpha_limit = v->alpha_limit;
-    w.round_through_float = v->round_through_float;
-    w.use_mask = solids ? 1 : 0;
+    WalkLaunch w = view_walk(d, v, p);
     w.write_steps = want_steps ? 1 : 0;
-    w.precision = v->precision ? v->precision : 64;
     w.channels = channels;
+    w.pass = pass;
     w.out = out_override ? out_override : d.out.p;
     w.mark_walk_done = d.ev_walk;
     w.mark_walk_done_tl = nullptr;
@@ -232,7 +241,6 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
         const size_t n = d.tl_events.size() / kTimelinePhases;
         w.mark_walk_done_tl = d.tl_events[(d.tl_views % n) * kTimelinePhases + 4];
     }
-    mesh_pixel_rect(d, v, p, w);
     if (!kHostSim) { // a band the mesh does not reach launches no walk kernels: the markers are recorded anyway
         C5_CUDA(cudaEventRecord(d.ev_walk, d.stream));
         if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
@@ -438,6 +446,33 @@ ViewResult wait_view(c5_ctx* lane) {
     return read_view(d, lane->pending.view, lane->pending.plan, true, lane->pending.flux_pairs);
 }
 
+// The stats of one view rendered as bands by several devices: counters and row costs add up, phase
+// times are the slowest device's.
+ViewResult merge_results(const std::vector<ViewResult>& results, int res_y) {
+    ViewResult total;
+    c5_stats& t = total.st;
+    total.row_cost.assign(static_cast<size_t>(res_y), 0);
+    for (const ViewResult& r : results) {
+        const c5_stats& s = r.st;
+        t.pixels += s.pixels;
+        t.tet_steps += s.tet_steps;
+        t.hit_pixels += s.hit_pixels;
+        t.solid_pixels += s.solid_pixels;
+        t.walk_errors += s.walk_errors;
+        t.grazing_rays += s.grazing_rays;
+        t.ms_rotate = std::max(t.ms_rotate, s.ms_rotate);
+        t.ms_bvh = std::max(t.ms_bvh, s.ms_bvh);
+        t.ms_mask = std::max(t.ms_mask, s.ms_mask);
+        t.ms_walk = std::max(t.ms_walk, s.ms_walk);
+        t.ms_graze = std::max(t.ms_graze, s.ms_graze);
+        t.ms_d2h = std::max(t.ms_d2h, s.ms_d2h);
+        t.ms_total = std::max(t.ms_total, s.ms_total);
+        for (size_t j = 0; j < total.row_cost.size(); j++) total.row_cost[j] += r.row_cost[j];
+    }
+    t.n_devices = static_cast<int32_t>(results.size());
+    return total;
+}
+
 // Multi-device contexts (c5_create with several devices): the context and each of its parts render
 // one cost-balanced row band, as c5_render does for a row band, straight into its final rows of the
 // caller's buffers. One host thread per device submits: a copy into pageable memory blocks the
@@ -484,28 +519,7 @@ void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* s
     for (auto& e : errors) {
         if (e) std::rethrow_exception(e);
     }
-    // counters and row costs add up, phase times are the slowest device's
-    ViewResult total;
-    c5_stats& t = total.st;
-    total.row_cost.assign(static_cast<size_t>(v->res_y), 0);
-    for (const ViewResult& r : results) {
-        const c5_stats& s = r.st;
-        t.pixels += s.pixels;
-        t.tet_steps += s.tet_steps;
-        t.hit_pixels += s.hit_pixels;
-        t.solid_pixels += s.solid_pixels;
-        t.walk_errors += s.walk_errors;
-        t.grazing_rays += s.grazing_rays;
-        t.ms_rotate = std::max(t.ms_rotate, s.ms_rotate);
-        t.ms_bvh = std::max(t.ms_bvh, s.ms_bvh);
-        t.ms_mask = std::max(t.ms_mask, s.ms_mask);
-        t.ms_walk = std::max(t.ms_walk, s.ms_walk);
-        t.ms_graze = std::max(t.ms_graze, s.ms_graze);
-        t.ms_d2h = std::max(t.ms_d2h, s.ms_d2h);
-        t.ms_total = std::max(t.ms_total, s.ms_total);
-        for (size_t j = 0; j < total.row_cost.size(); j++) total.row_cost[j] += r.row_cost[j];
-    }
-    t.n_devices = static_cast<int32_t>(n);
+    ViewResult total = merge_results(results, v->res_y);
     if (flux) {
         const size_t words = results[0].flux.size() / static_cast<size_t>(v->res_y);
         std::vector<double> rows(words * static_cast<size_t>(v->res_y), 0.0);
@@ -517,6 +531,79 @@ void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* s
         deliver_flux(rows, words, *flux);
     }
     report(ctx, total, st);
+}
+
+// ---- gradients (c5_render_grad) ------------------------------------------------------------------------
+
+// What one device returns for its band of a gradient render: the depth pass's stats and the band's
+// gradients, in the file order of the tets.
+struct GradResult {
+    ViewResult view;
+    std::vector<double> grad_alpha, grad_q; // empty unless asked for
+};
+
+// Band [row_begin,row_end) of v on ctx's device: the view prologue and the depth pass (enqueue_view),
+// then the gradient pass over the same rays, then the copies. Blocks until the results are on the host.
+// Events: 0..4 as for an image, 5 depth pass done, 6 gradients on the host.
+GradResult grad_band(c5_ctx* ctx, const c5_view* v, const double* g, bool want_alpha, bool want_q, double* out) {
+    follow_parent(ctx);
+    if (ctx->pending.active) fail(C5_E_STATE, "render_grad: this context still has a view in flight (c5_render_wait it first)");
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    const ViewPlan p = plan_view(v);
+    DeviceState& d = ctx->dev;
+    use_device(d);
+    const size_t n_t = static_cast<size_t>(d.n_tets);
+    const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
+    const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
+    ensure_host_staging(d, static_cast<size_t>(v->res_y));
+    // the gradient pass counts into the second half, so that the stats stay the depth pass's
+    d.counters.ensure(2 * kNumCounters);
+    d.row_cost.ensure(2 * static_cast<size_t>(v->res_y));
+    d.grad_alpha.ensure(n_t);
+    d.grad_q.ensure(n_t);
+    d.grad_in.ensure(2 * static_cast<size_t>(v->res_y) * v->res_x);
+    enqueue_view(d, v, p, false, nullptr, 0, kDepthPass);
+    record(d, 5);
+    dev_zero(d.grad_alpha.p, n_t * sizeof(double), d.stream);
+    dev_zero(d.grad_q.p, n_t * sizeof(double), d.stream);
+    dev_zero(d.counters.p + kNumCounters, kNumCounters * sizeof(unsigned long long), d.stream);
+    dev_zero(d.row_cost.p + v->res_y, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
+    h2d(d.grad_in.p, g + 2 * band_off, 2 * n_pix_band * sizeof(double), d.stream);
+    WalkLaunch w = view_walk(d, v, p);
+    w.pass = kGradPass;
+    w.depth = d.out.p;
+    w.grad_in = d.grad_in.p;
+    w.grad_alpha = d.grad_alpha.p;
+    w.grad_q = d.grad_q.p;
+    w.counters = d.counters.p + kNumCounters;
+    w.row_cost = d.row_cost.p + v->res_y;
+    launch_walk(d, w);
+    std::vector<double> morton[2];
+    for (int k = 0; k < 2; k++) {
+        if (!(k == 0 ? want_alpha : want_q)) continue;
+        morton[k].resize(n_t);
+        d2h(morton[k].data(), (k == 0 ? d.grad_alpha : d.grad_q).p, n_t * sizeof(double), d.stream);
+    }
+    record(d, 6);
+    d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
+    d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
+    std::vector<double> band(out ? 4 * n_pix_band : 0); // the depth pass's {tau, I, lam, 0} per pixel
+    if (out) d2h(band.data(), d.out.p, band.size() * sizeof(double), d.stream);
+    stream_sync(d.stream);
+    for (size_t k = 0; k < band.size() / 4; k++) { // its first pair is the image of c5_render_raw
+        out[2 * (band_off + k)] = band[4 * k];
+        out[2 * (band_off + k) + 1] = band[4 * k + 1];
+    }
+    GradResult r;
+    const std::vector<uint32_t>& tperm = (d.origin ? *d.origin : d).tperm; // new -> old tet
+    for (int k = 0; k < 2; k++) {
+        if (morton[k].empty()) continue;
+        std::vector<double>& file = k == 0 ? r.grad_alpha : r.grad_q;
+        file.resize(n_t);
+        for (size_t t = 0; t < n_t; t++) file[tperm[t]] = morton[k][t];
+    }
+    r.view = read_view(d, *v, p, true);
+    return r;
 }
 
 // The lanes of c5_render_submit: lane 0 is the context itself, the others are sibling contexts the
@@ -980,6 +1067,81 @@ int c5_render_channels(c5_ctx* ctx, const c5_view* view, double* out, uint32_t* 
         submit_view(ctx, view, out, steps, solid_mask, 0, true, true);
         ViewResult r = wait_view(ctx);
         report(ctx, r, stats);
+    });
+}
+
+int c5_update_fields(c5_ctx* ctx, const double* alpha, const double* q) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (ctx->parent) fail(C5_E_STATE, "update_fields: a sibling context shares its parent's fields; update through the parent");
+        if (!alpha || !q) fail(C5_E_INVALID, "update_fields: NULL array");
+        if (!ctx->has_mesh) fail(C5_E_STATE, "update_fields: no mesh uploaded");
+        for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
+            if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "update_fields: a submitted view is in flight");
+        }
+        if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize()); // siblings may be rendering from them
+        ctx->dev.mesh_version++; // siblings and lanes re-alias at their next render
+        for (c5_ctx* c : with_parts(ctx)) {
+            use_device(c->dev);
+            g_launch_counter = &c->dev.launches;
+            update_fields(c->dev, alpha, q);
+        }
+    });
+}
+
+int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* grad_alpha, double* grad_q, double* out,
+                   c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (!g) fail(C5_E_INVALID, "render_grad: g is NULL");
+        if (!grad_alpha && !grad_q) fail(C5_E_INVALID, "render_grad: grad_alpha and grad_q are both NULL");
+        if (view && view->precision == 32) fail(C5_E_INVALID, "render_grad: FP64 only (precision 64)");
+        if (view && view->round_through_float) {
+            fail(C5_E_INVALID, "render_grad: the float cast has no useful derivative; set round_through_float = 0");
+        }
+        follow_parent(ctx);
+        if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+        const ViewPlan p = plan_view(view);
+        const std::vector<c5_ctx*> parts = with_parts(ctx);
+        const size_t n = parts.size();
+        if (static_cast<size_t>(p.row_end - p.row_begin) < n) fail(C5_E_INVALID, "render: fewer rows than devices");
+        const auto bands = cut_bands(ctx, view, p, static_cast<int>(n));
+        std::vector<c5_view> band_views(n, *view);
+        std::vector<GradResult> results(n);
+        std::vector<std::exception_ptr> errors(n);
+        auto run = [&](size_t r) {
+            try {
+                band_views[r].row_begin = bands[r].first;
+                band_views[r].row_end = bands[r].second;
+                results[r] = grad_band(parts[r], &band_views[r], g, grad_alpha != nullptr, grad_q != nullptr, out);
+            } catch (...) {
+                errors[r] = std::current_exception();
+            }
+        };
+        if (kHostSim || n == 1) {
+            for (size_t r = 0; r < n; r++) run(r);
+        } else {
+            std::vector<std::thread> workers;
+            for (size_t r = 0; r < n; r++) workers.emplace_back(run, r);
+            for (auto& w : workers) w.join();
+        }
+        for (auto& e : errors) {
+            if (e) std::rethrow_exception(e);
+        }
+        // each device summed its own band: add them in device order
+        const size_t n_t = static_cast<size_t>(ctx->info.n_tets);
+        for (int k = 0; k < 2; k++) {
+            double* dst = k == 0 ? grad_alpha : grad_q;
+            if (!dst) continue;
+            for (size_t r = 0; r < n; r++) {
+                const std::vector<double>& src = k == 0 ? results[r].grad_alpha : results[r].grad_q;
+                for (size_t t = 0; t < n_t; t++) dst[t] = r == 0 ? src[t] : dst[t] + src[t];
+            }
+        }
+        std::vector<ViewResult> views(n);
+        for (size_t r = 0; r < n; r++) views[r] = std::move(results[r].view);
+        ViewResult total = n == 1 ? std::move(views[0]) : merge_results(views, view->res_y);
+        report(ctx, total, stats);
     });
 }
 

@@ -85,6 +85,8 @@ struct DeviceState {
     DevBuf<DeferredRay> queue;       // grazing rays of the current view (capacity: pixels of the band)
     DevBuf<double> ch_queue;         // their channel values {tau, I} (channel renders only)
     DevBuf<double> row_flux;         // flux renders: [res_y][pairs] {sum tau, sum I} of the band's rows
+    DevBuf<double> grad_alpha, grad_q; // c5_render_grad: [n_tets] Morton order, this device's band only
+    DevBuf<double> grad_in;          // c5_render_grad: the band's {g_tau, g_I} per pixel
     int sm_count = 0;
     cudaEvent_t ev_walk = nullptr;   // between the pixel kernel and the grazing-ray kernel (phase times)
     cudaEvent_t ev_done = nullptr;   // after the view's last copy: what c5_render_wait waits for
@@ -169,6 +171,8 @@ void launch_prepare_channels(DeviceState& d, double alpha_limit); // the same fo
 
 // c5_topology.cu — places n channels of file-order fields (channel-major) in ch_rec / ch_q0.
 void upload_channels(DeviceState& d, const double* alpha, const double* q, int n);
+// c5_topology.cu — replaces cells[].alpha and q0 by file-order fields (c5_update_fields).
+void update_fields(DeviceState& d, const double* alpha, const double* q);
 
 // c5_walk.cu
 struct WalkLaunch {
@@ -183,7 +187,18 @@ struct WalkLaunch {
     double* out; // {tau, I} per pixel (per channel) of the band, x fastest
     cudaEvent_t mark_walk_done;    // recorded between the pixel kernel and the grazing-ray kernel (may be null)
     cudaEvent_t mark_walk_done_tl; // the same moment for the timeline ring (may be null)
+    // c5_render_grad (channels 0, precision 64): kDepthPass stores {tau, I, lam, 0} per pixel into out;
+    // kGradPass reads them (depth) and the band's {g_tau, g_I} (grad_in), adds into grad_alpha / grad_q,
+    // stores no pixel and counts into its own counters / row_cost
+    int pass;
+    const double* depth;
+    const double* grad_in;
+    double* grad_alpha;
+    double* grad_q;
+    unsigned long long* counters;
+    unsigned long long* row_cost;
 };
+enum WalkPass { kImagePass = 0, kDepthPass = 1, kGradPass = 2 };
 void launch_walk(DeviceState& d, const WalkLaunch& w);
 // c5_flux.cu — row_flux[j] for the rows [row_begin,row_end) of d.out (pairs {tau, I} per pixel),
 // skipping pixels under d.mask when use_mask; the summation order is documented there.

@@ -314,6 +314,31 @@ struct ChannelGatherOp {
     }
 };
 
+// The alpha of channel record t (stride channel_stride(1)) into cell t: c5_update_fields gathers the
+// cells' new fields as one channel, then moves alpha beside the topology.
+struct CellAlphaOp {
+    const double* rec;
+    Cell* cells;
+    C5_HD void operator()(int64_t t) const { cells[t].alpha = rec[t * channel_stride(1)]; }
+};
+
+// n channel-major arrays of file-order alpha and q: record t of rec gets {alpha_c, 0} of old tet
+// tperm[t] for every channel, q0 gets Q in Morton order. Shared by c5_upload_channels and c5_update_fields.
+void gather_file_order(DeviceState& d, const double* alpha, const double* q, int n, double* rec, double* q0) {
+    cudaStream_t s = d.stream;
+    const size_t n_t = static_cast<size_t>(d.n_tets), n_all = n_t * static_cast<size_t>(n);
+    DevBuf<double> alpha_in, q_in;
+    DevBuf<uint32_t> tperm;
+    alpha_in.alloc(n_all);
+    q_in.alloc(n_all);
+    tperm.alloc(n_t);
+    h2d(alpha_in.p, alpha, alpha_in.bytes(), s);
+    h2d(q_in.p, q, q_in.bytes(), s);
+    h2d(tperm.p, d.tperm.data(), tperm.bytes(), s);
+    for_each(s, d.n_tets, ChannelGatherOp{alpha_in.p, q_in.p, tperm.p, d.n_tets, n, rec, q0});
+    stream_sync(s); // the staging buffers are freed on return
+}
+
 } // namespace
 
 void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t* tets, int64_t n_tets,
@@ -514,21 +539,20 @@ void upload_channels(DeviceState& d, const double* alpha, const double* q, int n
     d.n_channels = 0;
     d.ch_limit_valid = false;
     if (n == 0) return;
-    cudaStream_t s = d.stream;
-    const size_t n_t = static_cast<size_t>(d.n_tets), n_all = n_t * static_cast<size_t>(n);
-    DevBuf<double> alpha_in, q_in;
-    DevBuf<uint32_t> tperm;
-    alpha_in.alloc(n_all);
-    q_in.alloc(n_all);
-    tperm.alloc(n_t);
-    h2d(alpha_in.p, alpha, alpha_in.bytes(), s);
-    h2d(q_in.p, q, q_in.bytes(), s);
-    h2d(tperm.p, d.tperm.data(), tperm.bytes(), s);
+    const size_t n_t = static_cast<size_t>(d.n_tets);
     d.ch_rec.alloc(n_t * static_cast<size_t>(channel_stride(n)));
-    d.ch_q0.alloc(n_all);
-    for_each(s, d.n_tets, ChannelGatherOp{alpha_in.p, q_in.p, tperm.p, d.n_tets, n, d.ch_rec.p, d.ch_q0.p});
-    stream_sync(s);
+    d.ch_q0.alloc(n_t * static_cast<size_t>(n));
+    gather_file_order(d, alpha, q, n, d.ch_rec.p, d.ch_q0.p);
     d.n_channels = n;
+}
+
+void update_fields(DeviceState& d, const double* alpha, const double* q) {
+    DevBuf<double> rec;
+    rec.alloc(static_cast<size_t>(d.n_tets) * channel_stride(1));
+    gather_file_order(d, alpha, q, 1, rec.p, d.q0.p);
+    for_each(d.stream, d.n_tets, CellAlphaOp{rec.p, d.cells.p});
+    stream_sync(d.stream);
+    d.cells_limit_valid = false; // cells[].s is derived again from the new q0 at the next render
 }
 
 } // namespace c5

@@ -73,6 +73,15 @@ struct WalkParams {
     double* ch_queue;     // [deferred ray][K] {tau, I}: the channel values DeferredRay::tau/inten hold otherwise
 };
 
+// The gradient pass's kernels take these (the walk functions see the WalkParams part; the gradient
+// policy below casts back). A separate type keeps WalkParams, and so every other kernel, as it was.
+struct GradParams : WalkParams {
+    const double* grad_in; // band buffer: {g_tau, g_I} per pixel, indexed like out
+    const double* depth;   // the depth pass's band buffer: {tau, I, lam, 0} per pixel
+    double* grad_alpha;    // [n_tets] Morton order, accumulated with atomics
+    double* grad_q;
+};
+
 // ---- loads through the read-only path ----------------------------------------------------------
 struct CellData {
     int4 v, nbr, apex;
@@ -562,12 +571,15 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
 //   F::K                   {tau, I} pairs per pixel, stored at out[((j - row_begin) * res_x + i) * K + c];
 //   F::crossing<kAffine>   the crossing that integrates them into a Pairs<K>;
 //   F::kChanQueue          a deferred ray's values wait in WalkParams::ch_queue and DeferredRay::tau/inten
-//                          stay 0; otherwise they wait in DeferredRay::tau/inten.
+//                          stay 0; otherwise they wait in DeferredRay::tau/inten;
+//   F::kImage              the pixels are stored (false: the gradient pass, whose result is its atomics).
+// crossing() also gets the ray's pixel (j * res_x + i); only the gradient pass reads it.
 struct CellsF64 { // the cells' own fields
     static constexpr int K = 1;
     static constexpr bool kChanQueue = false;
+    static constexpr bool kImage = true;
     template <bool kAffine>
-    static C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<1>& v,
+    static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<1>& v,
                                  uint32_t& steps, uint32_t& error) {
         CellFields<kAffine> acc{v};
         return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
@@ -577,8 +589,9 @@ struct CellsF64 { // the cells' own fields
 struct CellsF32 { // the cells' own fields, FP32 step geometry
     static constexpr int K = 1;
     static constexpr bool kChanQueue = false;
+    static constexpr bool kImage = true;
     template <bool kAffine>
-    static C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<1>& v,
+    static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<1>& v,
                                  uint32_t& steps, uint32_t& error) {
         return crossing_f32<kAffine>(P, px, py, leaf, z_in, v.tau[0], v.inten[0], v.gain[0], steps, error);
     }
@@ -590,11 +603,161 @@ template <int N>
 struct Channels {
     static constexpr int K = N;
     static constexpr bool kChanQueue = true;
+    static constexpr bool kImage = true;
     template <bool kAffine>
-    static C5_HD double crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<K>& v,
+    static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<K>& v,
                                  uint32_t& steps, uint32_t& error) {
         ChanFields<K, kAffine> acc{P.rec, v};
         return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
+    }
+};
+
+// ---- gradients (c5_render_grad) ------------------------------------------------------------------------
+// The vector-Jacobian product of the pre-cast image with respect to every cell's alpha and Q, in two
+// passes over the same rays (DESIGN.md §5c). With a^ = min(alpha, limit), x = a^ dz, m = expm1(-x) and
+// e = 1 + m, a segment does I_out = I_in - (s - I_in) m, s = Q / a^, so
+//   dtau/dalpha  = dz                                       (every segment: tau uses the unclamped alpha)
+//   dI_out/dQ    = -m / a^                                   (a^ >= DBL_EPSILON; else the step is skipped)
+//   dI_out/dalpha = s a^ dz^2 f(x) - I_in dz e,  f(x) = ((1 + x) e^-x - 1) / x^2   (and alpha <= limit)
+// and a change of I_out reaches the viewer times T = exp(-(lam_ray - lam_through)): lam is the clamped
+// optical depth, the sum of x over the segments that change I, lam_ray its value for the whole ray and
+// lam_through its running value at the segment's exit. The difference of the two sums, unlike a ratio of
+// gains, does not underflow on an opaque ray.
+//   Depth pass (CellsDepth): the image of CellsF64 plus lam_ray, as a second pair {lam, 0} per pixel.
+//   Gradient pass (CellsGrad): the same rays again, carrying {lam_through, I}, adding into grad_alpha /
+//   grad_q with FP64 atomics. It defers exactly the rays the depth pass deferred: same search, same budget.
+
+// The clamped depth one segment adds (0 where the step leaves I alone). Both passes add the same rounded
+// product, so the last segment of a ray the pixel kernel finishes sees T = exp(0) = 1 exactly (a grazing
+// ray's sums are grouped by crossing and may differ in the last bits).
+C5_HD double lam_term(double alpha, double limit, double dzv) {
+    double a_c = alpha;
+    if (a_c > limit) a_c = limit;
+    return a_c < DBL_EPSILON ? 0.0 : mul_rn(a_c, dzv);
+}
+
+// f(x) = ((1 + x) e^-x - 1) / x^2 for x >= 0, m = expm1(-x). The numerator cancels to O(x^2) near 0, so
+// below 1/2 the Taylor series sum_{n>=2} (-1)^(n+1) (n-1)/n! x^(n-2) is summed instead (16 terms: the
+// next one is below 3e-18 relative); above, (1 + x)(1 + m) - 1 loses at most one digit.
+C5_HD double grad_f(double x, double m) {
+    if (x < 0.5) {
+        constexpr double c[16] = {-1.0 / 2.0, 1.0 / 3.0, -1.0 / 8.0, 1.0 / 30.0, -1.0 / 144.0, 1.0 / 840.0,
+                                  -1.0 / 5760.0, 1.0 / 45360.0, -1.0 / 403200.0, 1.0 / 3991680.0, -1.0 / 43545600.0,
+                                  1.0 / 518918400.0, -1.0 / 6706022400.0, 1.0 / 93405312000.0,
+                                  -1.0 / 1394852659200.0, 1.0 / 22230464256000.0};
+        double r = c[15];
+#pragma unroll
+        for (int k = 14; k >= 0; k--) r = r * x + c[k];
+        return r;
+    }
+    return ((1.0 + x) * (1.0 + m) - 1.0) / (x * x);
+}
+
+C5_HD void add_to(double* p, double v) {
+#ifdef __CUDA_ARCH__
+    atomicAdd(p, v);
+#else
+    *p += v;
+#endif
+}
+
+// What the gradient pass knows about a ray before it walks it: its upstream gradient and lam_ray.
+struct GradRay {
+    double g_tau, g_I, lam_ray;
+};
+
+C5_HD GradRay grad_ray(const GradParams& P, uint32_t pixel) {
+    const size_t o = pixel - static_cast<size_t>(P.row_begin) * static_cast<size_t>(P.res_x);
+    return GradRay{P.grad_in[2 * o], P.grad_in[2 * o + 1], P.depth[4 * o + 2]};
+}
+
+// One segment of the gradient pass through tet t; lam and inten are the ray's lam_through and I.
+C5_HD void grad_segment(const GradParams& P, int t, double alpha, double s, double dzv, const GradRay& r, double& lam,
+                        double& inten) {
+    double ga = r.g_tau * dzv;
+    double gq = 0.0;
+    double a_c = alpha;
+    if (a_c > P.alpha_limit) a_c = P.alpha_limit;
+    if (!(a_c < DBL_EPSILON)) {
+        const double x = mul_rn(a_c, dzv);
+        const double m = expm1(-x);
+        lam += x;
+        const double gt = r.g_I * exp(lam - r.lam_ray); // g_I T
+        gq = gt * (-m / a_c);
+        if (alpha <= P.alpha_limit) ga += gt * (s * x * dzv * grad_f(x, m) - inten * dzv * (1.0 + m));
+        inten = inten - (s - inten) * m;
+    }
+    if (ga != 0.0) add_to(P.grad_alpha + t, ga);
+    if (gq != 0.0) add_to(P.grad_q + t, gq);
+}
+
+// Depth pass: pair 0 is CellFields' {tau, I} (the same operations, so the same bits), tau[1] is lam.
+template <bool kAffine>
+struct DepthFields {
+    Pairs<2>& v;
+    C5_HD void fetch(int) {}
+    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
+        segment<kAffine>(c.alpha, c.s, P.alpha_limit, dzv, v.tau[0], v.inten[0], v.gain[0]);
+        v.tau[1] += lam_term(c.alpha, P.alpha_limit, dzv);
+    }
+};
+
+// A crossing of a grazing ray walked without the I it arrives with: tau[0] is its lam, inten[0] + gain[0] I
+// its exit I (the gradient kernel's first walk of a crossing).
+struct LamFields {
+    Pairs<1>& v;
+    C5_HD void fetch(int) {}
+    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
+        double tau = 0.0;
+        segment<true>(c.alpha, c.s, P.alpha_limit, dzv, tau, v.inten[0], v.gain[0]);
+        v.tau[0] += lam_term(c.alpha, P.alpha_limit, dzv);
+    }
+};
+
+// Gradient pass: tau[0] is lam_through, inten[0] is I, both from the ray's entry (or the deferred ray's state).
+struct GradFields {
+    const GradParams& G;
+    Pairs<1>& v;
+    GradRay r;
+    int t;
+    C5_HD void fetch(int t_) { t = t_; }
+    C5_HD void step(const WalkParams&, const CellData& c, double dzv) {
+        grad_segment(G, t, c.alpha, c.s, dzv, r, v.tau[0], v.inten[0]);
+    }
+};
+
+struct CellsDepth { // {tau, I} of CellsF64 and {lam, 0}
+    static constexpr int K = 2;
+    static constexpr bool kChanQueue = true;
+    static constexpr bool kImage = true;
+    template <bool kAffine>
+    static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<2>& v,
+                                 uint32_t& steps, uint32_t& error) {
+        DepthFields<kAffine> acc{v};
+        return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
+    }
+};
+
+struct CellsGrad { // the gradient pass: nothing is stored but the atomics; P is the WalkParams of a GradParams
+    static constexpr int K = 1;
+    static constexpr bool kChanQueue = false;
+    static constexpr bool kImage = false;
+    template <bool kAffine>
+    static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t pixel, int leaf, double z_in,
+                                 Pairs<1>& v, uint32_t& steps, uint32_t& error) {
+        static_assert(!kAffine, "grazing rays of the gradient pass walk through lam_crossing and grad_crossing");
+        return grad_crossing(P, px, py, pixel, leaf, z_in, v, steps, error);
+    }
+    static C5_HD double grad_crossing(const WalkParams& P, double px, double py, uint32_t pixel, int leaf, double z_in,
+                                      Pairs<1>& v, uint32_t& steps, uint32_t& error) {
+        const GradParams& G = static_cast<const GradParams&>(P);
+        GradFields acc{G, v, grad_ray(G, pixel), 0};
+        return crossing_walk<false>(P, px, py, leaf, z_in, acc, steps, error);
+    }
+    static C5_HD double lam_crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<1>& v,
+                                     uint32_t& steps, uint32_t& error) {
+        LamFields acc{v};
+        return crossing_walk<true>(P, px, py, leaf, z_in, acc, steps, error);
     }
 };
 
@@ -649,7 +812,7 @@ C5_HD RayResult<F::K> trace_ray(const WalkParams& P, double px, double py, uint3
     // B: first crossing
     const bool entered = !defer && L.n > 0;
     if (entered) {
-        z_after = F::template crossing<false>(P, px, py, L.leaf[0], L.z[0], r.v, r.steps, r.error);
+        z_after = F::template crossing<false>(P, px, py, pixel, L.leaf[0], L.z[0], r.v, r.steps, r.error);
     }
     sync_lanes(tracing);
     // C: anything above the exit?
@@ -664,7 +827,7 @@ C5_HD RayResult<F::K> trace_ray(const WalkParams& P, double px, double py, uint3
         // an entry at or below the ray's position is already behind it (two boundary faces sharing
         // the edge the ray passes through report the same depth)
         if (!defer && e < L.n && L.z[e] > z_after && !r.error) {
-            z_after = F::template crossing<false>(P, px, py, L.leaf[e], L.z[e], r.v, r.steps, r.error);
+            z_after = F::template crossing<false>(P, px, py, pixel, L.leaf[e], L.z[e], r.v, r.steps, r.error);
         }
         sync_lanes(tracing);
     }
@@ -755,13 +918,40 @@ C5_HD RayAcc<F::K> graze_ray_serial(const WalkParams& P, unsigned long long slot
             Pairs<F::K> k;
             k.reset();
             uint32_t steps_k = 0, error_k = 0;
-            const double z_out = F::template crossing<true>(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
+            const double z_out = F::template crossing<true>(P, px, py, P.queue[slot].pixel, L.leaf[e], L.z[e], k, steps_k,
+                                                            error_k);
             compose_crossing(a, L.z[e], z_out, k, steps_k, error_k);
             if (++crossings > 65536) a.error = 1;
         }
         if (L.n < P.serial_cap) break;
     }
     return a;
+}
+
+// The gradient pass's serial form: each crossing is walked affinely for its lam and (A, B), re-walked
+// with the gradient from the I and lam it is entered with, then composed — what the warp form does
+// for 32 crossings at a time.
+C5_HD void graze_ray_serial_grad(const WalkParams& P, unsigned long long slot, double px, double py) {
+    RayAcc<1> a = load_deferred<CellsGrad>(P, slot);
+    const uint32_t pixel = P.queue[slot].pixel;
+    EntryList<kSerialList> L;
+    int crossings = 0;
+    while (!a.error) {
+        if (!bvh_collect_entries(P, px, py, a.z_after, L, P.serial_cap, 0x7FFFFFFF)) a.error = 1;
+        for (int e = 0; e < L.n; e++) {
+            if (!(L.z[e] > a.z_after)) continue;
+            Pairs<1> k;
+            k.reset();
+            uint32_t steps_k = 0, error_k = 0;
+            const double z_out = CellsGrad::lam_crossing(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
+            Pairs<1> v = a.v;
+            uint32_t steps_g = 0, error_g = 0;
+            CellsGrad::grad_crossing(P, px, py, pixel, L.leaf[e], L.z[e], v, steps_g, error_g);
+            compose_crossing(a, L.z[e], z_out, k, steps_k, error_k);
+            if (++crossings > 65536) a.error = 1;
+        }
+        if (L.n < P.serial_cap) break;
+    }
 }
 
 C5_HD double __longlong_as_double_hd(long long bits) {
@@ -956,7 +1146,7 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
                 f.reset();
                 uint32_t steps_k = 0, error_k = 0;
                 if (have && z_in > a.z_after) { // a is the same in every lane
-                    z_out = F::template crossing<true>(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
+                    z_out = F::template crossing<true>(P, px, py, q_pixel, S.leaf[k], z_in, f, steps_k, error_k);
                 }
                 const int cnt = n - base < 32 ? n - base : 32;
                 for (int l = 0; l < cnt; l++) {
@@ -984,6 +1174,69 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
                 if (q_steps == 0) atomicAdd(&P.counters[kHitPixels], 1ull); // deferred before its first step
             }
             if (a.error) atomicAdd(&P.counters[kWalkErrors], 1ull);
+        }
+    }
+}
+
+// The gradient pass's grazing rays. Per batch of 32 crossings: (1) every lane walks its crossing
+// affinely, keeping its lam; (2) the warp folds the batch in z order exactly as graze_block does, and each
+// lane notes the {lam, I} its crossing is entered with (and whether the fold takes it); (3) the lanes
+// whose crossing was taken walk it again with the gradient.
+__device__ __forceinline__ void graze_block_grad(const WalkParams& P) {
+    __shared__ GrazeSmem smem[kGrazeWarps];
+    const unsigned full = 0xFFFFFFFFu;
+    const int lane = threadIdx.x & 31;
+    GrazeSmem& S = smem[threadIdx.x >> 5];
+    const unsigned long long n_rays = P.counters[kDeferred];
+    while (true) {
+        unsigned long long ticket = 0;
+        if (lane == 0) ticket = atomicAdd(&P.counters[kTicket], 1ull);
+        ticket = __shfl_sync(full, ticket, 0);
+        if (ticket >= n_rays) break;
+        const uint32_t q_pixel = P.queue[ticket].pixel;
+        const int i = static_cast<int>(q_pixel % static_cast<uint32_t>(P.res_x));
+        const int j = static_cast<int>(q_pixel / static_cast<uint32_t>(P.res_x));
+        const double px = P.xs[i], py = P.ys[j];
+        RayAcc<1> a = load_deferred<CellsGrad>(P, ticket);
+        int crossings = 0;
+        bool truncated = true;
+        while (truncated && !a.error) {
+            const int n = graze_collect(P, S, px, py, a.z_after, lane, truncated);
+            for (int base = 0; base < n; base += 32) {
+                const int k = base + lane;
+                const bool have = k < n;
+                const double z_in = have ? S.z[k] : INFINITY;
+                double z_out = z_in;
+                Pairs<1> f;
+                f.reset();
+                uint32_t steps_k = 0, error_k = 0;
+                if (have && z_in > a.z_after) {
+                    z_out = CellsGrad::lam_crossing(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
+                }
+                const int cnt = n - base < 32 ? n - base : 32;
+                Pairs<1> entered = a.v;
+                bool taken = false;
+                for (int l = 0; l < cnt; l++) {
+                    Pairs<1> g;
+                    g.tau[0] = __shfl_sync(full, f.tau[0], l);
+                    g.inten[0] = __shfl_sync(full, f.inten[0], l);
+                    g.gain[0] = __shfl_sync(full, f.gain[0], l);
+                    const double z_l = __shfl_sync(full, z_in, l);
+                    if (lane == l) {
+                        entered = a.v;
+                        taken = z_l > a.z_after;
+                    }
+                    compose_crossing(a, z_l, __shfl_sync(full, z_out, l), g, __shfl_sync(full, steps_k, l),
+                                     __shfl_sync(full, error_k, l));
+                }
+                if (taken) {
+                    uint32_t steps_g = 0, error_g = 0;
+                    CellsGrad::grad_crossing(P, px, py, q_pixel, S.leaf[k], z_in, entered, steps_g, error_g);
+                }
+            }
+            crossings += n;
+            if (crossings > 65536) a.error = 1;
+            __syncwarp();
         }
     }
 }
@@ -1030,16 +1283,18 @@ __device__ __forceinline__ void walk_block(const WalkParams& P) {
     const unsigned tracing = __ballot_sync(0xFFFFFFFFu, live && !solid && tile_sees_mesh);
     if (live) {
         if (solid) {
-            double nan[F::K];
-            fill_pairs(nan, __longlong_as_double(0x7FF8000000000000ll), std::make_integer_sequence<int, F::K>{}); // quiet NaN (config.hpp:26-27)
-            store_pixel(P, i, j, nan, nan, 0);
+            if (F::kImage) {
+                double nan[F::K];
+                fill_pairs(nan, __longlong_as_double(0x7FF8000000000000ll), std::make_integer_sequence<int, F::K>{}); // quiet NaN (config.hpp:26-27)
+                store_pixel(P, i, j, nan, nan, 0);
+            }
         } else {
             if (tile_sees_mesh) {
                 res = trace_ray<F>(P, P.xs[i], P.ys[j],
                                    static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
                                    tracing);
             }
-            if (!res.deferred) store_pixel(P, i, j, res.v.tau, res.v.inten, res.steps);
+            if (F::kImage && !res.deferred) store_pixel(P, i, j, res.v.tau, res.v.inten, res.steps);
         }
     }
 
@@ -1105,6 +1360,13 @@ __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_fp32(const Walk
 template <int K>
 __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_ch(const WalkParams P) { graze_block<Channels<K>>(P); }
 
+// The two passes of c5_render_grad: the depth pass stores {tau, I, lam, 0} per pixel, the gradient pass
+// adds into grad_alpha / grad_q. Their register counts are in DESIGN.md §5c (-Xptxas -v).
+__global__ void __launch_bounds__(kBlock) tet_walk_depth(const WalkParams P) { walk_block<CellsDepth>(P); }
+__global__ void __launch_bounds__(kBlock) tet_walk_grad(const GradParams P) { walk_block<CellsGrad>(P); }
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_depth(const WalkParams P) { graze_block<CellsDepth>(P); }
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad(const GradParams P) { graze_block_grad(P); }
+
 namespace {
 
 // The pixel and grazing-ray kernels of each field policy.
@@ -1125,6 +1387,16 @@ struct Kernels<Channels<K>> {
     static constexpr void (*walk)(WalkParams) = tet_walk_ch<K>;
     static constexpr void (*graze)(WalkParams) = grazing_rays_ch<K>;
 };
+template <>
+struct Kernels<CellsDepth> {
+    static constexpr void (*walk)(WalkParams) = tet_walk_depth;
+    static constexpr void (*graze)(WalkParams) = grazing_rays_depth;
+};
+template <>
+struct Kernels<CellsGrad> {
+    static constexpr void (*walk)(GradParams) = tet_walk_grad;
+    static constexpr void (*graze)(GradParams) = grazing_rays_grad;
+};
 
 void background_on_host(const WalkParams& P, int n) {
     for (int j = P.row_begin; j < P.row_end; j++) {
@@ -1140,15 +1412,17 @@ void walk_on_host(const WalkParams& P) {
     for (int j = P.j0; j < P.j1; j++) {
         for (int i = P.i0; i < P.i1; i++) {
             if (P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i]) {
-                double nan[F::K];
-                fill_pairs(nan, NAN, std::make_integer_sequence<int, F::K>{});
-                store_pixel(P, i, j, nan, nan, 0);
+                if (F::kImage) {
+                    double nan[F::K];
+                    fill_pairs(nan, NAN, std::make_integer_sequence<int, F::K>{});
+                    store_pixel(P, i, j, nan, nan, 0);
+                }
                 P.counters[kSolidPixels]++;
                 continue;
             }
             const uint32_t pixel = static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i);
             const RayResult<F::K> r = trace_ray<F>(P, P.xs[i], P.ys[j], pixel, 0);
-            if (!r.deferred) store_pixel(P, i, j, r.v.tau, r.v.inten, r.steps);
+            if (F::kImage && !r.deferred) store_pixel(P, i, j, r.v.tau, r.v.inten, r.steps);
             P.counters[kSteps] += r.steps;
             P.row_cost[j] += r.steps;
             if (r.steps) P.counters[kHitPixels]++;
@@ -1174,11 +1448,23 @@ void graze_on_host(const WalkParams& P) {
     P.counters[kTicket] = n_rays;
 }
 
+template <>
+void graze_on_host<CellsGrad>(const WalkParams& P) {
+    const unsigned long long n_rays = P.counters[kDeferred];
+    for (unsigned long long k = 0; k < n_rays; k++) {
+        const uint32_t pixel = P.queue[k].pixel;
+        const int i = static_cast<int>(pixel % static_cast<uint32_t>(P.res_x));
+        const int j = static_cast<int>(pixel / static_cast<uint32_t>(P.res_x));
+        graze_ray_serial_grad(P, k, P.xs[i], P.ys[j]);
+    }
+    P.counters[kTicket] = n_rays;
+}
+
 // Policy F's pixel kernel over `grid` blocks, then its grazing-ray kernel for the rays the pixel
 // kernel deferred: a fixed grid of persistent warps that draw tickets. The host-loop build runs both
 // as loops.
-template <class F>
-void launch_rays(DeviceState& d, const WalkLaunch& w, const WalkParams& P, unsigned grid) {
+template <class F, class Params>
+void launch_rays(DeviceState& d, const WalkLaunch& w, const Params& P, unsigned grid) {
     if (kHostSim) {
         walk_on_host<F>(P);
         count_launch();
@@ -1216,8 +1502,8 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     P.mask = w.use_mask ? d.mask.p : nullptr;
     P.out = w.out;
     P.steps = w.write_steps ? d.steps.p : nullptr;
-    P.counters = d.counters.p;
-    P.row_cost = d.row_cost.p;
+    P.counters = w.counters ? w.counters : d.counters.p;
+    P.row_cost = w.row_cost ? w.row_cost : d.row_cost.p;
     P.queue = d.queue.p;
     P.res_x = w.res_x;
     P.res_y = w.res_y;
@@ -1250,8 +1536,10 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
         P.rec = d.ch_rec.p;
         P.ch_queue = d.ch_queue.p;
     }
-    const int n_pairs = w.channels ? w.channels : 1;
-    if (!whole_band) {
+    if (w.pass != kImagePass && (w.channels || f32)) fail(C5_E_INVALID, "render_grad: FP64 over the cells' own fields only");
+    if (w.pass == kDepthPass) P.ch_queue = d.ch_queue.p;
+    const int n_pairs = w.channels ? w.channels : w.pass == kDepthPass ? 2 : 1;
+    if (!whole_band && w.pass != kGradPass) { // the gradient pass stores no pixel
         count_launch();
         if (kHostSim) {
             background_on_host(P, n_pairs);
@@ -1264,6 +1552,20 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     if (empty_rect) return; // the mesh is not in this band: no rays
     count_launch();
     const unsigned grid = static_cast<unsigned>(P.n_macro_x) * static_cast<unsigned>(n_macro_y) * 64u;
+    if (w.pass == kDepthPass) {
+        launch_rays<CellsDepth>(d, w, P, grid);
+        return;
+    }
+    if (w.pass == kGradPass) {
+        GradParams G{};
+        static_cast<WalkParams&>(G) = P;
+        G.grad_in = w.grad_in;
+        G.depth = w.depth;
+        G.grad_alpha = w.grad_alpha;
+        G.grad_q = w.grad_q;
+        launch_rays<CellsGrad>(d, w, G, grid);
+        return;
+    }
     switch (w.channels) {
     case 0:
         if (f32) {

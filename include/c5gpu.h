@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define C5_ABI_VERSION 4
+#define C5_ABI_VERSION 5
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
 #define C5_MAX_CHANNELS 8
@@ -207,6 +207,41 @@ int c5_render_flux(c5_ctx* ctx, const c5_view* view, int32_t channels, double* r
                    c5_stats* stats);
 int c5_render_flux_submit(c5_ctx* ctx, const c5_view* view, int32_t channels, double* rows, double* total,
                           uint64_t* ticket);
+
+/* ---- gradients: the derivative of a view with respect to every tet's alpha and Q --------------------
+ * c5_update_fields replaces the cells' own alpha and Q (n_tets doubles each, tets in the order given to
+ * c5_upload_mesh) without rebuilding topology or BVH; channels and solids stay. It goes through the
+ * parent like every upload and reaches the parts of a multi-device context; siblings and lanes see the
+ * new fields at their next render. Every render afterwards is bit-identical to one from a context
+ * uploaded with these fields. C5_E_INVALID: NULL array. C5_E_STATE: no mesh, a sibling context, or a
+ * submitted view in flight on the context or one of its lanes.
+ *
+ * c5_render_grad computes, for one view, the vector-Jacobian product of the pre-cast image (what
+ * c5_render_raw gives with round_through_float = 0) against an upstream gradient g: res_y * res_x * 2
+ * doubles, x fastest, {g_tau, g_I} per pixel, of which only the view's row band is read. It writes, in
+ * the tet order given to c5_upload_mesh and overwriting,
+ *   grad_alpha[t] = sum over pixels of g_tau dtau/dalpha_t + g_I dI/dalpha_t
+ *   grad_q[t]     = sum over pixels of g_I dI/dQ_t
+ * Pixels under the solid mask and background pixels contribute nothing. The derivative is that of the
+ * function the walk computes, segment lengths included: vertex positions and the view are not
+ * parameters. dtau/dalpha_t counts every segment (tau uses the unclamped alpha); a segment whose
+ * min(alpha, alpha_limit) is below DBL_EPSILON leaves I unchanged and adds nothing to dI; dI/dalpha_t is
+ * 0 where alpha_t > alpha_limit (the clamp) and flows where alpha_t == alpha_limit.
+ * Either gradient array may be NULL, not both. out (optional, res_y * res_x * 2 doubles) receives the
+ * {tau, I} image c5_render_raw gives for the view, bit for bit. stats mean what they mean for
+ * c5_render_raw, except that ms_d2h spans the gradient pass and the copies of the gradients.
+ * The call runs two walks over the same rays, a depth pass and a gradient pass: two kernel launches
+ * more than c5_render_raw of the same view (none more when the mesh is outside the band). Each device
+ * adds its band's contributions into its own buffers with FP64 atomics, so the gradients are NOT
+ * bit-reproducible from run to run (they agree to rounding, ~1e-15 relative); a multi-device context
+ * adds the devices' gradients on the host in device order. g and the gradients are host arrays
+ * (copied in and out on every call). C5_E_INVALID: NULL g, both gradient arrays NULL, precision 32, or
+ * round_through_float != 0 (the float cast is piecewise constant: ask for the raw values).
+ * C5_E_STATE: no mesh, or a submitted view in flight on this context. Single-device, multi-device and
+ * sibling contexts. Not covered: uploaded channels, the FP32 variant, a pipelined (submit) form. */
+int c5_update_fields(c5_ctx* ctx, const double* alpha, const double* q);
+int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* grad_alpha, double* grad_q, double* out,
+                   c5_stats* stats);
 
 /* Device-resident variant for callers that own device memory (e.g. a torch tensor that an NCCL
  * gather will read): d_out is a DEVICE pointer on the context's first device to
