@@ -91,6 +91,9 @@ SYMBOLS = {
     "c5_render_flux_submit": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, _dp, _dp, _u64p]),
     "c5_update_fields": (C.c_int, [C.c_void_p, _dp, _dp]),
     "c5_render_grad": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _dp, _dp, _dp, C.POINTER(Stats)]),
+    "c5_update_fields_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "c5_render_grad_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.POINTER(Stats)]),
     "c5_render_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_last_row_cost": (C.c_int, [C.c_void_p, _u64p, C.c_int32]),
     "c5_kernel_launches": (C.c_uint64, [C.c_void_p]),
@@ -107,7 +110,7 @@ SYMBOLS = {
 }
 IPC_HANDLE_BYTES = 80
 MAX_IN_FLIGHT = 8
-ABI_VERSION = 5        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
+ABI_VERSION = 6        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
 TIMELINE_PHASES = 6
 
 
@@ -173,6 +176,7 @@ class Context:
         if rc != OK:
             raise C5Error(rc, (self.lib.c5_last_error(None) or b"").decode())
         self._h = handle
+        self.devices = tuple(devices)
         self.n_devices = len(devices)
 
     def sibling(self) -> "Context":
@@ -183,6 +187,7 @@ class Context:
         self._check(self.lib.c5_create_sibling(self._h, C.byref(handle)))
         sib = Context.__new__(Context)
         sib.lib, sib._h, sib.n_devices, sib._parent = self.lib, handle, 1, self
+        sib.devices = self.devices
         return sib
 
     def debug_set(self, key: str, value: int):
@@ -376,8 +381,7 @@ class Context:
         g = np.ascontiguousarray(g, dtype=np.float64)
         if g.size != view.res_y * view.res_x * 2:
             raise ValueError("g must hold res_y * res_x * 2 doubles")
-        owner = getattr(self, "_parent", None) or self  # a sibling reports its parent's mesh only once it has rendered
-        n_tets = owner.mesh_info().n_tets
+        n_tets = self.n_tets
         ga = np.empty(n_tets, dtype=np.float64) if alpha else None
         gq = np.empty(n_tets, dtype=np.float64) if q else None
         out = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64) if image else None
@@ -386,6 +390,38 @@ class Context:
                                             _ptr(out, _dp), C.byref(st)))
         self.last_stats = st.as_dict()
         return (ga, gq, out) if image else (ga, gq)
+
+    @property
+    def n_tets(self) -> int:
+        """Tets of the uploaded mesh (0 before upload_mesh). A sibling reports its parent's: its own mesh
+        info is filled in only once it has rendered."""
+        owner = getattr(self, "_parent", None) or self
+        return int(owner.mesh_info().n_tets)
+
+    def update_fields_device(self, alpha_ptr: int, q_ptr: int, stream: int = 0):
+        """update_fields from DEVICE memory (c5_update_fields_device): alpha_ptr and q_ptr point to n_tets
+        doubles each on the context's device (e.g. tensor.data_ptr()), in the order given to upload_mesh.
+        The gather is enqueued on `stream` (a cudaStream_t handle, 0 = the legacy default stream) without a
+        host synchronisation; the library's later renders and later work on `stream` see the new fields.
+        The arrays must stay valid until the gather has run on `stream`."""
+        self._fields_version = self.fields_version + 1
+        self._check(self.lib.c5_update_fields_device(self._h, C.c_void_p(alpha_ptr), C.c_void_p(q_ptr),
+                                                     C.c_void_p(stream)))
+
+    def render_grad_device(self, view: View, g_ptr: int, grad_alpha_ptr: int, grad_q_ptr: int, out_ptr: int = 0,
+                           stream: int = 0, *, stats: bool = True) -> dict:
+        """render_grad on DEVICE memory (c5_render_grad_device), enqueued on `stream`. g_ptr: the view's row
+        band only, (row_end - row_begin) * res_x * 2 doubles {g_tau, g_I}; out_ptr (0 = none): the same size,
+        receives that band of render_raw's image; grad_alpha_ptr / grad_q_ptr (0 = not wanted, not both):
+        n_tets doubles each, overwritten. stats=False: enqueue only (no readback, no synchronisation, a ray
+        stopped by the step cap is not reported); returns {}."""
+        st = Stats() if stats else None
+        self._check(self.lib.c5_render_grad_device(self._h, C.byref(view), C.c_void_p(g_ptr),
+                                                   C.c_void_p(grad_alpha_ptr or None), C.c_void_p(grad_q_ptr or None),
+                                                   C.c_void_p(out_ptr or None), C.c_void_p(stream),
+                                                   C.byref(st) if stats else None))
+        self.last_stats = st.as_dict() if stats else {}
+        return self.last_stats
 
     def render_raw(self, view: View) -> RawImage:
         out = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64)

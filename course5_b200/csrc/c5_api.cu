@@ -542,9 +542,40 @@ struct GradResult {
     std::vector<double> grad_alpha, grad_q; // empty unless asked for
 };
 
-// Band [row_begin,row_end) of v on ctx's device: the view prologue and the depth pass (enqueue_view),
-// then the gradient pass over the same rays, then the copies. Blocks until the results are on the host.
-// Events: 0..4 as for an image, 5 depth pass done, 6 gradients on the host.
+// The depth pass (with the view prologue, enqueue_view) and the gradient pass of band [row_begin,row_end)
+// of v on d.stream, into d.grad_alpha / d.grad_q (Morton order). The band's {g_tau, g_I} per pixel are
+// g_host's rows (the whole image, copied to d.grad_in) or d_g (a device band buffer, read in place).
+// Events: 0..4 as for an image, 5 depth pass done.
+void enqueue_grad(DeviceState& d, const c5_view* v, const ViewPlan& p, const double* g_host, const double* d_g) {
+    const size_t n_t = static_cast<size_t>(d.n_tets);
+    const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
+    const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
+    // the gradient pass counts into the second half, so that the stats stay the depth pass's
+    d.counters.ensure(2 * kNumCounters);
+    d.row_cost.ensure(2 * static_cast<size_t>(v->res_y));
+    d.grad_alpha.ensure(n_t);
+    d.grad_q.ensure(n_t);
+    if (g_host) d.grad_in.ensure(2 * static_cast<size_t>(v->res_y) * v->res_x);
+    enqueue_view(d, v, p, false, nullptr, 0, kDepthPass);
+    record(d, 5);
+    dev_zero(d.grad_alpha.p, n_t * sizeof(double), d.stream);
+    dev_zero(d.grad_q.p, n_t * sizeof(double), d.stream);
+    dev_zero(d.counters.p + kNumCounters, kNumCounters * sizeof(unsigned long long), d.stream);
+    dev_zero(d.row_cost.p + v->res_y, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
+    if (g_host) h2d(d.grad_in.p, g_host + 2 * band_off, 2 * n_pix_band * sizeof(double), d.stream);
+    WalkLaunch w = view_walk(d, v, p);
+    w.pass = kGradPass;
+    w.depth = d.out.p;
+    w.grad_in = g_host ? d.grad_in.p : d_g; // indexed like the band's out
+    w.grad_alpha = d.grad_alpha.p;
+    w.grad_q = d.grad_q.p;
+    w.counters = d.counters.p + kNumCounters;
+    w.row_cost = d.row_cost.p + v->res_y;
+    launch_walk(d, w);
+}
+
+// Band [row_begin,row_end) of v on ctx's device: enqueue_grad, then the copies. Blocks until the results
+// are on the host. Events: 0..5 as for enqueue_grad, 6 gradients on the host.
 GradResult grad_band(c5_ctx* ctx, const c5_view* v, const double* g, bool want_alpha, bool want_q, double* out) {
     follow_parent(ctx);
     if (ctx->pending.active) fail(C5_E_STATE, "render_grad: this context still has a view in flight (c5_render_wait it first)");
@@ -556,28 +587,7 @@ GradResult grad_band(c5_ctx* ctx, const c5_view* v, const double* g, bool want_a
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
     const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
     ensure_host_staging(d, static_cast<size_t>(v->res_y));
-    // the gradient pass counts into the second half, so that the stats stay the depth pass's
-    d.counters.ensure(2 * kNumCounters);
-    d.row_cost.ensure(2 * static_cast<size_t>(v->res_y));
-    d.grad_alpha.ensure(n_t);
-    d.grad_q.ensure(n_t);
-    d.grad_in.ensure(2 * static_cast<size_t>(v->res_y) * v->res_x);
-    enqueue_view(d, v, p, false, nullptr, 0, kDepthPass);
-    record(d, 5);
-    dev_zero(d.grad_alpha.p, n_t * sizeof(double), d.stream);
-    dev_zero(d.grad_q.p, n_t * sizeof(double), d.stream);
-    dev_zero(d.counters.p + kNumCounters, kNumCounters * sizeof(unsigned long long), d.stream);
-    dev_zero(d.row_cost.p + v->res_y, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
-    h2d(d.grad_in.p, g + 2 * band_off, 2 * n_pix_band * sizeof(double), d.stream);
-    WalkLaunch w = view_walk(d, v, p);
-    w.pass = kGradPass;
-    w.depth = d.out.p;
-    w.grad_in = d.grad_in.p;
-    w.grad_alpha = d.grad_alpha.p;
-    w.grad_q = d.grad_q.p;
-    w.counters = d.counters.p + kNumCounters;
-    w.row_cost = d.row_cost.p + v->res_y;
-    launch_walk(d, w);
+    enqueue_grad(d, v, p, g, nullptr);
     std::vector<double> morton[2];
     for (int k = 0; k < 2; k++) {
         if (!(k == 0 ? want_alpha : want_q)) continue;
@@ -660,6 +670,75 @@ void check_flux_args(const c5_view* view, int32_t channels, const double* rows, 
     if (!rows && !total) fail(C5_E_INVALID, "render_flux: rows and total are both NULL");
     if (channels != 0 && channels != 1) fail(C5_E_INVALID, "render_flux: channels must be 0 or 1");
     if (channels && view && view->precision == 32) fail(C5_E_INVALID, "render_flux: channels are FP64 only (precision 64)");
+}
+
+// ---- gradients on device memory (c5_update_fields_device, c5_render_grad_device) ------------------------
+
+void check_device_array(const void* p, const char* what) {
+    if (!p) fail(C5_E_INVALID, std::string(what) + " is NULL");
+    if (reinterpret_cast<uintptr_t>(p) & 7u) fail(C5_E_INVALID, std::string(what) + " must be 8-byte aligned");
+}
+
+// The device copy of the tet permutation, on the state that owns the mesh: made by the first device-form
+// call (not at upload, so that contexts that never use it do not pay its 4 bytes per tet) and counted in
+// device_bytes from then on.
+const uint32_t* resident_tperm(c5_ctx* ctx) {
+    c5_ctx* owner = ctx->parent ? ctx->parent : ctx;
+    DeviceState& o = owner->dev;
+    if (!o.tperm_dev.p) {
+        use_device(o);
+        upload_tperm(o);
+        owner->info.device_bytes += static_cast<int64_t>(o.tperm_dev.bytes());
+        if (owner != ctx) ctx->info = owner->info;
+    }
+    return o.tperm_dev.p;
+}
+
+// The context's own stream and those of its lanes and siblings: the streams the library renders on.
+std::vector<DeviceState*> internal_streams(c5_ctx* ctx) {
+    std::vector<DeviceState*> all{&ctx->dev};
+    for (c5_ctx* s : ctx->siblings) all.push_back(&s->dev); // the caller's siblings and our lanes
+    return all;
+}
+
+// c5_render_grad_device on a single-device context or a sibling: enqueue_grad on the caller's stream with
+// d_g read in place, then the scatter into file order and the strided copy of the image.
+void grad_band_device(c5_ctx* ctx, const c5_view* v, const double* d_g, double* d_grad_alpha, double* d_grad_q,
+                      double* d_out, void* stream, c5_stats* stats) {
+    follow_parent(ctx);
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    if (ctx->pending.active) fail(C5_E_STATE, "render_grad_device: this context has a submitted view in flight");
+    const ViewPlan p = plan_view(v);
+    DeviceState& d = ctx->dev;
+    use_device(d);
+    const uint32_t* tperm = resident_tperm(ctx);
+    const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
+    if (stats) ensure_host_staging(d, static_cast<size_t>(v->res_y));
+    // run on the CALLER's stream, like c5_render_device: the scratch arrays are the context's own
+    cudaStream_t own = d.stream;
+    if (!kHostSim) d.stream = static_cast<cudaStream_t>(stream);
+    try {
+        enqueue_grad(d, v, p, nullptr, d_g);
+        scatter_grads(d.n_tets, tperm, d.grad_alpha.p, d.grad_q.p, d_grad_alpha, d_grad_q, d.stream);
+        // the depth pass left {tau, I, lam, 0} per pixel: its first pair is the image of c5_render_raw
+        if (d_out) d2d_2d(d_out, 2 * sizeof(double), d.out.p, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
+        record(d, 6);
+        if (!kHostSim && d.stream != own) { // the context's own later renders reuse these scratch arrays: they wait
+            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
+            C5_CUDA(cudaStreamWaitEvent(own, d.ev_fields, 0));
+        }
+        if (stats) {
+            d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
+            d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
+            stream_sync(d.stream);
+            ViewResult r = read_view(d, *v, p, true);
+            report(ctx, r, stats);
+        }
+    } catch (...) {
+        d.stream = own;
+        throw;
+    }
+    d.stream = own;
 }
 
 void upload_solids(c5_ctx* ctx, const double* pts, int64_t n, int follows) {
@@ -836,6 +915,7 @@ int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out) {
             for (auto& e : d.ev) C5_CUDA(cudaEventCreate(&e));
             C5_CUDA(cudaEventCreate(&d.ev_walk));
             C5_CUDA(cudaEventCreateWithFlags(&d.ev_done, cudaEventDisableTiming));
+            C5_CUDA(cudaEventCreateWithFlags(&d.ev_fields, cudaEventDisableTiming));
         }
         for (int k = 1; k < n_dev; k++) { // every further device: a single-device context of its own
             c5_ctx* part = nullptr;
@@ -916,6 +996,7 @@ void c5_destroy(c5_ctx* ctx) {
         for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
         if (d.ev_walk) cudaEventDestroy(d.ev_walk);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
+        if (d.ev_fields) cudaEventDestroy(d.ev_fields);
         for (auto& e : d.ev) {
             if (e) cudaEventDestroy(e);
         }
@@ -945,6 +1026,7 @@ int c5_upload_mesh(c5_ctx* ctx, const double* points_xyz, int64_t n_points, cons
             c->has_mesh = false;
             use_device(c->dev);
             upload_channels(c->dev, nullptr, nullptr, 0); // a new mesh drops the channels
+            c->dev.tperm_dev.release();                   // and the device copy of the old permutation
         }
         ctx->info.device_bytes -= ctx->channel_bytes;
         ctx->channel_bytes = 0;
@@ -1142,6 +1224,55 @@ int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* gr
         for (size_t r = 0; r < n; r++) views[r] = std::move(results[r].view);
         ViewResult total = n == 1 ? std::move(views[0]) : merge_results(views, view->res_y);
         report(ctx, total, stats);
+    });
+}
+
+int c5_update_fields_device(c5_ctx* ctx, const double* d_alpha, const double* d_q, void* stream) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (ctx->parent) fail(C5_E_STATE, "update_fields_device: a sibling context shares its parent's fields; update through the parent");
+        if (!ctx->parts.empty()) fail(C5_E_INVALID, "update_fields_device: single-device contexts only");
+        check_device_array(d_alpha, "update_fields_device: d_alpha");
+        check_device_array(d_q, "update_fields_device: d_q");
+        if (!ctx->has_mesh) fail(C5_E_STATE, "update_fields_device: no mesh uploaded");
+        for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
+            if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "update_fields_device: a submitted view is in flight");
+        }
+        DeviceState& d = ctx->dev;
+        use_device(d);
+        const uint32_t* tperm = resident_tperm(ctx);
+        cudaStream_t s = kHostSim ? d.stream : static_cast<cudaStream_t>(stream);
+        const std::vector<DeviceState*> internal = internal_streams(ctx);
+        if (!kHostSim) { // the gather waits for every render the library has enqueued on the old fields ...
+            for (DeviceState* x : internal) {
+                C5_CUDA(cudaEventRecord(x->ev_fields, x->stream));
+                C5_CUDA(cudaStreamWaitEvent(s, x->ev_fields, 0));
+            }
+        }
+        ctx->dev.mesh_version++; // siblings and lanes re-alias at their next render
+        gather_fields(d, tperm, d_alpha, d_q, s);
+        if (!kHostSim) { // ... and every later one waits for the gather
+            C5_CUDA(cudaEventRecord(d.ev_fields, s));
+            for (DeviceState* x : internal) C5_CUDA(cudaStreamWaitEvent(x->stream, d.ev_fields, 0));
+        }
+    });
+}
+
+int c5_render_grad_device(c5_ctx* ctx, const c5_view* view, const double* d_g, double* d_grad_alpha, double* d_grad_q,
+                          double* d_out, void* stream, c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        check_device_array(d_g, "render_grad_device: d_g");
+        if (!d_grad_alpha && !d_grad_q) fail(C5_E_INVALID, "render_grad_device: d_grad_alpha and d_grad_q are both NULL");
+        if (d_grad_alpha) check_device_array(d_grad_alpha, "render_grad_device: d_grad_alpha");
+        if (d_grad_q) check_device_array(d_grad_q, "render_grad_device: d_grad_q");
+        if (d_out) check_device_array(d_out, "render_grad_device: d_out");
+        if (view && view->precision == 32) fail(C5_E_INVALID, "render_grad_device: FP64 only (precision 64)");
+        if (view && view->round_through_float) {
+            fail(C5_E_INVALID, "render_grad_device: the float cast has no useful derivative; set round_through_float = 0");
+        }
+        if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_grad_device: single-device contexts only");
+        grad_band_device(ctx, view, d_g, d_grad_alpha, d_grad_q, d_out, stream, stats);
     });
 }
 

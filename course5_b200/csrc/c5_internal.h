@@ -55,6 +55,8 @@ struct DeviceState {
     DevBuf<int32_t> leaf_parent;     // per leaf: (parent << 1) | which child
     DevBuf<uint32_t> refit_flags;    // per internal node arrival counter
     std::vector<uint32_t> tperm;     // new -> old tet (host): places the file-order fields of c5_upload_channels
+    DevBuf<uint32_t> tperm_dev;      // the same on the device, made at the first device-form gradient call
+                                     // (siblings read their origin's)
 
     // channels (c5_upload_channels; aliased by siblings like the mesh)
     int n_channels = 0;
@@ -90,6 +92,7 @@ struct DeviceState {
     int sm_count = 0;
     cudaEvent_t ev_walk = nullptr;   // between the pixel kernel and the grazing-ray kernel (phase times)
     cudaEvent_t ev_done = nullptr;   // after the view's last copy: what c5_render_wait waits for
+    cudaEvent_t ev_fields = nullptr; // orders this stream and a caller's stream around the device-form gradient calls
     // results of the view in flight, copied by the stream into pinned host memory
     unsigned long long* h_counters = nullptr;   // [kNumCounters]
     uint64_t* h_row_cost = nullptr;             // [h_row_cost_n]
@@ -173,6 +176,15 @@ void launch_prepare_channels(DeviceState& d, double alpha_limit); // the same fo
 void upload_channels(DeviceState& d, const double* alpha, const double* q, int n);
 // c5_topology.cu — replaces cells[].alpha and q0 by file-order fields (c5_update_fields).
 void update_fields(DeviceState& d, const double* alpha, const double* q);
+// c5_topology.cu — what the device forms (c5_update_fields_device, c5_render_grad_device) need.
+// d.tperm_dev from d.tperm (allocates and blocks: made once, at the first device-form call)
+void upload_tperm(DeviceState& d);
+// The two ops below allocate nothing and launch one kernel on s.
+// cells[t].alpha = alpha[tperm[t]], q0[t] = q[tperm[t]]: file-order device fields into d's cells
+void gather_fields(DeviceState& d, const uint32_t* tperm, const double* alpha, const double* q, cudaStream_t s);
+// out[tperm[t]] = in[t] for both gradients (a null output is skipped): Morton order back to file order
+void scatter_grads(int64_t n_tets, const uint32_t* tperm, const double* in_alpha, const double* in_q, double* out_alpha,
+                   double* out_q, cudaStream_t s);
 
 // c5_walk.cu
 struct WalkLaunch {

@@ -106,6 +106,17 @@ void d2d(void* dst, const void* src, size_t bytes, cudaStream_t s) {
     }
 }
 
+void d2d_2d(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t height, cudaStream_t s) {
+    if (!width || !height) return;
+    if (kHostSim) {
+        for (size_t r = 0; r < height; r++) {
+            std::memcpy(static_cast<char*>(dst) + r * dpitch, static_cast<const char*>(src) + r * spitch, width);
+        }
+    } else {
+        C5_CUDA(cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, height, cudaMemcpyDeviceToDevice, s));
+    }
+}
+
 void* host_pinned_alloc(size_t bytes) {
     void* p = nullptr;
     if (kHostSim) {

@@ -50,6 +50,8 @@ void dev_zero(void* p, size_t bytes, cudaStream_t s);
 void h2d(void* dst, const void* src, size_t bytes, cudaStream_t s);
 void d2h(void* dst, const void* src, size_t bytes, cudaStream_t s);
 void d2d(void* dst, const void* src, size_t bytes, cudaStream_t s);
+// rows of `width` bytes, `height` of them, from src (pitch spitch) to dst (pitch dpitch), device to device
+void d2d_2d(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t height, cudaStream_t s);
 void stream_sync(cudaStream_t s);
 void* host_pinned_alloc(size_t bytes); // page-locked host memory (results the stream copies back while the host runs on)
 void host_pinned_free(void* p);

@@ -339,6 +339,34 @@ void gather_file_order(DeviceState& d, const double* alpha, const double* q, int
     stream_sync(s); // the staging buffers are freed on return
 }
 
+// c5_update_fields_device: file-order device fields straight into the cells (no staging, no allocation).
+struct FieldGatherOp {
+    const double* alpha;   // [n_tets], file order
+    const double* q;
+    const uint32_t* tperm; // new -> old tet
+    Cell* cells;
+    double* q0;            // Morton order
+    C5_HD void operator()(int64_t t) const {
+        const uint32_t old = tperm[t];
+        cells[t].alpha = alpha[old];
+        q0[t] = q[old];
+    }
+};
+
+// c5_render_grad_device: the gradient pass's Morton-order sums into the caller's file-order arrays.
+struct GradScatterOp {
+    const uint32_t* tperm; // new -> old tet
+    const double* in_alpha;
+    const double* in_q;
+    double* out_alpha;     // either may be null
+    double* out_q;
+    C5_HD void operator()(int64_t t) const {
+        const uint32_t old = tperm[t];
+        if (out_alpha) out_alpha[old] = in_alpha[t];
+        if (out_q) out_q[old] = in_q[t];
+    }
+};
+
 } // namespace
 
 void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t* tets, int64_t n_tets,
@@ -553,6 +581,22 @@ void update_fields(DeviceState& d, const double* alpha, const double* q) {
     for_each(d.stream, d.n_tets, CellAlphaOp{rec.p, d.cells.p});
     stream_sync(d.stream);
     d.cells_limit_valid = false; // cells[].s is derived again from the new q0 at the next render
+}
+
+void upload_tperm(DeviceState& d) {
+    d.tperm_dev.alloc(d.tperm.size());
+    h2d(d.tperm_dev.p, d.tperm.data(), d.tperm_dev.bytes(), d.stream);
+    stream_sync(d.stream); // the host vector is pageable and may change at the next upload_mesh
+}
+
+void gather_fields(DeviceState& d, const uint32_t* tperm, const double* alpha, const double* q, cudaStream_t s) {
+    for_each(s, d.n_tets, FieldGatherOp{alpha, q, tperm, d.cells.p, d.q0.p});
+    d.cells_limit_valid = false; // cells[].s is derived again from the new q0 at the next render
+}
+
+void scatter_grads(int64_t n_tets, const uint32_t* tperm, const double* in_alpha, const double* in_q, double* out_alpha,
+                   double* out_q, cudaStream_t s) {
+    for_each(s, n_tets, GradScatterOp{tperm, in_alpha, in_q, out_alpha, out_q});
 }
 
 } // namespace c5

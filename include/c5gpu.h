@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define C5_ABI_VERSION 5
+#define C5_ABI_VERSION 6
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
 #define C5_MAX_CHANNELS 8
@@ -235,13 +235,48 @@ int c5_render_flux_submit(c5_ctx* ctx, const c5_view* view, int32_t channels, do
  * adds its band's contributions into its own buffers with FP64 atomics, so the gradients are NOT
  * bit-reproducible from run to run (they agree to rounding, ~1e-15 relative); a multi-device context
  * adds the devices' gradients on the host in device order. g and the gradients are host arrays
- * (copied in and out on every call). C5_E_INVALID: NULL g, both gradient arrays NULL, precision 32, or
+ * (copied in and out on every call); c5_render_grad_device below is the same call on device memory.
+ * C5_E_INVALID: NULL g, both gradient arrays NULL, precision 32, or
  * round_through_float != 0 (the float cast is piecewise constant: ask for the raw values).
  * C5_E_STATE: no mesh, or a submitted view in flight on this context. Single-device, multi-device and
  * sibling contexts. Not covered: uploaded channels, the FP32 variant, a pipelined (submit) form. */
 int c5_update_fields(c5_ctx* ctx, const double* alpha, const double* q);
 int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* grad_alpha, double* grad_q, double* out,
                    c5_stats* stats);
+
+/* ---- gradients on device memory (fit loops whose fields, loss and optimiser live on the GPU) -------------
+ * c5_update_fields_device is c5_update_fields with d_alpha and d_q DEVICE pointers on the context's device
+ * (n_tets doubles each, tets in the order given to c5_upload_mesh), gathered into the cells on the device
+ * by one kernel through a device copy of the tet permutation. That copy (4 bytes per tet, shared with
+ * siblings) is made at the first call of either device form and counted in c5_mesh_info.device_bytes from
+ * then on; c5_upload_mesh drops it. Same semantics as c5_update_fields: channels and solids stay, and every
+ * render afterwards is bit-identical to one from a fresh upload of these fields.
+ * Ordering, without synchronising the host: the gather is enqueued on `stream` (a cudaStream_t; NULL = the
+ * legacy default stream) after `stream` has waited (events) for everything the library had enqueued on the
+ * internal streams of the context, its lanes and its siblings; those internal streams then wait for the
+ * gather, so the library's later renders (c5_render, c5_render_raw, c5_render_flux, submits, ...) and the
+ * caller's later work on `stream` see the new fields. Work the caller put on streams of its own (e.g.
+ * c5_render_device with stats == NULL) is the caller's to order, as for c5_render_device. d_alpha and d_q
+ * must stay valid until the gather has run on `stream`. C5_E_INVALID: a NULL or not 8-byte aligned pointer,
+ * or a multi-device context (single-device contexts only). C5_E_STATE: no mesh, a sibling context, or a
+ * submitted view in flight on the context or one of its lanes.
+ *
+ * c5_render_grad_device is c5_render_grad on device memory, enqueued on `stream`. Band-sized buffers, as
+ * for c5_render_device: d_g holds (row_end - row_begin) * res_x * 2 doubles, {g_tau, g_I} per pixel of the
+ * view's row band (0,0 = all rows), and the optional d_out the same number, receiving that band of the
+ * image c5_render_raw gives, bit for bit. d_grad_alpha and d_grad_q (n_tets doubles each, file order,
+ * overwritten; either may be NULL, not both) are scattered from the walk's Morton order on the device.
+ * stats == NULL: enqueue only — nothing is read back, the host is not synchronised, and a ray stopped by the
+ * step cap is not reported; successive calls and the caller's work on `stream` pipeline on the device.
+ * The context's own later renders wait for the call (an event; the host does not wait). Successive
+ * device-form calls on one context share its scratch buffers: keep them on one stream, or order them.
+ * stats != NULL: `stream` is synchronised and stats are those of c5_render_grad. Three kernel launches more
+ * than c5_render_raw of the same view (the gradient pass's two and the scatter). C5_E_INVALID: any cause
+ * c5_render_grad has, a pointer not 8-byte aligned, or a multi-device context. C5_E_STATE: no mesh, or a
+ * submitted view in flight on this context. Single-device contexts and siblings. */
+int c5_update_fields_device(c5_ctx* ctx, const double* d_alpha, const double* d_q, void* stream);
+int c5_render_grad_device(c5_ctx* ctx, const c5_view* view, const double* d_g, double* d_grad_alpha, double* d_grad_q,
+                          double* d_out, void* stream, c5_stats* stats);
 
 /* Device-resident variant for callers that own device memory (e.g. a torch tensor that an NCCL
  * gather will read): d_out is a DEVICE pointer on the context's first device to
