@@ -794,7 +794,8 @@ void alias_mesh(DeviceState& s, DeviceState& o) {
     s.px.alias(o.px);
     s.py.alias(o.py);
     s.pz.alias(o.pz);
-    s.cells.alias(o.cells);
+    s.conn.alias(o.conn);
+    s.fields.alias(o.fields);
     s.q0.alias(o.q0);
     s.n_channels = o.n_channels;
     s.ch_rec.alias(o.ch_rec);
@@ -1044,6 +1045,21 @@ int c5_upload_mesh(c5_ctx* ctx, const double* points_xyz, int64_t n_points, cons
         for (c5_ctx* c : all) c->has_mesh = true;
     });
 }
+
+#ifdef C5_HOSTSIM
+// Host-loop build only, for the layout tests: the topology as the walk reads it. conn gets 8 int32 per
+// tet (Conn), bfaces 8 int32 per boundary face (BFace), tperm the tet permutation (Morton -> file order).
+extern "C" int c5_hostsim_topology(c5_ctx* ctx, int32_t* conn, int32_t* bfaces, uint32_t* tperm) {
+    if (!ctx || !conn || !bfaces || !tperm) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (!ctx->has_mesh) fail(C5_E_STATE, "hostsim_topology: no mesh");
+        const c5::DeviceState& d = ctx->dev;
+        std::memcpy(conn, d.conn.p, d.conn.bytes());
+        std::memcpy(bfaces, d.bfaces.p, d.bfaces.bytes());
+        std::memcpy(tperm, d.tperm.data(), d.tperm.size() * sizeof(uint32_t));
+    });
+}
+#endif
 
 int c5_upload_solids(c5_ctx* ctx, const double* tet_points, int64_t n_tets, int32_t follows_view) {
     if (!ctx) return C5_E_INVALID;

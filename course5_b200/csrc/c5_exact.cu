@@ -673,8 +673,8 @@ C5_HD double source_fn(double alpha, const double* q, int64_t k, double limit) {
     return (alpha < DBL_EPSILON) ? 0.0 : q[k] / alpha;
 }
 
-C5_HD void prepare_cell_body(int64_t t, Cell* cells, const double* q0, double limit) {
-    cells[t].s = source_fn(cells[t].alpha, q0, t, limit);
+C5_HD void prepare_cell_body(int64_t t, Fields* fields, const double* q0, double limit) {
+    fields[t].s = source_fn(fields[t].alpha, q0, t, limit);
 }
 
 // Channel c of tet t (k = t * n + c): s_c from ch_q0[c][t] and the alpha_c beside it in the record.
@@ -689,9 +689,9 @@ C5_HD void prepare_channel_body(int64_t k, double* rec, const double* q0, int64_
 
 // Source function s = Q / min(alpha, limit) per cell; rerun only when --alpha_limit changes.
 __global__ void __launch_bounds__(256)
-prepare_cells(int64_t n, Cell* __restrict__ cells, const double* __restrict__ q0, double limit) {
+prepare_cells(int64_t n, Fields* __restrict__ fields, const double* __restrict__ q0, double limit) {
     const int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-    if (t < n) prepare_cell_body(t, cells, q0, limit);
+    if (t < n) prepare_cell_body(t, fields, q0, limit);
 }
 
 // The same for the uploaded channels (n_tets * n_channels records).
@@ -939,9 +939,9 @@ void prepare_for_limit(DeviceState& dd, double alpha_limit, double DeviceState::
 void launch_prepare_cells(DeviceState& dd, double alpha_limit) {
     prepare_for_limit(dd, alpha_limit, &DeviceState::cells_limit, &DeviceState::cells_limit_valid, [&](DeviceState& d) {
         if (kHostSim) {
-            for (int64_t t = 0; t < d.n_tets; t++) prepare_cell_body(t, d.cells.p, d.q0.p, alpha_limit);
+            for (int64_t t = 0; t < d.n_tets; t++) prepare_cell_body(t, d.fields.p, d.q0.p, alpha_limit);
         } else {
-            prepare_cells<<<grid_for(d.n_tets, 256), 256, 0, dd.stream>>>(d.n_tets, d.cells.p, d.q0.p, alpha_limit);
+            prepare_cells<<<grid_for(d.n_tets, 256), 256, 0, dd.stream>>>(d.n_tets, d.fields.p, d.q0.p, alpha_limit);
             C5_CUDA(cudaGetLastError());
         }
     });

@@ -42,9 +42,10 @@ struct DeviceState {
     int64_t n_pts = 0, n_tets = 0, n_bfaces = 0;
     double mesh_lo[3] = {0, 0, 0}, mesh_hi[3] = {0, 0, 0}; // bounding box in the file frame
     DevBuf<double> px, py, pz;       // Morton-ordered file-frame coordinates (SoA: the rotate kernel streams them)
-    DevBuf<Cell> cells;
-    DevBuf<double> q0;               // Q per tet (Morton order); cells[t].s is derived from it
-    double cells_limit = 0.0;        // the alpha_limit cells[].s was last prepared for
+    DevBuf<Conn> conn;               // per tet (Morton order): neighbours and apexes with their slot maps
+    DevBuf<Fields> fields;           // per tet (Morton order): alpha and s
+    DevBuf<double> q0;               // Q per tet (Morton order); fields[t].s is derived from it
+    double cells_limit = 0.0;        // the alpha_limit fields[].s was last prepared for
     bool cells_limit_valid = false;
     DeviceState* origin = nullptr;   // sibling context: the device state that owns the mesh (and these two flags)
     uint64_t mesh_version = 0;       // bumped by every upload; a sibling re-aliases when it falls behind
@@ -169,18 +170,18 @@ void launch_solid_mask(DeviceState& d, int res_x, int res_y, double x_min, doubl
                        double step_y, int row_begin, int row_end);
 void launch_bvh_refit(DeviceState& d);
 void dedupe_solid_faces(DeviceState& d, SolidSet& ss); // fills ss.faces / ss.n_faces from ss.pts0
-void launch_prepare_cells(DeviceState& d, double alpha_limit); // cells[t].s = q0[t] / min(alpha, limit)
+void launch_prepare_cells(DeviceState& d, double alpha_limit); // fields[t].s = q0[t] / min(alpha, limit)
 void launch_prepare_channels(DeviceState& d, double alpha_limit); // the same for every channel of ch_rec
 
 // c5_topology.cu — places n channels of file-order fields (channel-major) in ch_rec / ch_q0.
 void upload_channels(DeviceState& d, const double* alpha, const double* q, int n);
-// c5_topology.cu — replaces cells[].alpha and q0 by file-order fields (c5_update_fields).
+// c5_topology.cu — replaces fields[].alpha and q0 by file-order fields (c5_update_fields).
 void update_fields(DeviceState& d, const double* alpha, const double* q);
 // c5_topology.cu — what the device forms (c5_update_fields_device, c5_render_grad_device) need.
 // d.tperm_dev from d.tperm (allocates and blocks: made once, at the first device-form call)
 void upload_tperm(DeviceState& d);
 // The two ops below allocate nothing and launch one kernel on s.
-// cells[t].alpha = alpha[tperm[t]], q0[t] = q[tperm[t]]: file-order device fields into d's cells
+// fields[t].alpha = alpha[tperm[t]], q0[t] = q[tperm[t]]: file-order device fields into d's tets
 void gather_fields(DeviceState& d, const uint32_t* tperm, const double* alpha, const double* q, cudaStream_t s);
 // out[tperm[t]] = in[t] for both gradients (a null output is skipped): Morton order back to file order
 void scatter_grads(int64_t n_tets, const uint32_t* tperm, const double* in_alpha, const double* in_q, double* out_alpha,

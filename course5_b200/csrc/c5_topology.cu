@@ -4,9 +4,11 @@
 // The reference keeps a private copy of the 4 points in every tet and no connectivity
 // (object3d_base.cpp:37-51, tetra.hpp:42-45). Here:
 //   1. vertices are sorted along a 63-bit Morton curve (file frame) -> px/py/pz SoA;
-//   2. tets are sorted along the Morton curve of their centroids -> Cell records;
+//   2. tets are sorted along the Morton curve of their centroids -> Fields records and the tets'
+//      vertex ids (a buffer of the upload only);
 //   3. every tet face gets the key (sorted vertex triple); a radix sort brings the two copies of
-//      an interior face together -> Cell::nbr; unmatched faces are the domain boundary;
+//      an interior face together -> Conn::nbr and Conn::apex with the face's slot map; unmatched
+//      faces are the domain boundary;
 //   4. boundary faces are wound outward, Morton-sorted, and a Karras LBVH hierarchy is built over
 //      them (only the boxes are refitted per view, c5_exact.cu);
 //   5. the hierarchy is relabelled breadth-first on the host so the top levels are a contiguous
@@ -18,6 +20,8 @@
 #include "c5_internal.h"
 
 namespace c5 {
+
+static_assert(C5_MAX_POINTS == (1 << kApexIdBits), "a vertex id must fit the id bits of Conn::apex");
 
 namespace {
 
@@ -101,37 +105,34 @@ struct CellFillOp {
     const double* q;
     const uint32_t* tperm; // new -> old tet
     const uint32_t* vinv;  // old -> new vertex
-    Cell* cells;
+    int32_t* tv;           // [n_tets][4] vertex ids
+    Fields* fields;
     double* q0;
     C5_HD void operator()(int64_t t) const {
         const uint32_t old = tperm[t];
-        Cell c;
-        for (int k = 0; k < 4; k++) {
-            c.v[k] = static_cast<int32_t>(vinv[tets[4 * static_cast<int64_t>(old) + k]]);
-            c.nbr[k] = -1;
-            c.apex[k] = -1;
-        }
+        for (int k = 0; k < 4; k++) tv[4 * t + k] = static_cast<int32_t>(vinv[tets[4 * static_cast<int64_t>(old) + k]]);
+        Fields c;
         c.alpha = alpha[old];
         c.s = 0.0; // set by prepare_cells for the view's alpha_limit
         q0[t] = q[old];
-        cells[t] = c;
+        fields[t] = c;
     }
 };
 
 // -- 3. face keys and matching -------------------------------------------------------------------
 // Face f = 4 t + k is the face of tet t opposite its local vertex k.
 struct FaceKeyOp {
-    const Cell* cells;
+    const int32_t* tv;
     uint64_t* key_lo_mid;
     uint32_t* key_hi;
     uint32_t* hi_sort; // copy that gets sorted
     uint32_t* idx;
     C5_HD void operator()(int64_t f) const {
-        const Cell& c = cells[f >> 2];
+        const int32_t* v = tv + 4 * (f >> 2);
         const int k = static_cast<int>(f & 3);
-        uint32_t a = static_cast<uint32_t>(c.v[(k + 1) & 3]);
-        uint32_t b = static_cast<uint32_t>(c.v[(k + 2) & 3]);
-        uint32_t d = static_cast<uint32_t>(c.v[(k + 3) & 3]);
+        uint32_t a = static_cast<uint32_t>(v[(k + 1) & 3]);
+        uint32_t b = static_cast<uint32_t>(v[(k + 2) & 3]);
+        uint32_t d = static_cast<uint32_t>(v[(k + 3) & 3]);
         uint32_t t;
         if (a > b) { t = a; a = b; b = t; }
         if (b > d) { t = b; b = d; d = t; }
@@ -155,11 +156,28 @@ struct FaceMatchOp {
     const uint32_t* key_hi;     // by face
     const uint32_t* idx;        // faces sorted by (lo, mid, hi)
     int64_t n_faces;
-    Cell* cells;
+    const int32_t* tv;    // [n_tets][4] vertex ids
+    Conn* conn;
     uint8_t* is_boundary; // by face
     int* err;
     C5_HD bool same(uint32_t f, uint32_t g) const {
         return key_lo_mid[f] == key_lo_mid[g] && key_hi[f] == key_hi[g];
+    }
+    // Conn::apex of face f, whose twin is face g: g's apex id and the slots in g's tet of f's
+    // vertices at slots (k + 1) & 3, (k + 2) & 3, (k + 3) & 3 (the twins share these three vertices)
+    C5_HD uint32_t apex_word(uint32_t f, uint32_t g) const {
+        const int32_t* vf = tv + 4 * static_cast<int64_t>(f >> 2);
+        const int32_t* vg = tv + 4 * static_cast<int64_t>(g >> 2);
+        uint32_t map = 0;
+        for (uint32_t j = 1; j <= 3; j++) {
+            const int32_t x = vf[(f + j) & 3];
+            uint32_t slot = 0;
+            for (uint32_t m = 1; m < 4; m++) {
+                if (vg[m] == x) slot = m;
+            }
+            map |= slot << (2 * (j - 1));
+        }
+        return static_cast<uint32_t>(vg[g & 3]) | (map << kApexIdBits);
     }
     C5_HD void operator()(int64_t i) const {
         const uint32_t f = idx[i];
@@ -171,15 +189,15 @@ struct FaceMatchOp {
         }
         if (eq_next) {
             const uint32_t g = idx[i + 1];
-            cells[f >> 2].nbr[f & 3] = static_cast<int32_t>(g >> 2);
-            cells[g >> 2].nbr[g & 3] = static_cast<int32_t>(f >> 2);
-            cells[f >> 2].apex[f & 3] = cells[g >> 2].v[g & 3];
-            cells[g >> 2].apex[g & 3] = cells[f >> 2].v[f & 3];
+            conn[f >> 2].nbr[f & 3] = static_cast<int32_t>(g >> 2);
+            conn[g >> 2].nbr[g & 3] = static_cast<int32_t>(f >> 2);
+            conn[f >> 2].apex[f & 3] = apex_word(f, g);
+            conn[g >> 2].apex[g & 3] = apex_word(g, f);
             is_boundary[f] = 0;
             is_boundary[g] = 0;
         } else if (!eq_prev) {
-            cells[f >> 2].nbr[f & 3] = -1;
-            cells[f >> 2].apex[f & 3] = -1;
+            conn[f >> 2].nbr[f & 3] = -1;
+            conn[f >> 2].apex[f & 3] = 0;
             is_boundary[f] = 1;
         }
     }
@@ -187,7 +205,7 @@ struct FaceMatchOp {
 
 // -- 4. boundary faces and the LBVH hierarchy --------------------------------------------------
 struct BFaceOp {
-    const Cell* cells;
+    const int32_t* tv;
     const double *px, *py, *pz;
     const uint32_t* bface_ids; // face index f of each boundary face
     Box3 box;
@@ -196,10 +214,11 @@ struct BFaceOp {
     uint32_t* vals;
     C5_HD void operator()(int64_t i) const {
         const uint32_t f = bface_ids[i];
-        const Cell& c = cells[f >> 2];
+        const int32_t* v = tv + 4 * static_cast<int64_t>(f >> 2);
         const int k = static_cast<int>(f & 3);
-        int32_t a = c.v[(k + 1) & 3], b = c.v[(k + 2) & 3], cc = c.v[(k + 3) & 3];
-        const int32_t d = c.v[k];
+        int32_t a = v[(k + 1) & 3], b = v[(k + 2) & 3], cc = v[(k + 3) & 3];
+        int32_t sb = (k + 2) & 3, sc = (k + 3) & 3; // slots of b and cc
+        const int32_t d = v[k];
         const double ax = px[a], ay = py[a], az = pz[a];
         const double ux = px[b] - ax, uy = py[b] - ay, uz = pz[b] - az;
         const double vx = px[cc] - ax, vy = py[cc] - ay, vz = pz[cc] - az;
@@ -209,6 +228,9 @@ struct BFaceOp {
             const int32_t t = b;
             b = cc;
             cc = t;
+            const int32_t st = sb;
+            sb = sc;
+            sc = st;
         }
         BFace bf;
         bf.a = a;
@@ -216,7 +238,8 @@ struct BFaceOp {
         bf.c = cc;
         bf.tet = static_cast<int32_t>(f >> 2);
         bf.apex = d;
-        bf.pad[0] = bf.pad[1] = bf.pad[2] = 0;
+        bf.slots = ((k + 1) & 3) | (sc << 2) | (sb << 4); // a, c, b
+        bf.pad[0] = bf.pad[1] = 0;
         out[i] = bf;
         keys[i] = morton3((px[a] + px[b] + px[cc]) / 3.0, (py[a] + py[b] + py[cc]) / 3.0,
                           (pz[a] + pz[b] + pz[cc]) / 3.0, box.lo, box.inv);
@@ -314,12 +337,12 @@ struct ChannelGatherOp {
     }
 };
 
-// The alpha of channel record t (stride channel_stride(1)) into cell t: c5_update_fields gathers the
-// cells' new fields as one channel, then moves alpha beside the topology.
+// The alpha of channel record t (stride channel_stride(1)) into tet t: c5_update_fields gathers the
+// tets' new fields as one channel, then moves alpha into Fields.
 struct CellAlphaOp {
     const double* rec;
-    Cell* cells;
-    C5_HD void operator()(int64_t t) const { cells[t].alpha = rec[t * channel_stride(1)]; }
+    Fields* fields;
+    C5_HD void operator()(int64_t t) const { fields[t].alpha = rec[t * channel_stride(1)]; }
 };
 
 // n channel-major arrays of file-order alpha and q: record t of rec gets {alpha_c, 0} of old tet
@@ -339,16 +362,16 @@ void gather_file_order(DeviceState& d, const double* alpha, const double* q, int
     stream_sync(s); // the staging buffers are freed on return
 }
 
-// c5_update_fields_device: file-order device fields straight into the cells (no staging, no allocation).
+// c5_update_fields_device: file-order device fields straight into Fields (no staging, no allocation).
 struct FieldGatherOp {
     const double* alpha;   // [n_tets], file order
     const double* q;
     const uint32_t* tperm; // new -> old tet
-    Cell* cells;
+    Fields* fields;
     double* q0;            // Morton order
     C5_HD void operator()(int64_t t) const {
         const uint32_t old = tperm[t];
-        cells[t].alpha = alpha[old];
+        fields[t].alpha = alpha[old];
         q0[t] = q[old];
     }
 };
@@ -372,7 +395,7 @@ struct GradScatterOp {
 void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t* tets, int64_t n_tets,
                 const double* alpha, const double* q) {
     if (n_pts < 4 || n_tets < 1) fail(C5_E_INVALID, "upload_mesh: need at least 4 points and 1 tet");
-    if (n_pts >= (int64_t{1} << 31)) fail(C5_E_INVALID, "upload_mesh: more than 2^31 points");
+    if (n_pts > C5_MAX_POINTS) fail(C5_E_INVALID, "upload_mesh: more than C5_MAX_POINTS (2^26) points");
     if (n_tets >= (int64_t{1} << 29)) fail(C5_E_INVALID, "upload_mesh: more than 2^29 tets");
     cudaStream_t s = d.stream;
     const Box3 box = bounding_box(pts, n_pts);
@@ -415,8 +438,11 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
         for_each(s, n_pts, VertexScatterOp{xyz.p, perm.p, vinv.p, d.px.p, d.py.p, d.pz.p});
     }
 
-    // 2. tets -> cells in Morton order
-    d.cells.alloc(static_cast<size_t>(n_tets));
+    // 2. tets in Morton order: fields, and the vertex ids faces 3. and 4. are built from
+    d.conn.alloc(static_cast<size_t>(n_tets));
+    d.fields.alloc(static_cast<size_t>(n_tets));
+    DevBuf<int32_t> tv;
+    tv.alloc(static_cast<size_t>(4 * n_tets));
     {
         DevBuf<int32_t> tets_in;
         DevBuf<double> alpha_in, q_in;
@@ -434,7 +460,7 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
         check("upload_mesh");
         sort_pairs_u64(keys.p, tperm.p, static_cast<size_t>(n_tets), 63, s);
         d.q0.alloc(static_cast<size_t>(n_tets));
-        for_each(s, n_tets, CellFillOp{tets_in.p, alpha_in.p, q_in.p, tperm.p, vinv.p, d.cells.p, d.q0.p});
+        for_each(s, n_tets, CellFillOp{tets_in.p, alpha_in.p, q_in.p, tperm.p, vinv.p, tv.p, d.fields.p, d.q0.p});
         d.tperm.resize(static_cast<size_t>(n_tets));
         d2h(d.tperm.data(), tperm.p, tperm.bytes(), s);
         stream_sync(s);
@@ -454,7 +480,7 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
         key_hi.alloc(static_cast<size_t>(n_faces));
         hi_sort.alloc(static_cast<size_t>(n_faces));
         idx.alloc(static_cast<size_t>(n_faces));
-        for_each(s, n_faces, FaceKeyOp{d.cells.p, key_lm.p, key_hi.p, hi_sort.p, idx.p});
+        for_each(s, n_faces, FaceKeyOp{tv.p, key_lm.p, key_hi.p, hi_sort.p, idx.p});
         const int vbits = bits_for(static_cast<uint64_t>(n_pts));
         sort_pairs_u32(hi_sort.p, idx.p, static_cast<size_t>(n_faces), vbits, s); // by hi
         hi_sort.release();
@@ -464,7 +490,7 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
         key_sorted.release();
         is_boundary.alloc(static_cast<size_t>(n_faces));
         dev_zero(is_boundary.p, is_boundary.bytes(), s);
-        for_each(s, n_faces, FaceMatchOp{key_lm.p, key_hi.p, idx.p, n_faces, d.cells.p, is_boundary.p, err.p});
+        for_each(s, n_faces, FaceMatchOp{key_lm.p, key_hi.p, idx.p, n_faces, tv.p, d.conn.p, is_boundary.p, err.p});
         check("upload_mesh");
         bface_ids.alloc(static_cast<size_t>(n_faces));
         n_b = select_flagged(is_boundary.p, bface_ids.p, static_cast<size_t>(n_faces), s);
@@ -484,13 +510,14 @@ void build_mesh(DeviceState& d, const double* pts, int64_t n_pts, const int32_t*
         keys.alloc(n_b);
         perm.alloc(n_b);
         for_each(s, static_cast<int64_t>(n_b),
-                 BFaceOp{d.cells.p, d.px.p, d.py.p, d.pz.p, bface_ids.p, box, unsorted.p, keys.p, perm.p});
+                 BFaceOp{tv.p, d.px.p, d.py.p, d.pz.p, bface_ids.p, box, unsorted.p, keys.p, perm.p});
         sort_pairs_u64(keys.p, perm.p, n_b, 63, s);
         for_each(s, static_cast<int64_t>(n_b), GatherBFaceOp{unsorted.p, perm.p, d.bfaces.p});
         for_each(s, static_cast<int64_t>(n_b - 1), KarrasOp{keys.p, static_cast<int>(n_b), left.p, right.p});
         stream_sync(s);
     }
     bface_ids.release();
+    tv.release();
 
     // 5. breadth-first relabel on the host (n_b is small: the surface of the mesh)
     std::vector<int32_t> h_left(n_b - 1), h_right(n_b - 1);
@@ -578,9 +605,9 @@ void update_fields(DeviceState& d, const double* alpha, const double* q) {
     DevBuf<double> rec;
     rec.alloc(static_cast<size_t>(d.n_tets) * channel_stride(1));
     gather_file_order(d, alpha, q, 1, rec.p, d.q0.p);
-    for_each(d.stream, d.n_tets, CellAlphaOp{rec.p, d.cells.p});
+    for_each(d.stream, d.n_tets, CellAlphaOp{rec.p, d.fields.p});
     stream_sync(d.stream);
-    d.cells_limit_valid = false; // cells[].s is derived again from the new q0 at the next render
+    d.cells_limit_valid = false; // fields[].s is derived again from the new q0 at the next render
 }
 
 void upload_tperm(DeviceState& d) {
@@ -590,8 +617,8 @@ void upload_tperm(DeviceState& d) {
 }
 
 void gather_fields(DeviceState& d, const uint32_t* tperm, const double* alpha, const double* q, cudaStream_t s) {
-    for_each(s, d.n_tets, FieldGatherOp{alpha, q, tperm, d.cells.p, d.q0.p});
-    d.cells_limit_valid = false; // cells[].s is derived again from the new q0 at the next render
+    for_each(s, d.n_tets, FieldGatherOp{alpha, q, tperm, d.fields.p, d.q0.p});
+    d.cells_limit_valid = false; // fields[].s is derived again from the new q0 at the next render
 }
 
 void scatter_grads(int64_t n_tets, const uint32_t* tperm, const double* in_alpha, const double* in_q, double* out_alpha,

@@ -12,23 +12,33 @@ namespace c5 {
 
 // ---- data layout in HBM ----------------------------------------------------------------------
 //
-// Cell record: everything one tet-step reads about the tet it is in, in ONE 64-byte aligned
-// record (two 32-byte sectors of one 128-byte line): connectivity, the face-neighbour table, the
-// vertex ids across each face, and the two cell scalars. nbr[k] is the tet across the face
-// OPPOSITE local vertex k (the face that omits vertex k; the reference's face f omits vertex
-// 3 - f, plane.cpp:30-37), or -1 on the domain boundary; apex[k] is the vertex of THAT tet which
-// is not on the shared face. Knowing apex[k] when the ray leaves through face k lets the walk
-// issue the next cell load and the next vertex load together instead of one after the other.
-// s = Q / min(alpha, limit) (the source function) is refreshed when --alpha_limit changes, so the
-// I recurrence needs no divide: I <- I - (s - I) expm1(-a dz). Tets are in Morton order of centroids.
-struct alignas(64) Cell {
-    int32_t v[4];
+// A tet is two records at the same index, tets in Morton order of centroids: its connectivity
+// (Conn, one 32-byte sector) and its two scalars (Fields, half a sector). One tet-step reads both
+// and one vertex: 32 + 16 + 32 bytes.
+//
+// nbr[k] is the tet across the face OPPOSITE local vertex slot k (the face that omits slot k; the
+// reference's face f omits vertex 3 - f, plane.cpp:30-37), or -1 on the domain boundary. apex[k]
+// describes THAT tet, u: its low kApexIdBits hold the id of u's vertex that is not on the shared
+// face, so the walk issues the next Conn load and the next vertex load together instead of one
+// after the other; its top 6 bits are the slot map of the face: bits 2 (j - 1) .. 2 j - 1 hold
+// the slot in u of this tet's vertex at slot (k + j) & 3, j = 1, 2, 3 (u's apex has the slot left
+// over). The walk tracks the slots of the face it entered through and never compares vertex ids, so
+// the vertex ids of a tet are not stored: the upload builds them in a buffer it frees.
+constexpr int kApexIdBits = 26; // so a mesh has at most 2^26 points (C5_MAX_POINTS)
+constexpr uint32_t kApexIdMask = (1u << kApexIdBits) - 1u;
+struct alignas(32) Conn {
     int32_t nbr[4];
-    int32_t apex[4];
+    uint32_t apex[4]; // id | map << kApexIdBits (0 on the boundary)
+};
+static_assert(sizeof(Conn) == 32, "Conn must be 32 bytes");
+
+// s = Q / min(alpha, limit) (the source function) is refreshed when --alpha_limit changes, so the
+// I recurrence needs no divide: I <- I - (s - I) expm1(-a dz).
+struct alignas(16) Fields {
     double alpha; // "AbsorpCoef"
     double s;     // "radEnLooseRate" / min(alpha, alpha_limit)
 };
-static_assert(sizeof(Cell) == 64, "Cell must be 64 bytes");
+static_assert(sizeof(Fields) == 16, "Fields must be 16 bytes");
 
 // Rotated vertex: one 32-byte sector per vertex (a 24-byte record would straddle sectors half
 // the time). Vertices are stored in Morton order.
@@ -38,10 +48,11 @@ struct alignas(32) Vtx {
 static_assert(sizeof(Vtx) == 32, "Vtx must be 32 bytes");
 
 // Boundary face, wound so that (b-a)x(c-a) points OUT of the mesh. tet is the cell behind it and
-// apex that cell's fourth vertex.
+// apex that cell's fourth vertex. slots holds the local slots in tet of a, c and b (2 bits each, in
+// that order: the walk's counter-clockwise order of the face).
 struct alignas(32) BFace {
     int32_t a, b, c, tet;
-    int32_t apex, pad[3];
+    int32_t apex, slots, pad[2];
 };
 static_assert(sizeof(BFace) == 32, "BFace must be 32 bytes");
 

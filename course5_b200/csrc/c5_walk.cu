@@ -32,8 +32,10 @@
 // more orient2 of the two vertices that stay), so the exit z costs one divide; it is the entry z
 // of the next tet, i.e. each face plane is evaluated once per ray, not twice as in line.cpp:103-122.
 //
-// Per step the thread reads one 64-byte Cell and ONE new 32-byte vertex; the other three
-// vertices and their ids stay in registers (the 72 B/step algorithmic figure of SURVEY.md §8d).
+// Per step the thread reads the tet's 32-byte Conn and 16-byte Fields and ONE new 32-byte vertex; the
+// other three vertices stay in registers (the 72 B/step algorithmic figure of SURVEY.md §8d counts
+// 16 B of vertex ids the walk does without: it tracks which local slots of the tet hold the entry
+// face's vertices, c5_types.h).
 #include "c5_internal.h"
 
 #include <utility>
@@ -47,7 +49,8 @@ constexpr int kBlock = 128;       // 4 warps: 2 x 2 warp tiles of 8 x 4 pixels
 constexpr int kTileX = 16, kTileY = 8;
 
 struct WalkParams {
-    const Cell* cells;
+    const Conn* conn;
+    const Fields* fields;
     const Vtx* vrot;
     const BFace* bfaces;
     const BvhNode* nodes;
@@ -83,38 +86,78 @@ struct GradParams : WalkParams {
 };
 
 // ---- loads through the read-only path ----------------------------------------------------------
-struct CellData {
-    int4 v, nbr, apex;
-    double alpha, s;
+struct ConnData {
+    int4 nbr;
+    uint4 apex;
 };
 
-// sm_100 has 256-bit global loads (SASS LDG.E.ENL2.256): a 64-byte cell is two of them and a
-// 32-byte vertex one, i.e. 3 load instructions per tet-step instead of 6 LDG.128.
-C5_HD CellData load_cell(const Cell* cells, int t) {
-    CellData c;
+// sm_100 has 256-bit global loads (SASS LDG.E.ENL2.256): a 32-byte Conn is one of them, a 32-byte
+// vertex one, and the 16-byte Fields one LDG.128: 3 load instructions per tet-step.
+C5_HD ConnData load_conn(const Conn* conn, int t) {
+    ConnData c;
 #ifdef __CUDA_ARCH__
-    const char* p = reinterpret_cast<const char*>(cells + t);
-    asm volatile("ld.global.nc.v8.s32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(c.v.x), "=r"(c.v.y), "=r"(c.v.z), "=r"(c.v.w), "=r"(c.nbr.x), "=r"(c.nbr.y), "=r"(c.nbr.z),
-                   "=r"(c.nbr.w)
-                 : "l"(p));
-    int a0, a1, a2, a3;
-    int lo0, hi0, lo1, hi1;
-    asm volatile("ld.global.nc.v8.s32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(a3), "=r"(lo0), "=r"(hi0), "=r"(lo1), "=r"(hi1)
-                 : "l"(p + 32));
-    c.apex = make_int4(a0, a1, a2, a3);
-    c.alpha = __hiloint2double(hi0, lo0);
-    c.s = __hiloint2double(hi1, lo1);
+    asm volatile("ld.global.nc.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(c.nbr.x), "=r"(c.nbr.y), "=r"(c.nbr.z), "=r"(c.nbr.w), "=r"(c.apex.x), "=r"(c.apex.y),
+                   "=r"(c.apex.z), "=r"(c.apex.w)
+                 : "l"(conn + t));
 #else
-    const Cell& s = cells[t];
-    c.v = make_int4(s.v[0], s.v[1], s.v[2], s.v[3]);
+    const Conn& s = conn[t];
     c.nbr = make_int4(s.nbr[0], s.nbr[1], s.nbr[2], s.nbr[3]);
-    c.apex = make_int4(s.apex[0], s.apex[1], s.apex[2], s.apex[3]);
-    c.alpha = s.alpha;
-    c.s = s.s;
+    c.apex = make_uint4(s.apex[0], s.apex[1], s.apex[2], s.apex[3]);
 #endif
     return c;
+}
+
+// alpha and s of the tet being crossed, loaded by a field policy's fetch() together with its Conn
+struct TetFields {
+    double alpha, s;
+    C5_HD void load(const Fields* fields, int t) {
+#ifdef __CUDA_ARCH__
+        asm volatile("ld.global.nc.v2.f64 {%0,%1}, [%2];" : "=d"(alpha), "=d"(s) : "l"(fields + t));
+#else
+        alpha = fields[t].alpha;
+        s = fields[t].s;
+#endif
+    }
+};
+
+// Where the ray goes after leaving tet t through the face opposite local slot k: the next tet, its
+// new vertex, and the slots in it of the exit face's vertices. `slots` holds the slots in t of the
+// face the walk keeps (a, b, c: 2 bits each); the dropped vertex is the one at bit `sh`, and the new
+// vertex d of t, at the slot the three leave free, takes its place.
+C5_HD int step_across(const ConnData& c, uint32_t& slots, uint32_t sh, int& id_next) {
+    const uint32_t k = (slots >> sh) & 3u;
+    // two selects per word on the bits of k, without branches
+    const bool k0 = k & 1u, k1 = k & 2u;
+    const int t_next = k1 ? (k0 ? c.nbr.w : c.nbr.z) : (k0 ? c.nbr.y : c.nbr.x);
+    const uint32_t apex = k1 ? (k0 ? c.apex.w : c.apex.z) : (k0 ? c.apex.y : c.apex.x);
+    id_next = static_cast<int>(apex & kApexIdMask);
+    const uint32_t sd = (slots ^ (slots >> 2) ^ (slots >> 4)) & 3u; // 0 ^ 1 ^ 2 ^ 3 == 0
+    const uint32_t face = (slots & ~(3u << sh)) | (sd << sh);
+    // perm: 2-bit field s = the slot in the next tet of slot s of this one (s != k), i.e. the map
+    // rotated by k fields
+    const uint32_t rot = (apex >> kApexIdBits) << 2;
+    const uint32_t perm = ((rot << 8) | rot) >> (8u - 2u * k);
+    slots = ((perm >> (2u * (face & 3u))) & 3u) | (((perm >> (2u * ((face >> 2) & 3u))) & 3u) << 2) |
+            (((perm >> (2u * (face >> 4))) & 3u) << 4);
+    return t_next;
+}
+
+// The entry of a crossing through boundary face `leaf`: its vertices (a, c, b of the stored winding,
+// counter-clockwise in projection), tet, apex and their slots.
+struct Entry {
+    int ia, ib, ic, t, id;
+    uint32_t slots;
+};
+C5_HD Entry load_entry(const WalkParams& P, int leaf) {
+#ifdef __CUDA_ARCH__
+    const int4 f = __ldg(reinterpret_cast<const int4*>(P.bfaces + leaf));
+    const int2 e = __ldg(reinterpret_cast<const int2*>(&P.bfaces[leaf].apex));
+    return Entry{f.x, f.z, f.y, f.w, e.x, static_cast<uint32_t>(e.y)};
+#else
+    const BFace& bf = P.bfaces[leaf];
+    return Entry{bf.a, bf.c, bf.b, bf.tet, bf.apex, static_cast<uint32_t>(bf.slots)};
+#endif
 }
 
 C5_HD void load_vtx(const Vtx* vrot, int id, double& x, double& y, double& z) {
@@ -285,41 +328,34 @@ C5_HD bool bvh_collect_entries(const WalkParams& P, double px, double py, double
 // 1, and the crossing maps an arriving I to inten + gain * I (the recurrence of line.cpp:206-225 is
 // affine in I: s - (s - I) e = s (1 - e) + e I).
 //
-// `acc` integrates the fields along the crossing: fetch(t) is issued with tet t's cell load and
-// step(c, dz) adds one segment. CellFields below integrates the cells' own alpha and s; ChanFields
+// `acc` integrates the fields along the crossing: fetch(P, t) is issued with tet t's Conn load and
+// step(P, dz) adds one segment. CellFields below integrates the cells' own alpha and s; ChanFields
 // integrates K uploaded field pairs over the same steps.
 template <bool kAffine, class Acc>
 C5_HD double crossing_walk(const WalkParams& P, double px, double py, int leaf, double z_in, Acc& acc,
                            uint32_t& steps, uint32_t& error) {
-#ifdef __CUDA_ARCH__
-    const int4 f = __ldg(reinterpret_cast<const int4*>(P.bfaces + leaf));
-    int id = __ldg(&P.bfaces[leaf].apex);
-#else
-    const BFace& bf = P.bfaces[leaf];
-    const int4 f = make_int4(bf.a, bf.b, bf.c, bf.tet);
-    int id = bf.apex;
-#endif
-    // entry face (a, c, b) of the stored winding is counter-clockwise in projection
-    int ia = f.x, ib = f.z, ic = f.y;
+    const Entry e = load_entry(P, leaf);
+    int id = e.id;
+    uint32_t slots = e.slots;
     double ax, ay, az, bx, by, bz, cx, cy, cz;
-    load_vtx(P.vrot, ia, ax, ay, az);
-    load_vtx(P.vrot, ib, bx, by, bz);
-    load_vtx(P.vrot, ic, cx, cy, cz);
+    load_vtx(P.vrot, e.ia, ax, ay, az);
+    load_vtx(P.vrot, e.ib, bx, by, bz);
+    load_vtx(P.vrot, e.ic, cx, cy, cz);
     ax -= px; ay -= py;
     bx -= px; by -= py;
     cx -= px; cy -= py;
-    int t = f.w;
+    int t = e.t;
     double z_cur = z_in;
     while (true) {
         if (steps >= static_cast<uint32_t>(P.max_steps)) {
             error = 1;
             break;
         }
-        // id = the vertex of tet t that is not on the entry face. It is known BEFORE t's cell is
-        // read (Cell::apex of the previous tet, BFace::apex at entry), so the cell load and the
-        // vertex load of a step are independent and overlap: one memory latency per step, not two.
-        const CellData c = load_cell(P.cells, t);
-        acc.fetch(t);
+        // id = the vertex of tet t that is not on the entry face. It is known BEFORE t's Conn is
+        // read (Conn::apex of the previous tet, BFace::apex at entry), so the Conn, Fields and vertex
+        // loads of a step are independent and overlap: one memory latency per step, not two.
+        const ConnData c = load_conn(P.conn, t);
+        acc.fetch(P, t);
         double dx, dy, dz;
         load_vtx(P.vrot, id, dx, dy, dz);
         dx -= px;
@@ -330,27 +366,25 @@ C5_HD double crossing_walk(const WalkParams& P, double px, double py, int leaf, 
         // which face the ray leaves through, hence the next tet and its new vertex
         const bool drop_c = sa >= 0 && sb < 0;             // through (d, a, b)
         const bool drop_a = !drop_c && sb >= 0 && sc < 0;  // through (d, b, c)
-        const int dropped = drop_c ? ic : drop_a ? ia : ib; // else through (d, c, a)
-        const bool k0 = c.v.x == dropped, k1 = c.v.y == dropped, k2 = c.v.z == dropped;
-        const int t_next = k0 ? c.nbr.x : k1 ? c.nbr.y : k2 ? c.nbr.z : c.nbr.w;
-        const int id_next = k0 ? c.apex.x : k1 ? c.apex.y : k2 ? c.apex.z : c.apex.w;
+        int id_next;                                        // else through (d, c, a)
+        const int t_next = step_across(c, slots, drop_c ? 4u : drop_a ? 0u : 2u, id_next);
         // Barycentric weights of the pixel in the exit face (weight of a vertex = orient2 of the
         // other two, in cyclic order). Two of them are s values; the third belongs to d and is the
         // orient2 of the two vertices that stay — recomputed here (3 flops) rather than carried
         // from step to step (6 registers): same operands, same operations, so the same bits.
         double wa, wb, wc;
         if (drop_c) { // leaves through (d, a, b): c is replaced by d
-            ic = id; cx = dx; cy = dy; cz = dz;
+            cx = dx; cy = dy; cz = dz;
             wa = -sb;
             wb = sa;
             wc = orient2(ax, ay, bx, by);
         } else if (drop_a) { // through (d, b, c): a is replaced
-            ia = id; ax = dx; ay = dy; az = dz;
+            ax = dx; ay = dy; az = dz;
             wb = -sc;
             wc = sb;
             wa = orient2(bx, by, cx, cy);
         } else { // through (d, c, a): b is replaced
-            ib = id; bx = dx; by = dy; bz = dz;
+            bx = dx; by = dy; bz = dz;
             wc = -sa;
             wa = sc;
             wb = orient2(cx, cy, ax, ay);
@@ -358,7 +392,7 @@ C5_HD double crossing_walk(const WalkParams& P, double px, double py, int leaf, 
         const double wsum = wa + wb + wc;
         const double z_exit = (wsum != 0.0) ? (wa * az + wb * bz + wc * cz) / wsum : z_cur;
         const double dzv = fabs(z_exit - z_cur);
-        acc.step(P, c, dzv);
+        acc.step(P, dzv);
         steps++;
         z_cur = z_exit;
         t = t_next;
@@ -414,15 +448,16 @@ struct Pairs {
 template <bool kAffine>
 struct CellFields {
     Pairs<1>& v;
-    C5_HD void fetch(int) {}
-    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
+    TetFields c;
+    C5_HD void fetch(const WalkParams& P, int t) { c.load(P.fields, t); }
+    C5_HD void step(const WalkParams& P, double dzv) {
         segment<kAffine>(c.alpha, c.s, P.alpha_limit, dzv, v.tau[0], v.inten[0], v.gain[0]);
     }
 };
 
 // K uploaded field pairs. A step reads tet t's record of K {alpha_c, s_c} pairs (padded to 32-byte
-// sectors) together with t's cell, since t is known at the top of the step, so a channel adds FP64
-// work and a store but no further round trip.
+// sectors) together with t's Conn, since t is known at the top of the step, so a channel adds FP64
+// work and a store but no further round trip. The tet's own Fields are not read.
 template <int K, bool kAffine>
 struct ChanFields {
     const double* rec;
@@ -432,7 +467,7 @@ struct ChanFields {
     // f stays uninitialised: fetch fills it before every step (zeroing it costs the K = 3 grazing-ray
     // kernel 24 more bytes of spills)
     C5_HD ChanFields(const double* rec_, Pairs<K>& v_) : rec(rec_), v(v_) {}
-    C5_HD void fetch(int t) {
+    C5_HD void fetch(const WalkParams&, int t) {
         const double* p = rec + static_cast<size_t>(t) * channel_stride(K);
 #ifdef __CUDA_ARCH__
 #pragma unroll
@@ -445,7 +480,7 @@ struct ChanFields {
         for (int k = 0; k < channel_stride(K); k++) f[k] = p[k];
 #endif
     }
-    C5_HD void step(const WalkParams& P, const CellData&, double dzv) {
+    C5_HD void step(const WalkParams& P, double dzv) {
 #pragma unroll
         for (int c = 0; c < K; c++) segment<kAffine>(f[2 * c], f[2 * c + 1], P.alpha_limit, dzv, v.tau[c], v.inten[c], v.gain[c]);
     }
@@ -483,36 +518,32 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
                           double& inten, double& gain, uint32_t& steps, uint32_t& error) {
     const float limit = static_cast<float>(P.alpha_limit);
     const double z0 = z_in; // depths are kept relative to the entry point of the crossing
-#ifdef __CUDA_ARCH__
-    const int4 f = __ldg(reinterpret_cast<const int4*>(P.bfaces + leaf));
-    int id = __ldg(&P.bfaces[leaf].apex);
-#else
-    const BFace& bf = P.bfaces[leaf];
-    const int4 f = make_int4(bf.a, bf.b, bf.c, bf.tet);
-    int id = bf.apex;
-#endif
-    int ia = f.x, ib = f.z, ic = f.y;
+    const Entry e = load_entry(P, leaf);
+    int id = e.id;
+    uint32_t slots = e.slots;
     float ax, ay, az, bx, by, bz, cx, cy, cz;
     {
         double x, y, z;
-        load_vtx(P.vrot, ia, x, y, z);
+        load_vtx(P.vrot, e.ia, x, y, z);
         ax = static_cast<float>(x - px); ay = static_cast<float>(y - py); az = static_cast<float>(z - z0);
-        load_vtx(P.vrot, ib, x, y, z);
+        load_vtx(P.vrot, e.ib, x, y, z);
         bx = static_cast<float>(x - px); by = static_cast<float>(y - py); bz = static_cast<float>(z - z0);
-        load_vtx(P.vrot, ic, x, y, z);
+        load_vtx(P.vrot, e.ic, x, y, z);
         cx = static_cast<float>(x - px); cy = static_cast<float>(y - py); cz = static_cast<float>(z - z0);
     }
     float wa = orient2f(bx, by, cx, cy);
     float wb = orient2f(cx, cy, ax, ay);
     float wc = orient2f(ax, ay, bx, by);
-    int t = f.w;
+    int t = e.t;
     float z_cur = 0.f;
     while (true) {
         if (steps >= static_cast<uint32_t>(P.max_steps)) {
             error = 1;
             break;
         }
-        const CellData c = load_cell(P.cells, t);
+        const ConnData c = load_conn(P.conn, t);
+        TetFields fc;
+        fc.load(P.fields, t);
         float dx, dy, dz;
         {
             double x, y, z;
@@ -526,33 +557,31 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
         const float sc = orient2f(dx, dy, cx, cy);
         const bool drop_c = sa >= 0 && sb < 0;
         const bool drop_a = !drop_c && sb >= 0 && sc < 0;
-        const int dropped = drop_c ? ic : drop_a ? ia : ib;
-        const bool k0 = c.v.x == dropped, k1 = c.v.y == dropped, k2 = c.v.z == dropped;
-        const int t_next = k0 ? c.nbr.x : k1 ? c.nbr.y : k2 ? c.nbr.z : c.nbr.w;
-        const int id_next = k0 ? c.apex.x : k1 ? c.apex.y : k2 ? c.apex.z : c.apex.w;
+        int id_next;
+        const int t_next = step_across(c, slots, drop_c ? 4u : drop_a ? 0u : 2u, id_next);
         if (drop_c) {
-            ic = id; cx = dx; cy = dy; cz = dz;
+            cx = dx; cy = dy; cz = dz;
             wa = -sb;
             wb = sa;
         } else if (drop_a) {
-            ia = id; ax = dx; ay = dy; az = dz;
+            ax = dx; ay = dy; az = dz;
             wb = -sc;
             wc = sb;
         } else {
-            ib = id; bx = dx; by = dy; bz = dz;
+            bx = dx; by = dy; bz = dz;
             wc = -sa;
             wa = sc;
         }
         const float wsum = wa + wb + wc;
         const float z_exit = (wsum != 0.0f) ? (wa * az + wb * bz + wc * cz) / wsum : z_cur;
         const float dzv = fabsf(z_exit - z_cur);
-        tau += static_cast<double>(dzv) * c.alpha;
-        float a_c = static_cast<float>(c.alpha);
+        tau += static_cast<double>(dzv) * fc.alpha;
+        float a_c = static_cast<float>(fc.alpha);
         if (a_c > limit) a_c = limit;
-        const double a_d = c.alpha > P.alpha_limit ? P.alpha_limit : c.alpha;
+        const double a_d = fc.alpha > P.alpha_limit ? P.alpha_limit : fc.alpha;
         if (!(a_d < DBL_EPSILON)) { // the cancellation-free form of segment(), expm1f's error is relative
             const double m = static_cast<double>(expm1f(-a_c * dzv));
-            inten = inten - (c.s - inten) * m;
+            inten = inten - (fc.s - inten) * m;
             if (kAffine) gain *= 1.0 + m;
         }
         steps++;
@@ -695,8 +724,9 @@ C5_HD void grad_segment(const GradParams& P, int t, double alpha, double s, doub
 template <bool kAffine>
 struct DepthFields {
     Pairs<2>& v;
-    C5_HD void fetch(int) {}
-    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
+    TetFields c;
+    C5_HD void fetch(const WalkParams& P, int t) { c.load(P.fields, t); }
+    C5_HD void step(const WalkParams& P, double dzv) {
         segment<kAffine>(c.alpha, c.s, P.alpha_limit, dzv, v.tau[0], v.inten[0], v.gain[0]);
         v.tau[1] += lam_term(c.alpha, P.alpha_limit, dzv);
     }
@@ -706,8 +736,9 @@ struct DepthFields {
 // its exit I (the gradient kernel's first walk of a crossing).
 struct LamFields {
     Pairs<1>& v;
-    C5_HD void fetch(int) {}
-    C5_HD void step(const WalkParams& P, const CellData& c, double dzv) {
+    TetFields c;
+    C5_HD void fetch(const WalkParams& P, int t) { c.load(P.fields, t); }
+    C5_HD void step(const WalkParams& P, double dzv) {
         double tau = 0.0;
         segment<true>(c.alpha, c.s, P.alpha_limit, dzv, tau, v.inten[0], v.gain[0]);
         v.tau[0] += lam_term(c.alpha, P.alpha_limit, dzv);
@@ -720,8 +751,12 @@ struct GradFields {
     Pairs<1>& v;
     GradRay r;
     int t;
-    C5_HD void fetch(int t_) { t = t_; }
-    C5_HD void step(const WalkParams&, const CellData& c, double dzv) {
+    TetFields c;
+    C5_HD void fetch(const WalkParams& P, int t_) {
+        t = t_;
+        c.load(P.fields, t_);
+    }
+    C5_HD void step(const WalkParams&, double dzv) {
         grad_segment(G, t, c.alpha, c.s, dzv, r, v.tau[0], v.inten[0]);
     }
 };
@@ -1329,12 +1364,16 @@ constexpr int chan_blocks_per_sm(int K) {
 
 } // namespace
 
-// The product kernels. 7 blocks of 128 threads per SM = 72 registers: one more resident block than the
-// 80 the compiler picks on its own, measured faster (5.41 vs 5.64 ms on C3) despite a few spilled words
-// outside the step loop.
-__global__ void __launch_bounds__(kBlock, 7) tet_walk_fp64(const WalkParams P) { walk_block<CellsF64>(P); }
-// optional single-precision step geometry (north-star item (d)); entry search and accumulators stay FP64
-__global__ void __launch_bounds__(kBlock, 8) tet_walk_fp32(const WalkParams P) { walk_block<CellsF32>(P); }
+// The product kernels. 8 blocks of 128 threads per SM = 64 registers. With the 64-byte cell that cap
+// spilled in the step loop (8.9 ms on C3) and 7 blocks = 72 registers was the best bound (5.41 ms against
+// 5.64 with the compiler's own 80). Tracking face slots instead of vertex ids freed the registers: at 64
+// the kernel spills 28 bytes, none of them in the step loop (profiles/r09_ptxas_walk.txt,
+// r09_sass_step_loop.txt), and C3 takes 4.35 instead of 4.49 ms per view at 7 blocks (one B200,
+// profiles/r09_bench_c3_bounds_one_b200.jsonl).
+__global__ void __launch_bounds__(kBlock, 8) tet_walk_fp64(const WalkParams P) { walk_block<CellsF64>(P); }
+// optional single-precision step geometry (north-star item (d)); entry search and accumulators stay FP64.
+// 9 blocks = 56 registers, no spills: oblique view 1.90 against 2.03 ms at 8 blocks (same file).
+__global__ void __launch_bounds__(kBlock, 9) tet_walk_fp32(const WalkParams P) { walk_block<CellsF32>(P); }
 template <int K>
 __global__ void __launch_bounds__(kBlock, chan_blocks_per_sm(K)) tet_walk_ch(const WalkParams P) { walk_block<Channels<K>>(P); }
 
@@ -1493,7 +1532,8 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     if (w.precision != 64 && w.precision != 32) fail(C5_E_INVALID, "render: precision must be 64 or 32");
     const bool f32 = w.precision == 32;
     WalkParams P{};
-    P.cells = d.cells.p;
+    P.conn = d.conn.p;
+    P.fields = d.fields.p;
     P.vrot = d.vrot.p;
     P.bfaces = d.bfaces.p;
     P.nodes = d.nodes.p;

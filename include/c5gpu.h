@@ -29,6 +29,7 @@ extern "C" {
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
 #define C5_MAX_CHANNELS 8
+#define C5_MAX_POINTS (1 << 26) /* c5_upload_mesh: points per mesh (vertex ids are packed in 26 bits) */
 
 typedef struct c5_ctx c5_ctx;
 
@@ -113,7 +114,9 @@ int c5_abi_version(void);
  * per-tet point copies) by shared points + connectivity, which are flattened once into
  * device-resident arrays: Morton-reordered vertices and tets, a face-neighbour table, the
  * boundary-face list and an LBVH hierarchy over it. Caller keeps ownership of the host arrays;
- * the call blocks. alpha = "AbsorpCoef", q = "radEnLooseRate" (object3d_accretion_disk.cpp:4). */
+ * the call blocks. alpha = "AbsorpCoef", q = "radEnLooseRate" (object3d_accretion_disk.cpp:4).
+ * At most C5_MAX_POINTS points (67,108,864) and fewer than 2^29 tets; a larger mesh is C5_E_INVALID, refused
+ * before any of its arrays is read. */
 int c5_upload_mesh(c5_ctx* ctx, const double* points_xyz, int64_t n_points, const int32_t* tet_vertices,
                    int64_t n_tets, const double* alpha, const double* q);
 

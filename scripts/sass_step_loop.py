@@ -1,12 +1,13 @@
 #!/usr/bin/env python
 """Writes the SASS of the tet walk's step loop (first crossing of tet_walk_fp64) with an instruction
-census, from the built library — no GPU needed:
+census, from the built library (or another object given as the second argument) — no GPU needed:
 
-    python scripts/sass_step_loop.py > profiles/r02_sass_step_loop.txt
+    python scripts/sass_step_loop.py [kernel [library]] > profiles/r09_sass_step_loop.txt
 
-The loop is found structurally: the first backward branch whose body holds exactly three
-LDG.E.ENL2.256 (cell lower half, cell upper half, the one new vertex) and one MUFU.RCP64H (the
-divide of the exit depth).
+The loop is found structurally: the first backward branch whose body holds exactly three global
+loads, two or three of them LDG.E.ENL2.256 (the tet's Conn and Fields, the one new vertex; up to
+r06 the two halves of the 64-byte cell and the vertex), and one MUFU.RCP64H (the divide of the exit
+depth).
 """
 import collections
 import os
@@ -18,8 +19,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def main():
-    so = os.path.join(ROOT, "course5_b200", "libc5gpu.so")
     kernel = sys.argv[1] if len(sys.argv) > 1 else "tet_walk_fp64"
+    so = sys.argv[2] if len(sys.argv) > 2 else os.path.join(ROOT, "course5_b200", "libc5gpu.so")
     names = subprocess.run(["cuobjdump", "-res-usage", so], capture_output=True, text=True).stdout
     res = {}
     fn = None
@@ -47,8 +48,9 @@ def main():
             continue
         body = ins[addr_index[target]: i + 1]
         n256 = sum("LDG.E.ENL2.256" in t for _, t in body)
+        nldg = sum(re.search(r"\bLDG\.", t) is not None for _, t in body)
         nrcp = sum("MUFU.RCP64H" in t for _, t in body)
-        if n256 == 3 and nrcp == 1:
+        if nldg == 3 and n256 >= 2 and nrcp == 1:
             best = body
             break
     if best is None:
