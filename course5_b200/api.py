@@ -94,6 +94,8 @@ SYMBOLS = {
     "c5_update_fields_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "c5_render_grad_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_void_p, C.POINTER(Stats)]),
+    "c5_render_flux_grad_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_render_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_last_row_cost": (C.c_int, [C.c_void_p, _u64p, C.c_int32]),
     "c5_kernel_launches": (C.c_uint64, [C.c_void_p]),
@@ -110,7 +112,7 @@ SYMBOLS = {
 }
 IPC_HANDLE_BYTES = 80
 MAX_IN_FLIGHT = 8
-ABI_VERSION = 6        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
+ABI_VERSION = 7        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
 TIMELINE_PHASES = 6
 
 
@@ -178,6 +180,7 @@ class Context:
         self._h = handle
         self.devices = tuple(devices)
         self.n_devices = len(devices)
+        self._views_in_flight = 3  # c5_create's default
 
     def sibling(self) -> "Context":
         """A context on the same device that shares this one's mesh and solids and owns only per-view
@@ -207,6 +210,12 @@ class Context:
 
     def set_views_in_flight(self, n: int):
         self._check(self.lib.c5_set_views_in_flight(self._h, n))
+        self._views_in_flight = n
+
+    @property
+    def views_in_flight(self) -> int:
+        """The lanes of render_submit, render_flux_submit and render_flux_grad_device (set_views_in_flight)."""
+        return self._views_in_flight
 
     def _check(self, rc: int):
         if rc != OK:
@@ -420,6 +429,22 @@ class Context:
                                                    C.c_void_p(grad_alpha_ptr or None), C.c_void_p(grad_q_ptr or None),
                                                    C.c_void_p(out_ptr or None), C.c_void_p(stream),
                                                    C.byref(st) if stats else None))
+        self.last_stats = st.as_dict() if stats else {}
+        return self.last_stats
+
+    def render_flux_grad_device(self, views, g_ptr: int, grad_alpha_ptr: int, grad_q_ptr: int, stream: int = 0, *,
+                                stats: bool = True) -> dict:
+        """The gradient of sum_k g_k . total_k, total_k the {sum tau, sum I} of render_flux for views[k]
+        (round_through_float = 0), on DEVICE memory (c5_render_flux_grad_device), enqueued on `stream`. g_ptr:
+        len(views) * 2 doubles {g_tau_k, g_I_k}; grad_alpha_ptr / grad_q_ptr as for render_grad_device. The
+        views run on the context's views_in_flight lanes. stats=False: enqueue only; returns {}. With stats, the
+        counts are summed over the views and ms_total is the call's span on `stream`."""
+        views = list(views)
+        arr = (View * max(len(views), 1))(*views)
+        st = Stats() if stats else None
+        self._check(self.lib.c5_render_flux_grad_device(self._h, arr if views else None, len(views), C.c_void_p(g_ptr),
+                                                        C.c_void_p(grad_alpha_ptr or None), C.c_void_p(grad_q_ptr or None),
+                                                        C.c_void_p(stream), C.byref(st) if stats else None))
         self.last_stats = st.as_dict() if stats else {}
         return self.last_stats
 

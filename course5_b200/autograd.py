@@ -23,14 +23,18 @@ synchronisation, so a whole fit step (forward, loss, backward, optimiser) runs o
 a ray stopped by the step cap (C5_E_WALK, impossible on a valid mesh) is not reported.
 
 light_curve(ctx, views, alpha, q) is the differentiable {sum tau, sum I} of each view (c5_render_flux
-totals): its backward is one gradient per view against a constant upstream gradient.
+totals). On CUDA tensors its forward is the pipelined c5_render_flux_submit loop over the context's
+views_in_flight lanes (one host wait per curve), and its backward is one c5_render_flux_grad_device call
+over all views, on the same lanes, with grad_output read in place and no host synchronisation. On CPU
+tensors it renders the views one by one and its backward is one c5_render_grad per view against g filled
+with that view's upstream gradient.
 """
 from __future__ import annotations
 
 import numpy as np
 import torch
 
-from . import api
+from . import api, sweep
 
 
 def _raw_view(view: api.View) -> api.View:
@@ -134,7 +138,10 @@ class _LightCurve(torch.autograd.Function):
     def forward(fn_ctx, ctx: api.Context, views, alpha: torch.Tensor, q: torch.Tensor):
         vs = [_raw_view(v) for v in views]
         fn_ctx.version = _fields(ctx, alpha, q)
-        totals = np.stack([ctx.render_flux(v)[1][0] for v in vs])  # (n_views, 2): {sum tau, sum I}
+        if alpha.device.type == "cuda":
+            totals = sweep.render_light_curve(ctx, vs, in_flight=ctx.views_in_flight)[0][:, 0]
+        else:
+            totals = np.stack([ctx.render_flux(v)[1][0] for v in vs])  # (n_views, 2): {sum tau, sum I}
         fn_ctx.save_for_backward(alpha, q)
         fn_ctx.c5 = ctx
         fn_ctx.views = vs
@@ -149,21 +156,24 @@ class _LightCurve(torch.autograd.Function):
         want_alpha, want_q = fn_ctx.needs_input_grad[2], fn_ctx.needs_input_grad[3]
         if not (want_alpha or want_q):
             return None, None, None, None
-        on_device = alpha.device.type == "cuda"
-        go = grad_output.detach().to(dtype=torch.float64, device=alpha.device if on_device else "cpu")
+        if alpha.device.type == "cuda":
+            # every view's {g_tau, g_I} read in place by the kernels: no fill, no host synchronisation
+            go = grad_output.detach().to(dtype=torch.float64, device=alpha.device).contiguous()
+            ga = torch.empty_like(alpha) if want_alpha else None
+            gq = torch.empty_like(alpha) if want_q else None
+            ctx.render_flux_grad_device(fn_ctx.views, go.data_ptr(), ga.data_ptr() if want_alpha else 0,
+                                        gq.data_ptr() if want_q else 0, stream=_stream(alpha.device), stats=False)
+            return None, None, ga, gq
+        go = grad_output.detach().to(dtype=torch.float64, device="cpu")
         sums = [torch.zeros_like(alpha) if want_alpha else None, torch.zeros_like(alpha) if want_q else None]
         for k, v in enumerate(fn_ctx.views):
             # the flux is the image summed over the pixels outside the solid mask: its upstream gradient
             # is grad_output[k] in every pixel, and the gradient pass skips masked and background pixels
             rb, re = _band(v)
-            if on_device:
-                g = go[k].expand(re - rb, v.res_x, 2).contiguous()  # a device fill of the band
-                parts = _grad_device(ctx, v, g, alpha, want_alpha, want_q)
-            else:
-                g = np.zeros((v.res_y, v.res_x, 2))
-                g[rb:re] = go[k].numpy()
-                parts = [None if x is None else torch.from_numpy(x)
-                         for x in ctx.render_grad(v, g, alpha=want_alpha, q=want_q)]
+            g = np.zeros((v.res_y, v.res_x, 2))
+            g[rb:re] = go[k].numpy()
+            parts = [None if x is None else torch.from_numpy(x)
+                     for x in ctx.render_grad(v, g, alpha=want_alpha, q=want_q)]
             for s, p in zip(sums, parts):
                 if s is not None:
                     s += p

@@ -543,32 +543,40 @@ struct GradResult {
 };
 
 // The depth pass (with the view prologue, enqueue_view) and the gradient pass of band [row_begin,row_end)
-// of v on d.stream, into d.grad_alpha / d.grad_q (Morton order). The band's {g_tau, g_I} per pixel are
-// g_host's rows (the whole image, copied to d.grad_in) or d_g (a device band buffer, read in place).
+// of v on d.stream, into d.grad_alpha / d.grad_q (Morton order), zeroed first. The band's {g_tau, g_I} per
+// pixel are g_host's rows (the whole image, copied to d.grad_in) or d_g (a device band buffer, read in
+// place); with g_per_view, d_g is the view's one {g_tau, g_I}. acc != null: the pass adds into acc's
+// accumulators instead, which the caller has zeroed (the views of c5_render_flux_grad_device).
 // Events: 0..4 as for an image, 5 depth pass done.
-void enqueue_grad(DeviceState& d, const c5_view* v, const ViewPlan& p, const double* g_host, const double* d_g) {
+void enqueue_grad(DeviceState& d, const c5_view* v, const ViewPlan& p, const double* g_host, const double* d_g,
+                  DeviceState* acc = nullptr, bool g_per_view = false) {
     const size_t n_t = static_cast<size_t>(d.n_tets);
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
     const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
     // the gradient pass counts into the second half, so that the stats stay the depth pass's
     d.counters.ensure(2 * kNumCounters);
     d.row_cost.ensure(2 * static_cast<size_t>(v->res_y));
-    d.grad_alpha.ensure(n_t);
-    d.grad_q.ensure(n_t);
+    if (!acc) {
+        d.grad_alpha.ensure(n_t);
+        d.grad_q.ensure(n_t);
+    }
     if (g_host) d.grad_in.ensure(2 * static_cast<size_t>(v->res_y) * v->res_x);
     enqueue_view(d, v, p, false, nullptr, 0, kDepthPass);
     record(d, 5);
-    dev_zero(d.grad_alpha.p, n_t * sizeof(double), d.stream);
-    dev_zero(d.grad_q.p, n_t * sizeof(double), d.stream);
+    if (!acc) {
+        dev_zero(d.grad_alpha.p, n_t * sizeof(double), d.stream);
+        dev_zero(d.grad_q.p, n_t * sizeof(double), d.stream);
+    }
     dev_zero(d.counters.p + kNumCounters, kNumCounters * sizeof(unsigned long long), d.stream);
     dev_zero(d.row_cost.p + v->res_y, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
     if (g_host) h2d(d.grad_in.p, g_host + 2 * band_off, 2 * n_pix_band * sizeof(double), d.stream);
     WalkLaunch w = view_walk(d, v, p);
     w.pass = kGradPass;
     w.depth = d.out.p;
-    w.grad_in = g_host ? d.grad_in.p : d_g; // indexed like the band's out
-    w.grad_alpha = d.grad_alpha.p;
-    w.grad_q = d.grad_q.p;
+    w.grad_in = g_host ? d.grad_in.p : d_g; // indexed like the band's out, or the view's one pair
+    w.grad_per_view = g_per_view ? 1 : 0;
+    w.grad_alpha = (acc ? *acc : d).grad_alpha.p;
+    w.grad_q = (acc ? *acc : d).grad_q.p;
     w.counters = d.counters.p + kNumCounters;
     w.row_cost = d.row_cost.p + v->res_y;
     launch_walk(d, w);
@@ -739,6 +747,105 @@ void grad_band_device(c5_ctx* ctx, const c5_view* v, const double* d_g, double* 
         throw;
     }
     d.stream = own;
+}
+
+// Two timing events for the span of a call on a caller's stream (created only when stats are asked for).
+struct SpanEvents {
+    cudaEvent_t e[2] = {};
+    ~SpanEvents() {
+        for (cudaEvent_t x : e) {
+            if (x) cudaEventDestroy(x);
+        }
+    }
+};
+
+// c5_render_flux_grad_device: view k goes to lane k % views_in_flight, where the depth and the gradient pass
+// run on the lane's own stream with the view's one upstream pair d_g[2k..2k+1], all adding into the owner's
+// Morton-order accumulators; one scatter into file order on the caller's stream at the end.
+void flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_g, double* d_grad_alpha,
+                      double* d_grad_q, void* stream, c5_stats* stats) {
+    if (ctx->parent) fail(C5_E_STATE, "render_flux_grad_device: a sibling context; call through its parent");
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
+        if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "render_flux_grad_device: a submitted view is in flight");
+    }
+    std::vector<ViewPlan> plans;
+    for (int32_t k = 0; k < n_views; k++) plans.push_back(plan_view(&views[k]));
+    ensure_lanes(ctx);
+    const unsigned n_lanes = static_cast<unsigned>(ctx->lanes.size()) + 1;
+    for (unsigned k = 0; k < n_lanes; k++) follow_parent(lane_of(ctx, k));
+    DeviceState& o = ctx->dev;
+    use_device(o);
+    const uint32_t* tperm = resident_tperm(ctx);
+    const size_t n_t = static_cast<size_t>(o.n_tets);
+    o.grad_alpha.ensure(n_t);
+    o.grad_q.ensure(n_t);
+    if (stats && static_cast<size_t>(n_views) * kNumCounters > o.h_view_counters_n) {
+        host_pinned_free(o.h_view_counters);
+        o.h_view_counters = nullptr;
+        o.h_view_counters_n = 0;
+        const size_t n = static_cast<size_t>(n_views) * kNumCounters;
+        o.h_view_counters = static_cast<unsigned long long*>(host_pinned_alloc(n * sizeof(unsigned long long)));
+        o.h_view_counters_n = n;
+    }
+    cudaStream_t s = kHostSim ? o.stream : static_cast<cudaStream_t>(stream);
+    SpanEvents span;
+    if (stats && !kHostSim) {
+        for (cudaEvent_t& e : span.e) C5_CUDA(cudaEventCreate(&e));
+        C5_CUDA(cudaEventRecord(span.e[0], s));
+    }
+    // 1. the accumulators are zeroed on `stream` once the context's own stream is done with them (an earlier
+    // call's scatter, a host-form gradient), 2. every lane starts after that (and so after the caller's
+    // earlier work on `stream`, such as a field update or whatever wrote d_g)
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(o.ev_fields, o.stream));
+        C5_CUDA(cudaStreamWaitEvent(s, o.ev_fields, 0));
+    }
+    dev_zero(o.grad_alpha.p, n_t * sizeof(double), s);
+    dev_zero(o.grad_q.p, n_t * sizeof(double), s);
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(o.ev_fields, s));
+        for (unsigned k = 0; k < n_lanes; k++) C5_CUDA(cudaStreamWaitEvent(lane_of(ctx, k)->dev.stream, o.ev_fields, 0));
+    }
+    for (int32_t k = 0; k < n_views; k++) {
+        DeviceState& d = lane_of(ctx, static_cast<unsigned>(k) % n_lanes)->dev;
+        enqueue_grad(d, &views[k], plans[static_cast<size_t>(k)], nullptr, d_g + 2 * static_cast<size_t>(k), &o, true);
+        if (stats) d2h(o.h_view_counters + static_cast<size_t>(k) * kNumCounters, d.counters.p,
+                       kNumCounters * sizeof(unsigned long long), d.stream);
+    }
+    // 3. `stream` waits for every lane, then scatters
+    if (!kHostSim) {
+        for (unsigned k = 0; k < n_lanes; k++) {
+            DeviceState& d = lane_of(ctx, k)->dev;
+            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
+            C5_CUDA(cudaStreamWaitEvent(s, d.ev_fields, 0));
+        }
+    }
+    g_launch_counter = &o.launches;
+    scatter_grads(o.n_tets, tperm, o.grad_alpha.p, o.grad_q.p, d_grad_alpha, d_grad_q, s);
+    // 4. the context's own later renders (and the next call's zeroing) wait for the scatter
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(o.ev_fields, s));
+        C5_CUDA(cudaStreamWaitEvent(o.stream, o.ev_fields, 0));
+    }
+    if (!stats) return;
+    if (!kHostSim) C5_CUDA(cudaEventRecord(span.e[1], s));
+    stream_sync(s);
+    c5_stats st{};
+    for (int32_t k = 0; k < n_views; k++) {
+        const unsigned long long* c = o.h_view_counters + static_cast<size_t>(k) * kNumCounters;
+        const ViewPlan& p = plans[static_cast<size_t>(k)];
+        st.pixels += static_cast<uint64_t>(p.row_end - p.row_begin) * static_cast<uint64_t>(views[k].res_x);
+        st.tet_steps += c[kSteps];
+        st.hit_pixels += c[kHitPixels];
+        st.solid_pixels += c[kSolidPixels];
+        st.walk_errors += c[kWalkErrors];
+        st.grazing_rays += static_cast<int32_t>(c[kDeferred]);
+    }
+    if (!kHostSim) C5_CUDA(cudaEventElapsedTime(&st.ms_total, span.e[0], span.e[1]));
+    st.n_devices = 1;
+    *stats = st;
+    if (st.walk_errors) fail(C5_E_WALK, "render: " + std::to_string(st.walk_errors) + " ray(s) exceeded the step cap");
 }
 
 void upload_solids(c5_ctx* ctx, const double* pts, int64_t n, int follows) {
@@ -917,6 +1024,7 @@ int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out) {
             C5_CUDA(cudaEventCreate(&d.ev_walk));
             C5_CUDA(cudaEventCreateWithFlags(&d.ev_done, cudaEventDisableTiming));
             C5_CUDA(cudaEventCreateWithFlags(&d.ev_fields, cudaEventDisableTiming));
+            C5_CUDA(cudaEventCreateWithFlags(&d.ev_gather, cudaEventDisableTiming));
         }
         for (int k = 1; k < n_dev; k++) { // every further device: a single-device context of its own
             c5_ctx* part = nullptr;
@@ -944,6 +1052,16 @@ int c5_create_sibling(c5_ctx* parent, c5_ctx** out) {
     c5_ctx* ctx = nullptr;
     const int rc = c5_create(&device, 1, &ctx);
     if (rc != C5_OK) return rc;
+    // the internal streams made before a c5_update_fields_device wait for its gather; a sibling made after it
+    // waits here, so that its renders see the new fields too (an event never recorded is no wait)
+    if (!kHostSim) {
+        const cudaError_t e = cudaStreamWaitEvent(ctx->dev.stream, parent->dev.ev_gather, 0);
+        if (e != cudaSuccess) {
+            parent->err = std::string("create_sibling: ") + cudaGetErrorString(e);
+            c5_destroy(ctx);
+            return C5_E_CUDA;
+        }
+    }
     ctx->parent = parent;
     parent->siblings.push_back(ctx);
     DeviceState& from = parent->dev;
@@ -993,11 +1111,13 @@ void c5_destroy(c5_ctx* ctx) {
     host_pinned_free(d.h_counters);
     host_pinned_free(d.h_row_cost);
     host_pinned_free(d.h_row_flux);
+    host_pinned_free(d.h_view_counters);
     if (!kHostSim) {
         for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
         if (d.ev_walk) cudaEventDestroy(d.ev_walk);
         if (d.ev_done) cudaEventDestroy(d.ev_done);
         if (d.ev_fields) cudaEventDestroy(d.ev_fields);
+        if (d.ev_gather) cudaEventDestroy(d.ev_gather);
         for (auto& e : d.ev) {
             if (e) cudaEventDestroy(e);
         }
@@ -1267,9 +1387,9 @@ int c5_update_fields_device(c5_ctx* ctx, const double* d_alpha, const double* d_
         }
         ctx->dev.mesh_version++; // siblings and lanes re-alias at their next render
         gather_fields(d, tperm, d_alpha, d_q, s);
-        if (!kHostSim) { // ... and every later one waits for the gather
-            C5_CUDA(cudaEventRecord(d.ev_fields, s));
-            for (DeviceState* x : internal) C5_CUDA(cudaStreamWaitEvent(x->stream, d.ev_fields, 0));
+        if (!kHostSim) { // ... and every later one waits for the gather, also those of lanes made later
+            C5_CUDA(cudaEventRecord(d.ev_gather, s));
+            for (DeviceState* x : internal) C5_CUDA(cudaStreamWaitEvent(x->stream, d.ev_gather, 0));
         }
     });
 }
@@ -1289,6 +1409,26 @@ int c5_render_grad_device(c5_ctx* ctx, const c5_view* view, const double* d_g, d
         }
         if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_grad_device: single-device contexts only");
         grad_band_device(ctx, view, d_g, d_grad_alpha, d_grad_q, d_out, stream, stats);
+    });
+}
+
+int c5_render_flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_g,
+                               double* d_grad_alpha, double* d_grad_q, void* stream, c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (n_views < 1 || !views) fail(C5_E_INVALID, "render_flux_grad_device: need at least one view");
+        check_device_array(d_g, "render_flux_grad_device: d_g");
+        if (!d_grad_alpha && !d_grad_q) fail(C5_E_INVALID, "render_flux_grad_device: d_grad_alpha and d_grad_q are both NULL");
+        if (d_grad_alpha) check_device_array(d_grad_alpha, "render_flux_grad_device: d_grad_alpha");
+        if (d_grad_q) check_device_array(d_grad_q, "render_flux_grad_device: d_grad_q");
+        for (int32_t k = 0; k < n_views; k++) {
+            if (views[k].precision == 32) fail(C5_E_INVALID, "render_flux_grad_device: FP64 only (precision 64)");
+            if (views[k].round_through_float) {
+                fail(C5_E_INVALID, "render_flux_grad_device: the float cast has no useful derivative; set round_through_float = 0");
+            }
+        }
+        if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_flux_grad_device: single-device contexts only");
+        flux_grad_device(ctx, views, n_views, d_g, d_grad_alpha, d_grad_q, stream, stats);
     });
 }
 

@@ -94,12 +94,15 @@ struct DeviceState {
     cudaEvent_t ev_walk = nullptr;   // between the pixel kernel and the grazing-ray kernel (phase times)
     cudaEvent_t ev_done = nullptr;   // after the view's last copy: what c5_render_wait waits for
     cudaEvent_t ev_fields = nullptr; // orders this stream and a caller's stream around the device-form gradient calls
+    cudaEvent_t ev_gather = nullptr; // after the last c5_update_fields_device gather: a sibling made later waits on it
     // results of the view in flight, copied by the stream into pinned host memory
     unsigned long long* h_counters = nullptr;   // [kNumCounters]
     uint64_t* h_row_cost = nullptr;             // [h_row_cost_n]
     size_t h_row_cost_n = 0;
     double* h_row_flux = nullptr;               // [h_row_flux_n]: row_flux of a flux view
     size_t h_row_flux_n = 0;
+    unsigned long long* h_view_counters = nullptr; // c5_render_flux_grad_device with stats: [view][kNumCounters]
+    size_t h_view_counters_n = 0;
     // c5_debug_set (tests, diagnostics); 0 = default
     int opt_graze_list = 0, opt_query_budget = 0, opt_serial_list = 0, opt_mask_tile = 0;
     bool opt_no_zero_copy = false, opt_no_static_mask = false;
@@ -202,8 +205,10 @@ struct WalkLaunch {
     cudaEvent_t mark_walk_done_tl; // the same moment for the timeline ring (may be null)
     // c5_render_grad (channels 0, precision 64): kDepthPass stores {tau, I, lam, 0} per pixel into out;
     // kGradPass reads them (depth) and the band's {g_tau, g_I} (grad_in), adds into grad_alpha / grad_q,
-    // stores no pixel and counts into its own counters / row_cost
+    // stores no pixel and counts into its own counters / row_cost. grad_per_view: grad_in is the view's one
+    // {g_tau, g_I}, the upstream of every pixel (c5_render_flux_grad_device)
     int pass;
+    int grad_per_view;
     const double* depth;
     const double* grad_in;
     double* grad_alpha;

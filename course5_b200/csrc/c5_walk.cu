@@ -79,7 +79,8 @@ struct WalkParams {
 // The gradient pass's kernels take these (the walk functions see the WalkParams part; the gradient
 // policy below casts back). A separate type keeps WalkParams, and so every other kernel, as it was.
 struct GradParams : WalkParams {
-    const double* grad_in; // band buffer: {g_tau, g_I} per pixel, indexed like out
+    const double* grad_in; // band buffer: {g_tau, g_I} per pixel, indexed like out (the per-view kernels: the
+                           // view's one {g_tau, g_I}, c5_render_flux_grad_device)
     const double* depth;   // the depth pass's band buffer: {tau, I, lam, 0} per pixel
     double* grad_alpha;    // [n_tets] Morton order, accumulated with atomics
     double* grad_q;
@@ -695,8 +696,11 @@ struct GradRay {
     double g_tau, g_I, lam_ray;
 };
 
+// kViewG: every pixel of the view has the same upstream, the two doubles at grad_in.
+template <bool kViewG>
 C5_HD GradRay grad_ray(const GradParams& P, uint32_t pixel) {
     const size_t o = pixel - static_cast<size_t>(P.row_begin) * static_cast<size_t>(P.res_x);
+    if (kViewG) return GradRay{P.grad_in[0], P.grad_in[1], P.depth[4 * o + 2]};
     return GradRay{P.grad_in[2 * o], P.grad_in[2 * o + 1], P.depth[4 * o + 2]};
 }
 
@@ -773,7 +777,10 @@ struct CellsDepth { // {tau, I} of CellsF64 and {lam, 0}
     }
 };
 
-struct CellsGrad { // the gradient pass: nothing is stored but the atomics; P is the WalkParams of a GradParams
+// The gradient pass: nothing is stored but the atomics; P is the WalkParams of a GradParams. kViewG: one
+// upstream per view (grad_ray), the light-curve form.
+template <bool kViewG>
+struct CellsGradT {
     static constexpr int K = 1;
     static constexpr bool kChanQueue = false;
     static constexpr bool kImage = false;
@@ -786,7 +793,7 @@ struct CellsGrad { // the gradient pass: nothing is stored but the atomics; P is
     static C5_HD double grad_crossing(const WalkParams& P, double px, double py, uint32_t pixel, int leaf, double z_in,
                                       Pairs<1>& v, uint32_t& steps, uint32_t& error) {
         const GradParams& G = static_cast<const GradParams&>(P);
-        GradFields acc{G, v, grad_ray(G, pixel), 0};
+        GradFields acc{G, v, grad_ray<kViewG>(G, pixel), 0};
         return crossing_walk<false>(P, px, py, leaf, z_in, acc, steps, error);
     }
     static C5_HD double lam_crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<1>& v,
@@ -795,6 +802,8 @@ struct CellsGrad { // the gradient pass: nothing is stored but the atomics; P is
         return crossing_walk<true>(P, px, py, leaf, z_in, acc, steps, error);
     }
 };
+using CellsGrad = CellsGradT<false>;
+using CellsGradView = CellsGradT<true>;
 
 C5_HD void store2(double* p, double a, double b) {
 #ifdef __CUDA_ARCH__
@@ -966,8 +975,9 @@ C5_HD RayAcc<F::K> graze_ray_serial(const WalkParams& P, unsigned long long slot
 // The gradient pass's serial form: each crossing is walked affinely for its lam and (A, B), re-walked
 // with the gradient from the I and lam it is entered with, then composed — what the warp form does
 // for 32 crossings at a time.
+template <class F>
 C5_HD void graze_ray_serial_grad(const WalkParams& P, unsigned long long slot, double px, double py) {
-    RayAcc<1> a = load_deferred<CellsGrad>(P, slot);
+    RayAcc<1> a = load_deferred<F>(P, slot);
     const uint32_t pixel = P.queue[slot].pixel;
     EntryList<kSerialList> L;
     int crossings = 0;
@@ -978,10 +988,10 @@ C5_HD void graze_ray_serial_grad(const WalkParams& P, unsigned long long slot, d
             Pairs<1> k;
             k.reset();
             uint32_t steps_k = 0, error_k = 0;
-            const double z_out = CellsGrad::lam_crossing(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
+            const double z_out = F::lam_crossing(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
             Pairs<1> v = a.v;
             uint32_t steps_g = 0, error_g = 0;
-            CellsGrad::grad_crossing(P, px, py, pixel, L.leaf[e], L.z[e], v, steps_g, error_g);
+            F::grad_crossing(P, px, py, pixel, L.leaf[e], L.z[e], v, steps_g, error_g);
             compose_crossing(a, L.z[e], z_out, k, steps_k, error_k);
             if (++crossings > 65536) a.error = 1;
         }
@@ -1217,6 +1227,7 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
 // affinely, keeping its lam; (2) the warp folds the batch in z order exactly as graze_block does, and each
 // lane notes the {lam, I} its crossing is entered with (and whether the fold takes it); (3) the lanes
 // whose crossing was taken walk it again with the gradient.
+template <class F>
 __device__ __forceinline__ void graze_block_grad(const WalkParams& P) {
     __shared__ GrazeSmem smem[kGrazeWarps];
     const unsigned full = 0xFFFFFFFFu;
@@ -1232,7 +1243,7 @@ __device__ __forceinline__ void graze_block_grad(const WalkParams& P) {
         const int i = static_cast<int>(q_pixel % static_cast<uint32_t>(P.res_x));
         const int j = static_cast<int>(q_pixel / static_cast<uint32_t>(P.res_x));
         const double px = P.xs[i], py = P.ys[j];
-        RayAcc<1> a = load_deferred<CellsGrad>(P, ticket);
+        RayAcc<1> a = load_deferred<F>(P, ticket);
         int crossings = 0;
         bool truncated = true;
         while (truncated && !a.error) {
@@ -1246,7 +1257,7 @@ __device__ __forceinline__ void graze_block_grad(const WalkParams& P) {
                 f.reset();
                 uint32_t steps_k = 0, error_k = 0;
                 if (have && z_in > a.z_after) {
-                    z_out = CellsGrad::lam_crossing(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
+                    z_out = F::lam_crossing(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
                 }
                 const int cnt = n - base < 32 ? n - base : 32;
                 Pairs<1> entered = a.v;
@@ -1266,7 +1277,7 @@ __device__ __forceinline__ void graze_block_grad(const WalkParams& P) {
                 }
                 if (taken) {
                     uint32_t steps_g = 0, error_g = 0;
-                    CellsGrad::grad_crossing(P, px, py, q_pixel, S.leaf[k], z_in, entered, steps_g, error_g);
+                    F::grad_crossing(P, px, py, q_pixel, S.leaf[k], z_in, entered, steps_g, error_g);
                 }
             }
             crossings += n;
@@ -1404,7 +1415,12 @@ __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_ch(const WalkPa
 __global__ void __launch_bounds__(kBlock) tet_walk_depth(const WalkParams P) { walk_block<CellsDepth>(P); }
 __global__ void __launch_bounds__(kBlock) tet_walk_grad(const GradParams P) { walk_block<CellsGrad>(P); }
 __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_depth(const WalkParams P) { graze_block<CellsDepth>(P); }
-__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad(const GradParams P) { graze_block_grad(P); }
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad(const GradParams P) { graze_block_grad<CellsGrad>(P); }
+// The gradient pass with one {g_tau, g_I} per view (c5_render_flux_grad_device): registers in DESIGN.md §5c.
+__global__ void __launch_bounds__(kBlock) tet_walk_grad_view(const GradParams P) { walk_block<CellsGradView>(P); }
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad_view(const GradParams P) {
+    graze_block_grad<CellsGradView>(P);
+}
 
 namespace {
 
@@ -1435,6 +1451,11 @@ template <>
 struct Kernels<CellsGrad> {
     static constexpr void (*walk)(GradParams) = tet_walk_grad;
     static constexpr void (*graze)(GradParams) = grazing_rays_grad;
+};
+template <>
+struct Kernels<CellsGradView> {
+    static constexpr void (*walk)(GradParams) = tet_walk_grad_view;
+    static constexpr void (*graze)(GradParams) = grazing_rays_grad_view;
 };
 
 void background_on_host(const WalkParams& P, int n) {
@@ -1487,16 +1508,24 @@ void graze_on_host(const WalkParams& P) {
     P.counters[kTicket] = n_rays;
 }
 
-template <>
-void graze_on_host<CellsGrad>(const WalkParams& P) {
+template <class F>
+void graze_grad_on_host(const WalkParams& P) {
     const unsigned long long n_rays = P.counters[kDeferred];
     for (unsigned long long k = 0; k < n_rays; k++) {
         const uint32_t pixel = P.queue[k].pixel;
         const int i = static_cast<int>(pixel % static_cast<uint32_t>(P.res_x));
         const int j = static_cast<int>(pixel / static_cast<uint32_t>(P.res_x));
-        graze_ray_serial_grad(P, k, P.xs[i], P.ys[j]);
+        graze_ray_serial_grad<F>(P, k, P.xs[i], P.ys[j]);
     }
     P.counters[kTicket] = n_rays;
+}
+template <>
+void graze_on_host<CellsGrad>(const WalkParams& P) {
+    graze_grad_on_host<CellsGrad>(P);
+}
+template <>
+void graze_on_host<CellsGradView>(const WalkParams& P) {
+    graze_grad_on_host<CellsGradView>(P);
 }
 
 // Policy F's pixel kernel over `grid` blocks, then its grazing-ray kernel for the rays the pixel
@@ -1603,7 +1632,11 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
         G.depth = w.depth;
         G.grad_alpha = w.grad_alpha;
         G.grad_q = w.grad_q;
-        launch_rays<CellsGrad>(d, w, G, grid);
+        if (w.grad_per_view) {
+            launch_rays<CellsGradView>(d, w, G, grid);
+        } else {
+            launch_rays<CellsGrad>(d, w, G, grid);
+        }
         return;
     }
     switch (w.channels) {

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define C5_ABI_VERSION 6
+#define C5_ABI_VERSION 7
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
 #define C5_MAX_CHANNELS 8
@@ -242,7 +242,8 @@ int c5_render_flux_submit(c5_ctx* ctx, const c5_view* view, int32_t channels, do
  * C5_E_INVALID: NULL g, both gradient arrays NULL, precision 32, or
  * round_through_float != 0 (the float cast is piecewise constant: ask for the raw values).
  * C5_E_STATE: no mesh, or a submitted view in flight on this context. Single-device, multi-device and
- * sibling contexts. Not covered: uploaded channels, the FP32 variant, a pipelined (submit) form. */
+ * sibling contexts. Not covered: uploaded channels, the FP32 variant. The views of a light curve go through
+ * the lanes in one call, c5_render_flux_grad_device below. */
 int c5_update_fields(c5_ctx* ctx, const double* alpha, const double* q);
 int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* grad_alpha, double* grad_q, double* out,
                    c5_stats* stats);
@@ -256,8 +257,8 @@ int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* gr
  * render afterwards is bit-identical to one from a fresh upload of these fields.
  * Ordering, without synchronising the host: the gather is enqueued on `stream` (a cudaStream_t; NULL = the
  * legacy default stream) after `stream` has waited (events) for everything the library had enqueued on the
- * internal streams of the context, its lanes and its siblings; those internal streams then wait for the
- * gather, so the library's later renders (c5_render, c5_render_raw, c5_render_flux, submits, ...) and the
+ * internal streams of the context, its lanes and its siblings; those internal streams, and those of lanes
+ * and siblings made later, then wait for the gather, so the library's later renders (c5_render, c5_render_raw, c5_render_flux, submits, ...) and the
  * caller's later work on `stream` see the new fields. Work the caller put on streams of its own (e.g.
  * c5_render_device with stats == NULL) is the caller's to order, as for c5_render_device. d_alpha and d_q
  * must stay valid until the gather has run on `stream`. C5_E_INVALID: a NULL or not 8-byte aligned pointer,
@@ -280,6 +281,31 @@ int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* gr
 int c5_update_fields_device(c5_ctx* ctx, const double* d_alpha, const double* d_q, void* stream);
 int c5_render_grad_device(c5_ctx* ctx, const c5_view* view, const double* d_g, double* d_grad_alpha, double* d_grad_q,
                           double* d_out, void* stream, c5_stats* stats);
+
+/* c5_render_flux_grad_device is the gradient of a light curve, on device memory: with total_k view k's
+ * c5_render_flux total {sum tau, sum I} (round_through_float = 0), it gives the gradient of
+ * sum_k g_k . total_k, that is
+ *   grad_alpha[t] = sum_k sum_{p not under the solid mask} (g_tau_k dtau_p/dalpha_t + g_I_k dI_p/dalpha_t),
+ * and grad_q[t] likewise with g_I_k dI_p/dQ_t. d_g holds n_views * 2 doubles {g_tau_k, g_I_k} on the
+ * context's device; the kernels read it, the host does not. d_grad_alpha and d_grad_q (n_tets doubles
+ * each, file order, overwritten; either may be NULL, not both) as for c5_render_grad_device. Each view
+ * keeps its own resolution, window, rotations and row band; views of different sizes may be mixed.
+ * The views are dealt round-robin to the context's lanes (c5_set_views_in_flight, the lanes of
+ * c5_render_submit); each runs the depth pass and the gradient pass on its lane's stream, all lanes add
+ * into one accumulator, and one scatter to file order runs at the end. Ordering, without synchronising the
+ * host: the accumulator is zeroed on `stream` and every lane starts after that, so after the caller's
+ * earlier work on `stream` (a c5_update_fields_device, whatever wrote d_g); `stream` then waits for every
+ * lane and runs the scatter, and the context's own later renders wait for it. Launches: the sum over the
+ * views of what c5_render_grad_device launches for each, less n_views - 1 (one scatter per call).
+ * stats == NULL: enqueue only, as for c5_render_grad_device. stats != NULL: `stream` is synchronised; the
+ * counts are summed over the views, each counted as c5_render_raw counts it, ms_total is the call's span
+ * on `stream` and the other ms_* fields are 0; a ray stopped by the step cap is C5_E_WALK.
+ * c5_last_row_cost is not changed. C5_E_INVALID: n_views < 1, NULL views or d_g, a pointer not 8-byte
+ * aligned, both gradients NULL, precision 32, round_through_float != 0, or a multi-device context.
+ * C5_E_STATE: no mesh, a sibling context, or a submitted view in flight on the context or one of its
+ * lanes. */
+int c5_render_flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_g,
+                               double* d_grad_alpha, double* d_grad_q, void* stream, c5_stats* stats);
 
 /* Device-resident variant for callers that own device memory (e.g. a torch tensor that an NCCL
  * gather will read): d_out is a DEVICE pointer on the context's first device to
