@@ -96,6 +96,9 @@ SYMBOLS = {
                                         C.c_void_p, C.POINTER(Stats)]),
     "c5_render_flux_grad_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
+    "c5_render_jvp": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _dp, _dp, _dp, C.POINTER(Stats)]),
+    "c5_render_jvp_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.POINTER(Stats)]),
     "c5_render_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_last_row_cost": (C.c_int, [C.c_void_p, _u64p, C.c_int32]),
     "c5_kernel_launches": (C.c_uint64, [C.c_void_p]),
@@ -112,7 +115,7 @@ SYMBOLS = {
 }
 IPC_HANDLE_BYTES = 80
 MAX_IN_FLIGHT = 8
-ABI_VERSION = 7        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
+ABI_VERSION = 8        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
 TIMELINE_PHASES = 6
 
 
@@ -429,6 +432,44 @@ class Context:
                                                    C.c_void_p(grad_alpha_ptr or None), C.c_void_p(grad_q_ptr or None),
                                                    C.c_void_p(out_ptr or None), C.c_void_p(stream),
                                                    C.byref(st) if stats else None))
+        self.last_stats = st.as_dict() if stats else {}
+        return self.last_stats
+
+    def render_jvp(self, view: View, v_alpha, v_q, *, image: bool = False):
+        """Jacobian-vector product of the pre-cast image along the field direction (v_alpha, v_q), each of
+        shape (n_tets,) in the order given to upload_mesh or None for zero, not both (c5_render_jvp; the view
+        needs round_through_float = 0). Returns the (res_y, res_x, 2) tangent image {dtau, dI} per pixel, and
+        with image=True also render_raw's (res_y, res_x, 2) {tau, I} image. One walk, no atomics: bit for
+        bit the same from run to run, for any row band and device count. Rows outside the band are 0."""
+        n_tets = self.n_tets
+        if v_alpha is None and v_q is None:
+            raise ValueError("v_alpha and v_q are both None")
+        dirs = []
+        for d in (v_alpha, v_q):
+            if d is not None:
+                d = np.ascontiguousarray(d, dtype=np.float64)
+                if d.shape != (n_tets,):
+                    raise ValueError("v_alpha and v_q need one value per tet of the uploaded mesh")
+            dirs.append(d)
+        tangent = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64)
+        out = np.zeros((view.res_y, view.res_x, 2), dtype=np.float64) if image else None
+        st = Stats()
+        self._check(self.lib.c5_render_jvp(self._h, C.byref(view), _ptr(dirs[0], _dp), _ptr(dirs[1], _dp),
+                                           _ptr(tangent, _dp), _ptr(out, _dp), C.byref(st)))
+        self.last_stats = st.as_dict()
+        return (tangent, out) if image else tangent
+
+    def render_jvp_device(self, view: View, v_alpha_ptr: int, v_q_ptr: int, tangent_ptr: int, out_ptr: int = 0,
+                          stream: int = 0, *, stats: bool = True) -> dict:
+        """render_jvp on DEVICE memory (c5_render_jvp_device), enqueued on `stream`. v_alpha_ptr / v_q_ptr:
+        n_tets doubles each, file order (0 = zero, not both); tangent_ptr and out_ptr (0 = none): the view's row
+        band only, (row_end - row_begin) * res_x * 2 doubles, 16-byte aligned. stats=False: enqueue only (no
+        readback, no synchronisation); returns {}."""
+        st = Stats() if stats else None
+        self._check(self.lib.c5_render_jvp_device(self._h, C.byref(view), C.c_void_p(v_alpha_ptr or None),
+                                                  C.c_void_p(v_q_ptr or None), C.c_void_p(tangent_ptr or None),
+                                                  C.c_void_p(out_ptr or None), C.c_void_p(stream),
+                                                  C.byref(st) if stats else None))
         self.last_stats = st.as_dict() if stats else {}
         return self.last_stats
 

@@ -28,6 +28,14 @@ views_in_flight lanes (one host wait per curve), and its backward is one c5_rend
 over all views, on the same lanes, with grad_output read in place and no host synchronisation. On CPU
 tensors it renders the views one by one and its backward is one c5_render_grad per view against g filled
 with that view's upstream gradient.
+
+Forward mode: both Functions have a jvp, so torch.autograd.forward_ad dual tensors (and gradcheck with
+check_forward_ad=True) go through render and light_curve. The tangent of render is one c5_render_jvp: a
+single walk that carries {dtau, dI} beside {tau, I}, bit-reproducible from run to run; on CUDA tensors it is
+c5_render_jvp_device on torch.cuda.current_stream() with no host synchronisation. The tangent of light_curve
+sums each view's tangent image over the pixels outside the solid mask (its non-NaN pixels); that sum need
+not be bit-identical to the summation order of c5_render_flux. torch.func.jvp needs the Functions written
+with a separate setup_context, which they are not.
 """
 from __future__ import annotations
 
@@ -88,6 +96,7 @@ class _Render(torch.autograd.Function):
         v = _raw_view(view)
         fn_ctx.version = _fields(ctx, alpha, q)
         fn_ctx.save_for_backward(alpha, q)
+        fn_ctx.save_for_forward(alpha, q)
         fn_ctx.c5 = ctx
         fn_ctx.view = v
         if alpha.device.type == "cpu":
@@ -116,6 +125,32 @@ class _Render(torch.autograd.Function):
         ga, gq = _grad_device(ctx, fn_ctx.view, g, alpha, want_alpha, want_q)
         return None, None, ga, gq
 
+    @staticmethod
+    def jvp(fn_ctx, _ctx_t, _view_t, alpha_t, q_t):
+        return _tangent_image(fn_ctx, fn_ctx.view, alpha_t, q_t)
+
+
+def _tangent_image(fn_ctx, view, alpha_t, q_t) -> torch.Tensor:
+    """The (res_y, res_x, 2) {dtau, dI} of `view` along (alpha_t, q_t) (either may be None: zero), at the fields
+    fn_ctx's forward saw, on their device; rows outside the view's band are 0."""
+    ctx: api.Context = fn_ctx.c5
+    alpha, q = fn_ctx.saved_tensors
+    if ctx.fields_version != fn_ctx.version:
+        fn_ctx.version = _fields(ctx, alpha, q)
+    if alpha_t is None and q_t is None:
+        return torch.zeros((view.res_y, view.res_x, 2), dtype=torch.float64, device=alpha.device)
+    if alpha.device.type == "cpu":
+        dirs = [None if t is None else t.detach().to(torch.float64).contiguous().numpy() for t in (alpha_t, q_t)]
+        return torch.from_numpy(ctx.render_jvp(view, dirs[0], dirs[1]))
+    dirs = [None if t is None else t.detach().to(dtype=torch.float64, device=alpha.device).contiguous()
+            for t in (alpha_t, q_t)]
+    rb, re = _band(view)
+    tangent = torch.zeros((view.res_y, view.res_x, 2), dtype=torch.float64, device=alpha.device)
+    # stream-ordered, like _fields: the direction copies return to torch's cache only for later work on this stream
+    ctx.render_jvp_device(view, 0 if dirs[0] is None else dirs[0].data_ptr(), 0 if dirs[1] is None else dirs[1].data_ptr(),
+                          tangent[rb:re].data_ptr(), stream=_stream(alpha.device), stats=False)
+    return tangent
+
 
 def _grad_device(ctx, view, g, alpha, want_alpha, want_q):
     """c5_render_grad_device of band-sized g into new CUDA tensors (None for one not wanted), enqueued only."""
@@ -143,6 +178,7 @@ class _LightCurve(torch.autograd.Function):
         else:
             totals = np.stack([ctx.render_flux(v)[1][0] for v in vs])  # (n_views, 2): {sum tau, sum I}
         fn_ctx.save_for_backward(alpha, q)
+        fn_ctx.save_for_forward(alpha, q)
         fn_ctx.c5 = ctx
         fn_ctx.views = vs
         return torch.from_numpy(totals).to(alpha.device)
@@ -178,6 +214,11 @@ class _LightCurve(torch.autograd.Function):
                 if s is not None:
                     s += p
         return None, None, sums[0], sums[1]
+
+    @staticmethod
+    def jvp(fn_ctx, _ctx_t, _views_t, alpha_t, q_t):
+        # the flux sums the pixels outside the solid mask, where the tangent image is not NaN
+        return torch.stack([_tangent_image(fn_ctx, v, alpha_t, q_t).nansum(dim=(0, 1)) for v in fn_ctx.views])
 
 
 def light_curve(ctx: api.Context, views, alpha: torch.Tensor, q: torch.Tensor) -> torch.Tensor:

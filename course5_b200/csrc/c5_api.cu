@@ -193,8 +193,9 @@ WalkLaunch view_walk(const DeviceState& d, const c5_view* v, const ViewPlan& p) 
 // 0 start, 1 rotated, 2 bvh, 3 mask, 4 walk.
 // channels > 0: the walk integrates that many uploaded channels (c5_render_channels).
 // pass = kDepthPass: the first pass of c5_render_grad ({tau, I, lam, 0} per pixel into d.out).
+// pass = kJvpPass: c5_render_jvp ({tau, I, dtau, dI} per pixel into d.out, the tangent along dir).
 void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want_steps, double* out_override = nullptr,
-                  int channels = 0, int pass = kImagePass) {
+                  int channels = 0, int pass = kImagePass, const double* dir = nullptr) {
     use_device(d);
     g_launch_counter = &d.launches;
     ensure_pixel_tables(d, v, p);
@@ -203,12 +204,13 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     // synchronisation) and a cudaMalloc on the spot.
     const size_t n_pix = static_cast<size_t>(v->res_y) * v->res_x;
     const bool solids = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0;
-    const size_t words = 2 * static_cast<size_t>(channels ? channels : pass == kDepthPass ? 2 : 1); // doubles per pixel
+    const bool two_pairs = pass == kDepthPass || pass == kJvpPass;
+    const size_t words = 2 * static_cast<size_t>(channels ? channels : two_pairs ? 2 : 1); // doubles per pixel
     if (!out_override) d.out.ensure(words * n_pix);
     if (want_steps) d.steps.ensure(n_pix);
     d.counters.ensure(kNumCounters);
     d.queue.ensure(n_pix); // every ray may be deferred (reserved, hardly ever touched)
-    if (channels || pass == kDepthPass) d.ch_queue.ensure(words * n_pix);
+    if (channels || two_pairs) d.ch_queue.ensure(words * n_pix);
     d.row_cost.ensure(static_cast<size_t>(v->res_y));
     if (solids) d.mask.ensure(n_pix);
 
@@ -234,6 +236,7 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     w.write_steps = want_steps ? 1 : 0;
     w.channels = channels;
     w.pass = pass;
+    w.dir = dir;
     w.out = out_override ? out_override : d.out.p;
     w.mark_walk_done = d.ev_walk;
     w.mark_walk_done_tl = nullptr;
@@ -848,6 +851,126 @@ void flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const 
     if (st.walk_errors) fail(C5_E_WALK, "render: " + std::to_string(st.walk_errors) + " ray(s) exceeded the step cap");
 }
 
+// ---- forward mode (c5_render_jvp, c5_render_jvp_device) -------------------------------------------------
+
+// The tangent field of ctx's own device state, [n_tets][2] {v_alpha, v_q} in Morton order: made at the state's
+// first call and reused by every later one. The context that owns the mesh counts it in device_bytes from then on
+// (a sibling's, like its other per-view arrays, is not counted); c5_upload_mesh drops it.
+double* resident_dir(c5_ctx* ctx) {
+    DeviceState& d = ctx->dev;
+    const size_t n = 2 * static_cast<size_t>(d.n_tets);
+    if (d.jvp_dir.n != n) { // first call, or a sibling that followed its parent to a mesh of another size
+        if (!ctx->parent) ctx->info.device_bytes -= static_cast<int64_t>(d.jvp_dir.bytes());
+        d.jvp_dir.alloc(n);
+        if (!ctx->parent) ctx->info.device_bytes += static_cast<int64_t>(d.jvp_dir.bytes());
+    }
+    return d.jvp_dir.p;
+}
+
+// One launch gathers the file-order direction (device pointers; a null one is 0) into the tangent field, then the
+// view's walk stores {tau, I, dtau, dI} per pixel of the band into d.out. Events: 0..4 as for an image.
+void enqueue_jvp(DeviceState& d, const c5_view* v, const ViewPlan& p, const uint32_t* tperm, double* dir,
+                 const double* d_v_alpha, const double* d_v_q) {
+    g_launch_counter = &d.launches;
+    gather_direction(d.n_tets, tperm, d_v_alpha, d_v_q, dir, d.stream);
+    enqueue_view(d, v, p, false, nullptr, 0, kJvpPass, dir);
+}
+
+// Band [row_begin,row_end) of v on ctx's device from host arrays: the direction goes to the device through the
+// gradient's scratch arrays (file order, n_tets each), then enqueue_jvp and the copy of the band. Blocks until the
+// results are on the host. Events: 0..4 as for enqueue_jvp, 5..6 around the copy.
+ViewResult jvp_band(c5_ctx* ctx, const c5_view* v, const double* v_alpha, const double* v_q, double* tangent,
+                    double* out) {
+    follow_parent(ctx);
+    if (ctx->pending.active) fail(C5_E_STATE, "render_jvp: this context still has a view in flight (c5_render_wait it first)");
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    const ViewPlan p = plan_view(v);
+    DeviceState& d = ctx->dev;
+    use_device(d);
+    const uint32_t* tperm = resident_tperm(ctx);
+    double* dir = resident_dir(ctx);
+    const size_t n_t = static_cast<size_t>(d.n_tets);
+    const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
+    const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
+    ensure_host_staging(d, static_cast<size_t>(v->res_y));
+    if (v_alpha) {
+        d.grad_alpha.ensure(n_t);
+        h2d(d.grad_alpha.p, v_alpha, n_t * sizeof(double), d.stream);
+    }
+    if (v_q) {
+        d.grad_q.ensure(n_t);
+        h2d(d.grad_q.p, v_q, n_t * sizeof(double), d.stream);
+    }
+    enqueue_jvp(d, v, p, tperm, dir, v_alpha ? d.grad_alpha.p : nullptr, v_q ? d.grad_q.p : nullptr);
+    record(d, 5);
+    std::vector<double> band(4 * n_pix_band); // {tau, I, dtau, dI} per pixel
+    d2h(band.data(), d.out.p, band.size() * sizeof(double), d.stream);
+    record(d, 6);
+    d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
+    d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
+    stream_sync(d.stream);
+    for (size_t k = 0; k < n_pix_band; k++) {
+        tangent[2 * (band_off + k)] = band[4 * k + 2];
+        tangent[2 * (band_off + k) + 1] = band[4 * k + 3];
+        if (out) {
+            out[2 * (band_off + k)] = band[4 * k];
+            out[2 * (band_off + k) + 1] = band[4 * k + 1];
+        }
+    }
+    return read_view(d, *v, p, true);
+}
+
+// c5_render_jvp_device on a single-device context or a sibling: enqueue_jvp on the caller's stream, then the
+// strided copies of the two pairs into the caller's band buffers.
+void jvp_band_device(c5_ctx* ctx, const c5_view* v, const double* d_v_alpha, const double* d_v_q, double* d_tangent,
+                     double* d_out, void* stream, c5_stats* stats) {
+    follow_parent(ctx);
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    if (ctx->pending.active) fail(C5_E_STATE, "render_jvp_device: this context has a submitted view in flight");
+    const ViewPlan p = plan_view(v);
+    DeviceState& d = ctx->dev;
+    use_device(d);
+    const uint32_t* tperm = resident_tperm(ctx);
+    double* dir = resident_dir(ctx);
+    const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
+    if (stats) ensure_host_staging(d, static_cast<size_t>(v->res_y));
+    // run on the CALLER's stream, like c5_render_device: the scratch arrays are the context's own
+    cudaStream_t own = d.stream;
+    if (!kHostSim) d.stream = static_cast<cudaStream_t>(stream);
+    try {
+        enqueue_jvp(d, v, p, tperm, dir, d_v_alpha, d_v_q);
+        record(d, 5);
+        d2d_2d(d_tangent, 2 * sizeof(double), d.out.p + 2, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
+        if (d_out) d2d_2d(d_out, 2 * sizeof(double), d.out.p, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
+        record(d, 6);
+        if (!kHostSim && d.stream != own) { // the context's own later renders reuse these scratch arrays: they wait
+            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
+            C5_CUDA(cudaStreamWaitEvent(own, d.ev_fields, 0));
+        }
+        if (stats) {
+            d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
+            d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
+            stream_sync(d.stream);
+            ViewResult r = read_view(d, *v, p, true);
+            report(ctx, r, stats);
+        }
+    } catch (...) {
+        d.stream = own;
+        throw;
+    }
+    d.stream = own;
+}
+
+// Arguments c5_render_jvp and c5_render_jvp_device share.
+void check_jvp_args(const c5_view* view, const double* v_alpha, const double* v_q, const double* tangent, const char* who) {
+    if (!tangent) fail(C5_E_INVALID, std::string(who) + ": tangent is NULL");
+    if (!v_alpha && !v_q) fail(C5_E_INVALID, std::string(who) + ": v_alpha and v_q are both NULL");
+    if (view && view->precision == 32) fail(C5_E_INVALID, std::string(who) + ": FP64 only (precision 64)");
+    if (view && view->round_through_float) {
+        fail(C5_E_INVALID, std::string(who) + ": the float cast has no useful derivative; set round_through_float = 0");
+    }
+}
+
 void upload_solids(c5_ctx* ctx, const double* pts, int64_t n, int follows) {
     if (n < 0 || (n > 0 && !pts)) fail(C5_E_INVALID, "upload_solids: bad arguments");
     if (n == 0) return;
@@ -1148,6 +1271,7 @@ int c5_upload_mesh(c5_ctx* ctx, const double* points_xyz, int64_t n_points, cons
             use_device(c->dev);
             upload_channels(c->dev, nullptr, nullptr, 0); // a new mesh drops the channels
             c->dev.tperm_dev.release();                   // and the device copy of the old permutation
+            c->dev.jvp_dir.release();                     // and the tangent field of c5_render_jvp
         }
         ctx->info.device_bytes -= ctx->channel_bytes;
         ctx->channel_bytes = 0;
@@ -1429,6 +1553,59 @@ int c5_render_flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_view
         }
         if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_flux_grad_device: single-device contexts only");
         flux_grad_device(ctx, views, n_views, d_g, d_grad_alpha, d_grad_q, stream, stats);
+    });
+}
+
+int c5_render_jvp(c5_ctx* ctx, const c5_view* view, const double* v_alpha, const double* v_q, double* tangent,
+                  double* out, c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        check_jvp_args(view, v_alpha, v_q, tangent, "render_jvp");
+        follow_parent(ctx);
+        if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+        const ViewPlan p = plan_view(view);
+        const std::vector<c5_ctx*> parts = with_parts(ctx);
+        const size_t n = parts.size();
+        if (static_cast<size_t>(p.row_end - p.row_begin) < n) fail(C5_E_INVALID, "render: fewer rows than devices");
+        const auto bands = cut_bands(ctx, view, p, static_cast<int>(n));
+        std::vector<c5_view> band_views(n, *view);
+        std::vector<ViewResult> results(n);
+        std::vector<std::exception_ptr> errors(n);
+        auto run = [&](size_t r) {
+            try {
+                band_views[r].row_begin = bands[r].first;
+                band_views[r].row_end = bands[r].second;
+                results[r] = jvp_band(parts[r], &band_views[r], v_alpha, v_q, tangent, out);
+            } catch (...) {
+                errors[r] = std::current_exception();
+            }
+        };
+        if (kHostSim || n == 1) {
+            for (size_t r = 0; r < n; r++) run(r);
+        } else {
+            std::vector<std::thread> workers;
+            for (size_t r = 0; r < n; r++) workers.emplace_back(run, r);
+            for (auto& w : workers) w.join();
+        }
+        for (auto& e : errors) {
+            if (e) std::rethrow_exception(e);
+        }
+        ViewResult total = n == 1 ? std::move(results[0]) : merge_results(results, view->res_y);
+        report(ctx, total, stats);
+    });
+}
+
+int c5_render_jvp_device(c5_ctx* ctx, const c5_view* view, const double* d_v_alpha, const double* d_v_q,
+                         double* d_tangent, double* d_out, void* stream, c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        check_jvp_args(view, d_v_alpha, d_v_q, d_tangent, "render_jvp_device");
+        if (d_v_alpha) check_device_array(d_v_alpha, "render_jvp_device: d_v_alpha");
+        if (d_v_q) check_device_array(d_v_q, "render_jvp_device: d_v_q");
+        if (reinterpret_cast<uintptr_t>(d_tangent) & 15u) fail(C5_E_INVALID, "render_jvp_device: d_tangent must be 16-byte aligned");
+        if (reinterpret_cast<uintptr_t>(d_out) & 15u) fail(C5_E_INVALID, "render_jvp_device: d_out must be 16-byte aligned");
+        if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_jvp_device: single-device contexts only");
+        jvp_band_device(ctx, view, d_v_alpha, d_v_q, d_tangent, d_out, stream, stats);
     });
 }
 

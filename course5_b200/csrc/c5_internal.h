@@ -90,6 +90,8 @@ struct DeviceState {
     DevBuf<double> row_flux;         // flux renders: [res_y][pairs] {sum tau, sum I} of the band's rows
     DevBuf<double> grad_alpha, grad_q; // c5_render_grad: [n_tets] Morton order, this device's band only
     DevBuf<double> grad_in;          // c5_render_grad: the band's {g_tau, g_I} per pixel
+    DevBuf<double> jvp_dir;          // c5_render_jvp: [n_tets][2] {v_alpha, v_q}, Morton order; made at this state's
+                                     // first call, dropped by c5_upload_mesh (a sibling's when it follows a new mesh)
     int sm_count = 0;
     cudaEvent_t ev_walk = nullptr;   // between the pixel kernel and the grazing-ray kernel (phase times)
     cudaEvent_t ev_done = nullptr;   // after the view's last copy: what c5_render_wait waits for
@@ -186,6 +188,9 @@ void upload_tperm(DeviceState& d);
 // The two ops below allocate nothing and launch one kernel on s.
 // fields[t].alpha = alpha[tperm[t]], q0[t] = q[tperm[t]]: file-order device fields into d's tets
 void gather_fields(DeviceState& d, const uint32_t* tperm, const double* alpha, const double* q, cudaStream_t s);
+// dir[t] = {v_alpha[tperm[t]], v_q[tperm[t]]}, a null direction read as 0: c5_render_jvp's tangent field
+void gather_direction(int64_t n_tets, const uint32_t* tperm, const double* v_alpha, const double* v_q, double* dir,
+                      cudaStream_t s);
 // out[tperm[t]] = in[t] for both gradients (a null output is skipped): Morton order back to file order
 void scatter_grads(int64_t n_tets, const uint32_t* tperm, const double* in_alpha, const double* in_q, double* out_alpha,
                    double* out_q, cudaStream_t s);
@@ -215,8 +220,11 @@ struct WalkLaunch {
     double* grad_q;
     unsigned long long* counters;
     unsigned long long* row_cost;
+    // c5_render_jvp (channels 0, precision 64): kJvpPass stores {tau, I, dtau, dI} per pixel into out, the
+    // tangent along dir ([n_tets][2] {v_alpha, v_q}, Morton order)
+    const double* dir;
 };
-enum WalkPass { kImagePass = 0, kDepthPass = 1, kGradPass = 2 };
+enum WalkPass { kImagePass = 0, kDepthPass = 1, kGradPass = 2, kJvpPass = 3 };
 void launch_walk(DeviceState& d, const WalkLaunch& w);
 // c5_flux.cu — row_flux[j] for the rows [row_begin,row_end) of d.out (pairs {tau, I} per pixel),
 // skipping pixels under d.mask when use_mask; the summation order is documented there.

@@ -376,6 +376,19 @@ struct FieldGatherOp {
     }
 };
 
+// c5_render_jvp: a file-order direction into the walk's interleaved Morton-order tangent field.
+struct DirectionGatherOp {
+    const uint32_t* tperm; // new -> old tet
+    const double* v_alpha; // either may be null: 0
+    const double* v_q;
+    double* dir;           // [n_tets][2]
+    C5_HD void operator()(int64_t t) const {
+        const uint32_t old = tperm[t];
+        dir[2 * t] = v_alpha ? v_alpha[old] : 0.0;
+        dir[2 * t + 1] = v_q ? v_q[old] : 0.0;
+    }
+};
+
 // c5_render_grad_device: the gradient pass's Morton-order sums into the caller's file-order arrays.
 struct GradScatterOp {
     const uint32_t* tperm; // new -> old tet
@@ -619,6 +632,11 @@ void upload_tperm(DeviceState& d) {
 void gather_fields(DeviceState& d, const uint32_t* tperm, const double* alpha, const double* q, cudaStream_t s) {
     for_each(s, d.n_tets, FieldGatherOp{alpha, q, tperm, d.fields.p, d.q0.p});
     d.cells_limit_valid = false; // fields[].s is derived again from the new q0 at the next render
+}
+
+void gather_direction(int64_t n_tets, const uint32_t* tperm, const double* v_alpha, const double* v_q, double* dir,
+                      cudaStream_t s) {
+    for_each(s, n_tets, DirectionGatherOp{tperm, v_alpha, v_q, dir});
 }
 
 void scatter_grads(int64_t n_tets, const uint32_t* tperm, const double* in_alpha, const double* in_q, double* out_alpha,

@@ -86,6 +86,11 @@ struct GradParams : WalkParams {
     double* grad_q;
 };
 
+// The forward-mode kernels (c5_render_jvp) take these, for the same reason.
+struct JvpParams : WalkParams {
+    const double* dir;     // [n_tets][2] Morton order: the direction {v_alpha, v_q} of each tet
+};
+
 // ---- loads through the read-only path ----------------------------------------------------------
 struct ConnData {
     int4 nbr;
@@ -805,6 +810,90 @@ struct CellsGradT {
 using CellsGrad = CellsGradT<false>;
 using CellsGradView = CellsGradT<true>;
 
+// ---- forward mode (c5_render_jvp) ------------------------------------------------------------------------
+// The Jacobian-vector product of the pre-cast image along a field direction (v_alpha, v_Q), carried forward
+// along the ray beside {tau, I}, in the walk's +z order (DESIGN.md §5c, "Forward mode"). With the partials of
+// the gradient pass above, a segment does
+//   dtau  += v_alpha dz                                                   (every segment)
+//   dI_out = e dI_in + (-m / a^) v_Q + (s x dz f(x) - I_in dz e) v_a^       (a^ >= DBL_EPSILON; else unchanged)
+// with v_a^ = v_alpha where alpha <= limit, else 0: the coefficients grad_segment multiplies by g_I T (except that
+// e = exp(-x) past x = 1/2, where 1 + m loses digits), so <g, J v> and <J^T g, v> agree to rounding. A crossing
+// walked affinely (I_out = A + B I_in) also carries the tangent of B, held in gain[1]:
+// dI_out = dA + dB I_in + B dI_in, and per segment dB_out = e dB_in - B_in dz e v_a^.
+// Pair 0 goes through the operations of segment(), so it is c5_render_raw's {tau, I} bit for bit; dtau is
+// added like tau, so v_alpha = alpha gives dtau == tau bit for bit.
+template <bool kAffine>
+C5_HD void jvp_segment(double alpha, double s, double va, double vq, double limit, double dzv, Pairs<2>& v) {
+    v.tau[0] += dzv * alpha;
+    v.tau[1] += dzv * va;
+    double a_c = alpha;
+    if (a_c > limit) a_c = limit;
+    if (!(a_c < DBL_EPSILON)) {
+        const double m = expm1(-a_c * dzv);
+        const double x = mul_rn(a_c, dzv);
+        // 1 + m has an absolute error of an ulp of 1: past x = 1/2 it would cost the tangent digits in
+        // proportion to 1 / e (at x = 16, e ~ 1e-7: seven), so e is taken from exp there
+        const double e = x < 0.5 ? 1.0 + m : exp(-x);
+        const double i_in = v.inten[0];
+        double di = v.inten[1] * e + (-m / a_c) * vq;
+        if (alpha <= limit) {
+            di += (s * x * dzv * grad_f(x, m) - i_in * dzv * e) * va;
+            if (kAffine) v.gain[1] = v.gain[1] * e - (v.gain[0] * dzv * e) * va;
+        } else if (kAffine) {
+            v.gain[1] = v.gain[1] * e;
+        }
+        v.inten[1] = di;
+        v.inten[0] = i_in - (s - i_in) * m;
+        if (kAffine) v.gain[0] *= 1.0 + m;
+    }
+}
+
+template <bool kAffine>
+struct JvpFields {
+    const double* dir;
+    Pairs<2>& v;
+    TetFields c;
+    double va, vq;
+    C5_HD void fetch(const WalkParams& P, int t) {
+        c.load(P.fields, t);
+#ifdef __CUDA_ARCH__
+        asm volatile("ld.global.nc.v2.f64 {%0,%1}, [%2];" : "=d"(va), "=d"(vq) : "l"(dir + 2 * static_cast<size_t>(t)));
+#else
+        va = dir[2 * static_cast<size_t>(t)];
+        vq = dir[2 * static_cast<size_t>(t) + 1];
+#endif
+    }
+    C5_HD void step(const WalkParams& P, double dzv) {
+        jvp_segment<kAffine>(c.alpha, c.s, va, vq, P.alpha_limit, dzv, v);
+    }
+};
+
+// {tau, I} of CellsF64 and {dtau, dI}; P is the WalkParams of a JvpParams. A deferred ray's two pairs wait in
+// ch_queue. kTangent: the grazing-ray fold composes pair 1 as the tangent of pair 0 (compose_crossing).
+struct CellsJvp {
+    static constexpr int K = 2;
+    static constexpr bool kChanQueue = true;
+    static constexpr bool kImage = true;
+    static constexpr bool kTangent = true;
+    template <bool kAffine>
+    static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<2>& v,
+                                 uint32_t& steps, uint32_t& error) {
+        if (kAffine) v.gain[1] = 0.0; // an affine crossing starts from reset pairs: B = 1, and dB = 0
+        JvpFields<kAffine> acc{static_cast<const JvpParams&>(P).dir, v};
+        return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
+    }
+};
+
+// Policies whose pair 1 is the tangent of pair 0 (only CellsJvp) say so; every other policy's pairs are independent.
+template <class F, class = void>
+struct TangentPairs {
+    static constexpr bool value = false;
+};
+template <class F>
+struct TangentPairs<F, std::void_t<decltype(F::kTangent)>> {
+    static constexpr bool value = F::kTangent;
+};
+
 C5_HD void store2(double* p, double a, double b) {
 #ifdef __CUDA_ARCH__
     *reinterpret_cast<double2*>(p) = make_double2(a, b);
@@ -933,15 +1022,24 @@ C5_HD RayAcc<F::K> load_deferred(const WalkParams& P, unsigned long long slot) {
     return a;
 }
 
-// Folds crossing (z_in -> z_out) into the ray unless the ray is already past its entry.
-template <int K>
+// Folds crossing (z_in -> z_out) into the ray unless the ray is already past its entry. kTangent (CellsJvp):
+// pair 1 is the tangent of pair 0 and its gain the tangent of pair 0's, so the fold is the 2 x 2 lower-triangular
+// map dI_out = dA + dB I_in + B dI_in beside I_out = A + B I_in.
+template <int K, bool kTangent = false>
 C5_HD void compose_crossing(RayAcc<K>& a, double z_in, double z_out, const Pairs<K>& k, uint32_t steps_k,
                             uint32_t error_k) {
     if (!(z_in > a.z_after)) return;
+    if constexpr (kTangent) {
+        a.v.tau[0] += k.tau[0];
+        a.v.tau[1] += k.tau[1];
+        a.v.inten[1] = k.inten[1] + k.gain[1] * a.v.inten[0] + k.gain[0] * a.v.inten[1];
+        a.v.inten[0] = k.inten[0] + k.gain[0] * a.v.inten[0];
+    } else {
 #pragma unroll
-    for (int c = 0; c < K; c++) {
-        a.v.tau[c] += k.tau[c];
-        a.v.inten[c] = k.inten[c] + k.gain[c] * a.v.inten[c];
+        for (int c = 0; c < K; c++) {
+            a.v.tau[c] += k.tau[c];
+            a.v.inten[c] = k.inten[c] + k.gain[c] * a.v.inten[c];
+        }
     }
     a.steps += steps_k;
     a.error |= error_k;
@@ -964,7 +1062,7 @@ C5_HD RayAcc<F::K> graze_ray_serial(const WalkParams& P, unsigned long long slot
             uint32_t steps_k = 0, error_k = 0;
             const double z_out = F::template crossing<true>(P, px, py, P.queue[slot].pixel, L.leaf[e], L.z[e], k, steps_k,
                                                             error_k);
-            compose_crossing(a, L.z[e], z_out, k, steps_k, error_k);
+            compose_crossing<F::K, TangentPairs<F>::value>(a, L.z[e], z_out, k, steps_k, error_k);
             if (++crossings > 65536) a.error = 1;
         }
         if (L.n < P.serial_cap) break;
@@ -1202,8 +1300,10 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
                         g.inten[c] = __shfl_sync(full, f.inten[c], l);
                         g.gain[c] = __shfl_sync(full, f.gain[c], l);
                     }
-                    compose_crossing(a, __shfl_sync(full, z_in, l), __shfl_sync(full, z_out, l), g,
-                                     __shfl_sync(full, steps_k, l), __shfl_sync(full, error_k, l));
+                    compose_crossing<F::K, TangentPairs<F>::value>(a, __shfl_sync(full, z_in, l),
+                                                                   __shfl_sync(full, z_out, l), g,
+                                                                   __shfl_sync(full, steps_k, l),
+                                                                   __shfl_sync(full, error_k, l));
                 }
             }
             crossings += n;
@@ -1421,6 +1521,9 @@ __global__ void __launch_bounds__(kBlock) tet_walk_grad_view(const GradParams P)
 __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad_view(const GradParams P) {
     graze_block_grad<CellsGradView>(P);
 }
+// Forward mode (c5_render_jvp): {tau, I, dtau, dI} per pixel. Registers in DESIGN.md §5c.
+__global__ void __launch_bounds__(kBlock) tet_walk_jvp(const JvpParams P) { walk_block<CellsJvp>(P); }
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_jvp(const JvpParams P) { graze_block<CellsJvp>(P); }
 
 namespace {
 
@@ -1456,6 +1559,11 @@ template <>
 struct Kernels<CellsGradView> {
     static constexpr void (*walk)(GradParams) = tet_walk_grad_view;
     static constexpr void (*graze)(GradParams) = grazing_rays_grad_view;
+};
+template <>
+struct Kernels<CellsJvp> {
+    static constexpr void (*walk)(JvpParams) = tet_walk_jvp;
+    static constexpr void (*graze)(JvpParams) = grazing_rays_jvp;
 };
 
 void background_on_host(const WalkParams& P, int n) {
@@ -1606,8 +1714,8 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
         P.ch_queue = d.ch_queue.p;
     }
     if (w.pass != kImagePass && (w.channels || f32)) fail(C5_E_INVALID, "render_grad: FP64 over the cells' own fields only");
-    if (w.pass == kDepthPass) P.ch_queue = d.ch_queue.p;
-    const int n_pairs = w.channels ? w.channels : w.pass == kDepthPass ? 2 : 1;
+    if (w.pass == kDepthPass || w.pass == kJvpPass) P.ch_queue = d.ch_queue.p;
+    const int n_pairs = w.channels ? w.channels : (w.pass == kDepthPass || w.pass == kJvpPass) ? 2 : 1;
     if (!whole_band && w.pass != kGradPass) { // the gradient pass stores no pixel
         count_launch();
         if (kHostSim) {
@@ -1623,6 +1731,13 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     const unsigned grid = static_cast<unsigned>(P.n_macro_x) * static_cast<unsigned>(n_macro_y) * 64u;
     if (w.pass == kDepthPass) {
         launch_rays<CellsDepth>(d, w, P, grid);
+        return;
+    }
+    if (w.pass == kJvpPass) {
+        JvpParams J{};
+        static_cast<WalkParams&>(J) = P;
+        J.dir = w.dir;
+        launch_rays<CellsJvp>(d, w, J, grid);
         return;
     }
     if (w.pass == kGradPass) {

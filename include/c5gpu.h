@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define C5_ABI_VERSION 7
+#define C5_ABI_VERSION 8
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
 #define C5_MAX_CHANNELS 8
@@ -306,6 +306,43 @@ int c5_render_grad_device(c5_ctx* ctx, const c5_view* view, const double* d_g, d
  * lanes. */
 int c5_render_flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_g,
                                double* d_grad_alpha, double* d_grad_q, void* stream, c5_stats* stats);
+
+/* ---- forward mode: the Jacobian-vector product of a view along a field direction ------------------------
+ * c5_render_jvp gives, for one view, the change of the pre-cast image (what c5_render_raw gives with
+ * round_through_float = 0) when the cells' alpha and Q move along the direction (v_alpha, v_q):
+ *   tangent[p] = {sum_t dtau_p/dalpha_t v_alpha[t],  sum_t dI_p/dalpha_t v_alpha[t] + dI_p/dQ_t v_q[t]}
+ * with the derivatives c5_render_grad uses (the clamp, the DBL_EPSILON skip and the walk's segment lengths
+ * alike), so <g, J v> equals <c5_render_grad(g), v> to rounding. v_alpha and v_q are host arrays of n_tets
+ * doubles, in the tet order given to c5_upload_mesh; either may be NULL (zero), not both. tangent receives
+ * res_y * res_x * 2 doubles {dtau, dI} per pixel, x fastest, in the layout of c5_render_raw's out (a row band
+ * writes only its rows); pixels under the solid mask get NaN in both, background pixels 0. out (optional, the
+ * same size) receives the {tau, I} image c5_render_raw gives for the view, bit for bit. Only the cells' own
+ * fields are differentiated; uploaded channels are not.
+ * The tangent is carried forward along each ray beside {tau, I}, in ONE walk: no depth pass and no atomics,
+ * since each ray owns its pixel. The result is bit-reproducible from run to run, for any row band, any
+ * number of devices and on siblings, and the device form gives the host form's bits. Launches: what
+ * c5_render_raw launches for the same view, plus one gather of the direction into the walk's tet order.
+ * That tangent field (16 bytes per tet) is made at a context's first call and reused; the context that owns
+ * the mesh counts it in c5_mesh_info.device_bytes from then on (a sibling holds its own, not counted), and
+ * c5_upload_mesh drops it. stats mean what they mean for c5_render_raw, except that ms_d2h is the copy of
+ * both pairs. C5_E_INVALID: NULL tangent, both directions NULL, precision 32, or round_through_float != 0.
+ * C5_E_STATE: no mesh, or a submitted view in flight on this context. Single-device, multi-device (each
+ * device renders its band of both images) and sibling contexts.
+ *
+ * c5_render_jvp_device is c5_render_jvp on device memory, enqueued on `stream`, with the ordering contract of
+ * c5_render_grad_device: d_v_alpha and d_v_q are n_tets doubles each on the context's device (file order, read
+ * by the gather; either may be NULL, not both, 8-byte aligned); d_tangent and the optional d_out hold the view's
+ * row band only, (row_end - row_begin) * res_x * 2 doubles, 16-byte aligned as for c5_render_device.
+ * stats == NULL: enqueue only. stats != NULL: `stream` is synchronised and stats are those of c5_render_jvp.
+ * The context's own later renders wait for the call. C5_E_INVALID: any cause c5_render_jvp has, a misaligned
+ * pointer, or a multi-device context. C5_E_STATE as for c5_render_jvp. Single-device contexts and siblings.
+ *
+ * A Gauss-Newton step needs J^T J v: c5_render_jvp_device along v, then c5_render_grad_device with the
+ * tangent as d_g (INTEGRATION.md, section E). */
+int c5_render_jvp(c5_ctx* ctx, const c5_view* view, const double* v_alpha, const double* v_q, double* tangent,
+                  double* out, c5_stats* stats);
+int c5_render_jvp_device(c5_ctx* ctx, const c5_view* view, const double* d_v_alpha, const double* d_v_q,
+                         double* d_tangent, double* d_out, void* stream, c5_stats* stats);
 
 /* Device-resident variant for callers that own device memory (e.g. a torch tensor that an NCCL
  * gather will read): d_out is a DEVICE pointer on the context's first device to
