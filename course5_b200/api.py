@@ -99,6 +99,10 @@ SYMBOLS = {
     "c5_render_jvp": (C.c_int, [C.c_void_p, C.POINTER(View), _dp, _dp, _dp, _dp, C.POINTER(Stats)]),
     "c5_render_jvp_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.POINTER(Stats)]),
+    "c5_render_flux_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                        C.POINTER(Stats)]),
+    "c5_render_flux_jvp_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_render_device": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "c5_last_row_cost": (C.c_int, [C.c_void_p, _u64p, C.c_int32]),
     "c5_kernel_launches": (C.c_uint64, [C.c_void_p]),
@@ -115,7 +119,7 @@ SYMBOLS = {
 }
 IPC_HANDLE_BYTES = 80
 MAX_IN_FLIGHT = 8
-ABI_VERSION = 8        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
+ABI_VERSION = 9        # C5_ABI_VERSION of include/c5gpu.h this binding was written against
 TIMELINE_PHASES = 6
 
 
@@ -217,7 +221,8 @@ class Context:
 
     @property
     def views_in_flight(self) -> int:
-        """The lanes of render_submit, render_flux_submit and render_flux_grad_device (set_views_in_flight)."""
+        """The lanes of render_submit, render_flux_submit and the light-curve device calls (render_flux_device,
+        render_flux_jvp_device, render_flux_grad_device; set_views_in_flight)."""
         return self._views_in_flight
 
     def _check(self, rc: int):
@@ -486,6 +491,40 @@ class Context:
         self._check(self.lib.c5_render_flux_grad_device(self._h, arr if views else None, len(views), C.c_void_p(g_ptr),
                                                         C.c_void_p(grad_alpha_ptr or None), C.c_void_p(grad_q_ptr or None),
                                                         C.c_void_p(stream), C.byref(st) if stats else None))
+        self.last_stats = st.as_dict() if stats else {}
+        return self.last_stats
+
+    def render_flux_device(self, views, total_ptr: int, stream: int = 0, *, channels: bool = False,
+                           stats: bool = True) -> dict:
+        """The totals of render_flux for every view, on DEVICE memory (c5_render_flux_device), enqueued on `stream`:
+        total_ptr receives len(views) * n * 2 doubles, view k's (n, 2) total at k * n * 2, bit for bit render_flux's;
+        n = 1, or n_channels with channels=True. The views run on the context's views_in_flight lanes.
+        stats=False: enqueue only; returns {}. With stats, the counts are summed over the views and ms_total is
+        the call's span on `stream`."""
+        views = list(views)
+        arr = (View * max(len(views), 1))(*views)
+        st = Stats() if stats else None
+        self._check(self.lib.c5_render_flux_device(self._h, arr if views else None, len(views), 1 if channels else 0,
+                                                   C.c_void_p(total_ptr or None), C.c_void_p(stream),
+                                                   C.byref(st) if stats else None))
+        self.last_stats = st.as_dict() if stats else {}
+        return self.last_stats
+
+    def render_flux_jvp_device(self, views, v_alpha_ptr: int, v_q_ptr: int, tangent_ptr: int, total_ptr: int = 0,
+                               stream: int = 0, *, stats: bool = True) -> dict:
+        """The J v of a light curve on DEVICE memory (c5_render_flux_jvp_device), enqueued on `stream`: tangent_ptr
+        receives len(views) * 2 doubles, {sum dtau, sum dI} of each view's render_jvp tangent over the pixels
+        outside its solid mask, in render_flux's summation order; total_ptr (0 = none) the same size, the views'
+        render_flux totals bit for bit. v_alpha_ptr / v_q_ptr as for render_jvp_device (0 = zero, not both). The
+        views (FP64, round_through_float = 0) run on the context's views_in_flight lanes. The tangent is laid out
+        as render_flux_grad_device's g. stats as for render_flux_device."""
+        views = list(views)
+        arr = (View * max(len(views), 1))(*views)
+        st = Stats() if stats else None
+        self._check(self.lib.c5_render_flux_jvp_device(self._h, arr if views else None, len(views),
+                                                       C.c_void_p(v_alpha_ptr or None), C.c_void_p(v_q_ptr or None),
+                                                       C.c_void_p(tangent_ptr or None), C.c_void_p(total_ptr or None),
+                                                       C.c_void_p(stream), C.byref(st) if stats else None))
         self.last_stats = st.as_dict() if stats else {}
         return self.last_stats
 

@@ -23,26 +23,30 @@ synchronisation, so a whole fit step (forward, loss, backward, optimiser) runs o
 a ray stopped by the step cap (C5_E_WALK, impossible on a valid mesh) is not reported.
 
 light_curve(ctx, views, alpha, q) is the differentiable {sum tau, sum I} of each view (c5_render_flux
-totals). On CUDA tensors its forward is the pipelined c5_render_flux_submit loop over the context's
-views_in_flight lanes (one host wait per curve), and its backward is one c5_render_flux_grad_device call
-over all views, on the same lanes, with grad_output read in place and no host synchronisation. On CPU
-tensors it renders the views one by one and its backward is one c5_render_grad per view against g filled
-with that view's upstream gradient.
+totals). On CUDA tensors its forward is one c5_render_flux_device call over the context's views_in_flight
+lanes, into a CUDA tensor, and its backward is one c5_render_flux_grad_device call over all views, on the
+same lanes, with grad_output read in place; both are enqueued on torch.cuda.current_stream() with no host
+synchronisation. On CPU tensors it renders the views one by one and its backward is one c5_render_grad per
+view against g filled with that view's upstream gradient.
 
 Forward mode: both Functions have a jvp, so torch.autograd.forward_ad dual tensors (and gradcheck with
 check_forward_ad=True) go through render and light_curve. The tangent of render is one c5_render_jvp: a
 single walk that carries {dtau, dI} beside {tau, I}, bit-reproducible from run to run; on CUDA tensors it is
 c5_render_jvp_device on torch.cuda.current_stream() with no host synchronisation. The tangent of light_curve
-sums each view's tangent image over the pixels outside the solid mask (its non-NaN pixels); that sum need
-not be bit-identical to the summation order of c5_render_flux. torch.func.jvp needs the Functions written
-with a separate setup_context, which they are not.
+is each view's tangent summed over the pixels outside the solid mask. On CUDA tensors that is one
+c5_render_flux_jvp_device call over the lanes, on the current stream with no host synchronisation, summed
+in c5_render_flux's documented order and bit-reproducible; its (n_views, 2) result is laid out as the
+upstream gradient of c5_render_flux_grad_device, so a curve's J^T J v is two device calls. On CPU tensors it
+is each view's c5_render_jvp tangent image summed with torch over its non-NaN pixels, an order that need not
+match c5_render_flux's bit for bit. torch.func.jvp needs the Functions written with a separate
+setup_context, which they are not.
 """
 from __future__ import annotations
 
 import numpy as np
 import torch
 
-from . import api, sweep
+from . import api
 
 
 def _raw_view(view: api.View) -> api.View:
@@ -174,14 +178,17 @@ class _LightCurve(torch.autograd.Function):
         vs = [_raw_view(v) for v in views]
         fn_ctx.version = _fields(ctx, alpha, q)
         if alpha.device.type == "cuda":
-            totals = sweep.render_light_curve(ctx, vs, in_flight=ctx.views_in_flight)[0][:, 0]
+            # one call over the lanes, into the CUDA tensor: no host wait
+            totals = torch.empty((len(vs), 2), dtype=torch.float64, device=alpha.device)
+            ctx.render_flux_device(vs, totals.data_ptr(), _stream(alpha.device), stats=False)
         else:
-            totals = np.stack([ctx.render_flux(v)[1][0] for v in vs])  # (n_views, 2): {sum tau, sum I}
+            # (n_views, 2): {sum tau, sum I}
+            totals = torch.from_numpy(np.stack([ctx.render_flux(v)[1][0] for v in vs]))
         fn_ctx.save_for_backward(alpha, q)
         fn_ctx.save_for_forward(alpha, q)
         fn_ctx.c5 = ctx
         fn_ctx.views = vs
-        return torch.from_numpy(totals).to(alpha.device)
+        return totals
 
     @staticmethod
     def backward(fn_ctx, grad_output: torch.Tensor):
@@ -217,8 +224,23 @@ class _LightCurve(torch.autograd.Function):
 
     @staticmethod
     def jvp(fn_ctx, _ctx_t, _views_t, alpha_t, q_t):
-        # the flux sums the pixels outside the solid mask, where the tangent image is not NaN
-        return torch.stack([_tangent_image(fn_ctx, v, alpha_t, q_t).nansum(dim=(0, 1)) for v in fn_ctx.views])
+        alpha, q = fn_ctx.saved_tensors
+        if alpha.device.type == "cpu":
+            # the flux sums the pixels outside the solid mask, where the tangent image is not NaN
+            return torch.stack([_tangent_image(fn_ctx, v, alpha_t, q_t).nansum(dim=(0, 1)) for v in fn_ctx.views])
+        ctx: api.Context = fn_ctx.c5
+        if ctx.fields_version != fn_ctx.version:
+            fn_ctx.version = _fields(ctx, alpha, q)
+        if alpha_t is None and q_t is None:
+            return torch.zeros((len(fn_ctx.views), 2), dtype=torch.float64, device=alpha.device)
+        dirs = [None if t is None else t.detach().to(dtype=torch.float64, device=alpha.device).contiguous()
+                for t in (alpha_t, q_t)]
+        tangent = torch.empty((len(fn_ctx.views), 2), dtype=torch.float64, device=alpha.device)
+        # stream-ordered, like _fields: the direction copies return to torch's cache only for later work on this stream
+        ctx.render_flux_jvp_device(fn_ctx.views, 0 if dirs[0] is None else dirs[0].data_ptr(),
+                                   0 if dirs[1] is None else dirs[1].data_ptr(), tangent.data_ptr(),
+                                   stream=_stream(alpha.device), stats=False)
+        return tangent
 
 
 def light_curve(ctx: api.Context, views, alpha: torch.Tensor, q: torch.Tensor) -> torch.Tensor:

@@ -762,6 +762,40 @@ struct SpanEvents {
     }
 };
 
+// Page-locked room for the counters of n_views views, copied there one view at a time by the calls over the lanes.
+void ensure_view_counters(DeviceState& o, int32_t n_views) {
+    const size_t n = static_cast<size_t>(n_views) * kNumCounters;
+    if (n <= o.h_view_counters_n) return;
+    host_pinned_free(o.h_view_counters);
+    o.h_view_counters = nullptr;
+    o.h_view_counters_n = 0;
+    o.h_view_counters = static_cast<unsigned long long*>(host_pinned_alloc(n * sizeof(unsigned long long)));
+    o.h_view_counters_n = n;
+}
+
+// The stats of a call over the lanes, once `s` has waited for every lane: the views' counters summed (each view's
+// in o.h_view_counters), ms_total the call's span on s (span.e[0] recorded at its start), the other times 0.
+void report_views(DeviceState& o, const c5_view* views, const std::vector<ViewPlan>& plans, cudaStream_t s,
+                  const SpanEvents& span, c5_stats* stats) {
+    if (!kHostSim) C5_CUDA(cudaEventRecord(span.e[1], s));
+    stream_sync(s);
+    c5_stats st{};
+    for (size_t k = 0; k < plans.size(); k++) {
+        const unsigned long long* c = o.h_view_counters + k * kNumCounters;
+        const ViewPlan& p = plans[k];
+        st.pixels += static_cast<uint64_t>(p.row_end - p.row_begin) * static_cast<uint64_t>(views[k].res_x);
+        st.tet_steps += c[kSteps];
+        st.hit_pixels += c[kHitPixels];
+        st.solid_pixels += c[kSolidPixels];
+        st.walk_errors += c[kWalkErrors];
+        st.grazing_rays += static_cast<int32_t>(c[kDeferred]);
+    }
+    if (!kHostSim) C5_CUDA(cudaEventElapsedTime(&st.ms_total, span.e[0], span.e[1]));
+    st.n_devices = 1;
+    *stats = st;
+    if (st.walk_errors) fail(C5_E_WALK, "render: " + std::to_string(st.walk_errors) + " ray(s) exceeded the step cap");
+}
+
 // c5_render_flux_grad_device: view k goes to lane k % views_in_flight, where the depth and the gradient pass
 // run on the lane's own stream with the view's one upstream pair d_g[2k..2k+1], all adding into the owner's
 // Morton-order accumulators; one scatter into file order on the caller's stream at the end.
@@ -783,14 +817,7 @@ void flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const 
     const size_t n_t = static_cast<size_t>(o.n_tets);
     o.grad_alpha.ensure(n_t);
     o.grad_q.ensure(n_t);
-    if (stats && static_cast<size_t>(n_views) * kNumCounters > o.h_view_counters_n) {
-        host_pinned_free(o.h_view_counters);
-        o.h_view_counters = nullptr;
-        o.h_view_counters_n = 0;
-        const size_t n = static_cast<size_t>(n_views) * kNumCounters;
-        o.h_view_counters = static_cast<unsigned long long*>(host_pinned_alloc(n * sizeof(unsigned long long)));
-        o.h_view_counters_n = n;
-    }
+    if (stats) ensure_view_counters(o, n_views);
     cudaStream_t s = kHostSim ? o.stream : static_cast<cudaStream_t>(stream);
     SpanEvents span;
     if (stats && !kHostSim) {
@@ -831,24 +858,7 @@ void flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const 
         C5_CUDA(cudaEventRecord(o.ev_fields, s));
         C5_CUDA(cudaStreamWaitEvent(o.stream, o.ev_fields, 0));
     }
-    if (!stats) return;
-    if (!kHostSim) C5_CUDA(cudaEventRecord(span.e[1], s));
-    stream_sync(s);
-    c5_stats st{};
-    for (int32_t k = 0; k < n_views; k++) {
-        const unsigned long long* c = o.h_view_counters + static_cast<size_t>(k) * kNumCounters;
-        const ViewPlan& p = plans[static_cast<size_t>(k)];
-        st.pixels += static_cast<uint64_t>(p.row_end - p.row_begin) * static_cast<uint64_t>(views[k].res_x);
-        st.tet_steps += c[kSteps];
-        st.hit_pixels += c[kHitPixels];
-        st.solid_pixels += c[kSolidPixels];
-        st.walk_errors += c[kWalkErrors];
-        st.grazing_rays += static_cast<int32_t>(c[kDeferred]);
-    }
-    if (!kHostSim) C5_CUDA(cudaEventElapsedTime(&st.ms_total, span.e[0], span.e[1]));
-    st.n_devices = 1;
-    *stats = st;
-    if (st.walk_errors) fail(C5_E_WALK, "render: " + std::to_string(st.walk_errors) + " ray(s) exceeded the step cap");
+    if (stats) report_views(o, views, plans, s, span, stats);
 }
 
 // ---- forward mode (c5_render_jvp, c5_render_jvp_device) -------------------------------------------------
@@ -969,6 +979,112 @@ void check_jvp_args(const c5_view* view, const double* v_alpha, const double* v_
     if (view && view->round_through_float) {
         fail(C5_E_INVALID, std::string(who) + ": the float cast has no useful derivative; set round_through_float = 0");
     }
+}
+
+// ---- light curves on device memory (c5_render_flux_device, c5_render_flux_jvp_device) ---------------------
+
+// After a field update the first render derives fields[].s again (launch_prepare_cells), which on a mesh shared
+// with lanes is fenced by device-wide syncs: the host would wait for the caller's earlier work. Here the cells
+// (and channels) are prepared for alpha_limit on `s` instead, fenced by events: `s` waits for every stream the
+// library renders on, and they all wait for `s`. A view with another limit still takes the synced path.
+void prepare_fenced(c5_ctx* ctx, double alpha_limit, bool channels, cudaStream_t s) {
+    DeviceState& o = ctx->dev;
+    const bool cells = !(o.cells_limit_valid && o.cells_limit == alpha_limit);
+    const bool chans = channels && !(o.ch_limit_valid && o.ch_limit == alpha_limit);
+    if (!cells && !chans) return;
+    const std::vector<DeviceState*> internal = internal_streams(ctx);
+    if (!kHostSim) {
+        for (DeviceState* x : internal) {
+            C5_CUDA(cudaEventRecord(x->ev_fields, x->stream));
+            C5_CUDA(cudaStreamWaitEvent(s, x->ev_fields, 0));
+        }
+    }
+    cudaStream_t own = o.stream;
+    if (!kHostSim) o.stream = s;
+    try {
+        if (cells) launch_prepare_cells(o, alpha_limit, true);
+        if (chans) launch_prepare_channels(o, alpha_limit, true);
+    } catch (...) {
+        o.stream = own;
+        throw;
+    }
+    o.stream = own;
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(o.ev_fields, s));
+        for (DeviceState* x : internal) C5_CUDA(cudaStreamWaitEvent(x->stream, o.ev_fields, 0));
+    }
+}
+
+// View k goes to lane k % views_in_flight, where its walk, its row sums and its total run on the lane's own
+// stream, the total straight into the caller's array. jvp: the direction is gathered once, on `stream`, into the
+// owner's tangent field, which every lane's walk reads (lanes share the owner's tet order); the walk's
+// {tau, I, dtau, dI} per pixel is a two-pair band, so the row sums of a K = 2 channel image give the flux and the
+// tangent at once. Otherwise each view runs what c5_render_flux runs (n_ch pairs: 0 = the cells' own fields).
+void flux_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, int n_ch, bool jvp, const double* d_v_alpha,
+                 const double* d_v_q, double* d_tangent, double* d_total, void* stream, c5_stats* stats) {
+    const std::string who = jvp ? "render_flux_jvp_device" : "render_flux_device";
+    if (ctx->parent) fail(C5_E_STATE, who + ": a sibling context; call through its parent");
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
+        if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, who + ": a submitted view is in flight");
+    }
+    std::vector<ViewPlan> plans;
+    for (int32_t k = 0; k < n_views; k++) plans.push_back(plan_view(&views[k]));
+    ensure_lanes(ctx);
+    const unsigned n_lanes = static_cast<unsigned>(ctx->lanes.size()) + 1;
+    for (unsigned k = 0; k < n_lanes; k++) follow_parent(lane_of(ctx, k));
+    DeviceState& o = ctx->dev;
+    use_device(o);
+    const uint32_t* tperm = jvp ? resident_tperm(ctx) : nullptr;
+    double* dir = jvp ? resident_dir(ctx) : nullptr;
+    if (stats) ensure_view_counters(o, n_views);
+    cudaStream_t s = kHostSim ? o.stream : static_cast<cudaStream_t>(stream);
+    SpanEvents span;
+    if (stats && !kHostSim) {
+        for (cudaEvent_t& e : span.e) C5_CUDA(cudaEventCreate(&e));
+        C5_CUDA(cudaEventRecord(span.e[0], s));
+    }
+    // 1. `stream` waits for the context's own stream (an earlier call's lanes may still read the tangent field),
+    // 2. the gather, 3. every lane starts after that, and so after the caller's earlier work on `stream` (a
+    // c5_update_fields_device, whatever wrote the direction)
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(o.ev_fields, o.stream));
+        C5_CUDA(cudaStreamWaitEvent(s, o.ev_fields, 0));
+    }
+    g_launch_counter = &o.launches;
+    prepare_fenced(ctx, views[0].alpha_limit, n_ch > 0, s);
+    if (jvp) gather_direction(o.n_tets, tperm, d_v_alpha, d_v_q, dir, s);
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(o.ev_fields, s));
+        for (unsigned k = 0; k < n_lanes; k++) C5_CUDA(cudaStreamWaitEvent(lane_of(ctx, k)->dev.stream, o.ev_fields, 0));
+    }
+    const int pairs = jvp ? 2 : n_ch ? n_ch : 1;      // pairs per pixel of the walk's band
+    const int total_words = jvp ? 2 : 2 * pairs;      // d_total's doubles per view
+    for (int32_t k = 0; k < n_views; k++) {
+        DeviceState& d = lane_of(ctx, static_cast<unsigned>(k) % n_lanes)->dev;
+        const c5_view* v = &views[k];
+        const ViewPlan& p = plans[static_cast<size_t>(k)];
+        if (jvp) enqueue_view(d, v, p, false, nullptr, 0, kJvpPass, dir);
+        else enqueue_view(d, v, p, false, nullptr, n_ch);
+        const bool solids = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0;
+        launch_reduce_rows(d, v->res_x, v->res_y, p.row_begin, p.row_end, pairs, solids);
+        launch_total_rows(d, p.row_begin, p.row_end, 2 * pairs, total_words,
+                          d_total ? d_total + static_cast<size_t>(k) * total_words : nullptr,
+                          jvp ? d_tangent + 2 * static_cast<size_t>(k) : nullptr);
+        if (stats) d2h(o.h_view_counters + static_cast<size_t>(k) * kNumCounters, d.counters.p,
+                       kNumCounters * sizeof(unsigned long long), d.stream);
+    }
+    // 4. `stream` waits for every lane, and the context's own later renders (and the next call) wait for `stream`
+    if (!kHostSim) {
+        for (unsigned k = 0; k < n_lanes; k++) {
+            DeviceState& d = lane_of(ctx, k)->dev;
+            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
+            C5_CUDA(cudaStreamWaitEvent(s, d.ev_fields, 0));
+        }
+        C5_CUDA(cudaEventRecord(o.ev_fields, s));
+        C5_CUDA(cudaStreamWaitEvent(o.stream, o.ev_fields, 0));
+    }
+    if (stats) report_views(o, views, plans, s, span, stats);
 }
 
 void upload_solids(c5_ctx* ctx, const double* pts, int64_t n, int follows) {
@@ -1606,6 +1722,35 @@ int c5_render_jvp_device(c5_ctx* ctx, const c5_view* view, const double* d_v_alp
         if (reinterpret_cast<uintptr_t>(d_out) & 15u) fail(C5_E_INVALID, "render_jvp_device: d_out must be 16-byte aligned");
         if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_jvp_device: single-device contexts only");
         jvp_band_device(ctx, view, d_v_alpha, d_v_q, d_tangent, d_out, stream, stats);
+    });
+}
+
+int c5_render_flux_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, int32_t channels, double* d_total,
+                          void* stream, c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (n_views < 1 || !views) fail(C5_E_INVALID, "render_flux_device: need at least one view");
+        check_device_array(d_total, "render_flux_device: d_total");
+        for (int32_t k = 0; k < n_views; k++) check_flux_args(&views[k], channels, nullptr, d_total);
+        if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_flux_device: single-device contexts only");
+        if (channels) check_channels_ready(ctx);
+        flux_device(ctx, views, n_views, channels ? ctx->dev.n_channels : 0, false, nullptr, nullptr, nullptr, d_total,
+                    stream, stats);
+    });
+}
+
+int c5_render_flux_jvp_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_v_alpha,
+                              const double* d_v_q, double* d_tangent, double* d_total, void* stream, c5_stats* stats) {
+    if (!ctx) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        if (n_views < 1 || !views) fail(C5_E_INVALID, "render_flux_jvp_device: need at least one view");
+        check_device_array(d_tangent, "render_flux_jvp_device: d_tangent");
+        if (d_total) check_device_array(d_total, "render_flux_jvp_device: d_total");
+        if (d_v_alpha) check_device_array(d_v_alpha, "render_flux_jvp_device: d_v_alpha");
+        if (d_v_q) check_device_array(d_v_q, "render_flux_jvp_device: d_v_q");
+        for (int32_t k = 0; k < n_views; k++) check_jvp_args(&views[k], d_v_alpha, d_v_q, d_tangent, "render_flux_jvp_device");
+        if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_flux_jvp_device: single-device contexts only");
+        flux_device(ctx, views, n_views, 0, true, d_v_alpha, d_v_q, d_tangent, d_total, stream, stats);
     });
 }
 

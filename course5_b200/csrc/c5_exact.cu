@@ -914,13 +914,14 @@ DeviceState& mesh_owner(DeviceState& dd) {
 
 // Runs `prepare` on the context that owns the mesh unless its `limit` already holds alpha_limit.
 // What it writes belongs to that owner; its siblings read the same array, possibly on other streams
-// right now, so a change of --alpha_limit (rare) is fenced by device-wide syncs.
+// right now, so a change of --alpha_limit (rare) is fenced by device-wide syncs, unless the caller
+// has fenced every stream that reads the array with events (`fenced`).
 template <class Prepare>
 void prepare_for_limit(DeviceState& dd, double alpha_limit, double DeviceState::*limit, bool DeviceState::*valid,
-                       Prepare prepare) {
+                       bool fenced, Prepare prepare) {
     DeviceState& d = mesh_owner(dd);
     if (d.*valid && d.*limit == alpha_limit) return;
-    const bool shared = dd.origin != nullptr || d.mesh_shared;
+    const bool shared = !fenced && (dd.origin != nullptr || d.mesh_shared);
     if (shared && !kHostSim) C5_CUDA(cudaDeviceSynchronize());
     struct SyncAfter {
         bool on;
@@ -936,8 +937,8 @@ void prepare_for_limit(DeviceState& dd, double alpha_limit, double DeviceState::
 
 } // namespace
 
-void launch_prepare_cells(DeviceState& dd, double alpha_limit) {
-    prepare_for_limit(dd, alpha_limit, &DeviceState::cells_limit, &DeviceState::cells_limit_valid, [&](DeviceState& d) {
+void launch_prepare_cells(DeviceState& dd, double alpha_limit, bool fenced) {
+    prepare_for_limit(dd, alpha_limit, &DeviceState::cells_limit, &DeviceState::cells_limit_valid, fenced, [&](DeviceState& d) {
         if (kHostSim) {
             for (int64_t t = 0; t < d.n_tets; t++) prepare_cell_body(t, d.fields.p, d.q0.p, alpha_limit);
         } else {
@@ -947,9 +948,9 @@ void launch_prepare_cells(DeviceState& dd, double alpha_limit) {
     });
 }
 
-void launch_prepare_channels(DeviceState& dd, double alpha_limit) {
+void launch_prepare_channels(DeviceState& dd, double alpha_limit, bool fenced) {
     if (mesh_owner(dd).n_channels == 0) return;
-    prepare_for_limit(dd, alpha_limit, &DeviceState::ch_limit, &DeviceState::ch_limit_valid, [&](DeviceState& d) {
+    prepare_for_limit(dd, alpha_limit, &DeviceState::ch_limit, &DeviceState::ch_limit_valid, fenced, [&](DeviceState& d) {
         const int64_t n = d.n_tets * d.n_channels;
         if (kHostSim) {
             for (int64_t k = 0; k < n; k++) prepare_channel_body(k, d.ch_rec.p, d.ch_q0.p, d.n_tets, d.n_channels, alpha_limit);

@@ -1,6 +1,7 @@
 // c5_flux.cu — per-row sums of a rendered band (c5_render_flux, c5_render_flux_submit): the light
 // curve of a sweep needs 16 bytes per pair and VIEW, so the image stays on the device and only its
-// row sums are copied to the host.
+// row sums are copied to the host. The device forms (c5_render_flux_device, c5_render_flux_jvp_device)
+// also add the rows into the view's total on the device, in the host's order.
 //
 // Summation order (the contract of include/c5gpu.h, which makes the sums bit-identical for any band
 // cut, device count and number of views in flight): one block of 256 threads per row; thread t adds
@@ -59,6 +60,24 @@ __global__ void __launch_bounds__(kFluxThreads) reduce_rows(const double* out, c
     if (t < 2 * K) row_flux[static_cast<size_t>(j) * 2 * K + t] = p[t * kFluxThreads];
 }
 
+// The view's total on the device (c5_render_flux_device, c5_render_flux_jvp_device): thread c adds word c of the
+// band's rows of row_flux (`words` per row) in increasing j, starting from 0 — the host's order for the total,
+// where the rows outside the band are +0 and leave the sum's bits alone. Word c < split goes to lo[c], the others
+// to hi[c - split]; a null destination is skipped.
+C5_HD double band_total(const double* row_flux, int words, int row_begin, int row_end, int c) {
+    double s = 0.0;
+    for (int j = row_begin; j < row_end; j++) s += row_flux[static_cast<size_t>(j) * words + c];
+    return s;
+}
+
+__global__ void __launch_bounds__(32) total_rows(const double* row_flux, int words, int row_begin, int row_end, int split,
+                                                 double* lo, double* hi) {
+    const int c = static_cast<int>(threadIdx.x);
+    if (c >= words) return;
+    double* dst = c < split ? (lo ? lo + c : nullptr) : (hi ? hi + (c - split) : nullptr);
+    if (dst) *dst = band_total(row_flux, words, row_begin, row_end, c);
+}
+
 namespace {
 
 template <int K>
@@ -106,6 +125,19 @@ void launch_reduce_rows(DeviceState& d, int res_x, int res_y, int row_begin, int
     case 8: launch_k<8>(d, res_x, row_begin, row_end, mask); break;
     default: fail(C5_E_INVALID, "render_flux: 1 .. C5_MAX_CHANNELS pairs");
     }
+}
+
+void launch_total_rows(DeviceState& d, int row_begin, int row_end, int words, int split, double* lo, double* hi) {
+    count_launch();
+    if (kHostSim) {
+        for (int c = 0; c < words; c++) {
+            double* dst = c < split ? (lo ? lo + c : nullptr) : (hi ? hi + (c - split) : nullptr);
+            if (dst) *dst = band_total(d.row_flux.p, words, row_begin, row_end, c);
+        }
+        return;
+    }
+    total_rows<<<1, 32, 0, d.stream>>>(d.row_flux.p, words, row_begin, row_end, split, lo, hi);
+    C5_CUDA(cudaGetLastError());
 }
 
 } // namespace c5

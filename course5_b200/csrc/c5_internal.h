@@ -103,7 +103,7 @@ struct DeviceState {
     size_t h_row_cost_n = 0;
     double* h_row_flux = nullptr;               // [h_row_flux_n]: row_flux of a flux view
     size_t h_row_flux_n = 0;
-    unsigned long long* h_view_counters = nullptr; // c5_render_flux_grad_device with stats: [view][kNumCounters]
+    unsigned long long* h_view_counters = nullptr; // the light-curve device calls with stats: [view][kNumCounters]
     size_t h_view_counters_n = 0;
     // c5_debug_set (tests, diagnostics); 0 = default
     int opt_graze_list = 0, opt_query_budget = 0, opt_serial_list = 0, opt_mask_tile = 0;
@@ -175,8 +175,11 @@ void launch_solid_mask(DeviceState& d, int res_x, int res_y, double x_min, doubl
                        double step_y, int row_begin, int row_end);
 void launch_bvh_refit(DeviceState& d);
 void dedupe_solid_faces(DeviceState& d, SolidSet& ss); // fills ss.faces / ss.n_faces from ss.pts0
-void launch_prepare_cells(DeviceState& d, double alpha_limit); // fields[t].s = q0[t] / min(alpha, limit)
-void launch_prepare_channels(DeviceState& d, double alpha_limit); // the same for every channel of ch_rec
+// fields[t].s = q0[t] / min(alpha, limit), on d.stream, unless fields[] already hold that limit. A mesh shared with
+// siblings is fenced by device-wide syncs around the launch, unless `fenced`: the caller has ordered every stream
+// that reads the cells around d.stream with events.
+void launch_prepare_cells(DeviceState& d, double alpha_limit, bool fenced = false);
+void launch_prepare_channels(DeviceState& d, double alpha_limit, bool fenced = false); // the same for every channel of ch_rec
 
 // c5_topology.cu — places n channels of file-order fields (channel-major) in ch_rec / ch_q0.
 void upload_channels(DeviceState& d, const double* alpha, const double* q, int n);
@@ -229,6 +232,9 @@ void launch_walk(DeviceState& d, const WalkLaunch& w);
 // c5_flux.cu — row_flux[j] for the rows [row_begin,row_end) of d.out (pairs {tau, I} per pixel),
 // skipping pixels under d.mask when use_mask; the summation order is documented there.
 void launch_reduce_rows(DeviceState& d, int res_x, int res_y, int row_begin, int row_end, int pairs, bool use_mask);
+// c5_flux.cu — one launch: word c of the total of row_flux's rows [row_begin,row_end) (`words` doubles per row,
+// summed in increasing j from 0) into lo[c] for c < split, hi[c - split] otherwise; a null destination is skipped.
+void launch_total_rows(DeviceState& d, int row_begin, int row_end, int words, int split, double* lo, double* hi);
 // doubles per tet of ch_rec: n {alpha, s} pairs padded to 32 bytes (read with 256-bit loads)
 C5_HD constexpr int channel_stride(int n_channels) { return 4 * ((n_channels + 1) / 2); }
 

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define C5_ABI_VERSION 8
+#define C5_ABI_VERSION 9
 #define C5_MAX_IN_FLIGHT 8
 #define C5_MAX_ROT 8
 #define C5_MAX_CHANNELS 8
@@ -343,6 +343,40 @@ int c5_render_jvp(c5_ctx* ctx, const c5_view* view, const double* v_alpha, const
                   double* out, c5_stats* stats);
 int c5_render_jvp_device(c5_ctx* ctx, const c5_view* view, const double* d_v_alpha, const double* d_v_q,
                          double* d_tangent, double* d_out, void* stream, c5_stats* stats);
+
+/* ---- light curves on device memory: a curve and its J v in one call, the views on the lanes -------------
+ * c5_render_flux_device writes, for each view k in view order, the total c5_render_flux gives for it, bit for
+ * bit, to d_total: n_views * n * 2 doubles on the context's device, n = 1, or the number of uploaded channels
+ * with channels = 1. channels, precision and round_through_float mean what they mean for c5_render_flux.
+ *
+ * c5_render_flux_jvp_device writes d_tangent[k] = {sum_p dtau_p, sum_p dI_p} (n_views * 2 doubles): view k's
+ * c5_render_jvp tangent summed over the pixels outside its solid mask in the flux order above (each row in the
+ * order of its 256 threads and halving tree, then the rows in increasing j from 0). The optional d_total
+ * (n_views * 2 doubles) receives the views' c5_render_flux totals, bit for bit. d_v_alpha and d_v_q are as
+ * for c5_render_jvp_device (file order, either may be NULL, not both, 8-byte aligned). Views must be FP64 with
+ * round_through_float = 0; only the cells' own fields are differentiated. d_tangent has exactly the layout
+ * c5_render_flux_grad_device reads as d_g, so a light curve's J^T J v is two calls with nothing in between.
+ *
+ * Both calls deal the views as c5_render_flux_grad_device does: view k goes to lane k % views_in_flight and
+ * runs there, on the lane's stream, what c5_render_flux runs for it (the walk, then the row sums; the J v call
+ * walks with the tangent beside {tau, I}), then one small kernel that adds the view's rows into its slot of
+ * the output. The J v call gathers the direction once, on `stream`, into the context's tangent field (counted
+ * in c5_mesh_info.device_bytes as for c5_render_jvp), which every lane reads. Ordering, without synchronising
+ * the host: `stream` first waits for the context's own stream, every lane then waits for `stream`, so it sees
+ * the caller's earlier work there (a c5_update_fields_device, the writes of the direction), `stream` waits for
+ * every lane before the call returns, and the context's own stream waits for `stream`. No atomics: both
+ * results are bit-reproducible from run to run, for any number of lanes and any order of the views.
+ * Launches: the sum over the views of what c5_render_flux launches for each, plus n_views, plus one gather
+ * for the J v call. stats == NULL: enqueue only. stats != NULL: `stream` is synchronised; the counts are
+ * summed over the views, ms_total is the call's span on `stream` and the other ms_* fields are 0.
+ * C5_E_INVALID: n_views < 1, NULL views, a NULL or not 8-byte aligned output, any argument cause of
+ * c5_render_flux (c5_render_flux_device) or c5_render_jvp_device (c5_render_flux_jvp_device), or a multi-device
+ * context. C5_E_STATE: no mesh, a sibling context, a submitted view in flight on the context or one of its
+ * lanes, or channels = 1 with no channels uploaded. Single-device contexts that are not siblings. */
+int c5_render_flux_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, int32_t channels, double* d_total,
+                          void* stream, c5_stats* stats);
+int c5_render_flux_jvp_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_v_alpha,
+                              const double* d_v_q, double* d_tangent, double* d_total, void* stream, c5_stats* stats);
 
 /* Device-resident variant for callers that own device memory (e.g. a torch tensor that an NCCL
  * gather will read): d_out is a DEVICE pointer on the context's first device to
