@@ -3,6 +3,7 @@
 #include <cstring>
 #include <algorithm>
 #include <exception>
+#include <functional>
 #include <mutex>
 #include <thread>
 #include <utility>
@@ -41,6 +42,34 @@ int guarded(c5_ctx* ctx, Fn&& fn) {
 
 void use_device(const DeviceState& d) {
     if (!kHostSim) C5_CUDA(cudaSetDevice(d.device));
+}
+
+// d's enqueues go to a caller's stream while this lives (under hostsim they stay on d's own); d's own stream is put
+// back at the end of the scope, also when it is left by an exception. Ordering d's own stream after the borrowed
+// one is the caller's decision, not this guard's.
+struct BorrowStream {
+    DeviceState& d;
+    const cudaStream_t own;
+    BorrowStream(DeviceState& d, cudaStream_t s) : d(d), own(d.stream) {
+        if (!kHostSim) d.stream = s;
+    }
+    ~BorrowStream() { d.stream = own; }
+};
+
+// `waiter` waits for the work enqueued on `producer` so far, through `ev` (recorded on `producer`).
+void wait_for(cudaStream_t waiter, cudaStream_t producer, cudaEvent_t ev) {
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(ev, producer));
+        C5_CUDA(cudaStreamWaitEvent(waiter, ev, 0));
+    }
+}
+
+// Every stream in `waiters` waits for the work enqueued on `producer` so far, through one record of `ev`.
+void wait_for(const std::vector<DeviceState*>& waiters, cudaStream_t producer, cudaEvent_t ev) {
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(ev, producer));
+        for (DeviceState* w : waiters) C5_CUDA(cudaStreamWaitEvent(w->stream, ev, 0));
+    }
 }
 
 // The context and, for a multi-device context, its parts: one context per device.
@@ -439,6 +468,28 @@ void report(c5_ctx* owner, ViewResult& r, c5_stats* st) {
     }
 }
 
+// The start of a call that renders one view on ctx's own device state: the view's plan, once ctx has followed its
+// parent and has a mesh and no submitted view in flight (`busy` says so otherwise). stage: page-locked room for the
+// view's counters and row costs (finish_view).
+ViewPlan begin_view(c5_ctx* ctx, const c5_view* v, const char* busy, bool stage) {
+    follow_parent(ctx);
+    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
+    if (ctx->pending.active) fail(C5_E_STATE, busy);
+    const ViewPlan p = plan_view(v);
+    use_device(ctx->dev);
+    if (stage) ensure_host_staging(ctx->dev, static_cast<size_t>(v->res_y));
+    return p;
+}
+
+// The end of a call that rendered one view on d.stream: the counters and row costs are copied to the staging, the
+// stream is synchronised and the view is read (read_view).
+ViewResult finish_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool submitted) {
+    d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
+    d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
+    stream_sync(d.stream);
+    return read_view(d, *v, p, submitted);
+}
+
 // Waits for the view `lane` has in flight and reads it.
 ViewResult wait_view(c5_ctx* lane) {
     if (!lane->pending.active) fail(C5_E_STATE, "render_wait: no view in flight");
@@ -476,13 +527,14 @@ ViewResult merge_results(const std::vector<ViewResult>& results, int res_y) {
     return total;
 }
 
-// Multi-device contexts (c5_create with several devices): the context and each of its parts render
-// one cost-balanced row band, as c5_render does for a row band, straight into its final rows of the
-// caller's buffers. One host thread per device submits: a copy into pageable memory blocks the
-// submitting thread until its device is done, so one thread would render the bands one after another.
-// A flux render (flux != null) merges the parts' row sums and sums the total over all rows in order.
-void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, c5_stats* st,
-                         bool channels = false, const FluxOut* flux = nullptr) {
+// A view rendered as row bands by a context's devices (the context itself, then its parts): v's rows are cut into
+// one cost-balanced band per device, and part(r, device r's context, band r's view) runs on one host thread per
+// device (in turn under hostsim or with one device): a copy into pageable memory blocks the calling thread until
+// its device is done, so one thread would render the bands one after another. Returns the bands; errors[r] is
+// what part r threw.
+std::vector<std::pair<int, int>> over_bands(c5_ctx* ctx, const c5_view* v, std::vector<std::exception_ptr>& errors,
+                                            const std::function<void(size_t, c5_ctx*, const c5_view*)>& part) {
+    follow_parent(ctx);
     if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
     const ViewPlan p = plan_view(v);
     const std::vector<c5_ctx*> parts = with_parts(ctx);
@@ -490,24 +542,45 @@ void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* s
     if (static_cast<size_t>(p.row_end - p.row_begin) < n) fail(C5_E_INVALID, "render: fewer rows than devices");
     const auto bands = cut_bands(ctx, v, p, static_cast<int>(n));
     std::vector<c5_view> band_views(n, *v);
-    std::vector<std::exception_ptr> errors(n);
-    auto submit = [&](size_t r) {
+    errors.assign(n, nullptr);
+    auto run = [&](size_t r) {
         try {
             band_views[r].row_begin = bands[r].first;
             band_views[r].row_end = bands[r].second;
-            const FluxOut part_flux{}; // the merged sums are handed over below
-            submit_view(parts[r], &band_views[r], out, steps, solid_mask, 0, true, channels, flux ? &part_flux : nullptr);
+            part(r, parts[r], &band_views[r]);
         } catch (...) {
             errors[r] = std::current_exception();
         }
     };
-    if (kHostSim) {
-        for (size_t r = 0; r < n; r++) submit(r);
+    if (kHostSim || n == 1) {
+        for (size_t r = 0; r < n; r++) run(r);
     } else {
         std::vector<std::thread> workers;
-        for (size_t r = 0; r < n; r++) workers.emplace_back(submit, r);
+        for (size_t r = 0; r < n; r++) workers.emplace_back(run, r);
         for (auto& w : workers) w.join();
     }
+    return bands;
+}
+
+void rethrow_first(const std::vector<std::exception_ptr>& errors) {
+    for (const auto& e : errors) {
+        if (e) std::rethrow_exception(e);
+    }
+}
+
+// Multi-device contexts (c5_create with several devices): the context and each of its parts render
+// one cost-balanced row band, as c5_render does for a row band, straight into its final rows of the
+// caller's buffers. A flux render (flux != null) merges the parts' row sums and sums the total over all
+// rows in order.
+void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* steps, uint8_t* solid_mask, c5_stats* st,
+                         bool channels = false, const FluxOut* flux = nullptr) {
+    const std::vector<c5_ctx*> parts = with_parts(ctx);
+    const size_t n = parts.size();
+    std::vector<std::exception_ptr> errors;
+    const auto bands = over_bands(ctx, v, errors, [&](size_t, c5_ctx* part, const c5_view* band) {
+        const FluxOut part_flux{}; // the merged sums are handed over below
+        submit_view(part, band, out, steps, solid_mask, 0, true, channels, flux ? &part_flux : nullptr);
+    });
     // every band that was submitted is waited for, also when another failed: none may still be
     // writing into the caller's buffers once this returns
     std::vector<ViewResult> results(n);
@@ -519,9 +592,7 @@ void render_multi_device(c5_ctx* ctx, const c5_view* v, double* out, uint32_t* s
             if (!errors[r]) errors[r] = std::current_exception();
         }
     }
-    for (auto& e : errors) {
-        if (e) std::rethrow_exception(e);
-    }
+    rethrow_first(errors);
     ViewResult total = merge_results(results, v->res_y);
     if (flux) {
         const size_t words = results[0].flux.size() / static_cast<size_t>(v->res_y);
@@ -585,19 +656,22 @@ void enqueue_grad(DeviceState& d, const c5_view* v, const ViewPlan& p, const dou
     launch_walk(d, w);
 }
 
+// Pair `pair` (0 or 1) of every pixel of a {a, b, c, d}-per-pixel band, into the {x, y}-per-pixel image rows at `img`.
+void unpack_pair(const std::vector<double>& band, int pair, double* img) {
+    for (size_t k = 0; k < band.size() / 4; k++) {
+        img[2 * k] = band[4 * k + 2 * pair];
+        img[2 * k + 1] = band[4 * k + 2 * pair + 1];
+    }
+}
+
 // Band [row_begin,row_end) of v on ctx's device: enqueue_grad, then the copies. Blocks until the results
 // are on the host. Events: 0..5 as for enqueue_grad, 6 gradients on the host.
 GradResult grad_band(c5_ctx* ctx, const c5_view* v, const double* g, bool want_alpha, bool want_q, double* out) {
-    follow_parent(ctx);
-    if (ctx->pending.active) fail(C5_E_STATE, "render_grad: this context still has a view in flight (c5_render_wait it first)");
-    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    const ViewPlan p = plan_view(v);
+    const ViewPlan p = begin_view(ctx, v, "render_grad: this context still has a view in flight (c5_render_wait it first)", true);
     DeviceState& d = ctx->dev;
-    use_device(d);
     const size_t n_t = static_cast<size_t>(d.n_tets);
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
     const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
-    ensure_host_staging(d, static_cast<size_t>(v->res_y));
     enqueue_grad(d, v, p, g, nullptr);
     std::vector<double> morton[2];
     for (int k = 0; k < 2; k++) {
@@ -606,16 +680,11 @@ GradResult grad_band(c5_ctx* ctx, const c5_view* v, const double* g, bool want_a
         d2h(morton[k].data(), (k == 0 ? d.grad_alpha : d.grad_q).p, n_t * sizeof(double), d.stream);
     }
     record(d, 6);
-    d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
-    d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
     std::vector<double> band(out ? 4 * n_pix_band : 0); // the depth pass's {tau, I, lam, 0} per pixel
     if (out) d2h(band.data(), d.out.p, band.size() * sizeof(double), d.stream);
-    stream_sync(d.stream);
-    for (size_t k = 0; k < band.size() / 4; k++) { // its first pair is the image of c5_render_raw
-        out[2 * (band_off + k)] = band[4 * k];
-        out[2 * (band_off + k) + 1] = band[4 * k + 1];
-    }
     GradResult r;
+    r.view = finish_view(d, v, p, true);
+    if (out) unpack_pair(band, 0, out + 2 * band_off); // its first pair is the image of c5_render_raw
     const std::vector<uint32_t>& tperm = (d.origin ? *d.origin : d).tperm; // new -> old tet
     for (int k = 0; k < 2; k++) {
         if (morton[k].empty()) continue;
@@ -623,7 +692,6 @@ GradResult grad_band(c5_ctx* ctx, const c5_view* v, const double* g, bool want_a
         file.resize(n_t);
         for (size_t t = 0; t < n_t; t++) file[tperm[t]] = morton[k][t];
     }
-    r.view = read_view(d, *v, p, true);
     return r;
 }
 
@@ -639,6 +707,13 @@ void ensure_lanes(c5_ctx* ctx) {
         const int rc = c5_create_sibling(ctx, &lane);
         if (rc != C5_OK) fail(rc, "render_submit: cannot create a lane: " + ctx->err);
         ctx->lanes.push_back(lane);
+    }
+}
+
+// Fails with `text` while the context or one of its lanes has a submitted view in flight.
+void check_no_view_in_flight(c5_ctx* ctx, const std::string& text) {
+    for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
+        if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, text);
     }
 }
 
@@ -683,6 +758,14 @@ void check_flux_args(const c5_view* view, int32_t channels, const double* rows, 
     if (channels && view && view->precision == 32) fail(C5_E_INVALID, "render_flux: channels are FP64 only (precision 64)");
 }
 
+// A view the derivative calls can take (NULL is left to plan_view): FP64, and no float cast.
+void check_differentiable(const c5_view* view, const std::string& who) {
+    if (view && view->precision == 32) fail(C5_E_INVALID, who + ": FP64 only (precision 64)");
+    if (view && view->round_through_float) {
+        fail(C5_E_INVALID, who + ": the float cast has no useful derivative; set round_through_float = 0");
+    }
+}
+
 // ---- gradients on device memory (c5_update_fields_device, c5_render_grad_device) ------------------------
 
 void check_device_array(const void* p, const char* what) {
@@ -716,40 +799,24 @@ std::vector<DeviceState*> internal_streams(c5_ctx* ctx) {
 // d_g read in place, then the scatter into file order and the strided copy of the image.
 void grad_band_device(c5_ctx* ctx, const c5_view* v, const double* d_g, double* d_grad_alpha, double* d_grad_q,
                       double* d_out, void* stream, c5_stats* stats) {
-    follow_parent(ctx);
-    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    if (ctx->pending.active) fail(C5_E_STATE, "render_grad_device: this context has a submitted view in flight");
-    const ViewPlan p = plan_view(v);
+    const ViewPlan p = begin_view(ctx, v, "render_grad_device: this context has a submitted view in flight",
+                                stats != nullptr);
     DeviceState& d = ctx->dev;
-    use_device(d);
     const uint32_t* tperm = resident_tperm(ctx);
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
-    if (stats) ensure_host_staging(d, static_cast<size_t>(v->res_y));
     // run on the CALLER's stream, like c5_render_device: the scratch arrays are the context's own
-    cudaStream_t own = d.stream;
-    if (!kHostSim) d.stream = static_cast<cudaStream_t>(stream);
-    try {
-        enqueue_grad(d, v, p, nullptr, d_g);
-        scatter_grads(d.n_tets, tperm, d.grad_alpha.p, d.grad_q.p, d_grad_alpha, d_grad_q, d.stream);
-        // the depth pass left {tau, I, lam, 0} per pixel: its first pair is the image of c5_render_raw
-        if (d_out) d2d_2d(d_out, 2 * sizeof(double), d.out.p, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
-        record(d, 6);
-        if (!kHostSim && d.stream != own) { // the context's own later renders reuse these scratch arrays: they wait
-            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
-            C5_CUDA(cudaStreamWaitEvent(own, d.ev_fields, 0));
-        }
-        if (stats) {
-            d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
-            d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
-            stream_sync(d.stream);
-            ViewResult r = read_view(d, *v, p, true);
-            report(ctx, r, stats);
-        }
-    } catch (...) {
-        d.stream = own;
-        throw;
+    const BorrowStream on(d, static_cast<cudaStream_t>(stream));
+    enqueue_grad(d, v, p, nullptr, d_g);
+    scatter_grads(d.n_tets, tperm, d.grad_alpha.p, d.grad_q.p, d_grad_alpha, d_grad_q, d.stream);
+    // the depth pass left {tau, I, lam, 0} per pixel: its first pair is the image of c5_render_raw
+    if (d_out) d2d_2d(d_out, 2 * sizeof(double), d.out.p, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
+    record(d, 6);
+    // the context's own later renders reuse these scratch arrays: they wait
+    if (d.stream != on.own) wait_for(on.own, d.stream, d.ev_fields);
+    if (stats) {
+        ViewResult r = finish_view(d, v, p, true);
+        report(ctx, r, stats);
     }
-    d.stream = own;
 }
 
 // Two timing events for the span of a call on a caller's stream (created only when stats are asked for).
@@ -796,27 +863,32 @@ void report_views(DeviceState& o, const c5_view* views, const std::vector<ViewPl
     if (st.walk_errors) fail(C5_E_WALK, "render: " + std::to_string(st.walk_errors) + " ray(s) exceeded the step cap");
 }
 
-// c5_render_flux_grad_device: view k goes to lane k % views_in_flight, where the depth and the gradient pass
-// run on the lane's own stream with the view's one upstream pair d_g[2k..2k+1], all adding into the owner's
-// Morton-order accumulators; one scatter into file order on the caller's stream at the end.
-void flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_g, double* d_grad_alpha,
-                      double* d_grad_q, void* stream, c5_stats* stats) {
-    if (ctx->parent) fail(C5_E_STATE, "render_flux_grad_device: a sibling context; call through its parent");
+// A call over the lanes (c5_render_flux_grad_device, c5_render_flux_device, c5_render_flux_jvp_device): view k goes to
+// lane k % views_in_flight and enqueue(lane's state, k, view k's plan) runs it on the lane's own stream. Around the
+// views, prologue(stream) and epilogue(stream) run on the caller's stream, with launches counted on the owner:
+//  1. `stream` waits for the context's own stream (an earlier call's scatter or lanes, a host-form gradient),
+//     then runs the prologue,
+//  2. every lane starts after that, and so after the caller's earlier work on `stream` (a c5_update_fields_device,
+//     whatever wrote the call's inputs),
+//  3. `stream` waits for every lane, then runs the epilogue,
+//  4. the context's own later renders (and the next call) wait for `stream`.
+void over_lanes(c5_ctx* ctx, const std::string& who, const c5_view* views, int32_t n_views, void* stream,
+                c5_stats* stats, const std::function<void(cudaStream_t)>& prologue,
+                const std::function<void(DeviceState&, size_t, const ViewPlan&)>& enqueue,
+                const std::function<void(cudaStream_t)>& epilogue) {
+    if (ctx->parent) fail(C5_E_STATE, who + ": a sibling context; call through its parent");
     if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
-        if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "render_flux_grad_device: a submitted view is in flight");
-    }
+    check_no_view_in_flight(ctx, who + ": a submitted view is in flight");
     std::vector<ViewPlan> plans;
     for (int32_t k = 0; k < n_views; k++) plans.push_back(plan_view(&views[k]));
     ensure_lanes(ctx);
-    const unsigned n_lanes = static_cast<unsigned>(ctx->lanes.size()) + 1;
-    for (unsigned k = 0; k < n_lanes; k++) follow_parent(lane_of(ctx, k));
+    std::vector<DeviceState*> lanes;
+    for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
+        follow_parent(lane_of(ctx, k));
+        lanes.push_back(&lane_of(ctx, k)->dev);
+    }
     DeviceState& o = ctx->dev;
     use_device(o);
-    const uint32_t* tperm = resident_tperm(ctx);
-    const size_t n_t = static_cast<size_t>(o.n_tets);
-    o.grad_alpha.ensure(n_t);
-    o.grad_q.ensure(n_t);
     if (stats) ensure_view_counters(o, n_views);
     cudaStream_t s = kHostSim ? o.stream : static_cast<cudaStream_t>(stream);
     SpanEvents span;
@@ -824,41 +896,44 @@ void flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const 
         for (cudaEvent_t& e : span.e) C5_CUDA(cudaEventCreate(&e));
         C5_CUDA(cudaEventRecord(span.e[0], s));
     }
-    // 1. the accumulators are zeroed on `stream` once the context's own stream is done with them (an earlier
-    // call's scatter, a host-form gradient), 2. every lane starts after that (and so after the caller's
-    // earlier work on `stream`, such as a field update or whatever wrote d_g)
-    if (!kHostSim) {
-        C5_CUDA(cudaEventRecord(o.ev_fields, o.stream));
-        C5_CUDA(cudaStreamWaitEvent(s, o.ev_fields, 0));
-    }
-    dev_zero(o.grad_alpha.p, n_t * sizeof(double), s);
-    dev_zero(o.grad_q.p, n_t * sizeof(double), s);
-    if (!kHostSim) {
-        C5_CUDA(cudaEventRecord(o.ev_fields, s));
-        for (unsigned k = 0; k < n_lanes; k++) C5_CUDA(cudaStreamWaitEvent(lane_of(ctx, k)->dev.stream, o.ev_fields, 0));
-    }
-    for (int32_t k = 0; k < n_views; k++) {
-        DeviceState& d = lane_of(ctx, static_cast<unsigned>(k) % n_lanes)->dev;
-        enqueue_grad(d, &views[k], plans[static_cast<size_t>(k)], nullptr, d_g + 2 * static_cast<size_t>(k), &o, true);
-        if (stats) d2h(o.h_view_counters + static_cast<size_t>(k) * kNumCounters, d.counters.p,
-                       kNumCounters * sizeof(unsigned long long), d.stream);
-    }
-    // 3. `stream` waits for every lane, then scatters
-    if (!kHostSim) {
-        for (unsigned k = 0; k < n_lanes; k++) {
-            DeviceState& d = lane_of(ctx, k)->dev;
-            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
-            C5_CUDA(cudaStreamWaitEvent(s, d.ev_fields, 0));
-        }
-    }
+    wait_for(s, o.stream, o.ev_fields);
     g_launch_counter = &o.launches;
-    scatter_grads(o.n_tets, tperm, o.grad_alpha.p, o.grad_q.p, d_grad_alpha, d_grad_q, s);
-    // 4. the context's own later renders (and the next call's zeroing) wait for the scatter
-    if (!kHostSim) {
-        C5_CUDA(cudaEventRecord(o.ev_fields, s));
-        C5_CUDA(cudaStreamWaitEvent(o.stream, o.ev_fields, 0));
+    prologue(s);
+    wait_for(lanes, s, o.ev_fields);
+    for (size_t k = 0; k < plans.size(); k++) {
+        DeviceState& d = *lanes[k % lanes.size()];
+        enqueue(d, k, plans[k]);
+        if (stats) d2h(o.h_view_counters + k * kNumCounters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
     }
+    for (DeviceState* d : lanes) wait_for(s, d->stream, d->ev_fields);
+    g_launch_counter = &o.launches;
+    if (epilogue) epilogue(s);
+    wait_for(o.stream, s, o.ev_fields);
     if (stats) report_views(o, views, plans, s, span, stats);
+}
+
+// c5_render_flux_grad_device: on its lane, view k's depth and gradient pass take the view's one upstream pair
+// d_g[2k..2k+1] and add into the owner's Morton-order accumulators, zeroed first on the caller's stream; one scatter
+// into file order on the caller's stream at the end.
+void flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, const double* d_g, double* d_grad_alpha,
+                      double* d_grad_q, void* stream, c5_stats* stats) {
+    DeviceState& o = ctx->dev;
+    const uint32_t* tperm = nullptr;
+    auto zero = [&](cudaStream_t s) {
+        tperm = resident_tperm(ctx);
+        const size_t n_t = static_cast<size_t>(o.n_tets);
+        o.grad_alpha.ensure(n_t);
+        o.grad_q.ensure(n_t);
+        dev_zero(o.grad_alpha.p, n_t * sizeof(double), s);
+        dev_zero(o.grad_q.p, n_t * sizeof(double), s);
+    };
+    auto grad = [&](DeviceState& d, size_t k, const ViewPlan& p) {
+        enqueue_grad(d, &views[k], p, nullptr, d_g + 2 * k, &o, true);
+    };
+    auto scatter = [&](cudaStream_t s) {
+        scatter_grads(o.n_tets, tperm, o.grad_alpha.p, o.grad_q.p, d_grad_alpha, d_grad_q, s);
+    };
+    over_lanes(ctx, "render_flux_grad_device", views, n_views, stream, stats, zero, grad, scatter);
 }
 
 // ---- forward mode (c5_render_jvp, c5_render_jvp_device) -------------------------------------------------
@@ -891,18 +966,13 @@ void enqueue_jvp(DeviceState& d, const c5_view* v, const ViewPlan& p, const uint
 // results are on the host. Events: 0..4 as for enqueue_jvp, 5..6 around the copy.
 ViewResult jvp_band(c5_ctx* ctx, const c5_view* v, const double* v_alpha, const double* v_q, double* tangent,
                     double* out) {
-    follow_parent(ctx);
-    if (ctx->pending.active) fail(C5_E_STATE, "render_jvp: this context still has a view in flight (c5_render_wait it first)");
-    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    const ViewPlan p = plan_view(v);
+    const ViewPlan p = begin_view(ctx, v, "render_jvp: this context still has a view in flight (c5_render_wait it first)", true);
     DeviceState& d = ctx->dev;
-    use_device(d);
     const uint32_t* tperm = resident_tperm(ctx);
     double* dir = resident_dir(ctx);
     const size_t n_t = static_cast<size_t>(d.n_tets);
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
     const size_t band_off = static_cast<size_t>(p.row_begin) * v->res_x;
-    ensure_host_staging(d, static_cast<size_t>(v->res_y));
     if (v_alpha) {
         d.grad_alpha.ensure(n_t);
         h2d(d.grad_alpha.p, v_alpha, n_t * sizeof(double), d.stream);
@@ -916,69 +986,42 @@ ViewResult jvp_band(c5_ctx* ctx, const c5_view* v, const double* v_alpha, const 
     std::vector<double> band(4 * n_pix_band); // {tau, I, dtau, dI} per pixel
     d2h(band.data(), d.out.p, band.size() * sizeof(double), d.stream);
     record(d, 6);
-    d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
-    d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
-    stream_sync(d.stream);
-    for (size_t k = 0; k < n_pix_band; k++) {
-        tangent[2 * (band_off + k)] = band[4 * k + 2];
-        tangent[2 * (band_off + k) + 1] = band[4 * k + 3];
-        if (out) {
-            out[2 * (band_off + k)] = band[4 * k];
-            out[2 * (band_off + k) + 1] = band[4 * k + 1];
-        }
-    }
-    return read_view(d, *v, p, true);
+    ViewResult r = finish_view(d, v, p, true);
+    unpack_pair(band, 1, tangent + 2 * band_off);
+    if (out) unpack_pair(band, 0, out + 2 * band_off);
+    return r;
 }
 
 // c5_render_jvp_device on a single-device context or a sibling: enqueue_jvp on the caller's stream, then the
 // strided copies of the two pairs into the caller's band buffers.
 void jvp_band_device(c5_ctx* ctx, const c5_view* v, const double* d_v_alpha, const double* d_v_q, double* d_tangent,
                      double* d_out, void* stream, c5_stats* stats) {
-    follow_parent(ctx);
-    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    if (ctx->pending.active) fail(C5_E_STATE, "render_jvp_device: this context has a submitted view in flight");
-    const ViewPlan p = plan_view(v);
+    const ViewPlan p = begin_view(ctx, v, "render_jvp_device: this context has a submitted view in flight",
+                                  stats != nullptr);
     DeviceState& d = ctx->dev;
-    use_device(d);
     const uint32_t* tperm = resident_tperm(ctx);
     double* dir = resident_dir(ctx);
     const size_t n_pix_band = static_cast<size_t>(p.row_end - p.row_begin) * v->res_x;
-    if (stats) ensure_host_staging(d, static_cast<size_t>(v->res_y));
     // run on the CALLER's stream, like c5_render_device: the scratch arrays are the context's own
-    cudaStream_t own = d.stream;
-    if (!kHostSim) d.stream = static_cast<cudaStream_t>(stream);
-    try {
-        enqueue_jvp(d, v, p, tperm, dir, d_v_alpha, d_v_q);
-        record(d, 5);
-        d2d_2d(d_tangent, 2 * sizeof(double), d.out.p + 2, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
-        if (d_out) d2d_2d(d_out, 2 * sizeof(double), d.out.p, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
-        record(d, 6);
-        if (!kHostSim && d.stream != own) { // the context's own later renders reuse these scratch arrays: they wait
-            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
-            C5_CUDA(cudaStreamWaitEvent(own, d.ev_fields, 0));
-        }
-        if (stats) {
-            d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
-            d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(uint64_t), d.stream);
-            stream_sync(d.stream);
-            ViewResult r = read_view(d, *v, p, true);
-            report(ctx, r, stats);
-        }
-    } catch (...) {
-        d.stream = own;
-        throw;
+    const BorrowStream on(d, static_cast<cudaStream_t>(stream));
+    enqueue_jvp(d, v, p, tperm, dir, d_v_alpha, d_v_q);
+    record(d, 5);
+    d2d_2d(d_tangent, 2 * sizeof(double), d.out.p + 2, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
+    if (d_out) d2d_2d(d_out, 2 * sizeof(double), d.out.p, 4 * sizeof(double), 2 * sizeof(double), n_pix_band, d.stream);
+    record(d, 6);
+    // the context's own later renders reuse these scratch arrays: they wait
+    if (d.stream != on.own) wait_for(on.own, d.stream, d.ev_fields);
+    if (stats) {
+        ViewResult r = finish_view(d, v, p, true);
+        report(ctx, r, stats);
     }
-    d.stream = own;
 }
 
 // Arguments c5_render_jvp and c5_render_jvp_device share.
 void check_jvp_args(const c5_view* view, const double* v_alpha, const double* v_q, const double* tangent, const char* who) {
     if (!tangent) fail(C5_E_INVALID, std::string(who) + ": tangent is NULL");
     if (!v_alpha && !v_q) fail(C5_E_INVALID, std::string(who) + ": v_alpha and v_q are both NULL");
-    if (view && view->precision == 32) fail(C5_E_INVALID, std::string(who) + ": FP64 only (precision 64)");
-    if (view && view->round_through_float) {
-        fail(C5_E_INVALID, std::string(who) + ": the float cast has no useful derivative; set round_through_float = 0");
-    }
+    check_differentiable(view, who);
 }
 
 // ---- light curves on device memory (c5_render_flux_device, c5_render_flux_jvp_device) ---------------------
@@ -993,98 +1036,43 @@ void prepare_fenced(c5_ctx* ctx, double alpha_limit, bool channels, cudaStream_t
     const bool chans = channels && !(o.ch_limit_valid && o.ch_limit == alpha_limit);
     if (!cells && !chans) return;
     const std::vector<DeviceState*> internal = internal_streams(ctx);
-    if (!kHostSim) {
-        for (DeviceState* x : internal) {
-            C5_CUDA(cudaEventRecord(x->ev_fields, x->stream));
-            C5_CUDA(cudaStreamWaitEvent(s, x->ev_fields, 0));
-        }
-    }
-    cudaStream_t own = o.stream;
-    if (!kHostSim) o.stream = s;
-    try {
+    for (DeviceState* x : internal) wait_for(s, x->stream, x->ev_fields);
+    {
+        const BorrowStream on(o, s);
         if (cells) launch_prepare_cells(o, alpha_limit, true);
         if (chans) launch_prepare_channels(o, alpha_limit, true);
-    } catch (...) {
-        o.stream = own;
-        throw;
     }
-    o.stream = own;
-    if (!kHostSim) {
-        C5_CUDA(cudaEventRecord(o.ev_fields, s));
-        for (DeviceState* x : internal) C5_CUDA(cudaStreamWaitEvent(x->stream, o.ev_fields, 0));
-    }
+    wait_for(internal, s, o.ev_fields);
 }
 
-// View k goes to lane k % views_in_flight, where its walk, its row sums and its total run on the lane's own
-// stream, the total straight into the caller's array. jvp: the direction is gathered once, on `stream`, into the
-// owner's tangent field, which every lane's walk reads (lanes share the owner's tet order); the walk's
+// Each view's walk, its row sums and its total run on its lane, the total straight into the caller's array. jvp:
+// the direction is gathered once, on `stream`, into the owner's tangent field, which every lane's walk reads (lanes
+// share the owner's tet order; an earlier call's lanes may still read it, hence step 1 of over_lanes); the walk's
 // {tau, I, dtau, dI} per pixel is a two-pair band, so the row sums of a K = 2 channel image give the flux and the
 // tangent at once. Otherwise each view runs what c5_render_flux runs (n_ch pairs: 0 = the cells' own fields).
 void flux_device(c5_ctx* ctx, const c5_view* views, int32_t n_views, int n_ch, bool jvp, const double* d_v_alpha,
                  const double* d_v_q, double* d_tangent, double* d_total, void* stream, c5_stats* stats) {
-    const std::string who = jvp ? "render_flux_jvp_device" : "render_flux_device";
-    if (ctx->parent) fail(C5_E_STATE, who + ": a sibling context; call through its parent");
-    if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-    for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
-        if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, who + ": a submitted view is in flight");
-    }
-    std::vector<ViewPlan> plans;
-    for (int32_t k = 0; k < n_views; k++) plans.push_back(plan_view(&views[k]));
-    ensure_lanes(ctx);
-    const unsigned n_lanes = static_cast<unsigned>(ctx->lanes.size()) + 1;
-    for (unsigned k = 0; k < n_lanes; k++) follow_parent(lane_of(ctx, k));
     DeviceState& o = ctx->dev;
-    use_device(o);
-    const uint32_t* tperm = jvp ? resident_tperm(ctx) : nullptr;
-    double* dir = jvp ? resident_dir(ctx) : nullptr;
-    if (stats) ensure_view_counters(o, n_views);
-    cudaStream_t s = kHostSim ? o.stream : static_cast<cudaStream_t>(stream);
-    SpanEvents span;
-    if (stats && !kHostSim) {
-        for (cudaEvent_t& e : span.e) C5_CUDA(cudaEventCreate(&e));
-        C5_CUDA(cudaEventRecord(span.e[0], s));
-    }
-    // 1. `stream` waits for the context's own stream (an earlier call's lanes may still read the tangent field),
-    // 2. the gather, 3. every lane starts after that, and so after the caller's earlier work on `stream` (a
-    // c5_update_fields_device, whatever wrote the direction)
-    if (!kHostSim) {
-        C5_CUDA(cudaEventRecord(o.ev_fields, o.stream));
-        C5_CUDA(cudaStreamWaitEvent(s, o.ev_fields, 0));
-    }
-    g_launch_counter = &o.launches;
-    prepare_fenced(ctx, views[0].alpha_limit, n_ch > 0, s);
-    if (jvp) gather_direction(o.n_tets, tperm, d_v_alpha, d_v_q, dir, s);
-    if (!kHostSim) {
-        C5_CUDA(cudaEventRecord(o.ev_fields, s));
-        for (unsigned k = 0; k < n_lanes; k++) C5_CUDA(cudaStreamWaitEvent(lane_of(ctx, k)->dev.stream, o.ev_fields, 0));
-    }
+    double* dir = nullptr;
+    auto prepare = [&](cudaStream_t s) {
+        const uint32_t* tperm = jvp ? resident_tperm(ctx) : nullptr;
+        dir = jvp ? resident_dir(ctx) : nullptr;
+        prepare_fenced(ctx, views[0].alpha_limit, n_ch > 0, s);
+        if (jvp) gather_direction(o.n_tets, tperm, d_v_alpha, d_v_q, dir, s);
+    };
     const int pairs = jvp ? 2 : n_ch ? n_ch : 1;      // pairs per pixel of the walk's band
     const int total_words = jvp ? 2 : 2 * pairs;      // d_total's doubles per view
-    for (int32_t k = 0; k < n_views; k++) {
-        DeviceState& d = lane_of(ctx, static_cast<unsigned>(k) % n_lanes)->dev;
+    auto flux = [&](DeviceState& d, size_t k, const ViewPlan& p) {
         const c5_view* v = &views[k];
-        const ViewPlan& p = plans[static_cast<size_t>(k)];
         if (jvp) enqueue_view(d, v, p, false, nullptr, 0, kJvpPass, dir);
         else enqueue_view(d, v, p, false, nullptr, n_ch);
         const bool solids = v->use_solids && (d.solid_follow.n + d.solid_static.n) > 0;
         launch_reduce_rows(d, v->res_x, v->res_y, p.row_begin, p.row_end, pairs, solids);
-        launch_total_rows(d, p.row_begin, p.row_end, 2 * pairs, total_words,
-                          d_total ? d_total + static_cast<size_t>(k) * total_words : nullptr,
-                          jvp ? d_tangent + 2 * static_cast<size_t>(k) : nullptr);
-        if (stats) d2h(o.h_view_counters + static_cast<size_t>(k) * kNumCounters, d.counters.p,
-                       kNumCounters * sizeof(unsigned long long), d.stream);
-    }
-    // 4. `stream` waits for every lane, and the context's own later renders (and the next call) wait for `stream`
-    if (!kHostSim) {
-        for (unsigned k = 0; k < n_lanes; k++) {
-            DeviceState& d = lane_of(ctx, k)->dev;
-            C5_CUDA(cudaEventRecord(d.ev_fields, d.stream));
-            C5_CUDA(cudaStreamWaitEvent(s, d.ev_fields, 0));
-        }
-        C5_CUDA(cudaEventRecord(o.ev_fields, s));
-        C5_CUDA(cudaStreamWaitEvent(o.stream, o.ev_fields, 0));
-    }
-    if (stats) report_views(o, views, plans, s, span, stats);
+        launch_total_rows(d, p.row_begin, p.row_end, 2 * pairs, total_words, d_total ? d_total + k * total_words : nullptr,
+                          jvp ? d_tangent + 2 * k : nullptr);
+    };
+    over_lanes(ctx, jvp ? "render_flux_jvp_device" : "render_flux_device", views, n_views, stream, stats, prepare, flux,
+               nullptr);
 }
 
 void upload_solids(c5_ctx* ctx, const double* pts, int64_t n, int follows) {
@@ -1485,9 +1473,7 @@ int c5_upload_channels(c5_ctx* ctx, const double* alpha, const double* q, int32_
         if (!alpha || !q) fail(C5_E_INVALID, "upload_channels: NULL array");
         if (n_channels < 0 || n_channels > C5_MAX_CHANNELS) fail(C5_E_INVALID, "upload_channels: n_channels must be 0 .. C5_MAX_CHANNELS");
         if (!ctx->has_mesh) fail(C5_E_STATE, "upload_channels: no mesh uploaded");
-        for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
-            if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "upload_channels: a submitted view is in flight");
-        }
+        check_no_view_in_flight(ctx, "upload_channels: a submitted view is in flight");
         if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize()); // siblings may be rendering from them
         ctx->dev.mesh_version++; // siblings and lanes re-alias at their next render
         const std::vector<c5_ctx*> all = with_parts(ctx);
@@ -1534,9 +1520,7 @@ int c5_update_fields(c5_ctx* ctx, const double* alpha, const double* q) {
         if (ctx->parent) fail(C5_E_STATE, "update_fields: a sibling context shares its parent's fields; update through the parent");
         if (!alpha || !q) fail(C5_E_INVALID, "update_fields: NULL array");
         if (!ctx->has_mesh) fail(C5_E_STATE, "update_fields: no mesh uploaded");
-        for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
-            if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "update_fields: a submitted view is in flight");
-        }
+        check_no_view_in_flight(ctx, "update_fields: a submitted view is in flight");
         if (!ctx->siblings.empty() && !kHostSim) C5_CUDA(cudaDeviceSynchronize()); // siblings may be rendering from them
         ctx->dev.mesh_version++; // siblings and lanes re-alias at their next render
         for (c5_ctx* c : with_parts(ctx)) {
@@ -1553,39 +1537,14 @@ int c5_render_grad(c5_ctx* ctx, const c5_view* view, const double* g, double* gr
     return guarded(ctx, [&] {
         if (!g) fail(C5_E_INVALID, "render_grad: g is NULL");
         if (!grad_alpha && !grad_q) fail(C5_E_INVALID, "render_grad: grad_alpha and grad_q are both NULL");
-        if (view && view->precision == 32) fail(C5_E_INVALID, "render_grad: FP64 only (precision 64)");
-        if (view && view->round_through_float) {
-            fail(C5_E_INVALID, "render_grad: the float cast has no useful derivative; set round_through_float = 0");
-        }
-        follow_parent(ctx);
-        if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-        const ViewPlan p = plan_view(view);
-        const std::vector<c5_ctx*> parts = with_parts(ctx);
-        const size_t n = parts.size();
-        if (static_cast<size_t>(p.row_end - p.row_begin) < n) fail(C5_E_INVALID, "render: fewer rows than devices");
-        const auto bands = cut_bands(ctx, view, p, static_cast<int>(n));
-        std::vector<c5_view> band_views(n, *view);
+        check_differentiable(view, "render_grad");
+        const size_t n = ctx->parts.size() + 1;
         std::vector<GradResult> results(n);
-        std::vector<std::exception_ptr> errors(n);
-        auto run = [&](size_t r) {
-            try {
-                band_views[r].row_begin = bands[r].first;
-                band_views[r].row_end = bands[r].second;
-                results[r] = grad_band(parts[r], &band_views[r], g, grad_alpha != nullptr, grad_q != nullptr, out);
-            } catch (...) {
-                errors[r] = std::current_exception();
-            }
-        };
-        if (kHostSim || n == 1) {
-            for (size_t r = 0; r < n; r++) run(r);
-        } else {
-            std::vector<std::thread> workers;
-            for (size_t r = 0; r < n; r++) workers.emplace_back(run, r);
-            for (auto& w : workers) w.join();
-        }
-        for (auto& e : errors) {
-            if (e) std::rethrow_exception(e);
-        }
+        std::vector<std::exception_ptr> errors;
+        over_bands(ctx, view, errors, [&](size_t r, c5_ctx* part, const c5_view* band) {
+            results[r] = grad_band(part, band, g, grad_alpha != nullptr, grad_q != nullptr, out);
+        });
+        rethrow_first(errors);
         // each device summed its own band: add them in device order
         const size_t n_t = static_cast<size_t>(ctx->info.n_tets);
         for (int k = 0; k < 2; k++) {
@@ -1611,26 +1570,18 @@ int c5_update_fields_device(c5_ctx* ctx, const double* d_alpha, const double* d_
         check_device_array(d_alpha, "update_fields_device: d_alpha");
         check_device_array(d_q, "update_fields_device: d_q");
         if (!ctx->has_mesh) fail(C5_E_STATE, "update_fields_device: no mesh uploaded");
-        for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
-            if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "update_fields_device: a submitted view is in flight");
-        }
+        check_no_view_in_flight(ctx, "update_fields_device: a submitted view is in flight");
         DeviceState& d = ctx->dev;
         use_device(d);
         const uint32_t* tperm = resident_tperm(ctx);
         cudaStream_t s = kHostSim ? d.stream : static_cast<cudaStream_t>(stream);
         const std::vector<DeviceState*> internal = internal_streams(ctx);
-        if (!kHostSim) { // the gather waits for every render the library has enqueued on the old fields ...
-            for (DeviceState* x : internal) {
-                C5_CUDA(cudaEventRecord(x->ev_fields, x->stream));
-                C5_CUDA(cudaStreamWaitEvent(s, x->ev_fields, 0));
-            }
-        }
+        // the gather waits for every render the library has enqueued on the old fields ...
+        for (DeviceState* x : internal) wait_for(s, x->stream, x->ev_fields);
         ctx->dev.mesh_version++; // siblings and lanes re-alias at their next render
         gather_fields(d, tperm, d_alpha, d_q, s);
-        if (!kHostSim) { // ... and every later one waits for the gather, also those of lanes made later
-            C5_CUDA(cudaEventRecord(d.ev_gather, s));
-            for (DeviceState* x : internal) C5_CUDA(cudaStreamWaitEvent(x->stream, d.ev_gather, 0));
-        }
+        // ... and every later one waits for the gather, also those of lanes made later
+        wait_for(internal, s, d.ev_gather);
     });
 }
 
@@ -1643,10 +1594,7 @@ int c5_render_grad_device(c5_ctx* ctx, const c5_view* view, const double* d_g, d
         if (d_grad_alpha) check_device_array(d_grad_alpha, "render_grad_device: d_grad_alpha");
         if (d_grad_q) check_device_array(d_grad_q, "render_grad_device: d_grad_q");
         if (d_out) check_device_array(d_out, "render_grad_device: d_out");
-        if (view && view->precision == 32) fail(C5_E_INVALID, "render_grad_device: FP64 only (precision 64)");
-        if (view && view->round_through_float) {
-            fail(C5_E_INVALID, "render_grad_device: the float cast has no useful derivative; set round_through_float = 0");
-        }
+        check_differentiable(view, "render_grad_device");
         if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_grad_device: single-device contexts only");
         grad_band_device(ctx, view, d_g, d_grad_alpha, d_grad_q, d_out, stream, stats);
     });
@@ -1661,12 +1609,7 @@ int c5_render_flux_grad_device(c5_ctx* ctx, const c5_view* views, int32_t n_view
         if (!d_grad_alpha && !d_grad_q) fail(C5_E_INVALID, "render_flux_grad_device: d_grad_alpha and d_grad_q are both NULL");
         if (d_grad_alpha) check_device_array(d_grad_alpha, "render_flux_grad_device: d_grad_alpha");
         if (d_grad_q) check_device_array(d_grad_q, "render_flux_grad_device: d_grad_q");
-        for (int32_t k = 0; k < n_views; k++) {
-            if (views[k].precision == 32) fail(C5_E_INVALID, "render_flux_grad_device: FP64 only (precision 64)");
-            if (views[k].round_through_float) {
-                fail(C5_E_INVALID, "render_flux_grad_device: the float cast has no useful derivative; set round_through_float = 0");
-            }
-        }
+        for (int32_t k = 0; k < n_views; k++) check_differentiable(&views[k], "render_flux_grad_device");
         if (!ctx->parts.empty()) fail(C5_E_INVALID, "render_flux_grad_device: single-device contexts only");
         flux_grad_device(ctx, views, n_views, d_g, d_grad_alpha, d_grad_q, stream, stats);
     });
@@ -1677,35 +1620,13 @@ int c5_render_jvp(c5_ctx* ctx, const c5_view* view, const double* v_alpha, const
     if (!ctx) return C5_E_INVALID;
     return guarded(ctx, [&] {
         check_jvp_args(view, v_alpha, v_q, tangent, "render_jvp");
-        follow_parent(ctx);
-        if (!ctx->has_mesh) fail(C5_E_STATE, "render: no mesh uploaded");
-        const ViewPlan p = plan_view(view);
-        const std::vector<c5_ctx*> parts = with_parts(ctx);
-        const size_t n = parts.size();
-        if (static_cast<size_t>(p.row_end - p.row_begin) < n) fail(C5_E_INVALID, "render: fewer rows than devices");
-        const auto bands = cut_bands(ctx, view, p, static_cast<int>(n));
-        std::vector<c5_view> band_views(n, *view);
+        const size_t n = ctx->parts.size() + 1;
         std::vector<ViewResult> results(n);
-        std::vector<std::exception_ptr> errors(n);
-        auto run = [&](size_t r) {
-            try {
-                band_views[r].row_begin = bands[r].first;
-                band_views[r].row_end = bands[r].second;
-                results[r] = jvp_band(parts[r], &band_views[r], v_alpha, v_q, tangent, out);
-            } catch (...) {
-                errors[r] = std::current_exception();
-            }
-        };
-        if (kHostSim || n == 1) {
-            for (size_t r = 0; r < n; r++) run(r);
-        } else {
-            std::vector<std::thread> workers;
-            for (size_t r = 0; r < n; r++) workers.emplace_back(run, r);
-            for (auto& w : workers) w.join();
-        }
-        for (auto& e : errors) {
-            if (e) std::rethrow_exception(e);
-        }
+        std::vector<std::exception_ptr> errors;
+        over_bands(ctx, view, errors, [&](size_t r, c5_ctx* part, const c5_view* band) {
+            results[r] = jvp_band(part, band, v_alpha, v_q, tangent, out);
+        });
+        rethrow_first(errors);
         ViewResult total = n == 1 ? std::move(results[0]) : merge_results(results, view->res_y);
         report(ctx, total, stats);
     });
@@ -1759,9 +1680,7 @@ int c5_set_views_in_flight(c5_ctx* ctx, int32_t n) {
     return guarded(ctx, [&] {
         if (n < 1 || n > C5_MAX_IN_FLIGHT) fail(C5_E_INVALID, "set_views_in_flight: 1 .. C5_MAX_IN_FLIGHT");
         if (ctx->parent || !ctx->parts.empty()) fail(C5_E_INVALID, "set_views_in_flight: single-device contexts that are not siblings");
-        for (unsigned k = 0; k <= ctx->lanes.size(); k++) {
-            if (lane_of(ctx, k)->pending.active) fail(C5_E_STATE, "set_views_in_flight: views are in flight");
-        }
+        check_no_view_in_flight(ctx, "set_views_in_flight: views are in flight");
         while (static_cast<int>(ctx->lanes.size()) + 1 > n) { // lanes that are no longer wanted
             c5_destroy(ctx->lanes.back());
             ctx->lanes.pop_back();
@@ -1837,24 +1756,14 @@ int c5_render_device(c5_ctx* ctx, const c5_view* view, void* d_out, void* stream
         if (stats) ensure_host_staging(d, static_cast<size_t>(view->res_y));
         // run on the CALLER's stream (NULL = the legacy default stream, which is what torch's
         // default "current stream" is) so the result is ordered with the caller's later work
-        cudaStream_t own = d.stream;
-        if (!kHostSim) d.stream = static_cast<cudaStream_t>(stream);
-        try {
-            enqueue_view(d, view, p, false, static_cast<double*>(d_out)); // the walk stores into the caller's buffer
-            // stats == NULL: fire and forget — nothing is read back and the stream is not synchronised,
-            // so successive views (and the caller's gather) pipeline on the device
-            if (stats) {
-                d2h(d.h_counters, d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
-                d2h(d.h_row_cost, d.row_cost.p, static_cast<size_t>(view->res_y) * sizeof(uint64_t), d.stream);
-                stream_sync(d.stream);
-                ViewResult r = read_view(d, *view, p, false);
-                report(ctx, r, stats);
-            }
-        } catch (...) {
-            d.stream = own;
-            throw;
+        const BorrowStream on(d, static_cast<cudaStream_t>(stream));
+        enqueue_view(d, view, p, false, static_cast<double*>(d_out)); // the walk stores into the caller's buffer
+        // stats == NULL: fire and forget — nothing is read back and the stream is not synchronised,
+        // so successive views (and the caller's gather) pipeline on the device
+        if (stats) {
+            ViewResult r = finish_view(d, view, p, false);
+            report(ctx, r, stats);
         }
-        d.stream = own;
     });
 }
 
