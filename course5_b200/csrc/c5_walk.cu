@@ -19,7 +19,8 @@
 // FP32) -> field policies -> one ray, in warp-synchronised phases (trace_ray) -> grazing rays:
 // composition, serial form, warp-cooperative collection / sort / walk -> kernels (walk_block,
 // fill_background, graze_block) -> host loops -> launch_walk. Everything from trace_ray on is one
-// body over a field policy: FP64 cell fields, FP32 cell fields or K uploaded channels.
+// body over a field policy: FP64 cell fields, FP32 cell fields, K uploaded channels, or the depth,
+// gradient and tangent passes of the derivatives.
 //
 // Geometry of one step. All rays are parallel to z, so "which face does the ray leave through"
 // is a 2-D question about the projected tet. The entry face (a,b,c) is kept counter-clockwise in
@@ -607,12 +608,19 @@ C5_HD double crossing_f32(const WalkParams& P, double px, double py, int leaf, d
 //   F::crossing<kAffine>   the crossing that integrates them into a Pairs<K>;
 //   F::kChanQueue          a deferred ray's values wait in WalkParams::ch_queue and DeferredRay::tau/inten
 //                          stay 0; otherwise they wait in DeferredRay::tau/inten;
-//   F::kImage              the pixels are stored (false: the gradient pass, whose result is its atomics).
+//   F::kImage              the pixels are stored and a grazing ray's steps are counted (false: the gradient
+//                          pass, whose result is its atomics);
+//   F::kTangent            pair 1 is the tangent of pair 0, and a grazing ray's fold composes it as one
+//                          (compose_crossing);
+//   F::kRewalk             after a grazing ray's fold, each crossing the fold took is walked again with
+//                          crossing<false>, from the pairs it was entered with.
 // crossing() also gets the ray's pixel (j * res_x + i); only the gradient pass reads it.
 struct CellsF64 { // the cells' own fields
     static constexpr int K = 1;
     static constexpr bool kChanQueue = false;
     static constexpr bool kImage = true;
+    static constexpr bool kTangent = false;
+    static constexpr bool kRewalk = false;
     template <bool kAffine>
     static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<1>& v,
                                  uint32_t& steps, uint32_t& error) {
@@ -625,6 +633,8 @@ struct CellsF32 { // the cells' own fields, FP32 step geometry
     static constexpr int K = 1;
     static constexpr bool kChanQueue = false;
     static constexpr bool kImage = true;
+    static constexpr bool kTangent = false;
+    static constexpr bool kRewalk = false;
     template <bool kAffine>
     static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<1>& v,
                                  uint32_t& steps, uint32_t& error) {
@@ -639,6 +649,8 @@ struct Channels {
     static constexpr int K = N;
     static constexpr bool kChanQueue = true;
     static constexpr bool kImage = true;
+    static constexpr bool kTangent = false;
+    static constexpr bool kRewalk = false;
     template <bool kAffine>
     static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<K>& v,
                                  uint32_t& steps, uint32_t& error) {
@@ -774,6 +786,8 @@ struct CellsDepth { // {tau, I} of CellsF64 and {lam, 0}
     static constexpr int K = 2;
     static constexpr bool kChanQueue = true;
     static constexpr bool kImage = true;
+    static constexpr bool kTangent = false;
+    static constexpr bool kRewalk = false;
     template <bool kAffine>
     static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<2>& v,
                                  uint32_t& steps, uint32_t& error) {
@@ -783,28 +797,26 @@ struct CellsDepth { // {tau, I} of CellsF64 and {lam, 0}
 };
 
 // The gradient pass: nothing is stored but the atomics; P is the WalkParams of a GradParams. kViewG: one
-// upstream per view (grad_ray), the light-curve form.
+// upstream per view (grad_ray), the light-curve form. A grazing ray's crossing is walked affinely for its
+// lam and (A, B), and once the fold has given it the {lam, I} it is entered with, again with the gradient.
 template <bool kViewG>
 struct CellsGradT {
     static constexpr int K = 1;
     static constexpr bool kChanQueue = false;
     static constexpr bool kImage = false;
+    static constexpr bool kTangent = false;
+    static constexpr bool kRewalk = true;
     template <bool kAffine>
     static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t pixel, int leaf, double z_in,
                                  Pairs<1>& v, uint32_t& steps, uint32_t& error) {
-        static_assert(!kAffine, "grazing rays of the gradient pass walk through lam_crossing and grad_crossing");
-        return grad_crossing(P, px, py, pixel, leaf, z_in, v, steps, error);
-    }
-    static C5_HD double grad_crossing(const WalkParams& P, double px, double py, uint32_t pixel, int leaf, double z_in,
-                                      Pairs<1>& v, uint32_t& steps, uint32_t& error) {
-        const GradParams& G = static_cast<const GradParams&>(P);
-        GradFields acc{G, v, grad_ray<kViewG>(G, pixel), 0};
-        return crossing_walk<false>(P, px, py, leaf, z_in, acc, steps, error);
-    }
-    static C5_HD double lam_crossing(const WalkParams& P, double px, double py, int leaf, double z_in, Pairs<1>& v,
-                                     uint32_t& steps, uint32_t& error) {
-        LamFields acc{v};
-        return crossing_walk<true>(P, px, py, leaf, z_in, acc, steps, error);
+        if constexpr (kAffine) {
+            LamFields acc{v};
+            return crossing_walk<true>(P, px, py, leaf, z_in, acc, steps, error);
+        } else {
+            const GradParams& G = static_cast<const GradParams&>(P);
+            GradFields acc{G, v, grad_ray<kViewG>(G, pixel), 0};
+            return crossing_walk<false>(P, px, py, leaf, z_in, acc, steps, error);
+        }
     }
 };
 using CellsGrad = CellsGradT<false>;
@@ -869,12 +881,13 @@ struct JvpFields {
 };
 
 // {tau, I} of CellsF64 and {dtau, dI}; P is the WalkParams of a JvpParams. A deferred ray's two pairs wait in
-// ch_queue. kTangent: the grazing-ray fold composes pair 1 as the tangent of pair 0 (compose_crossing).
+// ch_queue.
 struct CellsJvp {
     static constexpr int K = 2;
     static constexpr bool kChanQueue = true;
     static constexpr bool kImage = true;
     static constexpr bool kTangent = true;
+    static constexpr bool kRewalk = false;
     template <bool kAffine>
     static C5_HD double crossing(const WalkParams& P, double px, double py, uint32_t, int leaf, double z_in, Pairs<2>& v,
                                  uint32_t& steps, uint32_t& error) {
@@ -882,16 +895,6 @@ struct CellsJvp {
         JvpFields<kAffine> acc{static_cast<const JvpParams&>(P).dir, v};
         return crossing_walk<kAffine>(P, px, py, leaf, z_in, acc, steps, error);
     }
-};
-
-// Policies whose pair 1 is the tangent of pair 0 (only CellsJvp) say so; every other policy's pairs are independent.
-template <class F, class = void>
-struct TangentPairs {
-    static constexpr bool value = false;
-};
-template <class F>
-struct TangentPairs<F, std::void_t<decltype(F::kTangent)>> {
-    static constexpr bool value = F::kTangent;
 };
 
 C5_HD void store2(double* p, double a, double b) {
@@ -1047,10 +1050,11 @@ C5_HD void compose_crossing(RayAcc<K>& a, double z_in, double z_out, const Pairs
 }
 
 // Serial form (one thread does everything): the host-loop build, and the reference the warp
-// version is tested against. Same crossing function, same composition.
+// version is tested against. Same crossing function, same composition, same re-walk.
 template <class F>
 C5_HD RayAcc<F::K> graze_ray_serial(const WalkParams& P, unsigned long long slot, double px, double py) {
     RayAcc<F::K> a = load_deferred<F>(P, slot);
+    const uint32_t pixel = P.queue[slot].pixel;
     EntryList<kSerialList> L;
     int crossings = 0;
     while (!a.error) {
@@ -1060,41 +1064,18 @@ C5_HD RayAcc<F::K> graze_ray_serial(const WalkParams& P, unsigned long long slot
             Pairs<F::K> k;
             k.reset();
             uint32_t steps_k = 0, error_k = 0;
-            const double z_out = F::template crossing<true>(P, px, py, P.queue[slot].pixel, L.leaf[e], L.z[e], k, steps_k,
-                                                            error_k);
-            compose_crossing<F::K, TangentPairs<F>::value>(a, L.z[e], z_out, k, steps_k, error_k);
+            const double z_out = F::template crossing<true>(P, px, py, pixel, L.leaf[e], L.z[e], k, steps_k, error_k);
+            if constexpr (F::kRewalk) {
+                Pairs<F::K> entered = a.v;
+                uint32_t steps_g = 0, error_g = 0;
+                F::template crossing<false>(P, px, py, pixel, L.leaf[e], L.z[e], entered, steps_g, error_g);
+            }
+            compose_crossing<F::K, F::kTangent>(a, L.z[e], z_out, k, steps_k, error_k);
             if (++crossings > 65536) a.error = 1;
         }
         if (L.n < P.serial_cap) break;
     }
     return a;
-}
-
-// The gradient pass's serial form: each crossing is walked affinely for its lam and (A, B), re-walked
-// with the gradient from the I and lam it is entered with, then composed — what the warp form does
-// for 32 crossings at a time.
-template <class F>
-C5_HD void graze_ray_serial_grad(const WalkParams& P, unsigned long long slot, double px, double py) {
-    RayAcc<1> a = load_deferred<F>(P, slot);
-    const uint32_t pixel = P.queue[slot].pixel;
-    EntryList<kSerialList> L;
-    int crossings = 0;
-    while (!a.error) {
-        if (!bvh_collect_entries(P, px, py, a.z_after, L, P.serial_cap, 0x7FFFFFFF)) a.error = 1;
-        for (int e = 0; e < L.n; e++) {
-            if (!(L.z[e] > a.z_after)) continue;
-            Pairs<1> k;
-            k.reset();
-            uint32_t steps_k = 0, error_k = 0;
-            const double z_out = F::lam_crossing(P, px, py, L.leaf[e], L.z[e], k, steps_k, error_k);
-            Pairs<1> v = a.v;
-            uint32_t steps_g = 0, error_g = 0;
-            F::grad_crossing(P, px, py, pixel, L.leaf[e], L.z[e], v, steps_g, error_g);
-            compose_crossing(a, L.z[e], z_out, k, steps_k, error_k);
-            if (++crossings > 65536) a.error = 1;
-        }
-        if (L.n < P.serial_cap) break;
-    }
 }
 
 C5_HD double __longlong_as_double_hd(long long bits) {
@@ -1292,6 +1273,8 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
                     z_out = F::template crossing<true>(P, px, py, q_pixel, S.leaf[k], z_in, f, steps_k, error_k);
                 }
                 const int cnt = n - base < 32 ? n - base : 32;
+                Pairs<F::K> entered = a.v; // kRewalk: the pairs this lane's crossing is entered with ...
+                bool taken = false;        // ... and whether the fold takes it
                 for (int l = 0; l < cnt; l++) {
                     Pairs<F::K> g;
 #pragma unroll
@@ -1300,89 +1283,38 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
                         g.inten[c] = __shfl_sync(full, f.inten[c], l);
                         g.gain[c] = __shfl_sync(full, f.gain[c], l);
                     }
-                    compose_crossing<F::K, TangentPairs<F>::value>(a, __shfl_sync(full, z_in, l),
-                                                                   __shfl_sync(full, z_out, l), g,
-                                                                   __shfl_sync(full, steps_k, l),
-                                                                   __shfl_sync(full, error_k, l));
-                }
-            }
-            crossings += n;
-            if (crossings > 65536) a.error = 1;
-            __syncwarp();
-        }
-        if (lane == 0) {
-            store_pixel(P, i, j, a.v.tau, a.v.inten, a.steps);
-            const unsigned long long more = a.steps - q_steps;
-            if (more) {
-                atomicAdd(&P.counters[kSteps], more);
-                atomicAdd(&P.row_cost[j], more);
-                if (q_steps == 0) atomicAdd(&P.counters[kHitPixels], 1ull); // deferred before its first step
-            }
-            if (a.error) atomicAdd(&P.counters[kWalkErrors], 1ull);
-        }
-    }
-}
-
-// The gradient pass's grazing rays. Per batch of 32 crossings: (1) every lane walks its crossing
-// affinely, keeping its lam; (2) the warp folds the batch in z order exactly as graze_block does, and each
-// lane notes the {lam, I} its crossing is entered with (and whether the fold takes it); (3) the lanes
-// whose crossing was taken walk it again with the gradient.
-template <class F>
-__device__ __forceinline__ void graze_block_grad(const WalkParams& P) {
-    __shared__ GrazeSmem smem[kGrazeWarps];
-    const unsigned full = 0xFFFFFFFFu;
-    const int lane = threadIdx.x & 31;
-    GrazeSmem& S = smem[threadIdx.x >> 5];
-    const unsigned long long n_rays = P.counters[kDeferred];
-    while (true) {
-        unsigned long long ticket = 0;
-        if (lane == 0) ticket = atomicAdd(&P.counters[kTicket], 1ull);
-        ticket = __shfl_sync(full, ticket, 0);
-        if (ticket >= n_rays) break;
-        const uint32_t q_pixel = P.queue[ticket].pixel;
-        const int i = static_cast<int>(q_pixel % static_cast<uint32_t>(P.res_x));
-        const int j = static_cast<int>(q_pixel / static_cast<uint32_t>(P.res_x));
-        const double px = P.xs[i], py = P.ys[j];
-        RayAcc<1> a = load_deferred<F>(P, ticket);
-        int crossings = 0;
-        bool truncated = true;
-        while (truncated && !a.error) {
-            const int n = graze_collect(P, S, px, py, a.z_after, lane, truncated);
-            for (int base = 0; base < n; base += 32) {
-                const int k = base + lane;
-                const bool have = k < n;
-                const double z_in = have ? S.z[k] : INFINITY;
-                double z_out = z_in;
-                Pairs<1> f;
-                f.reset();
-                uint32_t steps_k = 0, error_k = 0;
-                if (have && z_in > a.z_after) {
-                    z_out = F::lam_crossing(P, px, py, S.leaf[k], z_in, f, steps_k, error_k);
-                }
-                const int cnt = n - base < 32 ? n - base : 32;
-                Pairs<1> entered = a.v;
-                bool taken = false;
-                for (int l = 0; l < cnt; l++) {
-                    Pairs<1> g;
-                    g.tau[0] = __shfl_sync(full, f.tau[0], l);
-                    g.inten[0] = __shfl_sync(full, f.inten[0], l);
-                    g.gain[0] = __shfl_sync(full, f.gain[0], l);
                     const double z_l = __shfl_sync(full, z_in, l);
-                    if (lane == l) {
-                        entered = a.v;
-                        taken = z_l > a.z_after;
+                    if constexpr (F::kRewalk) {
+                        if (lane == l) {
+                            entered = a.v;
+                            taken = z_l > a.z_after;
+                        }
                     }
-                    compose_crossing(a, z_l, __shfl_sync(full, z_out, l), g, __shfl_sync(full, steps_k, l),
-                                     __shfl_sync(full, error_k, l));
+                    compose_crossing<F::K, F::kTangent>(a, z_l, __shfl_sync(full, z_out, l), g,
+                                                        __shfl_sync(full, steps_k, l), __shfl_sync(full, error_k, l));
                 }
-                if (taken) {
-                    uint32_t steps_g = 0, error_g = 0;
-                    F::grad_crossing(P, px, py, q_pixel, S.leaf[k], z_in, entered, steps_g, error_g);
+                if constexpr (F::kRewalk) {
+                    if (taken) {
+                        uint32_t steps_g = 0, error_g = 0;
+                        F::template crossing<false>(P, px, py, q_pixel, S.leaf[k], z_in, entered, steps_g, error_g);
+                    }
                 }
             }
             crossings += n;
             if (crossings > 65536) a.error = 1;
             __syncwarp();
+        }
+        if constexpr (F::kImage) {
+            if (lane == 0) {
+                store_pixel(P, i, j, a.v.tau, a.v.inten, a.steps);
+                const unsigned long long more = a.steps - q_steps;
+                if (more) {
+                    atomicAdd(&P.counters[kSteps], more);
+                    atomicAdd(&P.row_cost[j], more);
+                    if (q_steps == 0) atomicAdd(&P.counters[kHitPixels], 1ull); // deferred before its first step
+                }
+                if (a.error) atomicAdd(&P.counters[kWalkErrors], 1ull);
+            }
         }
     }
 }
@@ -1515,11 +1447,11 @@ __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_ch(const WalkPa
 __global__ void __launch_bounds__(kBlock) tet_walk_depth(const WalkParams P) { walk_block<CellsDepth>(P); }
 __global__ void __launch_bounds__(kBlock) tet_walk_grad(const GradParams P) { walk_block<CellsGrad>(P); }
 __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_depth(const WalkParams P) { graze_block<CellsDepth>(P); }
-__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad(const GradParams P) { graze_block_grad<CellsGrad>(P); }
+__global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad(const GradParams P) { graze_block<CellsGrad>(P); }
 // The gradient pass with one {g_tau, g_I} per view (c5_render_flux_grad_device): registers in DESIGN.md §5c.
 __global__ void __launch_bounds__(kBlock) tet_walk_grad_view(const GradParams P) { walk_block<CellsGradView>(P); }
 __global__ void __launch_bounds__(32 * kGrazeWarps) grazing_rays_grad_view(const GradParams P) {
-    graze_block_grad<CellsGradView>(P);
+    graze_block<CellsGradView>(P);
 }
 // Forward mode (c5_render_jvp): {tau, I, dtau, dI} per pixel. Registers in DESIGN.md §5c.
 __global__ void __launch_bounds__(kBlock) tet_walk_jvp(const JvpParams P) { walk_block<CellsJvp>(P); }
@@ -1607,33 +1539,15 @@ void graze_on_host(const WalkParams& P) {
         const int i = static_cast<int>(q.pixel % static_cast<uint32_t>(P.res_x));
         const int j = static_cast<int>(q.pixel / static_cast<uint32_t>(P.res_x));
         const RayAcc<F::K> a = graze_ray_serial<F>(P, k, P.xs[i], P.ys[j]);
-        store_pixel(P, i, j, a.v.tau, a.v.inten, a.steps);
-        P.counters[kSteps] += a.steps - q.steps;
-        P.row_cost[j] += a.steps - q.steps;
-        if (q.steps == 0 && a.steps > 0) P.counters[kHitPixels]++;
-        if (a.error) P.counters[kWalkErrors]++;
+        if constexpr (F::kImage) {
+            store_pixel(P, i, j, a.v.tau, a.v.inten, a.steps);
+            P.counters[kSteps] += a.steps - q.steps;
+            P.row_cost[j] += a.steps - q.steps;
+            if (q.steps == 0 && a.steps > 0) P.counters[kHitPixels]++;
+            if (a.error) P.counters[kWalkErrors]++;
+        }
     }
     P.counters[kTicket] = n_rays;
-}
-
-template <class F>
-void graze_grad_on_host(const WalkParams& P) {
-    const unsigned long long n_rays = P.counters[kDeferred];
-    for (unsigned long long k = 0; k < n_rays; k++) {
-        const uint32_t pixel = P.queue[k].pixel;
-        const int i = static_cast<int>(pixel % static_cast<uint32_t>(P.res_x));
-        const int j = static_cast<int>(pixel / static_cast<uint32_t>(P.res_x));
-        graze_ray_serial_grad<F>(P, k, P.xs[i], P.ys[j]);
-    }
-    P.counters[kTicket] = n_rays;
-}
-template <>
-void graze_on_host<CellsGrad>(const WalkParams& P) {
-    graze_grad_on_host<CellsGrad>(P);
-}
-template <>
-void graze_on_host<CellsGradView>(const WalkParams& P) {
-    graze_grad_on_host<CellsGradView>(P);
 }
 
 // Policy F's pixel kernel over `grid` blocks, then its grazing-ray kernel for the rays the pixel
