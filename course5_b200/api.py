@@ -110,6 +110,8 @@ SYMBOLS = {
     "c5_render_wait": (C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(Stats)]),
     "c5_set_views_in_flight": (C.c_int, [C.c_void_p, C.c_int32]),
     "c5_debug_set": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
+    "c5_debug_ray_order": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "c5_debug_ray_order_read": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, _i32p, _i32p]),
     "c5_timeline_read": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_float), C.c_int32, _i32p]),
     "c5_image_create": (C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p), _u8p]),
     "c5_image_open": (C.c_int, [C.c_void_p, _u8p, C.POINTER(C.c_void_p)]),

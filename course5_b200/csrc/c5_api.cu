@@ -165,7 +165,7 @@ void ensure_pixel_tables(DeviceState& d, const c5_view* v, const ViewPlan& p) {
 
 // Where on the screen the mesh can be: the view-frame box of the 8 corners of its file-frame box,
 // widened by a pixel. The walk's grid covers only that rectangle (the rest of the band is filled as
-// background); a conservative hint — inside it every tile is still tested against the BVH root.
+// background); a conservative hint — inside it every region is still tested against the BVH root.
 void mesh_pixel_rect(const DeviceState& d, const c5_view* v, const ViewPlan& p, WalkLaunch& w) {
     double lo[2] = {INFINITY, INFINITY}, hi[2] = {-INFINITY, -INFINITY};
     for (int corner = 0; corner < 8; corner++) {
@@ -242,6 +242,17 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     if (channels || two_pairs) d.ch_queue.ensure(words * n_pix);
     d.row_cost.ensure(static_cast<size_t>(v->res_y));
     if (solids) d.mask.ensure(n_pix);
+    // The walk deals its rays out by the steps this state's last view took at each pixel (launch_walk). Under a
+    // new pixel grid, window or mesh those are unknown: all 0, which gives the Morton order.
+    d.ray_cost.ensure(n_pix);
+    if (d.ray_cost_res[0] != v->res_x || d.ray_cost_res[1] != v->res_y || d.ray_cost_mesh != d.mesh_version ||
+        !std::equal(v->window, v->window + 4, d.ray_cost_win)) {
+        dev_zero(d.ray_cost.p, n_pix * sizeof(uint16_t), d.stream);
+        d.ray_cost_res[0] = v->res_x;
+        d.ray_cost_res[1] = v->res_y;
+        d.ray_cost_mesh = d.mesh_version;
+        std::copy(v->window, v->window + 4, d.ray_cost_win);
+    }
 
     record(d, 0);
     timeline_mark(d, 0);
@@ -1297,6 +1308,7 @@ int c5_create_sibling(c5_ctx* parent, c5_ctx** out) {
     to.opt_query_budget = from.opt_query_budget;
     to.opt_serial_list = from.opt_serial_list;
     to.opt_no_static_mask = from.opt_no_static_mask;
+    to.opt_no_ray_order = from.opt_no_ray_order;
     to.opt_mask_tile = from.opt_mask_tile;
     to.opt_no_zero_copy = from.opt_no_zero_copy;
     *out = ctx;
@@ -1896,6 +1908,7 @@ int c5_debug_set(c5_ctx* ctx, const char* key, int64_t value) {
                 d.mask_static_valid = false;
             }
             else if (k == "no_zero_copy") d.opt_no_zero_copy = value != 0;
+            else if (k == "no_ray_order") d.opt_no_ray_order = value != 0;
             else if (k == "timeline") {
                 if (value < 0 || value > 4096) fail(C5_E_INVALID, "debug_set: timeline 0 .. 4096 views");
                 if (kHostSim) continue;
@@ -1913,6 +1926,27 @@ int c5_debug_set(c5_ctx* ctx, const char* key, int64_t value) {
                 fail(C5_E_INVALID, "debug_set: unknown key '" + k + "'");
             }
         }
+    });
+}
+
+int c5_debug_ray_order(const uint16_t* cost, uint16_t* order, int32_t* bucket) {
+    if (!cost || !order || !bucket) return C5_E_INVALID;
+    return order_one_region(cost, order, bucket);
+}
+
+int c5_debug_ray_order_read(c5_ctx* ctx, int32_t region, uint16_t* order, int32_t* origin_xy, int32_t* n_regions) {
+    if (!ctx || !order || !origin_xy || !n_regions) return C5_E_INVALID;
+    return guarded(ctx, [&] {
+        DeviceState& d = ctx->dev;
+        const int* g = d.ray_order_grid;
+        if (region < 0 || region >= g[0]) fail(C5_E_INVALID, "debug_ray_order_read: no such region in the last view");
+        use_device(d);
+        const size_t n = static_cast<size_t>(g[2]) * g[2];
+        d2h(order, d.ray_order.p + static_cast<size_t>(region) * n, n * sizeof(uint16_t), d.stream);
+        stream_sync(d.stream);
+        origin_xy[0] = d.ray_order_origin[0] + (region % g[1]) * g[2];
+        origin_xy[1] = d.ray_order_origin[1] + (region / g[1]) * g[2];
+        *n_regions = g[0];
     });
 }
 

@@ -85,6 +85,14 @@ struct DeviceState {
     DevBuf<uint32_t> steps;
     DevBuf<unsigned long long> counters;
     DevBuf<unsigned long long> row_cost;
+    DevBuf<uint16_t> ray_cost;       // [res_y][res_x] tet-steps of each pixel's ray in this state's last view, saturating
+                                     // (0: a miss, a solid pixel, or unknown); the walk's pixel order is made from it
+    int ray_cost_res[2] = {0, 0};    // the key ray_cost was written under: pixel grid, window and mesh version
+    double ray_cost_win[4] = {0, 0, 0, 0};
+    uint64_t ray_cost_mesh = 0;
+    DevBuf<uint16_t> ray_order;      // per region of the walk's rectangle: its pixels in the order the walk takes them
+    int ray_order_grid[3] = {0, 0, 0};    // of the last order: regions, regions per row, region side, and ...
+    int ray_order_origin[2] = {0, 0};     // ... the rectangle's first pixel (c5_debug_ray_order_read)
     DevBuf<DeferredRay> queue;       // grazing rays of the current view (capacity: pixels of the band)
     DevBuf<double> ch_queue;         // their channel values {tau, I} (channel renders only)
     DevBuf<double> row_flux;         // flux renders: [res_y][pairs] {sum tau, sum I} of the band's rows
@@ -107,7 +115,7 @@ struct DeviceState {
     size_t h_view_counters_n = 0;
     // c5_debug_set (tests, diagnostics); 0 = default
     int opt_graze_list = 0, opt_query_budget = 0, opt_serial_list = 0, opt_mask_tile = 0;
-    bool opt_no_zero_copy = false, opt_no_static_mask = false;
+    bool opt_no_zero_copy = false, opt_no_static_mask = false, opt_no_ray_order = false;
     // c5_debug_set("timeline", n): phase events of the last n views, read by c5_timeline_read
     std::vector<cudaEvent_t> tl_events;         // [n][kTimelinePhases]
     uint64_t tl_views = 0;                      // views recorded since the timeline was enabled
@@ -229,6 +237,9 @@ struct WalkLaunch {
 };
 enum WalkPass { kImagePass = 0, kDepthPass = 1, kGradPass = 2, kJvpPass = 3 };
 void launch_walk(DeviceState& d, const WalkLaunch& w);
+// c5_walk.cu — the pixel order of one region of the walk (c5_debug_ray_order): cost_rows[y][x] in, order[k] = the
+// local Morton index of the k-th pixel and bucket[m] = the sort bucket of Morton index m out; returns the region side.
+int order_one_region(const uint16_t* cost_rows, uint16_t* order, int32_t* bucket);
 // c5_flux.cu — row_flux[j] for the rows [row_begin,row_end) of d.out (pairs {tau, I} per pixel),
 // skipping pixels under d.mask when use_mask; the summation order is documented there.
 void launch_reduce_rows(DeviceState& d, int res_x, int res_y, int row_begin, int row_end, int pairs, bool use_mask);

@@ -39,6 +39,7 @@
 // face's vertices, c5_types.h).
 #include "c5_internal.h"
 
+#include <algorithm>
 #include <utility>
 
 namespace c5 {
@@ -46,8 +47,26 @@ namespace c5 {
 namespace {
 
 constexpr int kStack = 64;        // private LBVH traversal stack; a search that would overflow it is an incomplete search
-constexpr int kBlock = 128;       // 4 warps: 2 x 2 warp tiles of 8 x 4 pixels
-constexpr int kTileX = 16, kTileY = 8;
+constexpr int kBlock = 128;       // 4 warps of 32 rays
+
+// The pixel kernels' rays are dealt out by region: the walk's rectangle is cut into regions of kRegion x kRegion
+// pixels from its origin (i0, j0), and each region into kBlocksPerRegion blocks of kBlock rays. A block keeps its
+// slots on the SM until its longest ray ends, and a warp issues until its longest ray does, so rays that take
+// about as many steps should share a block and a warp. order_rays sorts each region's pixels by the tet-steps the
+// state's previous view took there (DeviceState::ray_cost): stably by (cost_bucket, local Morton index), where that
+// saves enough (sort_pays), else in Morton order: warps of 8 x 4 pixels, blocks of 16 x 8. Every thread still
+// traces one pixel, fixed when its block starts, so the image and every count do not depend on the order.
+// The constants are measured (one B200, profiles/r13_ray_order_constants_one_b200.jsonl, every region sorted,
+// against the Morton order of the same build): regions of 16, 32 and 64 pixels all cut C3's time per view by
+// 11-14 %, but only 16 x 16 kept the oblique view near the Morton order (32 and 64: 1 % slower); larger regions
+// scatter a block's rays over more tets. Of buckets 1, 8 and 32 steps wide, 1 is the best over both views.
+constexpr int kRegionLog = 4;
+constexpr int kRegion = 1 << kRegionLog;
+constexpr int kRegionPix = kRegion * kRegion;
+constexpr int kBlocksPerRegion = kRegionPix / kBlock;
+constexpr int kBucketShift = 0;   // costs less than 2^kBucketShift steps apart may share a bucket
+constexpr int kBuckets = 128;     // bucket 0: cost 0 (a miss, a solid pixel, outside the rectangle, unknown)
+static_assert(kRegionPix % kBlock == 0, "a region is whole blocks");
 
 struct WalkParams {
     const Conn* conn;
@@ -64,8 +83,10 @@ struct WalkParams {
     unsigned long long* row_cost; // [res_y]
     DeferredRay* queue;   // rays handed to the grazing-ray kernel; counters[kDeferred] of them
     int res_x, res_y, row_begin, row_end;
-    int i0, i1, j0, j1;   // pixel rectangle [i0,i1) x [j0,j1) of the band that can see the mesh: the tiles cover it
-    int n_tiles_x, n_tiles_y, n_macro_x;
+    int i0, i1, j0, j1;   // pixel rectangle [i0,i1) x [j0,j1) of the band that can see the mesh: the regions cover it
+    int n_regions_x;      // regions per row of the rectangle
+    uint16_t* cost;       // [res_y][res_x] tet-steps of each pixel's ray (saturating), written by the pixel kernel
+    uint16_t* order;      // [region][kRegionPix] local Morton indices in walk order, written by order_rays
     int graze_cap;        // entries one cooperative collection may hold (<= kGrazeList)
     int serial_cap;       // same for the serial (host loop) form (<= kSerialList)
     int query_budget;     // BVH nodes one thread of the pixel kernel may visit per search before deferring the ray
@@ -1321,44 +1342,203 @@ __device__ __forceinline__ void graze_block(const WalkParams& P) {
 
 // ---- kernel ----------------------------------------------------------------------------------------
 
-// 3-bit Morton decode: bits 0,2,4 -> x, bits 1,3,5 -> y
-__device__ __forceinline__ int compact3(int v) {
-    return (v & 1) | ((v >> 1) & 2) | ((v >> 2) & 4);
+// Morton decode: bits 0, 2, 4, ... of v (x of a local Morton index m; y is compact_bits(m >> 1))
+C5_HD int compact_bits(uint32_t v) {
+    v &= 0x55555555u;
+    v = (v | (v >> 1)) & 0x33333333u;
+    v = (v | (v >> 2)) & 0x0F0F0F0Fu;
+    v = (v | (v >> 4)) & 0x00FF00FFu;
+    return static_cast<int>(v & 0xFFFFu);
 }
+
+// The sort key of a ray that took `cost` steps in the previous view, in a region whose least nonzero cost is
+// `least`: 0 for no steps, then one bucket per 2^kBucketShift steps from the least up, the last one open.
+C5_HD int cost_bucket(uint32_t cost, uint32_t least) {
+    if (cost == 0) return 0;
+    const uint32_t b = (cost >> kBucketShift) - (least >> kBucketShift);
+    return 1 + static_cast<int>(b < kBuckets - 2 ? b : kBuckets - 2);
+}
+
+// The cost of local Morton index m of region (rx, ry); pixels outside the rectangle cost 0.
+C5_HD uint32_t region_cost(const WalkParams& P, int rx, int ry, uint32_t m) {
+    const int i = P.i0 + rx * kRegion + compact_bits(m), j = P.j0 + ry * kRegion + compact_bits(m >> 1);
+    return i < P.i1 && j < P.j1 ? P.cost[static_cast<size_t>(j) * P.res_x + i] : 0u;
+}
+
+// A region keeps the Morton order unless sorting it saves at least kMinSaving percent of its warps' issue time,
+// modelled as the sum over its warps of the most steps any of their rays takes ("warp steps"). Where the previous
+// view's step counts are even (the oblique view, the 50 M-tet C5t) a sort saves little, and its blocks, spread over
+// the region instead of one compact 16 x 8 patch, share fewer tets in L1: those views then walk as they did in
+// Morton order. Measured (profiles/r14_ray_order_threshold_one_b200.jsonl): sorting every region (0 %) costs C5t 1.2 %
+// against the parent; 10 % keeps C3's gain (4.63 -> 4.14 ms) and C5t within 0.3 %; 20 % loses most of C3's gain.
+constexpr uint32_t kMinSaving = 10;
+
+// Warp steps of the sorted order: the last ray of a sorted warp takes the most steps of its warp, up to the width
+// of a bucket (one step, kBucketShift = 0) and the last, open bucket.
+C5_HD bool sort_pays(uint32_t morton_steps, uint32_t sorted_steps) {
+    return static_cast<uint64_t>(sorted_steps) * 100u <= static_cast<uint64_t>(morton_steps) * (100u - kMinSaving);
+}
+
+// One region's order, by one thread (the host-loop build): a stable counting sort, kept if sort_pays. cost[m] is
+// local Morton index m's.
+C5_HD void order_region(const uint16_t* cost, uint16_t* order) {
+    uint32_t least = 0xFFFFu;
+    for (int m = 0; m < kRegionPix; m++) {
+        if (cost[m] && cost[m] < least) least = cost[m];
+    }
+    int start[kBuckets] = {};
+    for (int m = 0; m < kRegionPix; m++) start[cost_bucket(cost[m], least)]++;
+    for (int b = 0, sum = 0; b < kBuckets; b++) {
+        const int n = start[b];
+        start[b] = sum;
+        sum += n;
+    }
+    for (int m = 0; m < kRegionPix; m++) order[start[cost_bucket(cost[m], least)]++] = static_cast<uint16_t>(m);
+    uint32_t morton_steps = 0, sorted_steps = 0;
+    for (int w = 0; w < kRegionPix; w += 32) {
+        uint32_t most = 0;
+        for (int l = 0; l < 32; l++) most = cost[w + l] > most ? cost[w + l] : most;
+        morton_steps += most;
+        sorted_steps += cost[order[w + 31]];
+    }
+    if (!sort_pays(morton_steps, sorted_steps)) {
+        for (int m = 0; m < kRegionPix; m++) order[m] = static_cast<uint16_t>(m);
+    }
+}
+
+// The same by one block per region, kOrderThreads threads taking kOrderItems local Morton indices each (m = q
+// kOrderThreads + thread). The bits of words[b][w] are the indices 32 w .. 32 w + 31 that fall into bucket b (one
+// __match_any_sync per warp of indices); an index's place is the start of its bucket plus the members of that
+// bucket below it. Shared memory is used here and not in the walk kernels, whose L1 capacity serves the tets.
+constexpr int kOrderThreads = kRegionPix < 1024 ? kRegionPix : 1024;
+constexpr int kOrderItems = kRegionPix / kOrderThreads;
+constexpr int kOrderWords = kRegionPix / 32;
+static_assert(sizeof(uint32_t) * kBuckets * (kOrderWords + 1) <= 40 * 1024, "order_rays' bitmaps fit static shared memory");
+
+__global__ void __launch_bounds__(kOrderThreads) order_rays(const WalkParams P) {
+    __shared__ uint32_t words[kBuckets][kOrderWords + 1]; // (+1: lanes reading different buckets hit different banks)
+    __shared__ uint32_t start[kBuckets];
+    __shared__ uint32_t least_all, morton_steps, sorted_steps, nonzero;
+    const unsigned full = 0xFFFFFFFFu;
+    const int lane = threadIdx.x & 31;
+    const int rx = static_cast<int>(blockIdx.x) % P.n_regions_x, ry = static_cast<int>(blockIdx.x) / P.n_regions_x;
+    for (int k = threadIdx.x; k < kBuckets * (kOrderWords + 1); k += kOrderThreads) (&words[0][0])[k] = 0u;
+    if (threadIdx.x == 0) {
+        least_all = 0xFFFFu;
+        morton_steps = 0;
+        sorted_steps = 0;
+        nonzero = 0;
+    }
+    uint32_t cost[kOrderItems];
+    uint32_t least = 0xFFFFu, most = 0, rays = 0;
+#pragma unroll
+    for (int q = 0; q < kOrderItems; q++) {
+        cost[q] = region_cost(P, rx, ry, static_cast<uint32_t>(q * kOrderThreads + threadIdx.x));
+        if (cost[q] && cost[q] < least) least = cost[q];
+        most += __reduce_max_sync(full, cost[q]); // the warp steps of Morton warp q
+        rays += __popc(__ballot_sync(full, cost[q] != 0));
+    }
+    least = __reduce_min_sync(full, least);
+    __syncthreads();
+    if (lane == 0) {
+        atomicMin(&least_all, least);
+        atomicAdd(&morton_steps, most);
+        atomicAdd(&nonzero, rays);
+    }
+    __syncthreads();
+    least = least_all;
+    // The sort puts the rays with steps last, ceil(nonzero / 32) warps of them, and the last ray of each of those
+    // warps takes at least `least` steps: when even that bound saves too little, the region keeps the Morton order
+    // without sorting (most regions of evenly costed views: the kernel then takes a fraction of its time).
+    if (nonzero == 0 || !sort_pays(morton_steps, (nonzero + 31u) / 32u * least)) {
+#pragma unroll
+        for (int q = 0; q < kOrderItems; q++) {
+            const uint32_t m = static_cast<uint32_t>(q * kOrderThreads + threadIdx.x);
+            P.order[static_cast<size_t>(blockIdx.x) * kRegionPix + m] = static_cast<uint16_t>(m);
+        }
+        return;
+    }
+    int bucket[kOrderItems];
+    unsigned same[kOrderItems];
+#pragma unroll
+    for (int q = 0; q < kOrderItems; q++) {
+        bucket[q] = cost_bucket(cost[q], least);
+        same[q] = __match_any_sync(full, bucket[q]);
+        if (lane == __ffs(same[q]) - 1) words[bucket[q]][(q * kOrderThreads + threadIdx.x) >> 5] = same[q];
+    }
+    __syncthreads();
+    if (threadIdx.x < 32) { // exclusive scan of the bucket sizes, kBuckets / 32 consecutive buckets per lane
+        constexpr int kPer = kBuckets / 32;
+        uint32_t n[kPer], sum = 0;
+#pragma unroll
+        for (int k = 0; k < kPer; k++) {
+            n[k] = 0;
+            for (int w = 0; w < kOrderWords; w++) n[k] += __popc(words[lane * kPer + k][w]);
+            sum += n[k];
+        }
+        uint32_t below = sum;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const uint32_t o = __shfl_up_sync(full, below, d);
+            if (lane >= d) below += o;
+        }
+        below -= sum;
+#pragma unroll
+        for (int k = 0; k < kPer; k++) {
+            start[lane * kPer + k] = below;
+            below += n[k];
+        }
+    }
+    __syncthreads();
+    const unsigned lower = (1u << lane) - 1u;
+    uint32_t pos[kOrderItems];
+#pragma unroll
+    for (int q = 0; q < kOrderItems; q++) {
+        const uint32_t m = static_cast<uint32_t>(q * kOrderThreads + threadIdx.x);
+        pos[q] = start[bucket[q]] + __popc(same[q] & lower);
+        for (uint32_t w = 0; w < (m >> 5); w++) pos[q] += __popc(words[bucket[q]][w]);
+        if ((pos[q] & 31u) == 31u) atomicAdd(&sorted_steps, cost[q]);
+    }
+    __syncthreads();
+    const bool sorted = sort_pays(morton_steps, sorted_steps);
+#pragma unroll
+    for (int q = 0; q < kOrderItems; q++) {
+        const uint32_t m = static_cast<uint32_t>(q * kOrderThreads + threadIdx.x);
+        P.order[static_cast<size_t>(blockIdx.x) * kRegionPix + (sorted ? pos[q] : m)] = static_cast<uint16_t>(m);
+    }
+}
+static_assert(kBuckets % 32 == 0, "the scan gives each lane the same number of buckets");
 
 template <class F>
 __device__ __forceinline__ void walk_block(const WalkParams& P) {
-    // screen-space order: macro tiles of 8 x 8 block tiles in row-major order, Morton inside, so that
-    // concurrently resident blocks cover a compact patch of the image and share tets in L2
-    const int b = blockIdx.x;
-    const int macro = b >> 6, r = b & 63;
-    const int tile_x = (macro % P.n_macro_x) * 8 + compact3(r);
-    const int tile_y = (macro / P.n_macro_x) * 8 + compact3(r >> 1);
-    if (tile_x >= P.n_tiles_x || tile_y >= P.n_tiles_y) return;
+    // block b takes slots kBlock (b % kBlocksPerRegion) .. of region b / kBlocksPerRegion's order; regions are in
+    // row-major order, so the blocks resident at one time cover a few rows of regions
+    const int region = static_cast<int>(blockIdx.x) / kBlocksPerRegion;
+    const int i_lo = P.i0 + (region % P.n_regions_x) * kRegion, j_lo = P.j0 + (region / P.n_regions_x) * kRegion;
 
-    // Tiles that cannot see the mesh (outside the root's two boxes) skip the rays.
-    const int i_lo = P.i0 + tile_x * kTileX, j_lo = P.j0 + tile_y * kTileY;
-    const int i_hi = min(i_lo + kTileX, P.i1) - 1, j_hi = min(j_lo + kTileY, P.j1) - 1;
-    bool tile_sees_mesh;
+    // Regions that cannot see the mesh (outside the root's two boxes) skip the rays.
+    const int i_hi = min(i_lo + kRegion, P.i1) - 1, j_hi = min(j_lo + kRegion, P.j1) - 1;
+    bool region_sees_mesh;
     {
         const BvhNode* root = P.nodes;
         const float x0 = f_round_down(P.xs[i_lo]), x1 = f_round_up(P.xs[i_hi]);
         const float y0 = f_round_down(P.ys[j_lo]), y1 = f_round_up(P.ys[j_hi]);
         const bool s0 = x1 >= root->xlo[0] && x0 <= root->xhi[0] && y1 >= root->ylo[0] && y0 <= root->yhi[0];
         const bool s1 = x1 >= root->xlo[1] && x0 <= root->xhi[1] && y1 >= root->ylo[1] && y0 <= root->yhi[1];
-        tile_sees_mesh = s0 || s1;
+        region_sees_mesh = s0 || s1;
     }
 
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int i = P.i0 + tile_x * kTileX + (warp % 2) * 8 + (lane & 7);
-    const int j = P.j0 + tile_y * kTileY + (warp / 2) * 4 + (lane >> 3);
+    const int lane = threadIdx.x & 31;
+    const uint32_t m = __ldg(P.order + static_cast<size_t>(blockIdx.x) * kBlock + threadIdx.x);
+    const int i = i_lo + compact_bits(m);
+    const int j = j_lo + compact_bits(m >> 1);
     const bool live = i < P.i1 && j < P.j1;
 
     RayResult<F::K> res{};
     bool solid = false;
     if (live) solid = P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i];
     // the lanes that will trace a ray, agreed on while the warp is whole (trace_ray synchronises on it)
-    const unsigned tracing = __ballot_sync(0xFFFFFFFFu, live && !solid && tile_sees_mesh);
+    const unsigned tracing = __ballot_sync(0xFFFFFFFFu, live && !solid && region_sees_mesh);
     if (live) {
         if (solid) {
             if (F::kImage) {
@@ -1367,25 +1547,28 @@ __device__ __forceinline__ void walk_block(const WalkParams& P) {
                 store_pixel(P, i, j, nan, nan, 0);
             }
         } else {
-            if (tile_sees_mesh) {
+            if (region_sees_mesh) {
                 res = trace_ray<F>(P, P.xs[i], P.ys[j],
                                    static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i),
                                    tracing);
             }
             if (F::kImage && !res.deferred) store_pixel(P, i, j, res.v.tau, res.v.inten, res.steps);
         }
+        // the next view's order (a deferred ray counts the steps it took here)
+        P.cost[static_cast<size_t>(j) * P.res_x + i] = static_cast<uint16_t>(min(res.steps, 0xFFFFu));
     }
 
-    // statistics: one atomic per warp per counter, one per warp-row for the row costs
+    // statistics: one atomic per warp per counter, one per row the warp's rays lie on for the row costs
     const unsigned full = 0xFFFFFFFFu;
-    unsigned row_steps = res.steps;
-    row_steps += __shfl_xor_sync(full, row_steps, 1);
-    row_steps += __shfl_xor_sync(full, row_steps, 2);
-    row_steps += __shfl_xor_sync(full, row_steps, 4);
-    if ((lane & 7) == 0 && live && row_steps) atomicAdd(&P.row_cost[j], static_cast<unsigned long long>(row_steps));
-    unsigned warp_steps = row_steps;
-    warp_steps += __shfl_xor_sync(full, warp_steps, 8);
-    warp_steps += __shfl_xor_sync(full, warp_steps, 16);
+    for (unsigned rows = full; rows;) { // the same trips in every lane
+        const int first = __ffs(rows) - 1;
+        const int jr = __shfl_sync(full, j, first);
+        const unsigned on_row = __ballot_sync(full, j == jr);
+        const unsigned row_steps = __reduce_add_sync(full, j == jr ? res.steps : 0u);
+        if (lane == first && row_steps) atomicAdd(&P.row_cost[jr], static_cast<unsigned long long>(row_steps));
+        rows &= ~on_row;
+    }
+    const unsigned warp_steps = __reduce_add_sync(full, res.steps);
     const unsigned hits = __popc(__ballot_sync(full, live && res.steps > 0));
     const unsigned solids = __popc(__ballot_sync(full, solid));
     const unsigned errors = __popc(__ballot_sync(full, res.error != 0));
@@ -1415,7 +1598,8 @@ constexpr int chan_blocks_per_sm(int K) {
 // profiles/r09_bench_c3_bounds_one_b200.jsonl).
 __global__ void __launch_bounds__(kBlock, 8) tet_walk_fp64(const WalkParams P) { walk_block<CellsF64>(P); }
 // optional single-precision step geometry (north-star item (d)); entry search and accumulators stay FP64.
-// 9 blocks = 56 registers, no spills: oblique view 1.90 against 2.03 ms at 8 blocks (same file).
+// 9 blocks = 56 registers: oblique view 1.90 against 2.03 ms at 8 blocks (same file). Since the pixel order
+// (order_rays) it spills 12 bytes outside the step loop (-Xptxas -v).
 __global__ void __launch_bounds__(kBlock, 9) tet_walk_fp32(const WalkParams P) { walk_block<CellsF32>(P); }
 template <int K>
 __global__ void __launch_bounds__(kBlock, chan_blocks_per_sm(K)) tet_walk_ch(const WalkParams P) { walk_block<Channels<K>>(P); }
@@ -1507,11 +1691,20 @@ void background_on_host(const WalkParams& P, int n) {
     }
 }
 
+void order_on_host(const WalkParams& P, int n_regions) {
+    uint16_t cost[kRegionPix];
+    for (int r = 0; r < n_regions; r++) {
+        for (int m = 0; m < kRegionPix; m++) cost[m] = static_cast<uint16_t>(region_cost(P, r % P.n_regions_x, r / P.n_regions_x, m));
+        order_region(cost, P.order + static_cast<size_t>(r) * kRegionPix);
+    }
+}
+
 template <class F>
 void walk_on_host(const WalkParams& P) {
     for (int j = P.j0; j < P.j1; j++) {
         for (int i = P.i0; i < P.i1; i++) {
             if (P.mask && P.mask[static_cast<size_t>(j) * P.res_x + i]) {
+                P.cost[static_cast<size_t>(j) * P.res_x + i] = 0;
                 if (F::kImage) {
                     double nan[F::K];
                     fill_pairs(nan, NAN, std::make_integer_sequence<int, F::K>{});
@@ -1523,6 +1716,7 @@ void walk_on_host(const WalkParams& P) {
             const uint32_t pixel = static_cast<uint32_t>(j) * static_cast<uint32_t>(P.res_x) + static_cast<uint32_t>(i);
             const RayResult<F::K> r = trace_ray<F>(P, P.xs[i], P.ys[j], pixel, 0);
             if (F::kImage && !r.deferred) store_pixel(P, i, j, r.v.tau, r.v.inten, r.steps);
+            P.cost[pixel] = static_cast<uint16_t>(std::min(r.steps, 0xFFFFu));
             P.counters[kSteps] += r.steps;
             P.row_cost[j] += r.steps;
             if (r.steps) P.counters[kHitPixels]++;
@@ -1574,8 +1768,20 @@ void launch_rays(DeviceState& d, const WalkLaunch& w, const Params& P, unsigned 
 
 } // namespace
 
-// One view's rays on d.stream: background fill, the pixel kernel, then the grazing-ray kernel for the
-// rays it deferred — three launches in stream order, no kernel ever waits for another one. (Round 1
+int order_one_region(const uint16_t* cost_rows, uint16_t* order, int32_t* bucket) {
+    uint16_t cost[kRegionPix];
+    uint32_t least = 0xFFFFu;
+    for (uint32_t m = 0; m < kRegionPix; m++) {
+        cost[m] = cost_rows[compact_bits(m >> 1) * kRegion + compact_bits(m)];
+        if (cost[m] && cost[m] < least) least = cost[m];
+    }
+    order_region(cost, order);
+    for (int m = 0; m < kRegionPix; m++) bucket[m] = cost_bucket(cost[m], least);
+    return kRegion;
+}
+
+// One view's rays on d.stream: background fill, the ray order, the pixel kernel, then the grazing-ray kernel for
+// the rays it deferred — four launches in stream order, no kernel ever waits for another one. (Round 1
 // ran the grazing-ray kernel BESIDE the pixel kernel, spinning on the queue; CUDA promises no forward
 // progress between kernels, and with three or four views in flight the ordered form is also the faster
 // one: profiles/r02_exp_lanes_graze_after.jsonl against r02_exp_lanes_graze_beside.jsonl.)
@@ -1608,10 +1814,19 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
     const bool empty_rect = P.i0 >= P.i1 || P.j0 >= P.j1;
     if (empty_rect) P.i0 = P.i1 = P.j0 = P.j1 = 0;
     const bool whole_band = P.i0 == 0 && P.i1 == w.res_x && P.j0 == w.row_begin && P.j1 == w.row_end;
-    P.n_tiles_x = (P.i1 - P.i0 + kTileX - 1) / kTileX;
-    P.n_tiles_y = (P.j1 - P.j0 + kTileY - 1) / kTileY;
-    P.n_macro_x = (P.n_tiles_x + 7) / 8;
-    const int n_macro_y = (P.n_tiles_y + 7) / 8;
+    P.n_regions_x = (P.i1 - P.i0 + kRegion - 1) / kRegion;
+    const int n_regions = P.n_regions_x * ((P.j1 - P.j0 + kRegion - 1) / kRegion);
+    // (sized for the whole image: the rectangle moves from view to view)
+    d.ray_order.ensure(static_cast<size_t>((w.res_x + kRegion - 1) / kRegion) * ((w.res_y + kRegion - 1) / kRegion) * kRegionPix);
+    P.cost = d.ray_cost.p;
+    P.order = d.ray_order.p;
+    if (w.pass != kGradPass) {
+        d.ray_order_grid[0] = n_regions;
+        d.ray_order_grid[1] = P.n_regions_x;
+        d.ray_order_grid[2] = kRegion;
+        d.ray_order_origin[0] = P.i0;
+        d.ray_order_origin[1] = P.j0;
+    }
     // c5_debug_set (tests shrink these to reach the overflow paths on small meshes); defaults otherwise
     P.graze_cap = d.opt_graze_list >= 128 && d.opt_graze_list <= kGrazeList ? (d.opt_graze_list & ~1) : kGrazeList;
     P.query_budget = d.opt_query_budget >= 1 ? d.opt_query_budget : 64;
@@ -1641,8 +1856,23 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
         }
     }
     if (empty_rect) return; // the mesh is not in this band: no rays
+    // The order of the view's rays, from the steps the state's last view took at each pixel (c5_debug_set
+    // "no_ray_order": from equal costs, the Morton order). The gradient pass walks the rays of the depth pass
+    // before it, over the same rectangle, and takes the same order.
+    // (Made on a stream of its own beside the view's prologue, the order cost the C4 sweep, three views in flight,
+    // 4.5 % against 1.2 % on the view's stream: profiles/r14_ray_order_threshold_one_b200.jsonl.)
+    if (w.pass != kGradPass) {
+        if (d.opt_no_ray_order) dev_zero(d.ray_cost.p, d.ray_cost.bytes(), d.stream);
+        count_launch();
+        if (kHostSim) {
+            order_on_host(P, n_regions);
+        } else {
+            order_rays<<<static_cast<unsigned>(n_regions), kOrderThreads, 0, d.stream>>>(P);
+            C5_CUDA(cudaGetLastError());
+        }
+    }
     count_launch();
-    const unsigned grid = static_cast<unsigned>(P.n_macro_x) * static_cast<unsigned>(n_macro_y) * 64u;
+    const unsigned grid = static_cast<unsigned>(n_regions) * kBlocksPerRegion;
     if (w.pass == kDepthPass) {
         launch_rays<CellsDepth>(d, w, P, grid);
         return;

@@ -438,6 +438,8 @@ uint64_t c5_kernel_launches(const c5_ctx* ctx);
  *   "no_static_mask" 1: solids that do not follow the view are scan-converted in every view, like the
  *                   others, instead of once per pixel grid (tests compare the two)
  *   "no_zero_copy"  1: page-locked output buffers get a device-to-host copy like pageable ones
+ *   "no_ray_order"  1: the pixel kernels take every region's pixels in Morton order instead of sorted by the
+ *                   tet-steps of the previous view (tests compare the two; images and counts are the same)
  *   "timeline"      n > 0: keep the phase events of the last n views of every lane (0 = off)
  * Unknown keys return C5_E_INVALID.
  * c5_timeline_read: for the last views rendered by ctx itself (not its lanes; oldest first, at most
@@ -445,6 +447,16 @@ uint64_t c5_kernel_launches(const c5_ctx* ctx);
  * on the same device): view start, vertices rotated, BVH refitted, solid mask done, pixel kernel
  * done, grazing-ray kernel done. Synchronises with the last of them. */
 int c5_debug_set(c5_ctx* ctx, const char* key, int64_t value);
+/* c5_debug_ray_order(cost, order, bucket) — the pixel order the walk gives one region of side R (the return
+ * value; every array holds R * R entries) whose pixels took cost[y * R + x] tet-steps in the previous view:
+ * order[k] is the local Morton index (x in bits 0, 2, 4, ..., y in bits 1, 3, 5, ...) of the pixel that takes ray
+ * slot k, bucket[m] the sort bucket of Morton index m. The order is the Morton order itself, or, where that saves
+ * enough of the region's warp time, the stable sort by (bucket, Morton index). Runs on the host.
+ * c5_debug_ray_order_read(ctx, region, order, origin_xy, n_regions) — the order ctx's last view walked region
+ * `region` in (R * R entries, read back from the device), the image pixel of the region's corner, and the number
+ * of regions of that view. */
+int c5_debug_ray_order(const uint16_t* cost, uint16_t* order, int32_t* bucket);
+int c5_debug_ray_order_read(c5_ctx* ctx, int32_t region, uint16_t* order, int32_t* origin_xy, int32_t* n_regions);
 int c5_timeline_read(c5_ctx* ctx, void* origin, float* ms_out, int32_t max_views, int32_t* n_views);
 
 #ifdef __cplusplus
