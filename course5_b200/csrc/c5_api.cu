@@ -56,14 +56,7 @@ struct BorrowStream {
     ~BorrowStream() { d.stream = own; }
 };
 
-// `waiter` waits for the work enqueued on `producer` so far, through `ev` (recorded on `producer`).
-void wait_for(cudaStream_t waiter, cudaStream_t producer, cudaEvent_t ev) {
-    if (!kHostSim) {
-        C5_CUDA(cudaEventRecord(ev, producer));
-        C5_CUDA(cudaStreamWaitEvent(waiter, ev, 0));
-    }
-}
-
+using c5::wait_for;
 // Every stream in `waiters` waits for the work enqueued on `producer` so far, through one record of `ev`.
 void wait_for(const std::vector<DeviceState*>& waiters, cudaStream_t producer, cudaEvent_t ev) {
     if (!kHostSim) {
@@ -245,50 +238,59 @@ void enqueue_view(DeviceState& d, const c5_view* v, const ViewPlan& p, bool want
     // The walk deals its rays out by the steps this state's last view took at each pixel (launch_walk). Under a
     // new pixel grid, window or mesh those are unknown: all 0, which gives the Morton order.
     d.ray_cost.ensure(n_pix);
-    if (d.ray_cost_res[0] != v->res_x || d.ray_cost_res[1] != v->res_y || d.ray_cost_mesh != d.mesh_version ||
-        !std::equal(v->window, v->window + 4, d.ray_cost_win)) {
-        dev_zero(d.ray_cost.p, n_pix * sizeof(uint16_t), d.stream);
-        d.ray_cost_res[0] = v->res_x;
-        d.ray_cost_res[1] = v->res_y;
-        d.ray_cost_mesh = d.mesh_version;
-        std::copy(v->window, v->window + 4, d.ray_cost_win);
-    }
+    // The pixel kernel runs on the call's stream, everything else on d.side (DeviceState::side), forked here and
+    // joined at the end: to the caller the view is still one stretch of its stream.
+    const cudaStream_t call = d.stream;
+    wait_for(d.side, call, d.ev_side);
+    {
+        const BorrowStream on_side(d, d.side);
+        if (d.ray_cost_res[0] != v->res_x || d.ray_cost_res[1] != v->res_y || d.ray_cost_mesh != d.mesh_version ||
+            !std::equal(v->window, v->window + 4, d.ray_cost_win)) {
+            dev_zero(d.ray_cost.p, n_pix * sizeof(uint16_t), d.stream);
+            d.ray_cost_res[0] = v->res_x;
+            d.ray_cost_res[1] = v->res_y;
+            d.ray_cost_mesh = d.mesh_version;
+            std::copy(v->window, v->window + 4, d.ray_cost_win);
+        }
 
-    record(d, 0);
-    timeline_mark(d, 0);
-    launch_prepare_cells(d, v->alpha_limit); // no-op unless --alpha_limit changed since the last view
-    if (channels) launch_prepare_channels(d, v->alpha_limit); // the same for the channels
-    launch_rotate_vertices(d, p.rot, p.n_rot);
-    if (solids) launch_rotate_solids(d, p.rot, p.n_rot);
-    record(d, 1);
-    timeline_mark(d, 1);
-    launch_bvh_refit(d);
-    record(d, 2);
-    timeline_mark(d, 2);
-    if (solids) {
-        launch_solid_mask(d, v->res_x, v->res_y, p.x_min, p.y_min, p.step_x, p.step_y, p.row_begin, p.row_end);
+        record(d, 0);
+        timeline_mark(d, 0);
+        launch_prepare_cells(d, v->alpha_limit); // no-op unless --alpha_limit changed since the last view
+        if (channels) launch_prepare_channels(d, v->alpha_limit); // the same for the channels
+        launch_rotate_vertices(d, p.rot, p.n_rot);
+        if (solids) launch_rotate_solids(d, p.rot, p.n_rot);
+        record(d, 1);
+        timeline_mark(d, 1);
+        launch_bvh_refit(d);
+        record(d, 2);
+        timeline_mark(d, 2);
+        if (solids) {
+            launch_solid_mask(d, v->res_x, v->res_y, p.x_min, p.y_min, p.step_x, p.step_y, p.row_begin, p.row_end);
+        }
+        record(d, 3);
+        timeline_mark(d, 3);
+        dev_zero(d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
+        dev_zero(d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
+        WalkLaunch w = view_walk(d, v, p);
+        w.write_steps = want_steps ? 1 : 0;
+        w.channels = channels;
+        w.pass = pass;
+        w.dir = dir;
+        w.out = out_override ? out_override : d.out.p;
+        w.pixel_stream = call;
+        w.mark_walk_done = d.ev_walk;
+        w.mark_walk_done_tl = nullptr;
+        if (!kHostSim && !d.tl_events.empty()) {
+            const size_t n = d.tl_events.size() / kTimelinePhases;
+            w.mark_walk_done_tl = d.tl_events[(d.tl_views % n) * kTimelinePhases + 4];
+        }
+        if (!kHostSim) { // a band the mesh does not reach launches no walk kernels: the markers are recorded anyway
+            C5_CUDA(cudaEventRecord(d.ev_walk, d.stream));
+            if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
+        }
+        launch_walk(d, w);
     }
-    record(d, 3);
-    timeline_mark(d, 3);
-    dev_zero(d.counters.p, kNumCounters * sizeof(unsigned long long), d.stream);
-    dev_zero(d.row_cost.p, static_cast<size_t>(v->res_y) * sizeof(unsigned long long), d.stream);
-    WalkLaunch w = view_walk(d, v, p);
-    w.write_steps = want_steps ? 1 : 0;
-    w.channels = channels;
-    w.pass = pass;
-    w.dir = dir;
-    w.out = out_override ? out_override : d.out.p;
-    w.mark_walk_done = d.ev_walk;
-    w.mark_walk_done_tl = nullptr;
-    if (!kHostSim && !d.tl_events.empty()) {
-        const size_t n = d.tl_events.size() / kTimelinePhases;
-        w.mark_walk_done_tl = d.tl_events[(d.tl_views % n) * kTimelinePhases + 4];
-    }
-    if (!kHostSim) { // a band the mesh does not reach launches no walk kernels: the markers are recorded anyway
-        C5_CUDA(cudaEventRecord(d.ev_walk, d.stream));
-        if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
-    }
-    launch_walk(d, w);
+    wait_for(call, d.side, d.ev_side);
     record(d, 4);
     timeline_mark(d, 5);
     if (!d.tl_events.empty()) d.tl_views++;
@@ -1258,6 +1260,10 @@ int c5_create(const int32_t* devices, int32_t n_dev, c5_ctx** out) {
         if (!kHostSim) {
             C5_CUDA(cudaSetDevice(d.device));
             C5_CUDA(cudaStreamCreateWithFlags(&d.stream, cudaStreamNonBlocking));
+            int least = 0, greatest = 0;
+            C5_CUDA(cudaDeviceGetStreamPriorityRange(&least, &greatest));
+            C5_CUDA(cudaStreamCreateWithPriority(&d.side, cudaStreamNonBlocking, greatest));
+            C5_CUDA(cudaEventCreateWithFlags(&d.ev_side, cudaEventDisableTiming));
             for (auto& e : d.ev) C5_CUDA(cudaEventCreate(&e));
             C5_CUDA(cudaEventCreate(&d.ev_walk));
             C5_CUDA(cudaEventCreateWithFlags(&d.ev_done, cudaEventDisableTiming));
@@ -1339,6 +1345,7 @@ void c5_destroy(c5_ctx* ctx) {
     if (!kHostSim && d.stream) {
         cudaSetDevice(d.device);
         cudaStreamSynchronize(d.stream);
+        if (d.side) cudaStreamSynchronize(d.side);
     }
     for (void* p : ctx->registered) {
         if (!kHostSim) cudaHostUnregister(p);
@@ -1357,10 +1364,12 @@ void c5_destroy(c5_ctx* ctx) {
         if (d.ev_done) cudaEventDestroy(d.ev_done);
         if (d.ev_fields) cudaEventDestroy(d.ev_fields);
         if (d.ev_gather) cudaEventDestroy(d.ev_gather);
+        if (d.ev_side) cudaEventDestroy(d.ev_side);
         for (auto& e : d.ev) {
             if (e) cudaEventDestroy(e);
         }
         if (d.stream) cudaStreamDestroy(d.stream);
+        if (d.side) cudaStreamDestroy(d.side);
     }
     delete ctx; // DevBuf destructors free on the current device, d.device
 }
@@ -1914,6 +1923,7 @@ int c5_debug_set(c5_ctx* ctx, const char* key, int64_t value) {
                 if (kHostSim) continue;
                 use_device(d);
                 C5_CUDA(cudaStreamSynchronize(d.stream));
+                C5_CUDA(cudaStreamSynchronize(d.side));
                 for (cudaEvent_t e : d.tl_events) cudaEventDestroy(e);
                 d.tl_events.clear();
                 d.tl_views = 0;

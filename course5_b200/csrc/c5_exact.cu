@@ -848,6 +848,7 @@ void mask_passes(DeviceState& d, SolidSet& ss, const MaskGrid& g, const TileGrid
     constexpr int kBlock = 32 * kMaskWarps;
     // pass 1: small faces are drawn, tall ones listed
     count_launch();
+    prefer_side_carveout(solid_mask_small, d.device);
     solid_mask_small<<<grid_for(ss.n_faces, kBlock), kBlock, 0, d.stream>>>(ss.n_faces, ss.faces.p, ss.pts_view.p, g,
                                                                              d.mask_tall.p, d.mask_counts.p);
     C5_CUDA(cudaGetLastError());
@@ -857,6 +858,7 @@ void mask_passes(DeviceState& d, SolidSet& ss, const MaskGrid& g, const TileGrid
     C5_CUDA(cudaGetLastError());
     // pass 3: tall faces, skipping tile rows that are solid already
     count_launch();
+    prefer_side_carveout(solid_mask_tall, d.device);
     solid_mask_tall<<<static_cast<unsigned>(d.sm_count) * 16u, kBlock, 0, d.stream>>>(d.mask_tall.p, d.mask_counts.p,
                                                                                       ss.pts_view.p, g, tg);
     C5_CUDA(cudaGetLastError());

@@ -36,6 +36,11 @@ struct SolidSet {
 struct DeviceState {
     int device = 0;
     cudaStream_t stream = nullptr;
+    // A view's prologue and grazing-ray kernel run on `side`, of the device's greatest priority, forked from and
+    // joined into the stream the view is enqueued on (enqueue_view); its pixel kernel runs on that stream. Their blocks
+    // then take the SM slots that another lane's pixel kernel frees, instead of waiting for its last wave.
+    cudaStream_t side = nullptr;
+    cudaEvent_t ev_side = nullptr;   // the fork and join edges between the view's stream and `side`
     cudaEvent_t ev[8] = {};
 
     // mesh (uploaded once)
@@ -217,6 +222,9 @@ struct WalkLaunch {
     int precision;
     int channels; // 0: the cells' own fields; n: the n uploaded channels, n {tau, I} per pixel
     double* out; // {tau, I} per pixel (per channel) of the band, x fastest
+    // the pixel kernel's stream, when it is not d.stream: the launch orders it after the prologue enqueued on
+    // d.stream so far and orders d.stream's grazing-ray kernel after it, through d.ev_side (null: d.stream)
+    cudaStream_t pixel_stream;
     cudaEvent_t mark_walk_done;    // recorded between the pixel kernel and the grazing-ray kernel (may be null)
     cudaEvent_t mark_walk_done_tl; // the same moment for the timeline ring (may be null)
     // c5_render_grad (channels 0, precision 64): kDepthPass stores {tau, I, lam, 0} per pixel into out;

@@ -138,6 +138,35 @@ void stream_sync(cudaStream_t s) {
     if (!kHostSim) C5_CUDA(cudaStreamSynchronize(s));
 }
 
+// 100 KB of shared memory per SM. Beside seven blocks of the pixel kernel (1 KB each, reserved by the hardware) that
+// holds four blocks of the solid mask (22 KB each) or seven of the grazing-ray kernel (11 KB each); alone, the
+// grazing-ray kernel gets eight blocks per SM (C3 on one B200: 0.52 ms, 0.47 with the twelve of its grid). The pixel
+// kernel alone pays 1 % for the L1 this takes (3.49 -> 3.53 ms); 64 KB cost the grazing-ray kernel alone 40 % and
+// the pipelined views half the gain (profiles/r15_arms_c3_one_b200.jsonl).
+constexpr int64_t kSideSmemBytes = 100 * 1024;
+
+void prefer_side_carveout(const void* kernel, int device) {
+    if (kHostSim) return;
+    static std::mutex mu;
+    static std::vector<std::pair<const void*, int>> done;
+    std::lock_guard<std::mutex> lock(mu);
+    const std::pair<const void*, int> key{kernel, device};
+    if (std::find(done.begin(), done.end(), key) != done.end()) return;
+    int per_sm = 0;
+    C5_CUDA(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, device));
+    // a percentage of the most an SM can hold, rounded down here and up by the driver to a split the SM has
+    const int percent = static_cast<int>(std::min<int64_t>(100, kSideSmemBytes * 100 / per_sm));
+    C5_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, percent));
+    done.push_back(key);
+}
+
+void wait_for(cudaStream_t waiter, cudaStream_t producer, cudaEvent_t ev) {
+    if (!kHostSim) {
+        C5_CUDA(cudaEventRecord(ev, producer));
+        C5_CUDA(cudaStreamWaitEvent(waiter, ev, 0));
+    }
+}
+
 #ifdef C5_HOSTSIM
 
 template <class K>

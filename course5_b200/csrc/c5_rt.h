@@ -53,6 +53,8 @@ void d2d(void* dst, const void* src, size_t bytes, cudaStream_t s);
 // rows of `width` bytes, `height` of them, from src (pitch spitch) to dst (pitch dpitch), device to device
 void d2d_2d(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t height, cudaStream_t s);
 void stream_sync(cudaStream_t s);
+// `waiter` waits for the work enqueued on `producer` so far, through `ev` (recorded on `producer`).
+void wait_for(cudaStream_t waiter, cudaStream_t producer, cudaEvent_t ev);
 void* host_pinned_alloc(size_t bytes); // page-locked host memory (results the stream copies back while the host runs on)
 void host_pinned_free(void* p);
 size_t dev_bytes_in_use();
@@ -118,6 +120,15 @@ extern thread_local uint64_t* g_launch_counter; // bumped once per kernel launch
 
 inline void count_launch() {
     if (g_launch_counter) ++*g_launch_counter;
+}
+
+// The pixel kernel and the kernels that run beside it on an SM (a view's prologue and grazing-ray kernel) ask for one
+// L1 / shared-memory split, so that a block of one can take the place a block of the other leaves without the SM
+// draining first to change its split. Once per kernel and device.
+void prefer_side_carveout(const void* kernel, int device);
+template <class... A>
+void prefer_side_carveout(void (*kernel)(A...), int device) {
+    prefer_side_carveout(reinterpret_cast<const void*>(kernel), device);
 }
 
 #ifdef __CUDACC__

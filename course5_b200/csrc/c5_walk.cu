@@ -1755,13 +1755,18 @@ void launch_rays(DeviceState& d, const WalkLaunch& w, const Params& P, unsigned 
         graze_on_host<F>(P);
         return;
     }
-    Kernels<F>::walk<<<grid, kBlock, 0, d.stream>>>(P);
+    const cudaStream_t ps = w.pixel_stream ? w.pixel_stream : d.stream;
+    if (ps != d.stream) wait_for(ps, d.stream, d.ev_side);
+    prefer_side_carveout(Kernels<F>::walk, d.device);
+    Kernels<F>::walk<<<grid, kBlock, 0, ps>>>(P);
     C5_CUDA(cudaGetLastError());
-    if (w.mark_walk_done) C5_CUDA(cudaEventRecord(w.mark_walk_done, d.stream));
-    if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, d.stream));
+    if (w.mark_walk_done) C5_CUDA(cudaEventRecord(w.mark_walk_done, ps));
+    if (w.mark_walk_done_tl) C5_CUDA(cudaEventRecord(w.mark_walk_done_tl, ps));
+    if (ps != d.stream) wait_for(d.stream, ps, d.ev_side);
     if (d.sm_count == 0) C5_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, d.device));
     const unsigned graze_grid = static_cast<unsigned>(d.sm_count) * static_cast<unsigned>(kGrazeBlocksPerSm);
     count_launch();
+    prefer_side_carveout(Kernels<F>::graze, d.device);
     Kernels<F>::graze<<<graze_grid, 32 * kGrazeWarps, 0, d.stream>>>(P);
     C5_CUDA(cudaGetLastError());
 }
@@ -1780,8 +1785,9 @@ int order_one_region(const uint16_t* cost_rows, uint16_t* order, int32_t* bucket
     return kRegion;
 }
 
-// One view's rays on d.stream: background fill, the ray order, the pixel kernel, then the grazing-ray kernel for
-// the rays it deferred — four launches in stream order, no kernel ever waits for another one. (Round 1
+// One view's rays on d.stream: background fill, the ray order, the pixel kernel (on w.pixel_stream when one is
+// given), then the grazing-ray kernel for the rays it deferred — four launches in stream order, no kernel ever
+// waits for another one. (Round 1
 // ran the grazing-ray kernel BESIDE the pixel kernel, spinning on the queue; CUDA promises no forward
 // progress between kernels, and with three or four views in flight the ordered form is also the faster
 // one: profiles/r02_exp_lanes_graze_after.jsonl against r02_exp_lanes_graze_beside.jsonl.)
@@ -1867,6 +1873,7 @@ void launch_walk(DeviceState& d, const WalkLaunch& w) {
         if (kHostSim) {
             order_on_host(P, n_regions);
         } else {
+            prefer_side_carveout(order_rays, d.device);
             order_rays<<<static_cast<unsigned>(n_regions), kOrderThreads, 0, d.stream>>>(P);
             C5_CUDA(cudaGetLastError());
         }
